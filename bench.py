@@ -216,6 +216,30 @@ class NvmlSampler:
                 "samples": len(sm), "source": "nvml, polled during the timed blocks"}
 
 
+MOMENT_SAMPLE = 1 << 20              # Adam moments dumped per buffer (of 5.77 M): keeps a dump near 32 MB
+
+
+def dump_outputs(out_dir: str, model, opt, loss: torch.Tensor) -> None:
+    """What a caller of the timed step holds after its last call, as float32 .npy files in out_dir: `loss.npy` (the
+    step's return value), `<parameter name>.npy` (every updated weight and bias, in full) and
+    `exp_avg.sample.npy` / `exp_avg_sq.sample.npy` (the optimizer's moments over all parameters in named_parameters()
+    order, at a fixed seeded sample of MOMENT_SAMPLE positions). The inputs of a run depend on the arguments only, so
+    two builds run with the same arguments can be compared file by file. Two runs of one build agree to rounding,
+    not bit for bit: split-K partial products are summed in arrival order, and Adam turns a rounding difference in a
+    near-zero gradient into up to one learning-rate step of a weight."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss.detach().float().cpu().numpy()}
+    named = list(model.named_parameters())
+    for name, p in named:
+        arrays[name] = p.detach().float().cpu().numpy()
+    idx = np.sort(np.random.default_rng(0).choice(sum(p.numel() for _, p in named), MOMENT_SAMPLE, replace=False))
+    for key in ("exp_avg", "exp_avg_sq"):
+        flat = torch.cat([opt.state[p][key].detach().float().flatten() for _, p in named]).cpu().numpy()
+        arrays[key + ".sample"] = flat[idx]
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     from rawaudiovae_kelsey_b200 import dist as rdist
     from rawaudiovae_kelsey_b200 import ops
@@ -256,20 +280,21 @@ def run_ours(args):
     # one eager call of that signature, and the pipelined signature contains the parity of the plan's double-buffered
     # input set: eager, eager, capture, capture, then replays. The untimed pre-steps therefore run for at least
     # --warmup steps AND until NEED consecutive steps were plain replays; the timed blocks assert that no capture and
-    # no eager step happened inside them.
+    # no eager step happened inside them. Each leg then runs one untimed lead-in block of --steps steps, shaped like a
+    # timed block and with the clock sampler already running: on a B200 (1000 W) a block timed straight after the
+    # set-up work measured ~2 % slower than every block after it.
     NEED = 4
     pre_steps = max(args.warmup, 2 * step_fn.graph_warmup + 2 + NEED) if args.graph else args.warmup
     est_ms = 0.35 if args.precision == "bf16" else 1.0
-    # Statistic. Every timed block is EXACTLY --steps steps between barrier + synchronize. `value` and `e2e` are the median
-    # of the first n_blocks blocks of their leg (>= 7 blocks, >= 200 steps: SURVEY.md 8d "timed over >= 200 steps after
-    # >= 20 warm-up"; the contract's own run is W + K = 25 steps long). A run that short is at boost clocks. Each leg then
-    # simply keeps going for sus_blocks more blocks (~0.4 s of continuous load): ~100 ms in, the board's power cap starts
-    # to pull the SM clock of a single busy GPU down, and it keeps drifting for seconds (under data parallelism the GPUs
-    # idle in the exchange and stay at boost). The median of the second half of those later blocks is reported as
-    # `sustained` - what a long job sees early on - and is never mixed into `value`. With --blocks B or --no-sustained a
-    # leg is B (n_blocks) blocks.
-    n_blocks = args.blocks if args.blocks > 0 else int(max(7, math.ceil(200.0 / args.steps)))
-    sus_blocks = 0 if (args.blocks > 0 or args.no_sustained) else int(min(200, math.ceil(400.0 / (args.steps * est_ms))))
+    # Statistic. Every timed block is EXACTLY --steps steps between barrier + synchronize, and a leg is --blocks blocks
+    # (default 1), so `value` and `e2e` time exactly --steps steps each unless --blocks asks for more; with several
+    # blocks they are the median block. A short run is at boost clocks. With --sustained each leg then simply keeps
+    # going for sus_blocks more blocks (~0.4 s of continuous load): ~100 ms in, the board's power cap starts to pull the
+    # SM clock of a single busy GPU down, and it keeps drifting for seconds (under data parallelism the GPUs idle in the
+    # exchange and stay at boost). The median of the second half of those later blocks is reported as `sustained` -
+    # what a long job sees early on - and is never mixed into `value`.
+    n_blocks = max(1, args.blocks)
+    sus_blocks = int(min(200, math.ceil(400.0 / (args.steps * est_ms)))) if args.sustained else 0
 
     def leg_stats(all_ms):
         """(median ms per block of the first n_blocks blocks, median of the second half of the later blocks or None)"""
@@ -281,7 +306,7 @@ def run_ours(args):
     # batch i = a fresh random 8192-frame gather; a pool of index sets is cycled (the pool's footprint is far larger
     # than L2). Step i also hands the step function batch i + 1, which it gathers (and draws the noise for) on its
     # background stream while the GEMMs of step i run - the device-side analogue of a prefetching DataLoader.
-    pool = min(256, pre_steps + (n_blocks + sus_blocks) * args.steps + 1)
+    pool = min(256, pre_steps + (1 + n_blocks + sus_blocks) * args.steps + 1)
     g = torch.Generator(device=dev).manual_seed(100 + rank)
     frame_idx = torch.randint(0, n_frames, (pool, BATCH), generator=g, device=dev, dtype=torch.int64)
     batches = [FrameBatch(audio, BATCH, HOP, S, frame_idx=frame_idx[i]) for i in range(pool)]
@@ -336,10 +361,13 @@ def run_ours(args):
     clocks = NvmlSampler(dev)
     if rank == 0:
         clocks.start()
+    _, i, _, _ = timed_blocks(device_step, i, blocks=1)     # lead-in block, untimed
     l0 = ops.launch_count(dev) + step_fn.replayed_launches
     block_ms, i, loss, delta = timed_blocks(device_step, i, blocks=n_blocks)
     launches = ops.launch_count(dev) + step_fn.replayed_launches - l0   # eager launches + kernels inside graph replays
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model, opt, loss)
     sus_clk = None
     if sus_blocks > 0:   # the leg simply continues (no gap beyond the per-block barrier); clocks sampled separately
         sclocks = NvmlSampler(dev)
@@ -361,7 +389,7 @@ def run_ours(args):
     chunk = (BATCH - 1) * HOP + S
     n_chunks = max(1, (len(corpus) - chunk) // (BATCH * HOP))
     host_audio = torch.from_numpy(corpus).pin_memory()
-    n_e2e = pre_steps + (n_blocks + sus_blocks) * args.steps
+    n_e2e = pre_steps + (1 + n_blocks + sus_blocks) * args.steps
     host_loss = torch.zeros(n_e2e, dtype=torch.float32).pin_memory()
     dbuf = [torch.empty(chunk, dtype=torch.float32, device=dev) for _ in range(2)]
     copy_stream = torch.cuda.Stream(device=dev)
@@ -402,7 +430,9 @@ def run_ours(args):
         freed[b].record(main)
     j = settle(e2e_step, 0)
     # a block ends when its last loss has reached the host buffer
-    e2e_block_ms, j, _, e2e_delta = timed_blocks(e2e_step, j, end_of_block=lambda: main.wait_stream(d2h_stream),
+    loss_on_host = lambda: main.wait_stream(d2h_stream)
+    _, j, _, _ = timed_blocks(e2e_step, j, end_of_block=loss_on_host, blocks=1)     # lead-in block, untimed
+    e2e_block_ms, j, _, e2e_delta = timed_blocks(e2e_step, j, end_of_block=loss_on_host,
                                                  blocks=n_blocks + sus_blocks)
     e2e_ms, e2e_sus_ms = leg_stats(e2e_block_ms)
     e2e_value = BATCH * world * args.steps / (e2e_ms * 1e-3)
@@ -504,9 +534,9 @@ def run_ours(args):
                              % (audio.numel() * audio.element_size() / 1e6, "16-bit PCM, lossless" if audio.dtype == torch.int16 else "float32"),
                        "corpus": f"{args.files} files x {args.seconds:.0f} s, 0.5*sin+0.05*noise, rng 1234"},
             "timing": {"blocks": n_blocks, "steps_per_block": args.steps,
-                       "statistic": "median of the first %d blocks of the leg; max over ranks per block" % n_blocks,
+                       "statistic": "median of the %d timed blocks of the leg; max over ranks per block" % n_blocks,
                        "later_blocks_for_sustained": sus_blocks,
-                       "pre_steps_untimed": pre_steps, "block_ms": [round(v, 4) for v in block_ms],
+                       "pre_steps_untimed": pre_steps, "lead_in_steps_untimed": args.steps, "block_ms": [round(v, 4) for v in block_ms],
                        "captures_in_timed_region": delta["captures"], "eager_steps_in_timed_region": delta["eager"],
                        "graph_replays_in_timed_region": delta["replays"],
                        "e2e_block_ms": [round(v, 4) for v in e2e_block_ms],
@@ -696,15 +726,20 @@ def main():
     ap.add_argument("--files", type=int, default=32)
     ap.add_argument("--seconds", type=float, default=30.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--no-sustained", action="store_true", help="skip the later blocks of each leg (key `sustained`)")
+    ap.add_argument("--sustained", action=argparse.BooleanOptionalAction, default=False,
+                    help="continue each leg for ~0.4 s of later blocks after the timed steps (key `sustained`)")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the side legs (fp32 mode, kelsey_iterable.ini streaming, widened-VAE inference)")
-    ap.add_argument("--blocks", type=int, default=0,
-                    help="timed blocks of --steps steps each (median reported); 0 = enough for >= 0.3 s of load, >= 7")
+    ap.add_argument("--blocks", type=int, default=1,
+                    help="timed blocks of --steps steps each per leg (median reported)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)")
     ap.add_argument("--no-graph", dest="graph", action="store_false", help="enqueue every step eagerly (no CUDA graph)")
     ap.add_argument("--no-prefetch", dest="prefetch", action="store_false",
                     help="every step gathers its own batch (no background prefetch of the next one)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU arm's step (--impl ours)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

@@ -9,6 +9,7 @@ it); `torchaudio.load` (needs the absent torchcodec) is replaced by a scipy.io.w
 """
 from __future__ import annotations
 
+import hashlib
 import importlib.util
 import json
 import sys
@@ -102,6 +103,52 @@ def model_case(ref_model, S, H, L, B, steps, kl_beta, lr, store_full):
             "param_group": {k: v for k, v in ost["param_groups"][0].items() if k in ("lr", "betas", "eps", "weight_decay", "amsgrad")}}
 
 
+def digest(a: np.ndarray) -> str:
+    """SHA-256 of an array's dtype, shape and bytes."""
+    a = np.ascontiguousarray(a)
+    return hashlib.sha256(f"{a.dtype.str}{a.shape}".encode() + a.tobytes()).hexdigest()
+
+
+def small_inputs(S, H, L, B, steps) -> dict:
+    """The seeded inputs of model_case: the initial weights of `torch.manual_seed(0); VAE(S, H, L)` (nn.Linear's
+    default init in the reference's creation order, rawvae/model.py:13-17), then x and one eps per step drawn from
+    Generator seed 1. The caller's global RNG state is left as it was."""
+    with torch.random.fork_rng(devices=[]):
+        torch.manual_seed(0)
+        layers = [("fc1", torch.nn.Linear(S, H)), ("fc21", torch.nn.Linear(H, L)), ("fc22", torch.nn.Linear(H, L)),
+                  ("fc3", torch.nn.Linear(L, H)), ("fc4", torch.nn.Linear(H, S))]
+    out = {f"init/{n}.{w}": getattr(m, w).detach().numpy() for n, m in layers for w in ("weight", "bias")}
+    gen = torch.Generator().manual_seed(1)
+    out["x"] = (torch.rand(B, S, generator=gen) * 2 - 1).numpy()
+    out["eps"] = torch.stack([torch.randn(B, L, generator=gen) for _ in range(steps)]).numpy()
+    return out
+
+
+def split_small(arrays: dict):
+    """model_case's arrays as the two files under tests/golden (each under 1 MB): model_small.npz holds the
+    reference's outputs and, for the inputs small_inputs regenerates, their digests; model_small_adam.npz holds the
+    Adam moments after the last step."""
+    regen = [k for k in arrays if k in ("x", "eps") or k.startswith("init/")]
+    main = {k: v for k, v in arrays.items() if k not in regen and not k.startswith("exp_avg")}
+    main.update({"sha256/" + k: np.array(digest(arrays[k])) for k in regen})
+    adam = {k: v for k, v in arrays.items() if k.startswith("exp_avg")}
+    return main, adam
+
+
+def load_small(golden_dir: Path = OUT) -> dict:
+    """The arrays model_case returned, from the files split_small wrote. Regenerated inputs are checked against the
+    reference's digests; a mismatch (torch's generators no longer reproduce the reference's draws) raises."""
+    arrays = dict(np.load(golden_dir / "model_small.npz"))
+    arrays.update(np.load(golden_dir / "model_small_adam.npz"))
+    S, H, L, B, steps = (int(v) for v in arrays["meta"])
+    for k, a in small_inputs(S, H, L, B, steps).items():
+        want = str(arrays.pop("sha256/" + k))
+        if digest(a) != want:
+            raise ValueError(f"regenerated {k} does not reproduce the reference's (sha256 {digest(a)}, want {want})")
+        arrays[k] = a
+    return arrays
+
+
 def dataset_case(ref_ds):
     import scipy.io.wavfile as wavfile
     import torchaudio
@@ -162,8 +209,10 @@ def dataset_case(ref_ds):
 def main():
     OUT.mkdir(parents=True, exist_ok=True)
     ref_model, ref_ds = load_reference()
-    small = model_case(ref_model, S=128, H=192, L=64, B=48, steps=3, kl_beta=1e-4, lr=1e-3, store_full=True)
+    small, adam = split_small(model_case(ref_model, S=128, H=192, L=64, B=48, steps=3, kl_beta=1e-4, lr=1e-3,
+                                         store_full=True))
     np.savez_compressed(OUT / "model_small.npz", **small)
+    np.savez_compressed(OUT / "model_small_adam.npz", **adam)
     # default.ini dims (default.ini:5,18-20,26): summary statistics only
     default = model_case(ref_model, S=1024, H=2048, L=256, B=256, steps=2, kl_beta=1e-4, lr=1e-4, store_full=False)
     (OUT / "model_default_summary.json").write_text(json.dumps(default, indent=1))

@@ -62,7 +62,8 @@ def dev():
 
 @pytest.fixture(scope="module")
 def small(golden_dir):
-    return np.load(golden_dir / "model_small.npz")
+    from oracle import gen_golden
+    return gen_golden.load_small(golden_dir)
 
 
 def make_model(small, prefix, dev, precision):

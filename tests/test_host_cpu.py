@@ -357,6 +357,35 @@ def test_bench_data_generator_matches_the_tests_generator():
         assert not re.search(r"^\s*(from|import)\s+oracle", f.read_text(), re.M), f
 
 
+def test_bench_dump_outputs_files(tmp_path):
+    """bench.py --dump-outputs at the benchmark's dimensions: the loss, every parameter in full and the same seeded
+    sample of both Adam moments on every call, all float32, 64 MB at most."""
+    import importlib
+    from rawvae.model import VAE
+    bench = importlib.import_module("bench")
+    torch.manual_seed(0)
+    model = VAE(bench.S, bench.H, bench.L)
+    opt = torch.optim.Adam(model.parameters(), lr=bench.LR)
+    for p in model.parameters():
+        p.grad = torch.randn_like(p)
+    opt.step()
+    loss = torch.tensor(0.25)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), model, opt, loss)
+    names = ["loss", "exp_avg.sample", "exp_avg_sq.sample"] + [k for k, _ in model.named_parameters()]
+    assert sorted(f.name for f in (tmp_path / "a").iterdir()) == sorted(n + ".npy" for n in names)
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= 64 * 2 ** 20
+    got = {n: np.load(tmp_path / "a" / (n + ".npy")) for n in names}
+    assert all(a.dtype == np.float32 for a in got.values())
+    assert got["loss"] == np.float32(0.25)
+    for k, p in model.named_parameters():
+        assert np.array_equal(got[k], p.detach().numpy()), k
+    for key in ("exp_avg", "exp_avg_sq"):
+        full = torch.cat([opt.state[p][key].flatten() for p in model.parameters()]).numpy()
+        assert got[key + ".sample"].size == bench.MOMENT_SAMPLE and np.isin(got[key + ".sample"], full).all()
+        assert np.array_equal(got[key + ".sample"], np.load(tmp_path / "b" / (key + ".sample.npy")))
+
+
 def test_pcm16_passthrough_view_equals_the_decoded_file(tmp_path):
     """The streaming ingest copies 16-bit PCM files into pinned memory as they are (audio_io.open_pcm16); the int16
     values it hands to the GPU are exactly the ones the float decode (int16 / 32768, what torchaudio.load returns,

@@ -1,11 +1,12 @@
 """Pin the CPU oracle (oracle/rawvae_oracle.py) against outputs of the reference itself (tests/golden/*,
-written by oracle/gen_golden.py from the unmodified /root/reference code). CPU only."""
+written by oracle/gen_golden.py from the unmodified reference code). CPU only."""
 import json
 
 import numpy as np
 import pytest
 import torch
 
+from oracle import gen_golden
 from oracle import rawvae_oracle as O
 
 
@@ -17,7 +18,7 @@ def _rel(a, b):
 
 @pytest.fixture(scope="module")
 def small(golden_dir):
-    return np.load(golden_dir / "model_small.npz")
+    return gen_golden.load_small(golden_dir)
 
 
 def _params(small, prefix, dtype):
