@@ -172,6 +172,28 @@ int rvae_adam_step(rvae_ctx* ctx, float* p, const float* g, float* m, float* v, 
                    double beta2, double eps, double weight_decay, float grad_scale, const float* step, void* shadow_hi,
                    void* shadow_lo, void* stream);
 
+/* TensorBoard parameter histograms: replaces `for name, param in model.named_parameters(): writer.add_histogram(name,
+ * param, step)` (train_iterable.py:216-217, train.py:203-204), which copies every parameter to the host and sorts it.
+ * One launch bins n_segs segments of the fp32 buffer `params` (segment s = params[seg_offsets_host[s] ..
+ * + seg_lengths_host[s]), lengths >= 1) against edges_host (n_edges strictly increasing finite doubles, e.g.
+ * SummaryWriter.default_bins), with the semantics of torch.utils.tensorboard.summary.make_histogram on the values
+ * converted to float64: bin i counts [edges[i], edges[i+1]), the last bin is closed, values outside
+ * [edges[0], edges[n_edges-1]] and NaN are not counted; num counts every value; min / max are NaN if any value is
+ * NaN. Counts, min, max and num are exact; sum and sum of squares are fp64, reduced in a fixed order (bitwise
+ * reproducible, not numpy's summation order).
+ * `record` (device, 16-byte aligned, rvae_param_histogram_bytes() bytes) receives, with nb = n_edges - 1 and
+ * ns = n_segs, at these byte offsets:
+ *   0                     int32  counts[ns][nb]
+ *   A = align8(4 ns nb)   double sum[ns];  A + 8 ns: double sum_squares[ns];  A + 16 ns: int64 num[ns];
+ *   A + 24 ns             float  min[ns];  A + 28 ns: float max[ns];
+ * i.e. A + 32 ns bytes of results, followed by the kernel's scratch (rewritten by every call). */
+#define RVAE_HIST_MAX_SEGS 16
+#define RVAE_HIST_MAX_EDGES 2048
+size_t rvae_param_histogram_bytes(int n_segs, int n_edges); /* 0 for unsupported sizes */
+int rvae_param_histogram(rvae_ctx* ctx, const float* params, const int64_t* seg_offsets_host,
+                         const int64_t* seg_lengths_host, int n_segs, const double* edges_host, int n_edges,
+                         void* record, void* stream);
+
 /* ---------------------------------------------------------------------------------------------------------
  * tcgen05 GEMMs with fused epilogues (rawvae/model.py:19-35 forward; autograd backward of the same)
  * ------------------------------------------------------------------------------------------------------- */

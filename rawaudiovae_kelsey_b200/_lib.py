@@ -67,6 +67,8 @@ SIGNATURES = {
     "rvae_step_inc": (c_int, [P, P, P]),
     "rvae_adam_step": (c_int, [P, P, P, P, P, c_int64, c_double, c_double, c_double, c_double, c_double, c_float, P, P,
                                P, P]),
+    "rvae_param_histogram_bytes": (c_size_t, [c_int, c_int]),
+    "rvae_param_histogram": (c_int, [P, P, P, P, c_int, P, c_int, P, P]),
     "rvae_linear_act_fwd": (c_int, [P, P, P, P, P, P, c_int, c_int, c_int, c_int, P, P, P, P]),
     "rvae_encode_head_fwd": (c_int, [P, P, P, P, P, P, c_int, c_int, c_int, P, P, P, P, P, P, P]),
     "rvae_out_tanh_mse_fwd": (c_int, [P, P, P, P, P, P, c_int, c_int, c_int, P, P, c_int, P, P, P, c_float, P, P, P]),

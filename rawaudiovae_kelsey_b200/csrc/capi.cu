@@ -372,6 +372,14 @@ int rvae_adam_step(rvae_ctx* ctx, float* p, const float* g, float* m, float* v, 
   return launch_adam(&ctx->c, p, const_cast<float*>(g), m, v, n, lr, beta1, beta2, eps, weight_decay, grad_scale, step,
                      BF(shadow_hi), BF(shadow_lo), 0, S_(stream));
 }
+size_t rvae_param_histogram_bytes(int n_segs, int n_edges) { return param_histogram_bytes(n_segs, n_edges); }
+int rvae_param_histogram(rvae_ctx* ctx, const float* params, const int64_t* seg_offsets_host,
+                         const int64_t* seg_lengths_host, int n_segs, const double* edges_host, int n_edges,
+                         void* record, void* stream) {
+  CTX_OR_FAIL(ctx);
+  return launch_param_histogram(&ctx->c, params, seg_offsets_host, seg_lengths_host, n_segs, edges_host, n_edges,
+                                record, S_(stream));
+}
 
 // ---------------------------------------------------------------------------------------------------------
 // GEMM-level ops

@@ -183,6 +183,10 @@ int launch_adam2(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, in
                  unsigned int* ticket, __nv_bfloat16* shadow_hi, __nv_bfloat16* shadow_lo, int zero_grads,
                  cudaStream_t stream);
 int launch_step_inc(Ctx* ctx, float* step, cudaStream_t stream);
+// TensorBoard parameter histograms (rvae_param_histogram): record layout and size in include/rvae_b200.h
+size_t param_histogram_bytes(int n_segs, int n_edges);
+int launch_param_histogram(Ctx* ctx, const float* params, const int64_t* seg_offsets, const int64_t* seg_lengths,
+                           int n_segs, const double* edges, int n_edges, void* record, cudaStream_t stream);
 
 // Peer-memory all-reduce (elementwise.cu): symmetric buffers of all ranks as mapped in THIS process.
 constexpr int kP2PMaxWorld = 8;

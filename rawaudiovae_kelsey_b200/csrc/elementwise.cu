@@ -1,8 +1,13 @@
 // HBM-bound kernels of the hot path: framing / overlap-add, Philox normal noise, bf16 plane splitting,
 // bias-gradient column sums, the fused reparameterisation + reconstruction/KL loss kernels, and fused Adam.
 // All are coalesced, 128-bit vectorised, grid-strided with grids sized in multiples of the SM count.
+#include <algorithm>
+#include <cmath>
 #include <cstdlib>
+#include <cstring>
+#include <memory>
 
+#include "../../include/rvae_b200.h"
 #include "common.h"
 
 namespace rvae {
@@ -1209,6 +1214,292 @@ int launch_allreduce_p2p(Ctx* ctx, const P2PArgs& a, const P2PSegs& sg, int buck
     RVAE_CUDA(launch_kernel(ctx, allreduce_p2p_kernel<4, 4>, dim3(ctas), dim3(512), (size_t)0, stream, a, sg, bucket, tr));
   else
     RVAE_CUDA(launch_kernel(ctx, allreduce_p2p_kernel<8, 2>, dim3(ctas), dim3(512), (size_t)0, stream, a, sg, bucket, tr));
+  RVAE_LAUNCH_CHECK(ctx);
+  return RVAE_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// TensorBoard parameter histograms (writer.add_histogram, train_iterable.py:216-217, train.py:203-204): one launch
+// bins every parameter segment of the flat buffer against the caller's edge table with the semantics of
+// make_histogram(values.astype(float64), edges): bin i holds [e[i], e[i+1]), the last bin is closed, values outside
+// [e[0], e[n]] and NaN are not counted; min / max / num / sum / sum of squares over all values, NaN and +-inf
+// propagating as in numpy.
+//
+// Bin search. A float's order-preserving 32-bit key (sign-flipped bits) is split at its top 12 bits: a bucket spans a
+// magnitude ratio of at most 1.125 (1 sign + 8 exponent + 3 mantissa bits). guide[j] = number of edges <= the
+// smallest float of bucket j (computed on the host, exact in fp64), so every value of bucket j has between guide[j]
+// and guide[j + 1] edges below or at it and the exact count is found by a forward scan over that window, comparing
+// in fp64 against the table. TensorBoard's edges grow by 1.1 per step, so a window holds at most two edges: one or two
+// fp64 compares per value instead of an 11-step binary search over 1549 edges. Nothing assumes the edges' spacing:
+// a denser table only widens some windows.
+//
+// Contention. Initialised (and trained) weights are roughly uniform in +-1/sqrt(fan_in), and on TensorBoard's
+// log-spaced bins ~90 % of them land in the top ~25 bins of each sign. Each warp therefore owns a private
+// shared-memory sub-histogram (no inter-warp contention); within a warp the hottest bin sees ~2-3 lanes per
+// instruction, which the shared atomic unit serialises cheaply. A warp whose 32 values all fall into one bin (a
+// constant tensor, e.g. zero biases) issues a single atomic with the count. Blocks add their non-zero bins to the
+// record with integer atomics - exact, so the counts do not depend on the order blocks finish in.
+//
+// Moments. sum and sum of squares are fp64 (each square of an fp32 value is exact in fp64) and reduced in a FIXED
+// order: each thread sums its elements in index order, warps and blocks combine in fixed trees, the per-block partials
+// land in the scratch tail of the record and the last block to finish (ticket) adds them in a fixed order. The grid
+// depends only on the element count, so repeated calls - on any GPU - give bitwise-identical records. min / max are
+// reduced through atomicMax on order-preserving keys (order-independent as well).
+//
+// Algorithmic traffic: read 4 B per parameter, write the record (6.2 KB per segment for TensorBoard's 1548 bins).
+// ------------------------------------------------------------------------------------------------
+constexpr int kHistGuideBits = 12;
+constexpr int kHistGuide = 1 << kHistGuideBits;
+constexpr int kHistThreads = 256;
+constexpr int kHistWarps = kHistThreads / 32;
+constexpr int kHistUnroll = 4;               // values per lane per iteration (independent loads in flight)
+constexpr int64_t kHistMinChunk = 16384;     // elements per block (64 per thread) before the grid is capped
+constexpr int kHistMaxBlocks = 1024;
+
+struct HistArgs {
+  int64_t seg_off[RVAE_HIST_MAX_SEGS];          // element offset of segment s in params
+  int64_t vstart[RVAE_HIST_MAX_SEGS + 1];       // prefix sums of the lengths: the segments concatenated
+  int64_t chunk;                                // concatenated elements per block
+  int n_segs, n_edges;
+  double edges[RVAE_HIST_MAX_EDGES];
+  uint16_t guide[kHistGuide + 1];
+};
+static_assert(sizeof(HistArgs) <= 32000, "kernel parameter space (32764 bytes on sm_70+)");
+
+struct HistLayout {   // byte offsets into the caller's record buffer (include/rvae_b200.h)
+  size_t sum, sum_sq, num, vmin, vmax, record_bytes, min_key, max_key, nan_flag, ticket, partials, total;
+};
+static HistLayout hist_layout(int n_segs, int n_edges) {
+  HistLayout L;
+  const size_t ns = static_cast<size_t>(n_segs), nb = static_cast<size_t>(n_edges - 1);
+  L.sum = (4 * ns * nb + 7) / 8 * 8;
+  L.sum_sq = L.sum + 8 * ns;
+  L.num = L.sum_sq + 8 * ns;
+  L.vmin = L.num + 8 * ns;
+  L.vmax = L.vmin + 4 * ns;
+  L.record_bytes = L.vmax + 4 * ns;
+  L.min_key = L.record_bytes;
+  L.max_key = L.min_key + 4 * ns;
+  L.nan_flag = L.max_key + 4 * ns;
+  L.ticket = L.nan_flag + 4 * ns;
+  L.partials = (L.ticket + 4 + 7) / 8 * 8;
+  L.total = L.partials + 16 * ns * kHistMaxBlocks;
+  return L;
+}
+
+__host__ __device__ __forceinline__ uint32_t hist_key(float x) {   // a < b <=> key(a) < key(b) (non-NaN, -0 < +0)
+  uint32_t u;
+  memcpy(&u, &x, 4);
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__host__ __device__ __forceinline__ float hist_unkey(uint32_t k) {
+  const uint32_t u = (k & 0x80000000u) ? (k & 0x7fffffffu) : ~k;
+  float x;
+  memcpy(&x, &u, 4);
+  return x;
+}
+
+__device__ __forceinline__ double warp_sum_f64(double v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+  return v;   // lane 0
+}
+
+__global__ void __launch_bounds__(kHistThreads) param_histogram_kernel(const float* __restrict__ params,
+                                                                       const __grid_constant__ HistArgs a,
+                                                                       uint8_t* __restrict__ rec, HistLayout lay) {
+  ptx::pdl_launch_dependents();
+  extern __shared__ __align__(16) uint8_t hist_smem[];
+  const int nb = a.n_edges - 1;
+  double* edges = reinterpret_cast<double*>(hist_smem);
+  uint16_t* guide = reinterpret_cast<uint16_t*>(edges + a.n_edges);
+  int* sub_all = reinterpret_cast<int*>(hist_smem + ((8 * a.n_edges + 2 * (kHistGuide + 1) + 15) / 16 * 16));
+  __shared__ double red_s[kHistWarps], red_ss[kHistWarps];
+  __shared__ float red_mn[kHistWarps], red_mx[kHistWarps];
+  __shared__ int red_nan[kHistWarps];
+  __shared__ bool is_last;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  int* sub = sub_all + warp * nb;
+  for (int i = tid; i < a.n_edges; i += kHistThreads) edges[i] = a.edges[i];
+  for (int i = tid; i <= kHistGuide; i += kHistThreads) guide[i] = a.guide[i];
+  for (int i = tid; i < kHistWarps * nb; i += kHistThreads) sub_all[i] = 0;
+  __syncthreads();
+  ptx::pdl_wait();
+
+  int* counts = reinterpret_cast<int*>(rec);
+  uint32_t* min_key = reinterpret_cast<uint32_t*>(rec + lay.min_key);
+  uint32_t* max_key = reinterpret_cast<uint32_t*>(rec + lay.max_key);
+  uint32_t* nan_flag = reinterpret_cast<uint32_t*>(rec + lay.nan_flag);
+  double* partials = reinterpret_cast<double*>(rec + lay.partials);   // [seg][block][2]
+  const int64_t c0 = static_cast<int64_t>(blockIdx.x) * a.chunk;
+  const int64_t c1 = min(c0 + a.chunk, a.vstart[a.n_segs]);
+  const double e_last = edges[nb];
+  for (int s = 0; s < a.n_segs; ++s) {
+    const int64_t lo = max(c0, a.vstart[s]), hi = min(c1, a.vstart[s + 1]);
+    if (lo >= hi) continue;   // block-uniform
+    const float* p = params + a.seg_off[s] - a.vstart[s];
+    double sum = 0.0, sum_sq = 0.0;
+    float mn = INFINITY, mx = -INFINITY;
+    int nan = 0;
+    for (int64_t base = lo + warp * 32 * kHistUnroll; base < hi; base += kHistThreads * kHistUnroll) {
+      float x[kHistUnroll];
+#pragma unroll
+      for (int u = 0; u < kHistUnroll; ++u) {
+        const int64_t v = base + u * 32 + lane;
+        x[u] = v < hi ? __ldg(p + v) : __int_as_float(0x7fffffff);   // NaN = nothing to count
+      }
+#pragma unroll
+      for (int u = 0; u < kHistUnroll; ++u) {
+        const bool in = base + u * 32 + lane < hi;
+        const double xd = static_cast<double>(x[u]);
+        int bin = -1;
+        if (in) {
+          sum += xd;
+          sum_sq += xd * xd;
+          if (x[u] != x[u]) {
+            nan = 1;
+          } else {
+            mn = fminf(mn, x[u]);
+            mx = fmaxf(mx, x[u]);
+            const uint32_t j = hist_key(x[u]) >> (32 - kHistGuideBits);
+            int c = guide[j];
+            const int c_end = guide[j + 1];
+            while (c < c_end && edges[c] <= xd) ++c;
+            bin = c - 1;                                  // edges <= x, minus one
+            if (bin == nb && xd == e_last) bin = nb - 1;  // the last bin is closed
+            if (bin >= nb) bin = -1;
+          }
+        }
+        const int b0 = __shfl_sync(0xffffffffu, bin, 0);
+        if (__all_sync(0xffffffffu, bin == b0)) {
+          if (lane == 0 && b0 >= 0) atomicAdd(sub + b0, 32);
+        } else if (bin >= 0) {
+          atomicAdd(sub + bin, 1);
+        }
+      }
+    }
+    // block totals of this segment (fixed trees)
+    sum = warp_sum_f64(sum);
+    sum_sq = warp_sum_f64(sum_sq);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o));
+      mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+    }
+    nan = __any_sync(0xffffffffu, nan);
+    if (lane == 0) { red_s[warp] = sum; red_ss[warp] = sum_sq; red_mn[warp] = mn; red_mx[warp] = mx; red_nan[warp] = nan; }
+    __syncthreads();
+    if (tid == 0) {
+      double ts = 0.0, tss = 0.0;
+      float tmn = INFINITY, tmx = -INFINITY;
+      int tnan = 0;
+      for (int w = 0; w < kHistWarps; ++w) {
+        ts += red_s[w]; tss += red_ss[w];
+        tmn = fminf(tmn, red_mn[w]); tmx = fmaxf(tmx, red_mx[w]);
+        tnan |= red_nan[w];
+      }
+      partials[(static_cast<size_t>(s) * kHistMaxBlocks + blockIdx.x) * 2] = ts;
+      partials[(static_cast<size_t>(s) * kHistMaxBlocks + blockIdx.x) * 2 + 1] = tss;
+      // key 0 is below every real value's key, so 0 (the memset) is the identity of both maxima
+      if (tmn <= tmx) {
+        atomicMax(min_key + s, ~hist_key(tmn));
+        atomicMax(max_key + s, hist_key(tmx));
+      }
+      if (tnan) atomicOr(nan_flag + s, 1u);
+    }
+    // fold the warps' sub-histograms into the record and clear them for the next segment
+    for (int b = tid; b < nb; b += kHistThreads) {
+      int t = 0;
+#pragma unroll
+      for (int w = 0; w < kHistWarps; ++w) { t += sub_all[w * nb + b]; sub_all[w * nb + b] = 0; }
+      if (t) atomicAdd(counts + static_cast<size_t>(s) * nb + b, t);
+    }
+    __syncthreads();
+  }
+
+  // the last block to finish adds the per-block moments in block order and writes the scalar fields
+  __threadfence();
+  __syncthreads();
+  if (tid == 0) is_last = atomicAdd(reinterpret_cast<unsigned int*>(rec + lay.ticket), 1u) == gridDim.x - 1;
+  __syncthreads();
+  if (!is_last) return;
+  __threadfence();
+  // one warp per segment: lane l adds blocks b0 + l, b0 + l + 32, ... in order, then a fixed shuffle tree (32 loads
+  // in flight instead of one dependent L2 round trip per block)
+  for (int s = warp; s < a.n_segs; s += kHistWarps) {
+    const int64_t b0 = a.vstart[s] / a.chunk, b1 = (a.vstart[s + 1] - 1) / a.chunk;
+    double ts = 0.0, tss = 0.0;
+    for (int64_t b = b0 + lane; b <= b1; b += 32) {
+      ts += __ldcg(partials + (static_cast<size_t>(s) * kHistMaxBlocks + b) * 2);
+      tss += __ldcg(partials + (static_cast<size_t>(s) * kHistMaxBlocks + b) * 2 + 1);
+    }
+    ts = warp_sum_f64(ts);
+    tss = warp_sum_f64(tss);
+    if (lane != 0) continue;
+    reinterpret_cast<double*>(rec + lay.sum)[s] = ts;
+    reinterpret_cast<double*>(rec + lay.sum_sq)[s] = tss;
+    reinterpret_cast<int64_t*>(rec + lay.num)[s] = a.vstart[s + 1] - a.vstart[s];
+    const bool has_nan = __ldcg(nan_flag + s) != 0u;
+    const uint32_t kmn = ~__ldcg(min_key + s), kmx = __ldcg(max_key + s);
+    reinterpret_cast<float*>(rec + lay.vmin)[s] = has_nan ? __int_as_float(0x7fffffff) : hist_unkey(kmn);
+    reinterpret_cast<float*>(rec + lay.vmax)[s] = has_nan ? __int_as_float(0x7fffffff) : hist_unkey(kmx);
+  }
+}
+
+size_t param_histogram_bytes(int n_segs, int n_edges) {
+  if (n_segs < 1 || n_segs > RVAE_HIST_MAX_SEGS || n_edges < 2 || n_edges > RVAE_HIST_MAX_EDGES) return 0;
+  return hist_layout(n_segs, n_edges).total;
+}
+
+int launch_param_histogram(Ctx* ctx, const float* params, const int64_t* seg_offsets, const int64_t* seg_lengths,
+                           int n_segs, const double* edges, int n_edges, void* record, cudaStream_t stream) {
+  RVAE_REQUIRE(params && seg_offsets && seg_lengths && edges && record, RVAE_ERR_INVALID, "param_histogram: null pointer");
+  RVAE_REQUIRE(n_segs >= 1 && n_segs <= RVAE_HIST_MAX_SEGS, RVAE_ERR_INVALID,
+               "param_histogram: n_segs = %d, must be 1..%d", n_segs, RVAE_HIST_MAX_SEGS);
+  RVAE_REQUIRE(n_edges >= 2 && n_edges <= RVAE_HIST_MAX_EDGES, RVAE_ERR_INVALID,
+               "param_histogram: n_edges = %d, must be 2..%d", n_edges, RVAE_HIST_MAX_EDGES);
+  RVAE_REQUIRE(reinterpret_cast<uintptr_t>(record) % 16 == 0 && reinterpret_cast<uintptr_t>(params) % 4 == 0,
+               RVAE_ERR_INVALID, "param_histogram: record must be 16-byte and params 4-byte aligned");
+  for (int i = 0; i < n_edges; ++i) {
+    RVAE_REQUIRE(std::isfinite(edges[i]), RVAE_ERR_INVALID, "param_histogram: edge %d is not finite", i);
+    RVAE_REQUIRE(i == 0 || edges[i] > edges[i - 1], RVAE_ERR_INVALID,
+                 "param_histogram: edges must increase strictly (edge %d)", i);
+  }
+  std::unique_ptr<HistArgs> ap(new HistArgs());   // 25 KB of kernel arguments: not on the stack
+  HistArgs& a = *ap;
+  a.n_segs = n_segs;
+  a.n_edges = n_edges;
+  a.vstart[0] = 0;
+  for (int s = 0; s < n_segs; ++s) {
+    RVAE_REQUIRE(seg_offsets[s] >= 0 && seg_lengths[s] >= 1, RVAE_ERR_INVALID,
+                 "param_histogram: segment %d (offset %lld, length %lld) is empty or out of range", s,
+                 (long long)seg_offsets[s], (long long)seg_lengths[s]);
+    a.seg_off[s] = seg_offsets[s];
+    a.vstart[s + 1] = a.vstart[s] + seg_lengths[s];
+  }
+  memcpy(a.edges, edges, sizeof(double) * n_edges);
+  // guide[j] = #edges <= smallest float of key bucket j (NaN buckets: below / above everything); a merge walk
+  int c = 0;
+  for (int j = 0; j < kHistGuide; ++j) {
+    const float lo = hist_unkey(static_cast<uint32_t>(j) << (32 - kHistGuideBits));
+    if (lo != lo) {
+      a.guide[j] = static_cast<uint16_t>(j < kHistGuide / 2 ? 0 : n_edges);
+      continue;
+    }
+    while (c < n_edges && edges[c] <= static_cast<double>(lo)) ++c;
+    a.guide[j] = static_cast<uint16_t>(c);
+  }
+  a.guide[kHistGuide] = static_cast<uint16_t>(n_edges);
+  const int64_t total = a.vstart[n_segs];
+  a.chunk = std::max<int64_t>(kHistMinChunk, (total + kHistMaxBlocks - 1) / kHistMaxBlocks);
+  const int grid = static_cast<int>((total + a.chunk - 1) / a.chunk);
+  const HistLayout lay = hist_layout(n_segs, n_edges);
+  const size_t smem = (8 * (size_t)n_edges + 2 * (kHistGuide + 1) + 15) / 16 * 16 + 4 * (size_t)kHistWarps * (n_edges - 1);
+  RVAE_CUDA(cudaFuncSetAttribute(param_histogram_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  // counts, min / max keys, NaN flags and the ticket start from zero; sums and partials are overwritten
+  RVAE_CUDA(cudaMemsetAsync(record, 0, lay.partials, stream));
+  RVAE_CUDA(launch_kernel(ctx, param_histogram_kernel, dim3(grid), dim3(kHistThreads), smem, stream, params, *ap,
+                          static_cast<uint8_t*>(record), lay));
   RVAE_LAUNCH_CHECK(ctx);
   return RVAE_OK;
 }

@@ -7,6 +7,7 @@ from __future__ import annotations
 import ctypes as C
 from typing import Optional, Tuple
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -234,6 +235,55 @@ def adam_step(p, g, m, v, step, lr, beta1=0.9, beta2=0.999, eps=1e-8, weight_dec
                              _ptr(v, torch.float32, "v"), p.numel(), lr, beta1, beta2, eps, weight_decay, grad_scale,
                              _ptr(step, torch.float32, "step"), _ptr(shadow_hi, torch.bfloat16),
                              _ptr(shadow_lo, torch.bfloat16), _stream()))
+
+
+def histogram_record_layout(n_segs: int, n_edges: int) -> dict:
+    """Byte offsets of the fields of an rvae_param_histogram record (include/rvae_b200.h); "bytes" = results only,
+    "total" = results + the kernel's scratch (what the device buffer must hold)."""
+    nb = n_edges - 1
+    a = (4 * n_segs * nb + 7) // 8 * 8
+    total = int(_lib.load().rvae_param_histogram_bytes(n_segs, n_edges))
+    if total == 0:
+        raise _lib.RvaeError(f"param_histogram: {n_segs} segments / {n_edges} edges are not supported")
+    return {"counts": 0, "sum": a, "sum_squares": a + 8 * n_segs, "num": a + 16 * n_segs, "min": a + 24 * n_segs,
+            "max": a + 28 * n_segs, "bytes": a + 32 * n_segs, "total": total}
+
+
+def param_histogram(params: torch.Tensor, seg_offsets, seg_lengths, edges, out: Optional[torch.Tensor] = None):
+    """TensorBoard histograms (make_histogram semantics) of the segments params[seg_offsets[s] : + seg_lengths[s]] of
+    a flat fp32 CUDA tensor against the float64 bin edges `edges`, in one launch on the current stream. Returns the
+    device record (uint8; `out` if given, at least histogram_record_layout(...)["total"] bytes): unpack a host copy
+    of its first ["bytes"] bytes with unpack_histogram_record."""
+    lib = _lib.load()
+    p = _ptr(params, torch.float32, "params")
+    offs = np.ascontiguousarray(seg_offsets, dtype=np.int64)
+    lens = np.ascontiguousarray(seg_lengths, dtype=np.int64)
+    e = np.ascontiguousarray(edges, dtype=np.float64)
+    if offs.shape != lens.shape or offs.ndim != 1:
+        raise _lib.RvaeError("param_histogram: seg_offsets and seg_lengths must be 1-D and of equal length")
+    if offs.size and (int((offs + lens).max()) > params.numel() or int(offs.min()) < 0):
+        raise _lib.RvaeError("param_histogram: a segment lies outside params")
+    lay = histogram_record_layout(offs.size, e.size)
+    if out is None:
+        out = torch.empty(lay["total"], dtype=torch.uint8, device=params.device)
+    elif out.numel() < lay["total"]:
+        raise _lib.RvaeError(f"param_histogram: record buffer holds {out.numel()} bytes, needs {lay['total']}")
+    check(lib.rvae_param_histogram(ctx(params.device), p, offs.ctypes.data,
+                                   lens.ctypes.data, offs.size, e.ctypes.data, e.size, _ptr(out, torch.uint8, "out"),
+                                   _stream()))
+    return out
+
+
+def unpack_histogram_record(buf, n_segs: int, n_edges: int) -> dict:
+    """numpy views of a host copy (uint8 tensor or array, at least ["bytes"] long) of a param_histogram record:
+    counts int32 [n_segs, n_edges - 1], sum / sum_squares float64, num int64, min / max float32, each [n_segs]."""
+    lay = histogram_record_layout(n_segs, n_edges)
+    raw = buf.numpy() if isinstance(buf, torch.Tensor) else np.asarray(buf)
+    raw = raw[:lay["bytes"]]
+    f = lambda key, dt, n: np.frombuffer(raw, dtype=dt, count=n, offset=lay[key])
+    return {"counts": f("counts", np.int32, n_segs * (n_edges - 1)).reshape(n_segs, n_edges - 1),
+            "sum": f("sum", np.float64, n_segs), "sum_squares": f("sum_squares", np.float64, n_segs),
+            "num": f("num", np.int64, n_segs), "min": f("min", np.float32, n_segs), "max": f("max", np.float32, n_segs)}
 
 
 # --------------------------------------------------------------------------------------------- GEMM-level ops

@@ -29,6 +29,7 @@ from . import audio_io, dist as rdist
 from .dataset import AudioDataset, IterableAudioDataset, ToTensor
 from .model import VAE, FusedTrainStep
 from .optim import Adam
+from .stats import ParamHistogramLogger
 from .testaudio import init_test_audio
 
 
@@ -217,6 +218,9 @@ def run_epoch_trainer(argv=None):
     else:
         step = FusedTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph)
 
+    # parameter histograms on the GPU (rank 0 only): one launch + one small asynchronous copy per set
+    hist = ParamHistogramLogger(model, writer) if rank == 0 else None
+
     train_loss_prev = 1000000
     best_loss = 1000000
     final_loss = 1000000
@@ -236,17 +240,20 @@ def run_epoch_trainer(argv=None):
             batch_id += 1
             if len(pending) >= log_interval:
                 train_loss += _flush_losses(writer, pending, world=world)
+                if hist is not None:
+                    hist.flush()
         train_loss += _flush_losses(writer, pending, world=world)
         print('====> Epoch: {} - Total loss: {} - Average loss: {:.9f}'.format(
             epoch, train_loss, train_loss / len(training_dataset)))
         writer.add_scalar('Loss/train_total', train_loss, epoch)
         writer.add_scalar('Loss/train_average', train_loss / len(training_dataset), epoch)
-        if rank == 0:
-            for name, param in model.named_parameters():
-                writer.add_histogram(name, param, epoch)
+        if hist is not None:
+            hist.record(epoch)
+            hist.flush()
 
         if rank == 0 and epoch % checkpoint_interval == 0 and epoch != 0:
             print('Checkpoint - Epoch {}'.format(epoch))
+            hist.flush(wait=True)
             state = {'epoch': epoch, 'state_dict': model.state_dict(), 'optimizer': optimizer.state_dict()}
             if generate_test:
                 audio_out = audio_log_dir.joinpath('test_reconst_{:05d}.wav'.format(epoch))
@@ -269,6 +276,7 @@ def run_epoch_trainer(argv=None):
         final_loss = train_loss
 
     if rank == 0:
+        hist.flush(wait=True)
         print('Last Checkpoint - Epoch {}'.format(epochs))
         state = {'epoch': epochs, 'state_dict': model.state_dict(), 'optimizer': optimizer.state_dict()}
         if generate_test:
@@ -368,6 +376,8 @@ def run_stream_trainer(argv=None):
         else:
             step = FusedTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph)
 
+        hist = ParamHistogramLogger(model, writer) if rank == 0 and histogram_interval > 0 else None
+
         train_loss_prev = 1000000
         best_loss = 1000000
         model.train()
@@ -382,11 +392,14 @@ def run_stream_trainer(argv=None):
             at_checkpoint = batch_id % checkpoint_interval == 0 and batch_id != 0
             if len(pending) >= log_interval or at_checkpoint:
                 train_loss += _flush_losses(writer, pending, fmt if rank == 0 else None, world=world)
-            if rank == 0 and histogram_interval > 0 and batch_id % histogram_interval == 0:
-                for name, param in model.named_parameters():
-                    writer.add_histogram(name, param, batch_id)
+                if hist is not None:
+                    hist.flush()
+            if hist is not None and batch_id % histogram_interval == 0:
+                hist.record(batch_id)   # same stream as the step: sees its Adam update, precedes the next step
             if rank == 0 and at_checkpoint:
                 print('Checkpoint - Epoch {}'.format(batch_id))
+                if hist is not None:
+                    hist.flush(wait=True)
                 state = {'batch_id': batch_id, 'state_dict': model.state_dict(), 'optimizer': optimizer.state_dict()}
                 if generate_test:
                     audio_out = audio_log_dir.joinpath('test_reconst_{:05d}.wav'.format(batch_id))
@@ -410,6 +423,8 @@ def run_stream_trainer(argv=None):
         final_loss = train_loss
 
         if rank == 0:
+            if hist is not None:
+                hist.flush(wait=True)
             print('Last Checkpoint - batch_id {}'.format(batch_id))
             state = {'batch_id': batch_id, 'state_dict': model.state_dict(), 'optimizer': optimizer.state_dict()}
             if generate_test:
