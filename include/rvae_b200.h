@@ -15,7 +15,11 @@
  *     as torch.nn.Linear stores them (rawvae/model.py:13-17);
  *   - bf16 planes: a tensor `t` is carried as t_hi = bf16(t) and, in fp32-emulation mode, t_lo = bf16(t - t_hi).
  *     Passing NULL for every *_lo pointer selects bf16 mode;
- *   - shape constraints of the sm_100a kernels: segment_length, n_units, latent_dim multiples of 64.
+ *   - shapes: a plan (rvae_plan_create) accepts any positive segment_length S, n_units H and latent_dim L. It computes
+ *     at Sp, Hp, Lp = the dims rounded up to multiples of 64 (rvae_param_layout_padded), with exact zeros in every
+ *     padded row, column and bias, and normalises the loss by the true dims; caller tensors keep their true shapes.
+ *     Dims that are multiples of 64 have no padding. The single-GEMM entry points (rvae_linear_act_fwd ..
+ *     rvae_wgrad) need their GEMM dims to be multiples of 64.
  */
 #ifndef RVAE_B200_H
 #define RVAE_B200_H
@@ -104,7 +108,7 @@ int rvae_dp_status(rvae_ctx* ctx, unsigned int* status);
  * 141-143, 61-63). Replaces AudioDataset.__getitem__ (dataset.py:108-118), TestDataset.__getitem__ (:147-157),
  * IterableAudioDataset.process_data's slicing loop (:68-75) and default_collate's stack.
  * audio is float32 (audio_is_i16 = 0) or int16 PCM scaled by 1/32768 (audio_is_i16 = 1). Any of the three
- * outputs may be NULL (at least one of out_hi / out_f32 required). Outputs are [n_frames, S]. */
+ * outputs may be NULL (at least one of out_hi / out_f32 required). Outputs are [n_frames, S], any S > 0. */
 int rvae_frame_gather(rvae_ctx* ctx, const void* audio, int audio_is_i16, int64_t n_samples,
                       const int64_t* frame_idx, int64_t first_frame, int64_t n_frames, int hop, int S,
                       void* out_hi, void* out_lo, float* out_f32, void* stream);
@@ -121,11 +125,11 @@ int rvae_overlap_add(rvae_ctx* ctx, const float* frames, int64_t n_frames, int S
 
 /* eps ~ N(0,1), Philox4x32-10 + Box-Muller keyed by (seed, offset). Replaces torch.randn_like (model.py:25).
  * out[i] is element (elem_base + i) of the logical noise tensor of that (seed, offset): a rank that owns rows
- * [r0, r1) of a global [B, L] batch passes elem_base = r0 * L (a multiple of 4) and draws exactly the values a
+ * [r0, r1) of a global [B, L] batch passes elem_base = r0 * L (any elem_base >= 0) and draws exactly the values a
  * single process would have drawn for those rows. */
 int rvae_randn(rvae_ctx* ctx, float* out, int64_t n, uint64_t seed, uint64_t offset, int64_t elem_base, void* stream);
 
-/* Latent interpolation of the inference pattern (tutorial.ipynb:496-510, 905-932): per row r,
+/* Latent interpolation of the inference pattern (tutorial.ipynb:496-510, 905-932), any L > 0: per row r,
  *   mu = (1 - alpha[r]) mu_a + alpha[r] mu_b, logvar likewise, z = mu + eps * exp(logvar / 2)   (eps NULL = 0).
  * alpha: `rows` floats, or doubles when alpha_is_f64 (the notebook's interp1d output); the lerp is then carried out
  * in double. Outputs (each may be NULL, not all): z, mu_out, logvar_out, fp32 [rows, L]. */
@@ -193,6 +197,13 @@ size_t rvae_param_histogram_bytes(int n_segs, int n_edges); /* 0 for unsupported
 int rvae_param_histogram(rvae_ctx* ctx, const float* params, const int64_t* seg_offsets_host,
                          const int64_t* seg_lengths_host, int n_segs, const double* edges_host, int n_edges,
                          void* record, void* stream);
+/* The same over strided segments: segment s = seg_rows_host[s] rows of seg_cols_host[s] values, row r starting at
+ * params[seg_offsets_host[s] + r * seg_pitch_host[s]] (seg_pitch >= seg_cols): a parameter of a padded plan inside its
+ * padded block, e.g. fc1.weight = H rows of S values at pitch Sp. num = rows * cols. rvae_param_histogram is the
+ * one-row case. */
+int rvae_param_histogram_rows(rvae_ctx* ctx, const float* params, const int64_t* seg_offsets_host,
+                              const int64_t* seg_rows_host, const int64_t* seg_cols_host, const int64_t* seg_pitch_host,
+                              int n_segs, const double* edges_host, int n_edges, void* record, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------
  * tcgen05 GEMMs with fused epilogues (rawvae/model.py:19-35 forward; autograd backward of the same)
@@ -253,7 +264,15 @@ typedef struct rvae_layout {
   int64_t total;                          /* total elements (5 772 800 for default.ini) */
 } rvae_layout;
 
-int rvae_param_layout(int S, int H, int L, rvae_layout* out);
+int rvae_param_layout(int S, int H, int L, rvae_layout* out);   /* S, H, L multiples of 64 */
+
+/* Layout of the padded blocks a plan of ANY positive dims uses: *Sp, *Hp, *Lp = S, H, L rounded up to multiples of 64;
+ * W1 [Hp,Sp] | W2 [2Lp,Hp] | W3 [Hp,Lp] | W4 [Sp,Hp] | b1 [Hp] | b2 [2Lp] | b3 [Hp] | b4 [Sp], i.e.
+ * rvae_param_layout(Sp, Hp, Lp). A parameter is the top-left corner of its block: fc1.weight = W1[:H, :S],
+ * fc21 = rows [0, L) of W2 and fc22 = rows [Lp, Lp + L), fc21.bias = b2[0:L], fc22.bias = b2[Lp:Lp+L], ... Everything
+ * outside those corners is zero and stays zero through training (gradients and Adam moments included). For multiples
+ * of 64 it equals rvae_param_layout. */
+int rvae_param_layout_padded(int S, int H, int L, rvae_layout* out, int* Sp, int* Hp, int* Lp);
 
 typedef struct rvae_plan_buffers {
   float* params;    /* [total] fp32 master weights */
@@ -280,7 +299,7 @@ int rvae_plan_sync_shadow(rvae_plan* plan, void* stream);
 int rvae_plan_load_frames(rvae_plan* plan, const void* audio, int audio_is_i16, int64_t n_samples,
                           const int64_t* frame_idx, int64_t first_frame, int count, int hop, int row_offset,
                           void* stream);
-/* ... or an fp32 [batch, S] matrix already on the device. */
+/* ... or an fp32 [batch, S] matrix already on the device (true S; a padded plan pads it on the way in). */
 int rvae_plan_load_batch(rvae_plan* plan, const float* x, int batch, void* stream);
 /* ... or a RUN of `count` consecutive frames (first_frame, first_frame + 1, ...: the stream of
  * IterableAudioDataset.process_data, rawvae/dataset.py:61-69, TestDataset with hop = S, tutorial.ipynb's inference
@@ -289,7 +308,8 @@ int rvae_plan_load_batch(rvae_plan* plan, const float* x, int batch, void* strea
  * gradient's operand then read frame i at row pitch `hop` through overlapping-row TMA tensor maps - the [count, S]
  * frame matrix is never materialised and every sample is touched once instead of S / hop times. Results are
  * bit-identical to rvae_plan_load_frames. first_frame_dev (device int64, may be NULL) overrides first_frame and is
- * read by the kernel, so a captured CUDA graph follows the stream. Needs hop % 8 == 0 and hop <= S
+ * read by the kernel, so a captured CUDA graph follows the stream. Needs hop % 8 == 0, hop <= S and S % 8 == 0; with
+ * S not a multiple of 64 (columns S..Sp read as zeros through the tensor maps) also bf16 mode
  * (rvae_plan_span_supported). */
 int rvae_plan_span_supported(const rvae_plan* plan, int count, int hop);
 int rvae_plan_load_span(rvae_plan* plan, const void* audio, int audio_is_i16, int64_t n_samples,
@@ -374,17 +394,19 @@ int rvae_plan_adam_buckets(rvae_plan* plan, unsigned bucket_mask, double lr, dou
 int rvae_plan_train_step(rvae_plan* plan, float kl_beta, double lr, double beta1, double beta2, double eps,
                          double weight_decay, int zero_grads, float* loss_out, int ring_size, void* stream);
 
-/* Device pointers into the workspace for the current batch (valid after forward): fp32 [batch, ...]. */
+/* Device pointers into the workspace for the current batch (valid after forward): fp32 [batch, ...] at the plan's
+ * padded row pitch - mu, logvar, eps [batch, Lp], xhat [batch, Sp] (rvae_param_layout_padded); only the first L (S)
+ * columns of a row are the model's, the rest are zeros. */
 const float* rvae_plan_mu(const rvae_plan* plan);
 const float* rvae_plan_logvar(const rvae_plan* plan);
 const float* rvae_plan_xhat(const rvae_plan* plan);
 const float* rvae_plan_eps(const rvae_plan* plan);
 /* Introspection (tests / debugging): device pointers to the bf16 planes of an intermediate of the current batch.
- * which: 0 x [B,S], 1 h1 [B,H], 2 z [B,L], 3 h3 [B,H], 4 da4 [B,S], 5 da3 [B,H], 6 d_ml [B,2L], 7 da1 [B,H].
- * *lo is NULL in bf16 mode. */
+ * which: 0 x [B,S], 1 h1 [B,H], 2 z [B,L], 3 h3 [B,H], 4 da4 [B,S], 5 da3 [B,H], 6 d_ml [B,2L], 7 da1 [B,H], all
+ * at the padded dims (*cols = the row pitch). *lo is NULL in bf16 mode. */
 int rvae_plan_activation(const rvae_plan* plan, int which, void** hi, void** lo, int* cols);
 /* gradient bucket s (see rvae_plan_backward): pointer into bufs.grads and element count. Buckets 0..3 are the
- * four weight matrices in backward-completion order; bucket 4 is the bias block. */
+ * four weight matrices in backward-completion order; bucket 4 is the bias block (padded blocks of a padded plan). */
 int rvae_plan_bucket(const rvae_plan* plan, int s, float** ptr, int64_t* count);
 
 /* Per-kernel device timing (bench.py roofline): when enabled, every launch of the plan is bracketed by CUDA events

@@ -69,6 +69,7 @@ SIGNATURES = {
                                P, P]),
     "rvae_param_histogram_bytes": (c_size_t, [c_int, c_int]),
     "rvae_param_histogram": (c_int, [P, P, P, P, c_int, P, c_int, P, P]),
+    "rvae_param_histogram_rows": (c_int, [P, P, P, P, P, P, c_int, P, c_int, P, P]),
     "rvae_linear_act_fwd": (c_int, [P, P, P, P, P, P, c_int, c_int, c_int, c_int, P, P, P, P]),
     "rvae_encode_head_fwd": (c_int, [P, P, P, P, P, P, c_int, c_int, c_int, P, P, P, P, P, P, P]),
     "rvae_out_tanh_mse_fwd": (c_int, [P, P, P, P, P, P, c_int, c_int, c_int, P, P, c_int, P, P, P, c_float, P, P, P]),
@@ -76,6 +77,8 @@ SIGNATURES = {
     "rvae_dgrad_latent": (c_int, [P, P, P, P, P, c_int, c_int, c_int, P, P, P, P, P, c_float, P, P, P, P, P]),
     "rvae_wgrad": (c_int, [P, P, P, P, P, c_int, c_int, c_int, P, c_int, c_int, P]),
     "rvae_param_layout": (c_int, [c_int, c_int, c_int, C.POINTER(Layout)]),
+    "rvae_param_layout_padded": (c_int, [c_int, c_int, c_int, C.POINTER(Layout), C.POINTER(c_int), C.POINTER(c_int),
+                                         C.POINTER(c_int)]),
     "rvae_plan_create": (c_int, [P, c_int, c_int, c_int, c_int, c_int, C.POINTER(P)]),
     "rvae_plan_destroy": (None, [P]),
     "rvae_plan_workspace_bytes": (c_size_t, [P]),

@@ -311,7 +311,7 @@ int rvae_frame_gather(rvae_ctx* ctx, const void* audio, int audio_is_i16, int64_
                       const int64_t* frame_idx, int64_t first_frame, int64_t n_frames, int hop, int S, void* out_hi,
                       void* out_lo, float* out_f32, void* stream) {
   CTX_OR_FAIL(ctx);
-  return launch_frame_gather(&ctx->c, audio, audio_is_i16, n_samples, frame_idx, first_frame, n_frames, hop, S,
+  return launch_frame_gather(&ctx->c, audio, audio_is_i16, n_samples, frame_idx, first_frame, n_frames, hop, S, S,
                              BF(out_hi), BF(out_lo), out_f32, S_(stream));
 }
 int rvae_overlap_add(rvae_ctx* ctx, const float* frames, int64_t n_frames, int S, int hop, float* out, int64_t t_begin,
@@ -322,13 +322,17 @@ int rvae_overlap_add(rvae_ctx* ctx, const float* frames, int64_t n_frames, int S
 int rvae_randn(rvae_ctx* ctx, float* out, int64_t n, uint64_t seed, uint64_t offset, int64_t elem_base,
                void* stream) {
   CTX_OR_FAIL(ctx);
+  RVAE_REQUIRE(elem_base >= 0, RVAE_ERR_INVALID, "randn: elem_base %lld", (long long)elem_base);
+  // a base that is not a multiple of 4 starts inside a Philox block (a shard of a [B, L] draw with odd L): one row
+  // of the element-wise kernel
+  if (elem_base % 4 != 0) return launch_randn_rows(&ctx->c, out, 1, n, n, seed, offset, nullptr, elem_base, S_(stream));
   return launch_randn(&ctx->c, out, n, seed, offset, nullptr, elem_base, S_(stream));
 }
 int rvae_lerp_reparameterize(rvae_ctx* ctx, const float* mu_a, const float* logvar_a, const float* mu_b,
                              const float* logvar_b, const void* alpha, int alpha_is_f64, const float* eps,
                              int64_t rows, int L, float* z, float* mu_out, float* logvar_out, void* stream) {
   CTX_OR_FAIL(ctx);
-  return launch_lerp_reparam(&ctx->c, mu_a, logvar_a, mu_b, logvar_b, alpha, alpha_is_f64, eps, rows, L, z, nullptr,
+  return launch_lerp_reparam(&ctx->c, mu_a, logvar_a, mu_b, logvar_b, alpha, alpha_is_f64, eps, rows, L, L, z, nullptr,
                              nullptr, mu_out, logvar_out, S_(stream));
 }
 int rvae_split_bf16(rvae_ctx* ctx, const float* src, int64_t n, void* hi, void* lo, void* stream) {
@@ -380,6 +384,13 @@ int rvae_param_histogram(rvae_ctx* ctx, const float* params, const int64_t* seg_
   return launch_param_histogram(&ctx->c, params, seg_offsets_host, seg_lengths_host, n_segs, edges_host, n_edges,
                                 record, S_(stream));
 }
+int rvae_param_histogram_rows(rvae_ctx* ctx, const float* params, const int64_t* seg_offsets_host,
+                              const int64_t* seg_rows_host, const int64_t* seg_cols_host, const int64_t* seg_pitch_host,
+                              int n_segs, const double* edges_host, int n_edges, void* record, void* stream) {
+  CTX_OR_FAIL(ctx);
+  return launch_param_histogram_rows(&ctx->c, params, seg_offsets_host, seg_rows_host, seg_cols_host, seg_pitch_host,
+                                     n_segs, edges_host, n_edges, record, S_(stream));
+}
 
 // ---------------------------------------------------------------------------------------------------------
 // GEMM-level ops
@@ -392,7 +403,7 @@ static GemmDesc desc_base(int epi, int M, int N, int K) {
 }
 static Operand op(const void* hi, const void* lo, int major, int ld) {
   Operand o;
-  o.hi = BF(hi); o.lo = BF(lo); o.major = major; o.ld = ld;
+  o.hi = BF(hi); o.lo = BF(lo); o.major = major; o.ld = ld; o.cols = 0;
   return o;
 }
 
@@ -501,6 +512,16 @@ int rvae_param_layout(int S, int H, int L, rvae_layout* out) {
   return RVAE_OK;
 }
 
+int rvae_param_layout_padded(int S, int H, int L, rvae_layout* out, int* Sp, int* Hp, int* Lp) {
+  RVAE_REQUIRE(out && Sp && Hp && Lp, RVAE_ERR_INVALID, "param_layout_padded: null out");
+  RVAE_REQUIRE(S > 0 && H > 0 && L > 0 && S <= (1 << 24) && H <= (1 << 24) && L <= (1 << 24), RVAE_ERR_UNSUPPORTED,
+               "segment_length=%d, n_units=%d, latent_dim=%d must be in 1..%d", S, H, L, 1 << 24);
+  const int sp = (S + 63) / 64 * 64, hp = (H + 63) / 64 * 64, lp = (L + 63) / 64 * 64;
+  RVAE_CHECK(rvae_param_layout(sp, hp, lp, out));
+  *Sp = sp; *Hp = hp; *Lp = lp;
+  return RVAE_OK;
+}
+
 }  // extern "C"
 
 // ---------------------------------------------------------------------------------------------------------
@@ -539,7 +560,11 @@ struct GemmSet {
 
 struct rvae_plan {
   rvae_ctx* ctx;
+  // S, H, L: the dims the plan computes at - the model's dims rounded up to multiples of 64 (rvae_param_layout_padded):
+  // workspace, GEMM shapes, tensor maps, parameter blocks. The padding holds exact zeros through every step.
+  // s_true, h_true, l_true: the model's dims - loss normalisation and the shapes of every caller tensor.
   int S, H, L, max_batch, precision;
+  int s_true, h_true, l_true;
   rvae_layout lay;
   rvae_plan_buffers bufs;
   bool bound;
@@ -547,6 +572,8 @@ struct rvae_plan {
   // workspace sections
   Planes x, h1, z, h3, da4, da3, dml, da1;
   float *mu, *lv, *eps, *dz, *xhat;
+  // padded plans only: the external upstream gradients of rvae_plan_backward_external at the padded row pitch
+  float *ext_gx, *ext_gmu, *ext_glv, *ext_lv;
   // second input set (frames + noise) the background stream fills for the NEXT step while this one runs
   Planes x_alt;
   float* eps_alt;
@@ -668,19 +695,26 @@ size_t carve(rvae_plan* p, uint8_t* base) {
   p->dz = reinterpret_cast<float*>(take(B * L * 4));
   p->xhat = reinterpret_cast<float*>(take(B * S * 4));
   p->loss_acc = reinterpret_cast<double*>(take(2 * sizeof(double)));
+  p->ext_gx = p->ext_gmu = p->ext_glv = p->ext_lv = nullptr;
+  if (p->S != (size_t)p->s_true) p->ext_gx = reinterpret_cast<float*>(take(B * S * 4));
+  if (p->L != (size_t)p->l_true) {
+    p->ext_gmu = reinterpret_cast<float*>(take(B * L * 4));
+    p->ext_glv = reinterpret_cast<float*>(take(B * L * 4));
+    p->ext_lv = reinterpret_cast<float*>(take(B * L * 4));
+  }
   return off;
 }
 
 Operand opnd(const Planes& pl, int major, int ld) {
   Operand o;
-  o.hi = pl.hi; o.lo = pl.lo; o.major = major; o.ld = ld;
+  o.hi = pl.hi; o.lo = pl.lo; o.major = major; o.ld = ld; o.cols = 0;
   return o;
 }
 Operand wopnd(const rvae_plan* p, int64_t off, int major, int ld) {
   Operand o;
   o.hi = BF(p->bufs.shadow_hi) + off;
   o.lo = p->bufs.shadow_lo ? BF(p->bufs.shadow_lo) + off : nullptr;
-  o.major = major; o.ld = ld;
+  o.major = major; o.ld = ld; o.cols = 0;
   return o;
 }
 
@@ -698,6 +732,7 @@ int prepare(rvae_plan* p, GemmSet& gs, int id) {
     case G_F1:
       d.epi = EPI_LINEAR; d.M = B; d.N = H; d.K = S;
       d.A = opnd(p->x, MAJOR_K, ldx); d.B = wopnd(p, ly.w1, MAJOR_K, S);
+      d.A.cols = p->s_true;   // frames read in place: the columns past segment_length are padding (zeros)
       d.args.bias = params + ly.b1; d.args.act = ACT_RELU; d.args.ldo = H;
       d.args.out_hi = p->h1.hi; d.args.out_lo = p->h1.lo;
       break;
@@ -720,7 +755,7 @@ int prepare(rvae_plan* p, GemmSet& gs, int id) {
       d.args.bias = params + ly.b4; d.args.in0 = p->x.hi; d.args.in1 = p->x.lo; d.args.out_f32 = p->xhat;
       d.args.out_hi = p->da4.hi; d.args.out_lo = p->da4.lo;
       d.args.act = bf16_mode ? ACT_TANH_APPROX : ACT_TANH;
-      d.args.loss_acc = p->loss_acc; d.args.ldo = S; d.args.ldi = ldx;
+      d.args.loss_acc = p->loss_acc; d.args.ldo = S; d.args.ldi = ldx; d.side_cols = p->s_true;
       d.args.colsum = grads ? grads + ly.b4 : nullptr;   // db4 = column sums of da4
       break;
     case G_F4_LIN:
@@ -773,7 +808,7 @@ int prepare(rvae_plan* p, GemmSet& gs, int id) {
       break;
     case G_B1W:
       d.epi = EPI_REDUCE; d.M = H; d.N = S; d.K = B;
-      d.A = opnd(p->da1, MAJOR_MN, H); d.B = opnd(p->x, MAJOR_MN, ldx);
+      d.A = opnd(p->da1, MAJOR_MN, H); d.B = opnd(p->x, MAJOR_MN, ldx); d.B.cols = p->s_true;
       d.args.out_f32 = grads + ly.w1; d.args.ldo = S; d.args.accumulate = 1;
       break;
     default:
@@ -849,6 +884,49 @@ int run(rvae_plan* p, int id, cudaStream_t st, const EpiArgs* override_args = nu
   const GemmParams& gp = gs->g[id].params;
   p->t_flops[tid] = 2.0 * gp.M * gp.N * gp.K;
   return RVAE_OK;
+}
+
+// Caller tensors of a padded plan cross the API at their true width `cols`; the plan's buffers have row pitch `ld`.
+// dst [rows, ld] <- src [rows, cols] with zeros in columns cols..ld
+int pad_rows(float* dst, const float* src, int rows, int cols, int ld, cudaStream_t st) {
+  RVAE_CUDA(cudaMemcpy2DAsync(dst, sizeof(float) * ld, src, sizeof(float) * cols, sizeof(float) * cols, rows,
+                              cudaMemcpyDeviceToDevice, st));
+  RVAE_CUDA(cudaMemset2DAsync(dst + cols, sizeof(float) * ld, 0, sizeof(float) * (ld - cols), rows, st));
+  return RVAE_OK;
+}
+// dst [rows, cols] <- the first cols columns of src [rows, ld]
+int strip_rows(float* dst, const float* src, int rows, int cols, int ld, cudaStream_t st) {
+  RVAE_CUDA(cudaMemcpy2DAsync(dst, sizeof(float) * cols, src, sizeof(float) * ld, sizeof(float) * cols, rows,
+                              cudaMemcpyDeviceToDevice, st));
+  return RVAE_OK;
+}
+// redirected mu / logvar of a plan with a padded latent_dim: copied out of the workspace
+int copy_latents_out(rvae_plan* p, cudaStream_t st) {
+  if (p->out_mu) RVAE_CHECK(strip_rows(p->out_mu, p->mu, p->batch, p->l_true, p->L, st));
+  if (p->out_lv) RVAE_CHECK(strip_rows(p->out_lv, p->lv, p->batch, p->l_true, p->L, st));
+  return RVAE_OK;
+}
+
+// Philox noise for `rows` rows of the batch starting at global row `row0`: element (r, c) is element
+// (row0 + r) * L + c of the unpadded [global batch, L] draw, whatever the padding of the plan's eps buffer
+int draw_eps(rvae_plan* p, float* out, int rows, uint64_t seed, uint64_t offset, const float* offset_src, int64_t row0,
+             cudaStream_t st) {
+  if (p->l_true == p->L)
+    return launch_randn(&p->ctx->c, out, (int64_t)rows * p->L, seed, offset, offset_src, row0 * p->L, st);
+  return launch_randn_rows(&p->ctx->c, out, rows, p->l_true, p->L, seed, offset, offset_src, row0 * p->l_true, st);
+}
+
+// decoder of rvae_plan_decode / rvae_plan_decode_lerp once z is in fc3's operand: fc3, fc4 + tanh -> xhat_out
+int decode_tail(rvae_plan* p, float* xhat_out, cudaStream_t st) {
+  RVAE_CHECK(run(p, G_F3, st));
+  GemmSet* gs;
+  RVAE_CHECK(get_set(p, &gs));
+  RVAE_CHECK(prepare(p, *gs, G_F4_LIN));
+  EpiArgs a = gs->g[G_F4_LIN].params.epi;
+  const bool rec_direct = p->S == p->s_true;
+  a.out_f32 = rec_direct ? xhat_out : p->xhat;
+  RVAE_CHECK(run(p, G_F4_LIN, st, &a));
+  return rec_direct ? RVAE_OK : strip_rows(xhat_out, p->xhat, p->batch, p->s_true, p->S, st);
 }
 
 int check_ready(const rvae_plan* p, bool need_batch) {
@@ -1170,10 +1248,12 @@ int rvae_plan_create(rvae_ctx* ctx, int S, int H, int L, int max_batch, int prec
   RVAE_REQUIRE(precision == RVAE_PRECISION_BF16 || precision == RVAE_PRECISION_FP32, RVAE_ERR_INVALID,
                "plan_create: precision %d", precision);
   rvae_layout lay;
-  RVAE_CHECK(rvae_param_layout(S, H, L, &lay));
+  int Sp, Hp, Lp;
+  RVAE_CHECK(rvae_param_layout_padded(S, H, L, &lay, &Sp, &Hp, &Lp));
   rvae_plan* p = new (std::nothrow) rvae_plan();
   RVAE_REQUIRE(p, RVAE_ERR_INVALID, "plan_create: out of host memory");
-  p->ctx = ctx; p->S = S; p->H = H; p->L = L; p->max_batch = max_batch; p->precision = precision;
+  p->ctx = ctx; p->S = Sp; p->H = Hp; p->L = Lp; p->max_batch = max_batch; p->precision = precision;
+  p->s_true = S; p->h_true = H; p->l_true = L;
   p->lay = lay; p->bound = false; p->batch = 0; p->have_eps = false; p->global_batch = 0; p->noise_row0 = 0;
   p->timing = false;
   p->kl_c0 = 0.f; p->dz_zeroed = false; p->dp_enabled = false;
@@ -1331,7 +1411,8 @@ int rvae_plan_load_frames(rvae_plan* plan, const void* audio, int audio_is_i16, 
   const size_t off = (size_t)row_offset * plan->S;
   TimedScope ts(plan, T_LOAD, S_(stream));
   return launch_frame_gather(&plan->ctx->c, audio, audio_is_i16, n_samples, frame_idx, first_frame, count, hop,
-                             plan->S, plan->x.hi + off, plan->x.lo ? plan->x.lo + off : nullptr, nullptr, S_(stream));
+                             plan->s_true, plan->S, plan->x.hi + off, plan->x.lo ? plan->x.lo + off : nullptr, nullptr,
+                             S_(stream));
 }
 
 int rvae_plan_load_batch(rvae_plan* plan, const float* x, int batch, void* stream) {
@@ -1343,6 +1424,9 @@ int rvae_plan_load_batch(rvae_plan* plan, const float* x, int batch, void* strea
   plan->x_pitch = 0;
   plan->have_eps = false;
   TimedScope ts(plan, T_LOAD, S_(stream));
+  if (plan->s_true != plan->S)
+    return launch_split_bf16_rows(&plan->ctx->c, x, batch, plan->s_true, plan->s_true, plan->S, plan->x.hi, plan->x.lo,
+                                  S_(stream));
   return launch_split_bf16(&plan->ctx->c, x, (int64_t)batch * plan->S, plan->x.hi, plan->x.lo, S_(stream));
 }
 
@@ -1351,16 +1435,20 @@ int rvae_plan_load_batch(rvae_plan* plan, const float* x, int batch, void* strea
 // and let the GEMMs read frame i at row pitch hop. Every sample is touched once instead of S / hop times and the
 // [count, S] operand is never materialised (rawvae/dataset.py:61-69: sequential frames of a stream).
 static int span_eligible(const rvae_plan* p, int count, int hop) {
-  // 16-byte row pitch for the tensor maps; the span must fit the planes (hop <= S)
-  return hop > 0 && hop % 8 == 0 && hop <= p->S && p->S % 8 == 0 && count > 0 && count <= p->max_batch;
+  // 16-byte row pitch for the tensor maps; the span must fit the planes (hop <= S). A padded segment_length reads
+  // zeros past S through the tensor maps; the fp32 mode's residual plane of x is read by the fc4 epilogue straight
+  // from memory, where a frame's columns past S are the next frame's samples, so that mode gathers padded rows.
+  const int S = p->s_true;
+  return hop > 0 && hop % 8 == 0 && hop <= S && S % 8 == 0 && count > 0 && count <= p->max_batch &&
+         (S == p->S || p->precision == RVAE_PRECISION_BF16);
 }
 static int convert_span(rvae_plan* p, const void* audio, int audio_is_i16, int64_t n_samples,
                         const int64_t* first_frame_dev, int64_t first_frame, int count, int hop, Planes& dst,
                         cudaStream_t st) {
-  const int64_t span = (int64_t)(count - 1) * hop + p->S;
+  const int64_t span = (int64_t)(count - 1) * hop + p->s_true;
   RVAE_REQUIRE(span <= (int64_t)INT32_MAX, RVAE_ERR_UNSUPPORTED, "plan span: %lld samples", (long long)span);
   return launch_frame_gather(&p->ctx->c, audio, audio_is_i16, n_samples, first_frame_dev, first_frame, 1, hop,
-                             (int)span, dst.hi, dst.lo, nullptr, st);
+                             (int)span, (int)span, dst.hi, dst.lo, nullptr, st);
 }
 
 int rvae_plan_span_supported(const rvae_plan* plan, int count, int hop) {
@@ -1371,8 +1459,8 @@ int rvae_plan_load_span(rvae_plan* plan, const void* audio, int audio_is_i16, in
                         const int64_t* first_frame_dev, int64_t first_frame, int count, int hop, void* stream) {
   RVAE_CHECK(check_ready(plan, false));
   RVAE_REQUIRE(audio && span_eligible(plan, count, hop), RVAE_ERR_UNSUPPORTED,
-               "plan_load_span: count %d (max %d), hop %d (needs hop %% 8 == 0 and hop <= S = %d)", count,
-               plan->max_batch, hop, plan->S);
+               "plan_load_span: count %d (max %d), hop %d (needs hop %% 8 == 0 and hop <= S = %d; S %% 8 == 0; bf16 "
+               "mode if S %% 64 != 0)", count, plan->max_batch, hop, plan->s_true);
   // (samples past n_samples read as zeros, exactly as in the gather: the zero-padded tail of a file)
   RVAE_REQUIRE(first_frame_dev || first_frame >= 0, RVAE_ERR_INVALID, "plan_load_span: first_frame %lld",
                (long long)first_frame);
@@ -1387,8 +1475,11 @@ int rvae_plan_load_span(rvae_plan* plan, const void* audio, int audio_is_i16, in
 int rvae_plan_set_eps(rvae_plan* plan, const float* eps, void* stream) {
   RVAE_CHECK(check_ready(plan, true));
   RVAE_REQUIRE(eps, RVAE_ERR_INVALID, "plan_set_eps: null eps");
-  RVAE_CUDA(cudaMemcpyAsync(plan->eps, eps, sizeof(float) * (size_t)plan->batch * plan->L, cudaMemcpyDeviceToDevice,
-                            S_(stream)));
+  if (plan->l_true != plan->L)
+    RVAE_CHECK(pad_rows(plan->eps, eps, plan->batch, plan->l_true, plan->L, S_(stream)));
+  else
+    RVAE_CUDA(cudaMemcpyAsync(plan->eps, eps, sizeof(float) * (size_t)plan->batch * plan->L, cudaMemcpyDeviceToDevice,
+                              S_(stream)));
   plan->have_eps = true;
   return RVAE_OK;
 }
@@ -1404,15 +1495,15 @@ int rvae_plan_gen_eps(rvae_plan* plan, uint64_t seed, uint64_t offset, int add_s
     RVAE_CHECK(ensure_side_stream(plan));
     RVAE_CUDA(cudaEventRecord(plan->ev_fork, st));
     RVAE_CUDA(cudaStreamWaitEvent(plan->adam_stream, plan->ev_fork, 0));
-    RVAE_CHECK(launch_randn(&plan->ctx->c, plan->eps, (int64_t)plan->batch * plan->L, seed, offset,
-                            add_step ? plan->bufs.step : nullptr, plan->noise_row0 * plan->L, plan->adam_stream));
+    RVAE_CHECK(draw_eps(plan, plan->eps, plan->batch, seed, offset, add_step ? plan->bufs.step : nullptr,
+                        plan->noise_row0, plan->adam_stream));
     RVAE_CUDA(cudaEventRecord(plan->ev_eps, plan->adam_stream));
     plan->eps_pending = true;
     return RVAE_OK;
   }
   TimedScope ts(plan, T_EPS, st);
-  return launch_randn(&plan->ctx->c, plan->eps, (int64_t)plan->batch * plan->L, seed, offset,
-                      add_step ? plan->bufs.step : nullptr, plan->noise_row0 * plan->L, st);
+  return draw_eps(plan, plan->eps, plan->batch, seed, offset, add_step ? plan->bufs.step : nullptr, plan->noise_row0,
+                  st);
 }
 
 int rvae_plan_set_outputs(rvae_plan* plan, float* mu, float* logvar, float* xhat) {
@@ -1453,7 +1544,9 @@ int rvae_plan_forward(rvae_plan* plan, float kl_beta, int fused_loss, int want_x
   cudaStream_t st = S_(stream);
   rvae_plan* p = plan;
   const double nb = p->global_batch > 0 ? (double)p->global_batch : (double)p->batch;
-  const double BL = nb * p->L, BS = nb * p->S;
+  const double BL = nb * p->l_true, BS = nb * p->s_true;
+  // caller tensors of a padded plan: the epilogues write the workspace, the true columns are copied out afterwards
+  const bool lat_direct = p->L == p->l_true, rec_direct = p->S == p->s_true;
   GemmSet* gs;
   RVAE_CHECK(get_set(p, &gs));
 
@@ -1504,11 +1597,12 @@ int rvae_plan_forward(rvae_plan* plan, float kl_beta, int fused_loss, int want_x
   {
     RVAE_CHECK(prepare(p, *gs, G_F2));
     EpiArgs a = gs->g[G_F2].params.epi;
-    if (p->out_mu) a.out_f32 = p->out_mu;
-    if (p->out_lv) a.out_f32_b = p->out_lv;
+    if (p->out_mu && lat_direct) a.out_f32 = p->out_mu;
+    if (p->out_lv && lat_direct) a.out_f32_b = p->out_lv;
     if (fused_loss) p->kl_c0 = (float)((double)kl_beta / BL);
     else a.loss_acc = nullptr;
     RVAE_CHECK(run(p, G_F2, st, &a));
+    if (!lat_direct) RVAE_CHECK(copy_latents_out(p, st));
   }
   RVAE_CHECK(run(p, G_F3, st));
   if (fused_loss) {
@@ -1520,13 +1614,15 @@ int rvae_plan_forward(rvae_plan* plan, float kl_beta, int fused_loss, int want_x
     RVAE_CHECK(prepare(p, *gs, G_F4_OUT));
     EpiArgs a = gs->g[G_F4_OUT].params.epi;
     a.c0 = (float)(2.0 / BS);
-    a.out_f32 = want_xhat ? (p->out_xhat ? p->out_xhat : p->xhat) : nullptr;
+    a.out_f32 = want_xhat ? (p->out_xhat && rec_direct ? p->out_xhat : p->xhat) : nullptr;
     RVAE_CHECK(run(p, G_F4_OUT, st, &a));
+    if (want_xhat && p->out_xhat && !rec_direct) RVAE_CHECK(strip_rows(p->out_xhat, p->xhat, p->batch, p->s_true, p->S, st));
   } else {
     RVAE_CHECK(prepare(p, *gs, G_F4_LIN));
     EpiArgs a = gs->g[G_F4_LIN].params.epi;
-    a.out_f32 = p->out_xhat ? p->out_xhat : p->xhat;
+    a.out_f32 = p->out_xhat && rec_direct ? p->out_xhat : p->xhat;
     RVAE_CHECK(run(p, G_F4_LIN, st, &a));
+    if (p->out_xhat && !rec_direct) RVAE_CHECK(strip_rows(p->out_xhat, p->xhat, p->batch, p->s_true, p->S, st));
   }
   return RVAE_OK;
 }
@@ -1552,6 +1648,20 @@ int rvae_plan_backward_external(rvae_plan* plan, const float* g_xhat, const floa
                "plan_backward_external: null argument");
   rvae_plan* p = plan;
   cudaStream_t st = S_(stream);
+  if (p->S != p->s_true) {   // padded plan: the caller's [batch, S] tensors at the padded row pitch, zero padding
+    RVAE_CHECK(pad_rows(p->ext_gx, g_xhat, p->batch, p->s_true, p->S, st));
+    RVAE_CHECK(pad_rows(p->xhat, xhat, p->batch, p->s_true, p->S, st));
+    g_xhat = p->ext_gx;
+    xhat = p->xhat;
+  }
+  if (p->L != p->l_true) {
+    RVAE_CHECK(pad_rows(p->ext_gmu, g_mu, p->batch, p->l_true, p->L, st));
+    RVAE_CHECK(pad_rows(p->ext_glv, g_logvar, p->batch, p->l_true, p->L, st));
+    RVAE_CHECK(pad_rows(p->ext_lv, logvar, p->batch, p->l_true, p->L, st));
+    g_mu = p->ext_gmu;
+    g_logvar = p->ext_glv;
+    logvar = p->ext_lv;
+  }
   RVAE_CHECK(ensure_bias_zeroed(p, st));
   p->grads_zeroed[4] = false;
   { TimedScope ts(p, T_TANHBWD, st); RVAE_CHECK(launch_tanh_bwd(&p->ctx->c, g_xhat, xhat, (int64_t)p->batch * p->S, p->da4.hi, p->da4.lo, st)); }
@@ -1571,14 +1681,14 @@ int rvae_plan_finish_loss(rvae_plan* plan, float kl_beta, float* loss_out, int r
   // The reported loss is the mean over THIS rank's frames (under data parallelism: an unbiased estimate of the
   // global mean that needs no collective); the gradients use the global-batch normalisation set on the plan.
   TimedScope ts(plan, T_FINALIZE, S_(stream));
-  return launch_loss_finalize(&plan->ctx->c, plan->loss_acc, plan->batch, plan->S, plan->L, kl_beta, loss_out, ring_size,
-                              plan->bufs.step, S_(stream));
+  return launch_loss_finalize(&plan->ctx->c, plan->loss_acc, plan->batch, plan->s_true, plan->l_true, kl_beta, loss_out,
+                              ring_size, plan->bufs.step, S_(stream));
 }
 
 int rvae_plan_finish_loss_deferred(rvae_plan* plan, float kl_beta, float* loss_out, int ring_size) {
   RVAE_CHECK(check_ready(plan, true));
   RVAE_REQUIRE(ring_size >= 1, RVAE_ERR_INVALID, "plan_finish_loss_deferred: ring_size %d", ring_size);
-  plan->fin = make_loss_finalize(plan->loss_acc, plan->batch, plan->S, plan->L, kl_beta, loss_out, ring_size,
+  plan->fin = make_loss_finalize(plan->loss_acc, plan->batch, plan->s_true, plan->l_true, kl_beta, loss_out, ring_size,
                                  plan->bufs.step);
   plan->fin_pending = true;
   return RVAE_OK;
@@ -1604,8 +1714,8 @@ int rvae_plan_prefetch_span(rvae_plan* plan, const void* audio, int audio_is_i16
                             uint64_t offset, int add_step) {
   RVAE_CHECK(check_ready(plan, false));
   RVAE_REQUIRE(audio && span_eligible(plan, count, hop), RVAE_ERR_UNSUPPORTED,
-               "plan_prefetch_span: count %d (max %d), hop %d (needs hop %% 8 == 0 and hop <= S = %d)", count,
-               plan->max_batch, hop, plan->S);
+               "plan_prefetch_span: count %d (max %d), hop %d (needs hop %% 8 == 0 and hop <= S = %d; S %% 8 == 0; "
+               "bf16 mode if S %% 64 != 0)", count, plan->max_batch, hop, plan->s_true);
   RVAE_REQUIRE(first_frame_dev || first_frame >= 0, RVAE_ERR_INVALID, "plan_prefetch_span: first_frame %lld",
                (long long)first_frame);
   RVAE_CHECK(rvae_plan_prefetch_frames(plan, audio, audio_is_i16, n_samples, first_frame_dev, first_frame, count, hop,
@@ -1706,12 +1816,12 @@ int rvae_plan_train_step(rvae_plan* plan, float kl_beta, double lr, double beta1
       p->x_pitch_alt = f.hop;
     } else {
       RVAE_CHECK(launch_frame_gather(&p->ctx->c, f.audio, f.audio_is_i16, f.n_samples, f.frame_idx, f.first_frame,
-                                     f.count, f.hop, p->S, p->x_alt.hi, p->x_alt.lo, nullptr, bg));
+                                     f.count, f.hop, p->s_true, p->S, p->x_alt.hi, p->x_alt.lo, nullptr, bg));
       p->x_pitch_alt = 0;
     }
     // the consumer sees a step counter advanced by one
-    RVAE_CHECK(launch_randn(&p->ctx->c, p->eps_alt, (int64_t)f.count * p->L, f.seed, f.offset + (f.add_step ? 1 : 0),
-                            f.add_step ? b.step : nullptr, f.noise_row0 * p->L, bg));
+    RVAE_CHECK(draw_eps(p, p->eps_alt, f.count, f.seed, f.offset + (f.add_step ? 1 : 0), f.add_step ? b.step : nullptr,
+                        f.noise_row0, bg));
     p->pf.ready_batch = f.count;
     p->pf.registered = false;
     return RVAE_OK;
@@ -1872,14 +1982,11 @@ int rvae_plan_decode(rvae_plan* plan, const float* z, int batch, float* xhat_out
   cudaStream_t st = S_(stream);
   p->batch = batch;
   p->have_eps = false;
-  RVAE_CHECK(launch_split_bf16(&p->ctx->c, z, (int64_t)batch * p->L, p->z.hi, p->z.lo, st));
-  RVAE_CHECK(run(p, G_F3, st));
-  GemmSet* gs;
-  RVAE_CHECK(get_set(p, &gs));
-  RVAE_CHECK(prepare(p, *gs, G_F4_LIN));
-  EpiArgs a = gs->g[G_F4_LIN].params.epi;
-  a.out_f32 = xhat_out;
-  return run(p, G_F4_LIN, st, &a);
+  if (p->l_true != p->L)
+    RVAE_CHECK(launch_split_bf16_rows(&p->ctx->c, z, batch, p->l_true, p->l_true, p->L, p->z.hi, p->z.lo, st));
+  else
+    RVAE_CHECK(launch_split_bf16(&p->ctx->c, z, (int64_t)batch * p->L, p->z.hi, p->z.lo, st));
+  return decode_tail(p, xhat_out, st);
 }
 
 int rvae_plan_decode_lerp(rvae_plan* plan, const float* mu_a, const float* logvar_a, const float* mu_b,
@@ -1894,15 +2001,9 @@ int rvae_plan_decode_lerp(rvae_plan* plan, const float* mu_a, const float* logva
   p->batch = batch;
   p->have_eps = false;
   // interpolated latents -> z written straight into fc3's bf16 operand planes (no fp32 z, no split pass)
-  RVAE_CHECK(launch_lerp_reparam(&p->ctx->c, mu_a, logvar_a, mu_b, logvar_b, alpha, alpha_is_f64, eps, batch, p->L, nullptr,
-                                 p->z.hi, p->z.lo, nullptr, nullptr, st));
-  RVAE_CHECK(run(p, G_F3, st));
-  GemmSet* gs;
-  RVAE_CHECK(get_set(p, &gs));
-  RVAE_CHECK(prepare(p, *gs, G_F4_LIN));
-  EpiArgs a = gs->g[G_F4_LIN].params.epi;
-  a.out_f32 = xhat_out;
-  return run(p, G_F4_LIN, st, &a);
+  RVAE_CHECK(launch_lerp_reparam(&p->ctx->c, mu_a, logvar_a, mu_b, logvar_b, alpha, alpha_is_f64, eps, batch, p->l_true,
+                                 p->L, nullptr, p->z.hi, p->z.lo, nullptr, nullptr, st));
+  return decode_tail(p, xhat_out, st);
 }
 
 int rvae_plan_encode(rvae_plan* plan, void* stream) {
@@ -1914,11 +2015,13 @@ int rvae_plan_encode(rvae_plan* plan, void* stream) {
   RVAE_CHECK(get_set(p, &gs));
   RVAE_CHECK(prepare(p, *gs, G_F2));
   EpiArgs a = gs->g[G_F2].params.epi;
-  if (p->out_mu) a.out_f32 = p->out_mu;
-  if (p->out_lv) a.out_f32_b = p->out_lv;
+  const bool lat_direct = p->L == p->l_true;
+  if (p->out_mu && lat_direct) a.out_f32 = p->out_mu;
+  if (p->out_lv && lat_direct) a.out_f32_b = p->out_lv;
   a.in0 = nullptr; a.out_hi = nullptr; a.out_lo = nullptr;
   a.loss_acc = nullptr;
-  return run(p, G_F2, st, &a);
+  RVAE_CHECK(run(p, G_F2, st, &a));
+  return lat_direct ? RVAE_OK : copy_latents_out(p, st);
 }
 
 }  // extern "C"

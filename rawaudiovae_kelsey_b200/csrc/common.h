@@ -100,7 +100,9 @@ struct Operand {
   const __nv_bfloat16* hi;
   const __nv_bfloat16* lo;  // optional residual plane (fp32 emulation)
   int major;
-  int ld;  // elements
+  int ld;    // elements
+  int cols;  // > 0: only the first `cols` elements of each row are data, the rest read as zeros through the tensor
+             // map (frames read in place whose segment_length is padded up to the GEMM's extent); 0 = the full extent
 };
 
 struct GemmDesc {
@@ -110,6 +112,7 @@ struct GemmDesc {
   EpiArgs args;
   int head_L;    // EPI_HEAD: latent width L (B holds 2L stacked rows, N must equal 2L)
   int k_splits;  // EPI_WGRAD: requested split-K (0 = choose)
+  int side_cols; // EPI_OUT: > 0 = columns of the side input x that are data (as Operand::cols); 0 = N
 };
 
 struct PreparedGemm {
@@ -122,6 +125,7 @@ struct PreparedGemm {
   int epi;
   int a_major, b_major, cg;
   int out_rows, out_cols_bf16, out_ld_bf16, out_cols_f32, out_ld_f32;
+  int side_cols;  // GemmDesc::side_cols
 };
 
 int gemm_bind_outputs(PreparedGemm* g, const EpiArgs& args, bool force);
@@ -151,12 +155,16 @@ int gemm_launch(Ctx* ctx, const GemmDesc& d, cudaStream_t stream);  // prepare +
 
 // Elementwise launchers (elementwise.cu)
 int launch_frame_gather(Ctx* ctx, const void* audio, int audio_is_i16, int64_t n_samples, const int64_t* frame_idx,
-                        int64_t first_frame, int64_t n_frames, int hop, int S, __nv_bfloat16* out_hi,
+                        int64_t first_frame, int64_t n_frames, int hop, int S, int W, __nv_bfloat16* out_hi,
                         __nv_bfloat16* out_lo, float* out_f32, cudaStream_t stream);
 int launch_overlap_add(Ctx* ctx, const float* frames, int64_t n_frames, int S, int hop, float* out, int64_t t_begin,
                        int64_t n_out, cudaStream_t stream);
 int launch_randn(Ctx* ctx, float* out, int64_t n, uint64_t seed, uint64_t offset, const float* offset_src,
                  int64_t elem_base, cudaStream_t stream);
+int launch_randn_rows(Ctx* ctx, float* out, int64_t rows, int64_t cols, int64_t ld, uint64_t seed, uint64_t offset,
+                      const float* offset_src, int64_t elem_base, cudaStream_t stream);
+int launch_split_bf16_rows(Ctx* ctx, const float* src, int64_t rows, int cols, int ld_src, int ld_dst,
+                           __nv_bfloat16* hi, __nv_bfloat16* lo, cudaStream_t stream);
 int launch_split_bf16(Ctx* ctx, const float* src, int64_t n, __nv_bfloat16* hi, __nv_bfloat16* lo,
                       cudaStream_t stream);
 int launch_colsum(Ctx* ctx, const __nv_bfloat16* hi, const __nv_bfloat16* lo, int64_t M, int N, int ld, float* out,
@@ -171,8 +179,9 @@ int launch_tanh_bwd(Ctx* ctx, const float* g_xhat, const float* xhat, int64_t n,
 int launch_reparam(Ctx* ctx, const float* mu, const float* lv, const float* eps, int64_t n, float* z,
                    cudaStream_t stream);
 int launch_lerp_reparam(Ctx* ctx, const float* mu_a, const float* lv_a, const float* mu_b, const float* lv_b,
-                        const void* alpha, int alpha_is_f64, const float* eps, int64_t rows, int L, float* z_f32,
-                        __nv_bfloat16* z_hi, __nv_bfloat16* z_lo, float* mu_out, float* lv_out, cudaStream_t stream);
+                        const void* alpha, int alpha_is_f64, const float* eps, int64_t rows, int L, int ld_z,
+                        float* z_f32, __nv_bfloat16* z_hi, __nv_bfloat16* z_lo, float* mu_out, float* lv_out,
+                        cudaStream_t stream);
 int launch_loss_finalize(Ctx* ctx, double* acc, int64_t B, int S, int L, float beta, float* loss_out, int ring_size,
                          float* step, cudaStream_t stream);
 int launch_adam(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, double lr, double beta1, double beta2,
@@ -187,6 +196,10 @@ int launch_step_inc(Ctx* ctx, float* step, cudaStream_t stream);
 size_t param_histogram_bytes(int n_segs, int n_edges);
 int launch_param_histogram(Ctx* ctx, const float* params, const int64_t* seg_offsets, const int64_t* seg_lengths,
                            int n_segs, const double* edges, int n_edges, void* record, cudaStream_t stream);
+// the same over segments of seg_rows[s] rows of seg_cols[s] values at row pitch seg_pitch[s] (host arrays)
+int launch_param_histogram_rows(Ctx* ctx, const float* params, const int64_t* seg_offsets, const int64_t* seg_rows,
+                                const int64_t* seg_cols, const int64_t* seg_pitch, int n_segs, const double* edges,
+                                int n_edges, void* record, cudaStream_t stream);
 
 // Peer-memory all-reduce (elementwise.cu): symmetric buffers of all ranks as mapped in THIS process.
 constexpr int kP2PMaxWorld = 8;

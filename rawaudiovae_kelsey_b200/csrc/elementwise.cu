@@ -56,17 +56,19 @@ __device__ __forceinline__ float block_sum_to_warp0(float v, float* smem) {
 // ------------------------------------------------------------------------------------------------
 // K-D1 framing: frame f = audio_pad[idx*hop : idx*hop + S], zero beyond n_samples (the reference zero-pads the
 // tail, rawvae/dataset.py:102-104,141-143). idx = frame_idx[f] (shuffled map-style batches) or first_frame + f
-// (streaming / sequential). One thread converts 8 consecutive samples.
+// (streaming / sequential). One thread converts 8 consecutive samples. Output rows are W >= S elements wide: columns
+// S..W are written as zeros (the zero padding of a plan whose segment_length is not a multiple of 64).
 // ------------------------------------------------------------------------------------------------
 template <bool I16, int U>
 __global__ void frame_gather_kernel(const void* __restrict__ audio, int64_t n_samples,
                                     const int64_t* __restrict__ frame_idx, int64_t first_frame, int64_t n_frames,
-                                    int hop, int S, __nv_bfloat16* __restrict__ out_hi,
+                                    int hop, int S, int W, __nv_bfloat16* __restrict__ out_hi,
                                     __nv_bfloat16* __restrict__ out_lo, float* __restrict__ out_f32, AuxTrace tr) {
   ptx::pdl_launch_dependents();
   ptx::pdl_wait();
   aux_begin(tr, 1);
-  const int vec_per_frame = S >> 3;
+  const int vec_per_frame = (W + 7) >> 3;
+  const bool vec_store = (W & 7) == 0;   // 16-byte rows: vector stores (else the row width is the caller's odd S)
   const int64_t total = n_frames * vec_per_frame;
   // U groups of 8 samples per thread and trip: the U frame indices are fetched first, then all 2 U 16-byte loads are
   // issued before the first convert / store (U = 1 by default: occupancy beats per-thread unrolling here)
@@ -87,7 +89,7 @@ __global__ void frame_gather_kernel(const void* __restrict__ audio, int64_t n_sa
       s0[u] = fi * hop + col[u];
       // 16-byte aligned source address (the buffer base may itself be an unaligned view of a longer stream)
       const uintptr_t addr = reinterpret_cast<uintptr_t>(audio) + static_cast<uintptr_t>(s0[u]) * (I16 ? 2 : 4);
-      fast[u] = fr[u] >= 0 && s0[u] >= 0 && s0[u] + 8 <= n_samples && (addr & 15) == 0;
+      fast[u] = fr[u] >= 0 && col[u] + 8 <= S && s0[u] >= 0 && s0[u] + 8 <= n_samples && (addr & 15) == 0;
     }
     float v[U][8];
     uint4 raw[U][2];
@@ -115,19 +117,28 @@ __global__ void frame_gather_kernel(const void* __restrict__ audio, int64_t n_sa
 #pragma unroll
           for (int j = 0; j < 8; ++j) v[u][j] = f[j];
         }
-      } else {   // unaligned start, or the zero-padded tail beyond n_samples
+      } else {   // unaligned start, the zero-padded tail beyond n_samples, or columns at and past S
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
           const int64_t sidx = s0[u] + j;
           float x = 0.f;
-          if (sidx >= 0 && sidx < n_samples) {
+          if (col[u] + j < S && sidx >= 0 && sidx < n_samples) {
             if constexpr (I16) x = __ldg(reinterpret_cast<const int16_t*>(audio) + sidx) * (1.0f / 32768.0f);
             else x = __ldg(reinterpret_cast<const float*>(audio) + sidx);
           }
           v[u][j] = x;
         }
       }
-      const int64_t o = fr[u] * S + col[u];
+      const int64_t o = fr[u] * W + col[u];
+      if (!vec_store) {
+        for (int j = 0; j < 8 && col[u] + j < W; ++j) {
+          const __nv_bfloat16 h = __float2bfloat16_rn(v[u][j]);
+          if (out_hi) out_hi[o + j] = h;
+          if (out_lo) out_lo[o + j] = __float2bfloat16_rn(v[u][j] - __bfloat162float(h));
+          if (out_f32) out_f32[o + j] = v[u][j];
+        }
+        continue;
+      }
       if (out_hi) {
         *reinterpret_cast<uint4*>(out_hi + o) = make_uint4(pack2(v[u][0], v[u][1]), pack2(v[u][2], v[u][3]),
                                                            pack2(v[u][4], v[u][5]), pack2(v[u][6], v[u][7]));
@@ -150,10 +161,10 @@ __global__ void frame_gather_kernel(const void* __restrict__ audio, int64_t n_sa
 }
 
 int launch_frame_gather(Ctx* ctx, const void* audio, int audio_is_i16, int64_t n_samples, const int64_t* frame_idx,
-                        int64_t first_frame, int64_t n_frames, int hop, int S, __nv_bfloat16* out_hi,
+                        int64_t first_frame, int64_t n_frames, int hop, int S, int W, __nv_bfloat16* out_hi,
                         __nv_bfloat16* out_lo, float* out_f32, cudaStream_t stream) {
   RVAE_REQUIRE(audio && (out_hi || out_f32), RVAE_ERR_INVALID, "frame_gather: null buffer");
-  RVAE_REQUIRE(S > 0 && S % 8 == 0 && hop > 0, RVAE_ERR_UNSUPPORTED, "frame_gather: S=%d must be a multiple of 8", S);
+  RVAE_REQUIRE(S > 0 && hop > 0 && W >= S, RVAE_ERR_UNSUPPORTED, "frame_gather: S=%d, row width %d, hop %d", S, W, hop);
   if (n_frames <= 0) return RVAE_OK;
   const int threads = 256;
   // RVAE_GATHER_UNROLL (1 / 2 / 4 groups of 8 samples per thread and trip), RVAE_GATHER_WAVES: tuning knobs
@@ -162,11 +173,11 @@ int launch_frame_gather(Ctx* ctx, const void* audio, int audio_is_i16, int64_t n
   static const int unroll = getenv("RVAE_GATHER_UNROLL") ? atoi(getenv("RVAE_GATHER_UNROLL")) : 1;
   static const int waves = getenv("RVAE_GATHER_WAVES") ? atoi(getenv("RVAE_GATHER_WAVES")) : 16;
   const int u = unroll == 1 ? 1 : (unroll == 2 ? 2 : 4);
-  const int grid = grid_for(ctx, (n_frames * (S / 8) + u - 1) / u, threads, waves > 0 ? waves : 8);
+  const int grid = grid_for(ctx, (n_frames * ((W + 7) / 8) + u - 1) / u, threads, waves > 0 ? waves : 8);
   const AuxTrace tr = next_aux(ctx, 1);
   auto go = [&](auto kern) {
     return launch_kernel(ctx, kern, dim3(grid), dim3(threads), (size_t)0, stream, audio, n_samples, frame_idx,
-                         first_frame, n_frames, hop, S, out_hi, out_lo, out_f32, tr);
+                         first_frame, n_frames, hop, S, W, out_hi, out_lo, out_f32, tr);
   };
   if (audio_is_i16) {
     if (u == 1) RVAE_CUDA(go(frame_gather_kernel<true, 1>));
@@ -295,6 +306,23 @@ __device__ __forceinline__ void philox4x32_10(uint32_t (&c)[4], uint32_t k0, uin
   }
 }
 
+// the four normal values of Philox counter ci (elements 4 ci .. 4 ci + 3 of the logical noise tensor)
+__device__ __forceinline__ void randn4(int64_t ci, uint64_t seed, uint64_t offset, float (&z)[4]) {
+  uint32_t c[4] = {static_cast<uint32_t>(ci), static_cast<uint32_t>(ci >> 32), static_cast<uint32_t>(offset),
+                   static_cast<uint32_t>(offset >> 32)};
+  philox4x32_10(c, static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32));
+#pragma unroll
+  for (int h = 0; h < 2; ++h) {
+    const float u1 = (static_cast<float>(c[2 * h] >> 8) + 0.5f) * (1.0f / 16777216.0f);  // (0,1)
+    const float u2 = (static_cast<float>(c[2 * h + 1] >> 8) + 0.5f) * (1.0f / 16777216.0f);
+    const float r = sqrtf(-2.0f * __logf(u1));
+    float s, co;
+    __sincosf(6.283185307179586f * u2, &s, &co);
+    z[2 * h] = r * co;
+    z[2 * h + 1] = r * s;
+  }
+}
+
 __global__ void randn_kernel(float* __restrict__ out, int64_t n, uint64_t seed, uint64_t offset,
                              const float* __restrict__ offset_src, int64_t vec_base, AuxTrace tr) {
   ptx::pdl_launch_dependents();
@@ -306,21 +334,8 @@ __global__ void randn_kernel(float* __restrict__ out, int64_t n, uint64_t seed, 
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < nvec; i += (int64_t)gridDim.x * blockDim.x) {
     // vec_base: this buffer is elements [4 * vec_base, ...) of a larger logical tensor (a rank's rows of the global
     // batch under data parallelism): the ranks draw disjoint pieces of ONE stream, the single-process draw
-    const int64_t ci = i + vec_base;
-    uint32_t c[4] = {static_cast<uint32_t>(ci), static_cast<uint32_t>(ci >> 32), static_cast<uint32_t>(offset),
-                     static_cast<uint32_t>(offset >> 32)};
-    philox4x32_10(c, static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32));
     float z[4];
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {
-      const float u1 = (static_cast<float>(c[2 * h] >> 8) + 0.5f) * (1.0f / 16777216.0f);  // (0,1)
-      const float u2 = (static_cast<float>(c[2 * h + 1] >> 8) + 0.5f) * (1.0f / 16777216.0f);
-      const float r = sqrtf(-2.0f * __logf(u1));
-      float s, co;
-      __sincosf(6.283185307179586f * u2, &s, &co);
-      z[2 * h] = r * co;
-      z[2 * h + 1] = r * s;
-    }
+    randn4(i + vec_base, seed, offset, z);
     const int64_t o = i << 2;
     if (o + 4 <= n) {
       *reinterpret_cast<float4*>(out + o) = make_float4(z[0], z[1], z[2], z[3]);
@@ -329,6 +344,42 @@ __global__ void randn_kernel(float* __restrict__ out, int64_t n, uint64_t seed, 
     }
   }
   aux_end(tr);
+}
+
+// Row-pitched draw: out[r * ld + c] = element elem_base + r * cols + c of the logical noise tensor for c < cols, 0 for
+// cols <= c < ld (the zero padding of a plan whose latent_dim is not a multiple of 64). Any elem_base. One thread per
+// output element; each evaluates the Philox block of its element (the noise is a few hundred KB per step).
+__global__ void randn_rows_kernel(float* __restrict__ out, int64_t rows, int64_t cols, int64_t ld, uint64_t seed,
+                                  uint64_t offset, const float* __restrict__ offset_src, int64_t elem_base, AuxTrace tr) {
+  ptx::pdl_launch_dependents();
+  ptx::pdl_wait();
+  aux_begin(tr, 2);
+  if (offset_src) offset += static_cast<uint64_t>(__ldg(offset_src));
+  const int64_t n = rows * ld;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = i / ld;
+    const int64_t c = i - r * ld;
+    float v = 0.f;
+    if (c < cols) {
+      const int64_t e = elem_base + r * cols + c;
+      float z[4];
+      randn4(e >> 2, seed, offset, z);
+      v = z[e & 3];
+    }
+    out[i] = v;
+  }
+  aux_end(tr);
+}
+
+int launch_randn_rows(Ctx* ctx, float* out, int64_t rows, int64_t cols, int64_t ld, uint64_t seed, uint64_t offset,
+                      const float* offset_src, int64_t elem_base, cudaStream_t stream) {
+  RVAE_REQUIRE(out && cols > 0 && ld >= cols && elem_base >= 0, RVAE_ERR_INVALID, "randn_rows: bad arguments");
+  if (rows <= 0) return RVAE_OK;
+  const int threads = 256;
+  RVAE_CUDA(launch_kernel(ctx, randn_rows_kernel, dim3(grid_for(ctx, rows * ld, threads, 8)), dim3(threads), (size_t)0,
+                          stream, out, rows, cols, ld, seed, offset, offset_src, elem_base, next_aux(ctx, 2)));
+  RVAE_LAUNCH_CHECK(ctx);
+  return RVAE_OK;
 }
 
 int launch_randn(Ctx* ctx, float* out, int64_t n, uint64_t seed, uint64_t offset, const float* offset_src,
@@ -373,6 +424,34 @@ __global__ void split_bf16_kernel(const float* __restrict__ src, int64_t n, __nv
       if (lo) lo[j] = __float2bfloat16_rn(v - __bfloat162float(h));
     }
   }
+}
+
+// fp32 [rows, cols] at row pitch ld_src -> bf16 planes [rows, ld_dst], zeros in columns cols..ld_dst (caller tensors
+// of a plan whose dims are not multiples of 64, on their way into the padded operands)
+__global__ void split_bf16_rows_kernel(const float* __restrict__ src, int64_t rows, int cols, int ld_src, int ld_dst,
+                                       __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo) {
+  ptx::pdl_launch_dependents();
+  ptx::pdl_wait();
+  const int64_t n = rows * ld_dst;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = i / ld_dst;
+    const int c = static_cast<int>(i - r * ld_dst);
+    const float v = c < cols ? src[r * ld_src + c] : 0.f;
+    const __nv_bfloat16 h = __float2bfloat16_rn(v);
+    hi[i] = h;
+    if (lo) lo[i] = __float2bfloat16_rn(v - __bfloat162float(h));
+  }
+}
+
+int launch_split_bf16_rows(Ctx* ctx, const float* src, int64_t rows, int cols, int ld_src, int ld_dst,
+                           __nv_bfloat16* hi, __nv_bfloat16* lo, cudaStream_t stream) {
+  RVAE_REQUIRE(src && hi && cols > 0 && ld_src >= cols && ld_dst >= cols, RVAE_ERR_INVALID, "split_bf16_rows: bad arguments");
+  if (rows <= 0) return RVAE_OK;
+  const int threads = 256;
+  RVAE_CUDA(launch_kernel(ctx, split_bf16_rows_kernel, dim3(grid_for(ctx, rows * ld_dst, threads, 8)), dim3(threads),
+                          (size_t)0, stream, src, rows, cols, ld_src, ld_dst, hi, lo));
+  RVAE_LAUNCH_CHECK(ctx);
+  return RVAE_OK;
 }
 
 int launch_split_bf16(Ctx* ctx, const float* src, int64_t n, __nv_bfloat16* hi, __nv_bfloat16* lo,
@@ -698,14 +777,65 @@ __global__ void lerp_reparam_kernel(const float* __restrict__ mu_a, const float*
   }
 }
 
+// Any L: one thread per element of [rows, ld_z]. The fp32 outputs are [rows, L]; the bf16 z planes have row pitch
+// ld_z >= L and zeros in columns L..ld_z (fc3's operand of a plan whose latent_dim is not a multiple of 64). Same
+// arithmetic as the vector kernel, so the same bits.
+template <typename AT>
+__global__ void lerp_reparam_rows_kernel(const float* __restrict__ mu_a, const float* __restrict__ lv_a,
+                                         const float* __restrict__ mu_b, const float* __restrict__ lv_b,
+                                         const AT* __restrict__ alpha, const float* __restrict__ eps, int64_t rows,
+                                         int L, int ld_z, float* __restrict__ z_f32, __nv_bfloat16* __restrict__ z_hi,
+                                         __nv_bfloat16* __restrict__ z_lo, float* __restrict__ mu_out,
+                                         float* __restrict__ lv_out) {
+  ptx::pdl_launch_dependents();
+  ptx::pdl_wait();
+  const int64_t n = rows * ld_z;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = i / ld_z;
+    const int c = static_cast<int>(i - r * ld_z);
+    float z = 0.f;
+    if (c < L) {
+      const int64_t k = r * L + c;
+      const AT al = alpha[r];
+      const float e = eps ? eps[k] : 0.f;
+      const float m = static_cast<float>((AT(1) - al) * AT(mu_a[k]) + al * AT(mu_b[k]));
+      const float l = static_cast<float>((AT(1) - al) * AT(lv_a[k]) + al * AT(lv_b[k]));
+      z = fmaf(e, expf(0.5f * l), m);
+      if (mu_out) mu_out[k] = m;
+      if (lv_out) lv_out[k] = l;
+      if (z_f32) z_f32[k] = z;
+    }
+    if (z_hi) z_hi[i] = __float2bfloat16_rn(z);
+    if (z_lo) z_lo[i] = __float2bfloat16_rn(z - __bfloat162float(__float2bfloat16_rn(z)));
+  }
+}
+
 int launch_lerp_reparam(Ctx* ctx, const float* mu_a, const float* lv_a, const float* mu_b, const float* lv_b,
-                        const void* alpha, int alpha_is_f64, const float* eps, int64_t rows, int L, float* z_f32,
-                        __nv_bfloat16* z_hi, __nv_bfloat16* z_lo, float* mu_out, float* lv_out, cudaStream_t stream) {
+                        const void* alpha, int alpha_is_f64, const float* eps, int64_t rows, int L, int ld_z,
+                        float* z_f32, __nv_bfloat16* z_hi, __nv_bfloat16* z_lo, float* mu_out, float* lv_out,
+                        cudaStream_t stream) {
   RVAE_REQUIRE(mu_a && lv_a && mu_b && lv_b && alpha, RVAE_ERR_INVALID, "lerp_reparam: null buffer");
   RVAE_REQUIRE(z_f32 || z_hi || mu_out, RVAE_ERR_INVALID, "lerp_reparam: no output buffer");
-  RVAE_REQUIRE(L > 0 && L % 4 == 0, RVAE_ERR_UNSUPPORTED, "lerp_reparam: latent_dim=%d must be a multiple of 4", L);
+  RVAE_REQUIRE(L > 0 && ld_z >= L, RVAE_ERR_UNSUPPORTED, "lerp_reparam: latent_dim=%d, z row pitch %d", L, ld_z);
   if (rows <= 0) return RVAE_OK;
   const int threads = 256;
+  const bool vec = L % 4 == 0 && ld_z == L &&
+                   ((reinterpret_cast<uintptr_t>(mu_a) | reinterpret_cast<uintptr_t>(lv_a) | reinterpret_cast<uintptr_t>(mu_b) |
+                     reinterpret_cast<uintptr_t>(lv_b) | reinterpret_cast<uintptr_t>(eps) | reinterpret_cast<uintptr_t>(z_f32) |
+                     reinterpret_cast<uintptr_t>(mu_out) | reinterpret_cast<uintptr_t>(lv_out)) & 15) == 0;
+  if (!vec) {
+    const dim3 grid(grid_for(ctx, rows * ld_z, threads, 8));
+    if (alpha_is_f64)
+      RVAE_CUDA(launch_kernel(ctx, lerp_reparam_rows_kernel<double>, grid, dim3(threads), (size_t)0, stream, mu_a, lv_a,
+                              mu_b, lv_b, reinterpret_cast<const double*>(alpha), eps, rows, L, ld_z, z_f32, z_hi, z_lo,
+                              mu_out, lv_out));
+    else
+      RVAE_CUDA(launch_kernel(ctx, lerp_reparam_rows_kernel<float>, grid, dim3(threads), (size_t)0, stream, mu_a, lv_a,
+                              mu_b, lv_b, reinterpret_cast<const float*>(alpha), eps, rows, L, ld_z, z_f32, z_hi, z_lo,
+                              mu_out, lv_out));
+    RVAE_LAUNCH_CHECK(ctx);
+    return RVAE_OK;
+  }
   const dim3 grid(grid_for(ctx, rows * (L / 4), threads, 8));
   if (alpha_is_f64)
     RVAE_CUDA(launch_kernel(ctx, lerp_reparam_kernel<double>, grid, dim3(threads), (size_t)0, stream, mu_a, lv_a, mu_b, lv_b,
@@ -1258,6 +1388,8 @@ constexpr int kHistMaxBlocks = 1024;
 
 struct HistArgs {
   int64_t seg_off[RVAE_HIST_MAX_SEGS];          // element offset of segment s in params
+  int64_t seg_cols[RVAE_HIST_MAX_SEGS];         // segment s = rows of seg_cols values at row pitch seg_pitch
+  int64_t seg_pitch[RVAE_HIST_MAX_SEGS];
   int64_t vstart[RVAE_HIST_MAX_SEGS + 1];       // prefix sums of the lengths: the segments concatenated
   int64_t chunk;                                // concatenated elements per block
   int n_segs, n_edges;
@@ -1337,7 +1469,9 @@ __global__ void __launch_bounds__(kHistThreads) param_histogram_kernel(const flo
   for (int s = 0; s < a.n_segs; ++s) {
     const int64_t lo = max(c0, a.vstart[s]), hi = min(c1, a.vstart[s + 1]);
     if (lo >= hi) continue;   // block-uniform
-    const float* p = params + a.seg_off[s] - a.vstart[s];
+    const float* p = params + a.seg_off[s];
+    const int64_t v0 = a.vstart[s], cols = a.seg_cols[s], pitch = a.seg_pitch[s];
+    const bool dense = cols == pitch;   // block-uniform: one contiguous run, no index arithmetic
     double sum = 0.0, sum_sq = 0.0;
     float mn = INFINITY, mx = -INFINITY;
     int nan = 0;
@@ -1345,8 +1479,9 @@ __global__ void __launch_bounds__(kHistThreads) param_histogram_kernel(const flo
       float x[kHistUnroll];
 #pragma unroll
       for (int u = 0; u < kHistUnroll; ++u) {
-        const int64_t v = base + u * 32 + lane;
-        x[u] = v < hi ? __ldg(p + v) : __int_as_float(0x7fffffff);   // NaN = nothing to count
+        const int64_t v = base + u * 32 + lane - v0;   // index within the segment
+        x[u] = v < hi - v0 ? __ldg(p + (dense ? v : v / cols * pitch + v % cols))
+                           : __int_as_float(0x7fffffff);   // NaN = nothing to count
       }
 #pragma unroll
       for (int u = 0; u < kHistUnroll; ++u) {
@@ -1453,7 +1588,20 @@ size_t param_histogram_bytes(int n_segs, int n_edges) {
 
 int launch_param_histogram(Ctx* ctx, const float* params, const int64_t* seg_offsets, const int64_t* seg_lengths,
                            int n_segs, const double* edges, int n_edges, void* record, cudaStream_t stream) {
-  RVAE_REQUIRE(params && seg_offsets && seg_lengths && edges && record, RVAE_ERR_INVALID, "param_histogram: null pointer");
+  RVAE_REQUIRE(seg_lengths, RVAE_ERR_INVALID, "param_histogram: null pointer");
+  RVAE_REQUIRE(n_segs >= 1 && n_segs <= RVAE_HIST_MAX_SEGS, RVAE_ERR_INVALID,
+               "param_histogram: n_segs = %d, must be 1..%d", n_segs, RVAE_HIST_MAX_SEGS);
+  int64_t ones[RVAE_HIST_MAX_SEGS];
+  for (int s = 0; s < n_segs; ++s) ones[s] = 1;
+  return launch_param_histogram_rows(ctx, params, seg_offsets, ones, seg_lengths, seg_lengths, n_segs, edges, n_edges,
+                                     record, stream);
+}
+
+int launch_param_histogram_rows(Ctx* ctx, const float* params, const int64_t* seg_offsets, const int64_t* seg_rows,
+                                const int64_t* seg_cols, const int64_t* seg_pitch, int n_segs, const double* edges,
+                                int n_edges, void* record, cudaStream_t stream) {
+  RVAE_REQUIRE(params && seg_offsets && seg_rows && seg_cols && seg_pitch && edges && record, RVAE_ERR_INVALID,
+               "param_histogram: null pointer");
   RVAE_REQUIRE(n_segs >= 1 && n_segs <= RVAE_HIST_MAX_SEGS, RVAE_ERR_INVALID,
                "param_histogram: n_segs = %d, must be 1..%d", n_segs, RVAE_HIST_MAX_SEGS);
   RVAE_REQUIRE(n_edges >= 2 && n_edges <= RVAE_HIST_MAX_EDGES, RVAE_ERR_INVALID,
@@ -1471,11 +1619,14 @@ int launch_param_histogram(Ctx* ctx, const float* params, const int64_t* seg_off
   a.n_edges = n_edges;
   a.vstart[0] = 0;
   for (int s = 0; s < n_segs; ++s) {
-    RVAE_REQUIRE(seg_offsets[s] >= 0 && seg_lengths[s] >= 1, RVAE_ERR_INVALID,
-                 "param_histogram: segment %d (offset %lld, length %lld) is empty or out of range", s,
-                 (long long)seg_offsets[s], (long long)seg_lengths[s]);
+    RVAE_REQUIRE(seg_offsets[s] >= 0 && seg_rows[s] >= 1 && seg_cols[s] >= 1 && seg_pitch[s] >= seg_cols[s],
+                 RVAE_ERR_INVALID, "param_histogram: segment %d (offset %lld, %lld rows of %lld at pitch %lld) is empty "
+                 "or out of range", s, (long long)seg_offsets[s], (long long)seg_rows[s], (long long)seg_cols[s],
+                 (long long)seg_pitch[s]);
     a.seg_off[s] = seg_offsets[s];
-    a.vstart[s + 1] = a.vstart[s] + seg_lengths[s];
+    a.seg_cols[s] = seg_cols[s];
+    a.seg_pitch[s] = seg_rows[s] == 1 ? seg_cols[s] : seg_pitch[s];   // one row: contiguous, whatever the pitch
+    a.vstart[s + 1] = a.vstart[s] + seg_rows[s] * seg_cols[s];
   }
   memcpy(a.edges, edges, sizeof(double) * n_edges);
   // guide[j] = #edges <= smallest float of key bucket j (NaN buckets: below / above everything); a merge walk

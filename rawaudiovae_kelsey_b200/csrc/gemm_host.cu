@@ -93,7 +93,7 @@ int gemm_bind_outputs(PreparedGemm* g, const EpiArgs& a, bool force) {
     if (g->epi == EPI_HEAD)  // eps, fp32 [M, L]
       RVAE_CHECK(encode_2d(&p.tmSide, a.in0, true, g->out_cols_f32, g->out_rows, g->out_ld_f32, 32, 128));
     else if (g->epi == EPI_OUT || g->epi == EPI_DRELU)  // x / ReLU mask, bf16 [M, N]
-      RVAE_CHECK(encode_2d(&p.tmSide, a.in0, false, g->out_cols_bf16, g->out_rows,
+      RVAE_CHECK(encode_2d(&p.tmSide, a.in0, false, g->side_cols > 0 ? g->side_cols : g->out_cols_bf16, g->out_rows,
                            (g->epi == EPI_OUT && a.ldi > 0) ? a.ldi : g->out_ld_bf16, 64, 128));
   }
   return RVAE_OK;
@@ -257,20 +257,23 @@ int gemm_prepare(const Ctx* ctx, const GemmDesc& d, PreparedGemm* out) {
   p.num_passes = np;
 
   const int b_rows = (d.epi == EPI_HEAD) ? d.N : d.N;
+  // extent of an operand's contiguous dimension in its tensor map: columns past Operand::cols read as zeros
+  auto dim0 = [](const Operand& o, int extent) { return (uint64_t)(o.cols > 0 && o.cols < extent ? o.cols : extent); };
   for (int i = 0; i < np; ++i) {
     if (d.A.major == MAJOR_K)
-      RVAE_CHECK(encode_bf16_2d(&p.tmA[i], a_ptr[i], d.K, d.M, d.A.ld, kBlockK, kBlockM));
+      RVAE_CHECK(encode_bf16_2d(&p.tmA[i], a_ptr[i], dim0(d.A, d.K), d.M, d.A.ld, kBlockK, kBlockM));
     else
-      RVAE_CHECK(encode_bf16_2d(&p.tmA[i], a_ptr[i], d.M, d.K, d.A.ld, 64, kBlockK));
+      RVAE_CHECK(encode_bf16_2d(&p.tmA[i], a_ptr[i], dim0(d.A, d.M), d.K, d.A.ld, 64, kBlockK));
     if (d.B.major == MAJOR_K)
-      RVAE_CHECK(encode_bf16_2d(&p.tmB[i], b_ptr[i], d.K, b_rows, d.B.ld, kBlockK, block_n / 2));
+      RVAE_CHECK(encode_bf16_2d(&p.tmB[i], b_ptr[i], dim0(d.B, d.K), b_rows, d.B.ld, kBlockK, block_n / 2));
     else
-      RVAE_CHECK(encode_bf16_2d(&p.tmB[i], b_ptr[i], d.N, d.K, d.B.ld, 64, kBlockK));
+      RVAE_CHECK(encode_bf16_2d(&p.tmB[i], b_ptr[i], dim0(d.B, d.N), d.K, d.B.ld, 64, kBlockK));
   }
 
   // epilogue tensors (what the TMA stores write and the side-input loads read)
   g.epi = d.epi;
   g.out_rows = d.M;
+  g.side_cols = d.epi == EPI_OUT ? d.side_cols : 0;
   if (d.epi == EPI_HEAD) {            // z [M, L] bf16; mu, logvar, eps [M, L] fp32
     g.out_cols_bf16 = d.head_L; g.out_ld_bf16 = d.head_L;
     g.out_cols_f32 = d.head_L; g.out_ld_f32 = d.head_L;

@@ -1,8 +1,10 @@
 """Host-side engine: flat parameter storage + the rvae_plan (C ABI) that runs whole steps.
 
 `FlatState` owns the fp32 master weights, gradients, Adam moments, the device step counter and the bf16 shadow
-planes in the layout of `rvae_param_layout` (W1 | W2=[fc21;fc22] | W3 | W4 | b1 | b2 | b3 | b4). The nn.Module
-parameters are views into it, so `state_dict()` stays reference-compatible while one kernel can update everything.
+planes in the layout of `rvae_param_layout_padded` (W1 | W2=[fc21;fc22] | W3 | W4 | b1 | b2 | b3 | b4, each block
+at the dims rounded up to multiples of 64). The nn.Module parameters are views into it - the top-left corners of their
+blocks, strided when a dim is padded - so `state_dict()` stays reference-compatible while one kernel can update
+everything.
 `Plan` binds those buffers plus a workspace to an rvae_plan for a maximum batch size.
 """
 from __future__ import annotations
@@ -45,16 +47,29 @@ def param_layout(S: int, H: int, L: int) -> _lib.Layout:
     return lay
 
 
+def param_layout_padded(S: int, H: int, L: int) -> Tuple[_lib.Layout, int, int, int]:
+    """(layout of the padded blocks, Sp, Hp, Lp): any positive dims, rounded up to multiples of 64."""
+    lay, sp, hp, lp = _lib.Layout(), C.c_int(), C.c_int(), C.c_int()
+    check(_lib.load().rvae_param_layout_padded(S, H, L, C.byref(lay), C.byref(sp), C.byref(hp), C.byref(lp)))
+    return lay, sp.value, hp.value, lp.value
+
+
+def param_geometry(S: int, H: int, L: int) -> Dict[str, Tuple[int, Tuple[int, ...], Tuple[int, ...]]]:
+    """name -> (element offset in the flat buffer, shape, strides): each parameter is the top-left corner of its
+    padded block (row pitch = the block's padded width); contiguous when the dims are multiples of 64."""
+    lay, Sp, Hp, Lp = param_layout_padded(S, H, L)
+    return {
+        "fc1.weight": (lay.w1, (H, S), (Sp, 1)), "fc1.bias": (lay.b1, (H,), (1,)),
+        "fc21.weight": (lay.w2, (L, H), (Hp, 1)), "fc21.bias": (lay.b2, (L,), (1,)),
+        "fc22.weight": (lay.w2 + Lp * Hp, (L, H), (Hp, 1)), "fc22.bias": (lay.b2 + Lp, (L,), (1,)),
+        "fc3.weight": (lay.w3, (H, L), (Lp, 1)), "fc3.bias": (lay.b3, (H,), (1,)),
+        "fc4.weight": (lay.w4, (S, H), (Hp, 1)), "fc4.bias": (lay.b4, (S,), (1,)),
+    }
+
+
 def param_offsets(S: int, H: int, L: int) -> Dict[str, Tuple[int, Tuple[int, ...]]]:
     """name -> (element offset in the flat buffer, shape)."""
-    lay = param_layout(S, H, L)
-    return {
-        "fc1.weight": (lay.w1, (H, S)), "fc1.bias": (lay.b1, (H,)),
-        "fc21.weight": (lay.w2, (L, H)), "fc21.bias": (lay.b2, (L,)),
-        "fc22.weight": (lay.w2 + L * H, (L, H)), "fc22.bias": (lay.b2 + L, (L,)),
-        "fc3.weight": (lay.w3, (H, L)), "fc3.bias": (lay.b3, (H,)),
-        "fc4.weight": (lay.w4, (S, H)), "fc4.bias": (lay.b4, (S,)),
-    }
+    return {n: (off, shape) for n, (off, shape, _) in param_geometry(S, H, L).items()}
 
 
 class FlatState:
@@ -64,8 +79,10 @@ class FlatState:
         self.S, self.H, self.L = S, H, L
         self.device = device
         self.precision = precision
-        self.offsets = param_offsets(S, H, L)
-        self.total = int(param_layout(S, H, L).total)
+        self.geometry = param_geometry(S, H, L)
+        self.offsets = {n: (off, shape) for n, (off, shape, _) in self.geometry.items()}
+        lay, self.Sp, self.Hp, self.Lp = param_layout_padded(S, H, L)
+        self.total = int(lay.total)
         z = lambda dt: torch.zeros(self.total, dtype=dt, device=device)
         self.params = z(torch.float32)
         self.grads = z(torch.float32)
@@ -77,7 +94,9 @@ class FlatState:
         self.shadow_version = -1  # sum of parameter version counters at the last shadow refresh
 
     def view(self, buf: torch.Tensor, name: str) -> torch.Tensor:
-        off, shape = self.offsets[name]
+        off, shape, strides = self.geometry[name]
+        if len(shape) == 2 and strides[0] != shape[1]:   # a padded block: strided view of its top-left corner
+            return buf[off:off + shape[0] * strides[0]].view(shape[0], strides[0])[:, :shape[1]]
         n = 1
         for s in shape:
             n *= s
@@ -331,12 +350,14 @@ class Plan:
 
     def latent(self, name: str) -> torch.Tensor:
         """fp32 view [batch, L] of the current batch's `eps` (the noise the step used - Philox or injected), `mu` or
-        `logvar` in the workspace. Introspection for tests: aliases the workspace, overwritten by the next step."""
+        `logvar` in the workspace. Introspection for tests: aliases the workspace, overwritten by the next step.
+        (A strided view when latent_dim is padded: the workspace rows are Lp wide.)"""
         fn = {"eps": self.lib.rvae_plan_eps, "mu": self.lib.rvae_plan_mu, "logvar": self.lib.rvae_plan_logvar}[name]
         ptr = int(fn(self.handle))
         off = ptr - self.workspace.data_ptr()
-        n = self.batch * self.flat.L
-        return self.workspace[off:off + 4 * n].view(torch.float32).view(self.batch, self.flat.L)
+        L, Lp = self.flat.L, self.flat.Lp
+        n = self.batch * Lp
+        return self.workspace[off:off + 4 * n].view(torch.float32).view(self.batch, Lp)[:, :L]
 
     def bucket(self, s: int) -> torch.Tensor:
         """Gradient bucket s as a view of flat.grads (0..3 = W4, W3, W2, W1 in backward order; 4 = biases)."""

@@ -144,8 +144,9 @@ class VAE(nn.Module):
         if ok:
             base = flat.params.data_ptr()
             for n, p in named:
-                off, shape = flat.offsets[n]
-                if p.data_ptr() != base + 4 * off or tuple(p.shape) != shape or p.dtype != torch.float32:
+                off, shape, strides = flat.geometry[n]
+                if (p.data_ptr() != base + 4 * off or tuple(p.shape) != shape or p.stride() != strides
+                        or p.dtype != torch.float32):
                     ok = False
                     break
         if not ok:
@@ -168,6 +169,11 @@ class VAE(nn.Module):
             flat.sync_shadow()
             flat.shadow_version = version
         return flat
+
+    def _in_place(self, fb: "FrameBatch") -> bool:
+        """Does this model read the frames of `fb` in place (FrameBatch.span)? A segment_length that is not a multiple
+        of 64 is padded inside the model; in fp32 mode such frames are gathered instead (rvae_plan_span_supported)."""
+        return fb.span and (self.segment_length % 64 == 0 or self.precision == "bf16")
 
     def _plan_for(self, batch: int) -> engine.Plan:
         flat = self._ensure_flat()
@@ -209,9 +215,10 @@ class VAE(nn.Module):
             for r in src:
                 if r.segment_length != self.segment_length:
                     raise _lib.RvaeError("FrameBatch segment_length does not match the model")
-                span = len(src) == 1 and r.span and r.n_frames <= plan.max_batch
+                span = len(src) == 1 and self._in_place(r) and r.n_frames <= plan.max_batch
                 if r.frame_idx is not None and r.run and not span:
-                    raise _lib.RvaeError("a device-side run (FrameBatch(run=True)) needs hop % 8 == 0 and hop <= S")
+                    raise _lib.RvaeError("a device-side run (FrameBatch(run=True)) needs hop % 8 == 0, hop <= S, "
+                                         "S % 8 == 0, and bf16 precision when S % 64 != 0")
                 plan.load_frames(r.audio, r.n_frames, r.hop, frame_idx=r.frame_idx, first_frame=r.first_frame,
                                  row_offset=row, span=span)
                 row += r.n_frames
@@ -419,7 +426,8 @@ class _StepBase:
     def _graph_key(self, data):
         """Input signature for graph reuse, or None when the input cannot be served by a replay."""
         if isinstance(data, FrameBatch):
-            return ("frames", data.audio.data_ptr(), data.n_frames, data.hop, data.segment_length, data.span)
+            return ("frames", data.audio.data_ptr(), data.n_frames, data.hop, data.segment_length,
+                    self.model._in_place(data))
         if isinstance(data, torch.Tensor) and data.is_cuda:
             return ("tensor", data.numel())
         return None
@@ -500,7 +508,7 @@ class _StepBase:
             key = None
             if graphable and do_pf and isinstance(data, FrameBatch):
                 key = ("pf", plan.handle.value, next_data.audio.data_ptr(), plan.batch, next_data.n_frames,
-                       next_data.hop, self._plan_cur(plan), plan.pitch, next_data.span) \
+                       next_data.hop, self._plan_cur(plan), plan.pitch, model._in_place(next_data)) \
                     + self._key_extra(data) + self._key_extra(next_data)
             if key is not None and key in self._graphs:
                 st = self._graphs[key]
@@ -536,7 +544,8 @@ class _StepBase:
     def _prefetch(self, plan, data, next_data, frame_idx, first_frame):
         """Register next_data (frames + noise) as the batch the coming train step gathers in the background."""
         plan.prefetch_frames(next_data.audio, next_data.n_frames, next_data.hop, frame_idx=frame_idx,
-                             first_frame=first_frame, seed=self._seed(), offset=0, add_step=True, span=next_data.span)
+                             first_frame=first_frame, seed=self._seed(), offset=0, add_step=True,
+                             span=self.model._in_place(next_data))
 
     def _count(self, what):
         self.stats[what] += 1
@@ -548,7 +557,7 @@ class _StepBase:
 
     def _mark_prefetched(self, plan, next_data):
         # a replayed graph performed the prefetch on the device; mirror it in the plan's host-side state
-        plan.note_prefetched(next_data.n_frames, next_data.hop if next_data.span else 0)
+        plan.note_prefetched(next_data.n_frames, next_data.hop if self.model._in_place(next_data) else 0)
         self._pf = (plan, next_data)
 
     def _fill_idx(self, st, nxt):
@@ -582,7 +591,7 @@ class _StepBase:
             st["idx"] = torch.empty(data.n_frames, dtype=torch.int64, device=dev)
             st["arange"] = torch.arange(data.n_frames, dtype=torch.int64, device=dev)
             static_in = FrameBatch(data.audio, data.n_frames, data.hop, data.segment_length, frame_idx=st["idx"],
-                                   run=data.span)
+                                   run=model._in_place(data))
         else:
             st["x"] = torch.empty((data.numel() // model.segment_length, model.segment_length), dtype=torch.float32,
                                   device=dev)

@@ -136,7 +136,7 @@ def overlap_add(frames: torch.Tensor, hop: int, n_out: Optional[int] = None, *, 
 
 # --------------------------------------------------------------------------------------------- elementwise
 def randn(shape, seed: int, offset: int = 0, device=None, elem_base: int = 0) -> torch.Tensor:
-    """eps ~ N(0,1) from Philox (seed, offset); `elem_base` (a multiple of 4) makes the result elements
+    """eps ~ N(0,1) from Philox (seed, offset); `elem_base` (any value >= 0) makes the result elements
     [elem_base, elem_base + n) of the logical noise tensor - a rank's rows of a global batch."""
     lib = _lib.load()
     out = torch.empty(shape, dtype=torch.float32, device=device or "cuda")
@@ -249,11 +249,14 @@ def histogram_record_layout(n_segs: int, n_edges: int) -> dict:
             "max": a + 28 * n_segs, "bytes": a + 32 * n_segs, "total": total}
 
 
-def param_histogram(params: torch.Tensor, seg_offsets, seg_lengths, edges, out: Optional[torch.Tensor] = None):
+def param_histogram(params: torch.Tensor, seg_offsets, seg_lengths, edges, out: Optional[torch.Tensor] = None, *,
+                    seg_rows=None, seg_pitch=None):
     """TensorBoard histograms (make_histogram semantics) of the segments params[seg_offsets[s] : + seg_lengths[s]] of
     a flat fp32 CUDA tensor against the float64 bin edges `edges`, in one launch on the current stream. Returns the
     device record (uint8; `out` if given, at least histogram_record_layout(...)["total"] bytes): unpack a host copy
-    of its first ["bytes"] bytes with unpack_histogram_record."""
+    of its first ["bytes"] bytes with unpack_histogram_record.
+    seg_rows / seg_pitch (given together): segment s is seg_rows[s] rows of seg_lengths[s] values, row r starting at
+    seg_offsets[s] + r * seg_pitch[s] (a parameter inside the padded block of a padded model)."""
     lib = _lib.load()
     p = _ptr(params, torch.float32, "params")
     offs = np.ascontiguousarray(seg_offsets, dtype=np.int64)
@@ -261,16 +264,27 @@ def param_histogram(params: torch.Tensor, seg_offsets, seg_lengths, edges, out: 
     e = np.ascontiguousarray(edges, dtype=np.float64)
     if offs.shape != lens.shape or offs.ndim != 1:
         raise _lib.RvaeError("param_histogram: seg_offsets and seg_lengths must be 1-D and of equal length")
-    if offs.size and (int((offs + lens).max()) > params.numel() or int(offs.min()) < 0):
+    if (seg_rows is None) != (seg_pitch is None):
+        raise _lib.RvaeError("param_histogram: seg_rows and seg_pitch come together")
+    rows = np.ones_like(offs) if seg_rows is None else np.ascontiguousarray(seg_rows, dtype=np.int64)
+    pitch = lens if seg_pitch is None else np.ascontiguousarray(seg_pitch, dtype=np.int64)
+    if rows.shape != offs.shape or pitch.shape != offs.shape:
+        raise _lib.RvaeError("param_histogram: seg_rows and seg_pitch must match seg_offsets")
+    if offs.size and (int((offs + (rows - 1) * pitch + lens).max()) > params.numel() or int(offs.min()) < 0):
         raise _lib.RvaeError("param_histogram: a segment lies outside params")
     lay = histogram_record_layout(offs.size, e.size)
     if out is None:
         out = torch.empty(lay["total"], dtype=torch.uint8, device=params.device)
     elif out.numel() < lay["total"]:
         raise _lib.RvaeError(f"param_histogram: record buffer holds {out.numel()} bytes, needs {lay['total']}")
-    check(lib.rvae_param_histogram(ctx(params.device), p, offs.ctypes.data,
-                                   lens.ctypes.data, offs.size, e.ctypes.data, e.size, _ptr(out, torch.uint8, "out"),
-                                   _stream()))
+    if seg_rows is None:
+        check(lib.rvae_param_histogram(ctx(params.device), p, offs.ctypes.data,
+                                       lens.ctypes.data, offs.size, e.ctypes.data, e.size, _ptr(out, torch.uint8, "out"),
+                                       _stream()))
+    else:
+        check(lib.rvae_param_histogram_rows(ctx(params.device), p, offs.ctypes.data, rows.ctypes.data, lens.ctypes.data,
+                                            pitch.ctypes.data, offs.size, e.ctypes.data, e.size,
+                                            _ptr(out, torch.uint8, "out"), _stream()))
     return out
 
 

@@ -97,11 +97,15 @@ class Adam(torch.optim.Optimizer):
                     st["step"] = torch.zeros((), dtype=torch.float32, device=p.device)
                     st["exp_avg"] = torch.zeros_like(p, memory_format=torch.contiguous_format)
                     st["exp_avg_sq"] = torch.zeros_like(p, memory_format=torch.contiguous_format)
-                if p.dtype != torch.float32 or not p.is_contiguous():
-                    raise _lib.RvaeError("fused Adam: parameters must be contiguous float32")
-                ops.adam_step(p.data.view(-1), p.grad.contiguous().view(-1), st["exp_avg"].view(-1),
+                if p.dtype != torch.float32:
+                    raise _lib.RvaeError("fused Adam: parameters must be float32")
+                # a VAE parameter of a padded model is a strided view of its block: update a contiguous copy
+                pc = p.data if p.is_contiguous() else p.data.contiguous()
+                ops.adam_step(pc.view(-1), p.grad.contiguous().view(-1), st["exp_avg"].view(-1),
                               st["exp_avg_sq"].view(-1), st["step"], group["lr"], b1, b2, group["eps"],
                               group["weight_decay"])
+                if pc is not p.data:
+                    p.data.copy_(pc)
                 tag = engine.flat_of(p)
                 if tag is not None:
                     tag[0].shadow_version = -1  # shadows are stale; refreshed at the next forward

@@ -80,22 +80,31 @@ class ParamHistogramLogger:
     def _segments(self):
         flat = self.model._ensure_flat()
         if self._segs is None or self._segs[0] is not flat.params:
-            offs, lens = [], []
+            # each parameter as rows of its padded block (one row when contiguous): the padding is not counted
+            offs, rows, cols, pitch = [], [], [], []
             for n in self.names:
-                off, shape = flat.offsets[n]
+                off, shape, strides = flat.geometry[n]
                 offs.append(off)
-                lens.append(int(np.prod(shape)))
-            self._segs = (flat.params, np.asarray(offs, np.int64), np.asarray(lens, np.int64))
+                if len(shape) == 2 and strides[0] != shape[1]:
+                    rows.append(shape[0]); cols.append(shape[1]); pitch.append(strides[0])
+                else:
+                    n_el = int(np.prod(shape))
+                    rows.append(1); cols.append(n_el); pitch.append(n_el)
+            a = lambda v: np.asarray(v, np.int64)
+            self._segs = (flat.params, a(offs), a(rows), a(cols), a(pitch))
         return self._segs
 
     def record(self, step: int) -> None:
-        params, offs, lens = self._segments()
+        params, offs, rows, cols, pitch = self._segments()
         if not self._free:
             self._write(self._pending.popleft())
         slot = self._free.pop()
         if self._dev is None or self._dev.device != params.device:
             self._dev = torch.empty(self.layout["total"], dtype=torch.uint8, device=params.device)
-        ops.param_histogram(params, offs, lens, self.edges, out=self._dev)
+        if (rows == 1).all():
+            ops.param_histogram(params, offs, cols, self.edges, out=self._dev)
+        else:
+            ops.param_histogram(params, offs, cols, self.edges, out=self._dev, seg_rows=rows, seg_pitch=pitch)
         self._host[slot].copy_(self._dev[:self.layout["bytes"]], non_blocking=True)
         self._events[slot].record()
         self._pending.append((slot, int(step), time.time()))
