@@ -149,6 +149,22 @@ int rvae_reparameterize(rvae_ctx* ctx, const float* mu, const float* logvar, con
 int rvae_loss_fwd(rvae_ctx* ctx, const float* xhat, const float* x, const float* mu, const float* logvar,
                   int64_t B, int S, int L, float beta, double* acc, float* loss_out, void* stream);
 
+/* Per-frame loss of held-out audio: what loss_function (rawvae/model.py:38-46) measures, one value per frame instead
+ * of one batch mean - the score of the reference's test_dataset (train.py:153-155, train_iterable.py:170-172), which
+ * the reference only resynthesises. For f < rows, with frame f = audio[(first_frame + f) * hop + s], s < S (the
+ * framing rule of rvae_frame_gather: float32, or int16 * (1/32768); zeros at and beyond n_samples):
+ *   rec_out[f] = (1/S) sum_s (xhat[f,s] - x[f,s])^2
+ *   kl_out[f]  = -(0.5/L) sum_l (1 + logvar[f,l] - mu[f,l]^2 - exp(logvar[f,l]))        (accurate expf)
+ * so that mean_f(rec_out[f] + beta * kl_out[f]) is loss_function(xhat, x, mu, logvar, beta, S). xhat is read at row
+ * pitch ld_xhat >= S, mu and logvar at ld_lat >= L: a plan's rvae_plan_xhat / rvae_plan_mu / rvae_plan_logvar can be
+ * passed directly (pitches Sp, Lp). x is read from the audio itself, exact, never rounded to bf16. Each frame is
+ * reduced by one fixed group of threads in a fixed order (fp64 sums, no atomics): repeated calls are bitwise equal.
+ * Returns 1 for null pointers, rows, S or L <= 0, ld_xhat < S, ld_lat < L, hop <= 0, n_samples < 0 or
+ * first_frame < 0 (checked before ctx is used). */
+int rvae_frame_loss(rvae_ctx* ctx, const float* xhat, int ld_xhat, const float* mu, const float* logvar, int ld_lat,
+                    int64_t rows, int S, int L, const void* audio, int audio_is_i16, int64_t n_samples,
+                    int64_t first_frame, int hop, float* rec_out, float* kl_out, void* stream);
+
 /* Gradients of that loss w.r.t. xhat, mu, logvar, times the upstream scalar *grad_out (NULL = 1). */
 int rvae_loss_bwd(rvae_ctx* ctx, const float* xhat, const float* x, const float* mu, const float* logvar,
                   int64_t B, int S, int L, float beta, const float* grad_out, float* g_xhat, float* g_mu,

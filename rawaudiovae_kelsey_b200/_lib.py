@@ -61,6 +61,8 @@ SIGNATURES = {
     "rvae_split_bf16": (c_int, [P, P, c_int64, P, P, P]),
     "rvae_reparameterize": (c_int, [P, P, P, P, c_int64, P, P]),
     "rvae_loss_fwd": (c_int, [P, P, P, P, P, c_int64, c_int, c_int, c_float, P, P, P]),
+    "rvae_frame_loss": (c_int, [P, P, c_int, P, P, c_int, c_int64, c_int, c_int, P, c_int, c_int64, c_int64, c_int, P,
+                                P, P]),
     "rvae_loss_bwd": (c_int, [P, P, P, P, P, c_int64, c_int, c_int, c_float, P, P, P, P, P]),
     "rvae_tanh_bwd": (c_int, [P, P, P, c_int64, P, P, P]),
     "rvae_colsum": (c_int, [P, P, P, c_int64, c_int, c_int, P, c_int, P]),

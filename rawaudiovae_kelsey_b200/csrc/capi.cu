@@ -349,6 +349,22 @@ int rvae_loss_fwd(rvae_ctx* ctx, const float* xhat, const float* x, const float*
   CTX_OR_FAIL(ctx);
   return launch_loss_fwd(&ctx->c, xhat, x, mu, logvar, B, S, L, beta, acc, loss_out, S_(stream));
 }
+int rvae_frame_loss(rvae_ctx* ctx, const float* xhat, int ld_xhat, const float* mu, const float* logvar, int ld_lat,
+                    int64_t rows, int S, int L, const void* audio, int audio_is_i16, int64_t n_samples,
+                    int64_t first_frame, int hop, float* rec_out, float* kl_out, void* stream) {
+  // arguments first: a malformed call is reported the same way with or without a device
+  RVAE_REQUIRE(xhat && mu && logvar && audio && rec_out && kl_out, RVAE_ERR_INVALID, "frame_loss: null buffer");
+  RVAE_REQUIRE(rows > 0 && S > 0 && L > 0, RVAE_ERR_INVALID, "frame_loss: rows %lld, S %d, L %d (need > 0)",
+               (long long)rows, S, L);
+  RVAE_REQUIRE(ld_xhat >= S && ld_lat >= L, RVAE_ERR_INVALID, "frame_loss: row pitch ld_xhat %d < S %d or ld_lat %d < L %d",
+               ld_xhat, S, ld_lat, L);
+  RVAE_REQUIRE(hop > 0 && n_samples >= 0 && first_frame >= 0, RVAE_ERR_INVALID,
+               "frame_loss: hop %d, n_samples %lld, first_frame %lld (need hop > 0, n_samples >= 0, first_frame >= 0)",
+               hop, (long long)n_samples, (long long)first_frame);
+  CTX_OR_FAIL(ctx);
+  return launch_frame_loss(&ctx->c, xhat, ld_xhat, mu, logvar, ld_lat, rows, S, L, audio, audio_is_i16, n_samples,
+                           first_frame, hop, rec_out, kl_out, S_(stream));
+}
 int rvae_loss_bwd(rvae_ctx* ctx, const float* xhat, const float* x, const float* mu, const float* logvar, int64_t B,
                   int S, int L, float beta, const float* grad_out, float* g_xhat, float* g_mu, float* g_logvar,
                   void* stream) {

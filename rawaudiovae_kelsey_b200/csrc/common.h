@@ -171,6 +171,9 @@ int launch_colsum(Ctx* ctx, const __nv_bfloat16* hi, const __nv_bfloat16* lo, in
                   int accumulate, cudaStream_t stream);
 int launch_loss_fwd(Ctx* ctx, const float* xhat, const float* x, const float* mu, const float* lv, int64_t B, int S,
                     int L, float beta, double* acc, float* loss_out, cudaStream_t stream);
+int launch_frame_loss(Ctx* ctx, const float* xhat, int ld_xhat, const float* mu, const float* lv, int ld_lat,
+                      int64_t rows, int S, int L, const void* audio, int audio_is_i16, int64_t n_samples,
+                      int64_t first_frame, int hop, float* rec_out, float* kl_out, cudaStream_t stream);
 int launch_loss_bwd(Ctx* ctx, const float* xhat, const float* x, const float* mu, const float* lv, int64_t B, int S,
                     int L, float beta, const float* grad_out, float* g_xhat, float* g_mu, float* g_lv,
                     cudaStream_t stream);

@@ -53,6 +53,12 @@ __device__ __forceinline__ float block_sum_to_warp0(float v, float* smem) {
   return t;
 }
 
+__device__ __forceinline__ double warp_sum_f64(double v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+  return v;   // lane 0
+}
+
 // ------------------------------------------------------------------------------------------------
 // K-D1 framing: frame f = audio_pad[idx*hop : idx*hop + S], zero beyond n_samples (the reference zero-pads the
 // tail, rawvae/dataset.py:102-104,141-143). idx = frame_idx[f] (shuffled map-style batches) or first_frame + f
@@ -621,6 +627,107 @@ int launch_loss_fwd(Ctx* ctx, const float* xhat, const float* x, const float* mu
   RVAE_CUDA(launch_kernel(ctx, loss_fwd_kernel, dim3(grid), dim3(threads), (size_t)0, stream, xhat, x, mu, lv, B * S, B * L, acc));
   RVAE_LAUNCH_CHECK(ctx);
   return launch_loss_finalize(ctx, acc, B, S, L, beta, loss_out, 1, nullptr, stream);
+}
+
+// ------------------------------------------------------------------------------------------------
+// K-L3 per-frame loss of held-out audio (rawvae/model.py:38-46 per frame, no mean over the batch):
+//   rec[f] = (1/S) sum_s (xhat[f,s] - x[f,s])^2,   kl[f] = -(0.5/L) sum_l (1 + lv[f,l] - mu[f,l]^2 - exp(lv[f,l]))
+// x is framed straight from the audio (the rule of frame_gather_kernel: exact fp32 or int16 / 32768 samples, zeros
+// at and beyond n_samples), so no bf16 rounding of x enters the score. One warp owns a frame: every lane sums a
+// fixed set of columns, then a fixed shuffle tree combines the lanes - no atomics, repeated calls are bitwise equal.
+// The differences and KL terms are fp32, as in the reference; their sums are fp64.
+// VEC: S, ld_xhat and hop multiples of 4, xhat / audio 16-byte (int16: 8-byte) aligned: 4 columns per load.
+// ------------------------------------------------------------------------------------------------
+template <bool I16>
+__device__ __forceinline__ float audio_sample(const void* audio, int64_t i, int64_t n_samples) {
+  if (i >= n_samples) return 0.f;
+  if constexpr (I16) return __ldg(reinterpret_cast<const int16_t*>(audio) + i) * (1.0f / 32768.0f);
+  else return __ldg(reinterpret_cast<const float*>(audio) + i);
+}
+
+template <bool I16, bool VEC>
+__global__ void frame_loss_kernel(const float* __restrict__ xhat, int ld_xhat, const float* __restrict__ mu,
+                                  const float* __restrict__ lv, int ld_lat, int64_t rows, int S, int L,
+                                  const void* __restrict__ audio, int64_t n_samples, int64_t first_frame, int hop,
+                                  float* __restrict__ rec_out, float* __restrict__ kl_out) {
+  ptx::pdl_launch_dependents();
+  ptx::pdl_wait();
+  const int lane = threadIdx.x & 31;
+  const int64_t warps = (int64_t)gridDim.x * (blockDim.x >> 5);
+  for (int64_t f = blockIdx.x * (int64_t)(blockDim.x >> 5) + (threadIdx.x >> 5); f < rows; f += warps) {
+    const float* xr = xhat + f * ld_xhat;
+    const int64_t s0 = (first_frame + f) * hop;
+    double rec = 0.0;
+    if constexpr (VEC) {
+#pragma unroll 4
+      for (int c = lane * 4; c < S; c += 128) {
+        const float4 a = __ldg(reinterpret_cast<const float4*>(xr + c));
+        const int64_t si = s0 + c;
+        float b[4];
+        if (si + 4 <= n_samples) {
+          if constexpr (I16) {
+            const uint2 r = __ldg(reinterpret_cast<const uint2*>(reinterpret_cast<const int16_t*>(audio) + si));
+            const int16_t* h = reinterpret_cast<const int16_t*>(&r);
+#pragma unroll
+            for (int j = 0; j < 4; ++j) b[j] = h[j] * (1.0f / 32768.0f);
+          } else {
+            const float4 r = __ldg(reinterpret_cast<const float4*>(reinterpret_cast<const float*>(audio) + si));
+            b[0] = r.x; b[1] = r.y; b[2] = r.z; b[3] = r.w;
+          }
+        } else {
+#pragma unroll
+          for (int j = 0; j < 4; ++j) b[j] = audio_sample<I16>(audio, si + j, n_samples);
+        }
+        const float d0 = a.x - b[0], d1 = a.y - b[1], d2 = a.z - b[2], d3 = a.w - b[3];
+        rec = fma((double)d0, (double)d0, rec);
+        rec = fma((double)d1, (double)d1, rec);
+        rec = fma((double)d2, (double)d2, rec);
+        rec = fma((double)d3, (double)d3, rec);
+      }
+    } else {
+#pragma unroll 4
+      for (int c = lane; c < S; c += 32) {
+        const float d = __ldg(xr + c) - audio_sample<I16>(audio, s0 + c, n_samples);
+        rec = fma((double)d, (double)d, rec);
+      }
+    }
+    const float* mr = mu + f * ld_lat;
+    const float* lr = lv + f * ld_lat;
+    double kl = 0.0;
+    for (int l = lane; l < L; l += 32) {
+      const float m = __ldg(mr + l), v = __ldg(lr + l);
+      kl += (double)(1.f + v - m * m - expf(v));
+    }
+    rec = warp_sum_f64(rec);
+    kl = warp_sum_f64(kl);
+    if (lane == 0) {
+      rec_out[f] = static_cast<float>(rec / S);
+      kl_out[f] = static_cast<float>(-0.5 * kl / L);
+    }
+  }
+}
+
+int launch_frame_loss(Ctx* ctx, const float* xhat, int ld_xhat, const float* mu, const float* lv, int ld_lat,
+                      int64_t rows, int S, int L, const void* audio, int audio_is_i16, int64_t n_samples,
+                      int64_t first_frame, int hop, float* rec_out, float* kl_out, cudaStream_t stream) {
+  const int threads = 256;   // 8 frames in flight per block
+  const int grid = grid_for(ctx, rows * 32, threads, 8);
+  const uintptr_t align = audio_is_i16 ? 7 : 15;
+  const bool vec = S % 4 == 0 && ld_xhat % 4 == 0 && hop % 4 == 0 &&
+                   (reinterpret_cast<uintptr_t>(xhat) & 15) == 0 && (reinterpret_cast<uintptr_t>(audio) & align) == 0;
+  auto go = [&](auto kern) {
+    return launch_kernel(ctx, kern, dim3(grid), dim3(threads), (size_t)0, stream, xhat, ld_xhat, mu, lv, ld_lat, rows,
+                         S, L, audio, n_samples, first_frame, hop, rec_out, kl_out);
+  };
+  if (audio_is_i16) {
+    if (vec) RVAE_CUDA(go(frame_loss_kernel<true, true>));
+    else RVAE_CUDA(go(frame_loss_kernel<true, false>));
+  } else {
+    if (vec) RVAE_CUDA(go(frame_loss_kernel<false, true>));
+    else RVAE_CUDA(go(frame_loss_kernel<false, false>));
+  }
+  RVAE_LAUNCH_CHECK(ctx);
+  return RVAE_OK;
 }
 
 // d loss / d xhat, mu, logvar scaled by the upstream gradient (a device scalar; nullptr = 1).
@@ -1429,12 +1536,6 @@ __host__ __device__ __forceinline__ float hist_unkey(uint32_t k) {
   float x;
   memcpy(&x, &u, 4);
   return x;
-}
-
-__device__ __forceinline__ double warp_sum_f64(double v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
-  return v;   // lane 0
 }
 
 __global__ void __launch_bounds__(kHistThreads) param_histogram_kernel(const float* __restrict__ params,

@@ -353,11 +353,17 @@ class Plan:
         `logvar` in the workspace. Introspection for tests: aliases the workspace, overwritten by the next step.
         (A strided view when latent_dim is padded: the workspace rows are Lp wide.)"""
         fn = {"eps": self.lib.rvae_plan_eps, "mu": self.lib.rvae_plan_mu, "logvar": self.lib.rvae_plan_logvar}[name]
-        ptr = int(fn(self.handle))
+        return self._rows(int(fn(self.handle)), self.flat.L, self.flat.Lp)
+
+    def xhat(self) -> torch.Tensor:
+        """fp32 view [batch, S] of the current batch's xhat in the workspace (after a forward that left xhat there:
+        set_outputs without an xhat tensor). Aliases the workspace; rows are Sp wide when segment_length is padded."""
+        return self._rows(int(self.lib.rvae_plan_xhat(self.handle)), self.flat.S, self.flat.Sp)
+
+    def _rows(self, ptr: int, cols: int, pitch: int) -> torch.Tensor:
         off = ptr - self.workspace.data_ptr()
-        L, Lp = self.flat.L, self.flat.Lp
-        n = self.batch * Lp
-        return self.workspace[off:off + 4 * n].view(torch.float32).view(self.batch, Lp)[:, :L]
+        n = self.batch * pitch
+        return self.workspace[off:off + 4 * n].view(torch.float32).view(self.batch, pitch)[:, :cols]
 
     def bucket(self, s: int) -> torch.Tensor:
         """Gradient bucket s as a view of flat.grads (0..3 = W4, W3, W2, W1 in backward order; 4 = biases)."""

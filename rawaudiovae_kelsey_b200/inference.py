@@ -8,12 +8,15 @@
                                                   overlap-add of hop-strided frames ('ola', new - SURVEY.md Q8)
     interpolate(model, ...)                       the whole chain lerp -> reparameterize -> decode as ONE enqueue per
                                                   batch: z is written straight into fc3's bf16 operand
+    evaluate_audio(model, wav, kl_beta)           per-frame loss_function terms of held-out audio (rawvae/model.py:
+                                                  38-46 on the test_dataset of train.py:153-155) and their mean
 
 The audio lives in HBM once; frames are gathered by index into fc1's operand (never materialised in fp32); latents
 of all frames are written into one preallocated tensor (no per-batch torch.cat). CUDA only - CPU tensors raise.
 """
 from __future__ import annotations
 
+from dataclasses import dataclass
 from typing import Optional, Sequence, Tuple, Union
 
 import numpy as np
@@ -178,6 +181,59 @@ def resynthesize(frames: torch.Tensor, mode: str = "concat", hop: Optional[int] 
     if hop is None:
         raise ValueError("mode='ola' needs the hop the frames were cut with")
     return ops.overlap_add(frames, int(hop), n_out)
+
+
+@dataclass
+class Evaluation:
+    """evaluate_audio's result. reconstruction / kl: fp32 [n_frames], the per-frame terms of loss_function;
+    loss = mean(reconstruction + kl_beta * kl), reconstruction_mean = mean(reconstruction), kl_mean = mean(kl), each
+    summed in float64."""
+    reconstruction: torch.Tensor
+    kl: torch.Tensor
+    loss: float
+    reconstruction_mean: float
+    kl_mean: float
+
+
+@torch.no_grad()
+def evaluate_audio(model: VAE, wav, kl_beta: float, *, hop: Optional[int] = None, batch_size: int = 16384,
+                   sample: bool = True, seed: int = 0) -> Evaluation:
+    """Score held-out audio: per frame, the reconstruction error and KL divergence of loss_function
+    (rawvae/model.py:38-46), and their dataset mean - the number the reference's test_dataset never produces
+    (train.py:153-155, train_iterable.py:170-172 load it for listening only).
+
+    Framing as encode_audio: TestDataset by default, AudioDataset at stride `hop` when given. Per batch: the frames are
+    loaded into the model's plan, run through a plain forward and scored by rvae_frame_loss against the exact audio
+    samples (x is never rounded to bf16). Noise: sample=True draws eps from Philox(seed, offset 0) keyed by frame
+    index, so results do not depend on batch_size and evaluations of different checkpoints share their noise;
+    sample=False is the mean path (eps = 0). The model's noise counter, parameters, gradients, optimizer state and a
+    batch a FusedTrainStep has prefetched are left as they were."""
+    dev = _device_of(model)
+    S, L = model.segment_length, model.latent_dim
+    step = S if hop is None else int(hop)
+    if S % step != 0:
+        raise ValueError("segment_length {} is not a multiple of hop_size {}".format(S, step))
+    if batch_size <= 0:
+        raise ValueError("batch_size must be positive")
+    n = int(wav.shape[0])
+    audio = _audio_to_device(wav, dev, step)
+    N = frame_count(n, S, hop)
+    if N <= 0:
+        raise ValueError("{} samples give no frame of {} samples".format(n, S))
+    rec = torch.empty(N, dtype=torch.float32, device=dev)
+    kl = torch.empty_like(rec)
+    zero = None if sample else torch.zeros((min(batch_size, N), L), dtype=torch.float32, device=dev)
+    for lo in range(0, N, batch_size):
+        hi = min(N, lo + batch_size)
+        b = hi - lo
+        plan = model._load(FrameBatch(audio, b, step, S, first_frame=lo))
+        plan.set_eps(ops.randn((b, L), int(seed) & 0xFFFFFFFFFFFFFFFF, 0, device=dev, elem_base=lo * L) if sample
+                     else zero[:b])
+        plan.forward(0.0, fused_loss=False, want_xhat=True)
+        ops.frame_loss(plan.xhat(), plan.latent("mu"), plan.latent("logvar"), audio, lo, step, rec[lo:hi], kl[lo:hi])
+    r64, k64 = rec.double(), kl.double()
+    sums = torch.stack([(r64 + float(kl_beta) * k64).sum(), r64.sum(), k64.sum()]).cpu().tolist()
+    return Evaluation(rec, kl, sums[0] / N, sums[1] / N, sums[2] / N)
 
 
 @torch.no_grad()

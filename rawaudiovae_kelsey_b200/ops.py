@@ -190,6 +190,47 @@ def loss_fwd(xhat, x, mu, logvar, beta: float) -> torch.Tensor:
     return out
 
 
+def _rows(t: torch.Tensor, name: str) -> Tuple[int, int]:
+    """(data pointer, row pitch) of an fp32 CUDA matrix whose rows are contiguous (a strided row view is fine)."""
+    if not t.is_cuda or t.dtype != torch.float32 or t.dim() != 2:
+        raise _lib.RvaeError(f"{name} must be a 2-D float32 CUDA tensor")
+    if t.shape[1] > 1 and t.stride(1) != 1:
+        raise _lib.RvaeError(f"{name} must have contiguous rows")
+    return t.data_ptr(), max(t.stride(0), t.shape[1])
+
+
+def frame_loss(xhat: torch.Tensor, mu: torch.Tensor, logvar: torch.Tensor, audio: torch.Tensor, first_frame: int,
+               hop: int, rec: Optional[torch.Tensor] = None, kl: Optional[torch.Tensor] = None
+               ) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Per-frame reconstruction and KL terms (rvae_frame_loss) of the frames first_frame, first_frame + 1, ... of the
+    wav buffer `audio` (float32 / int16), cut at stride hop: rec[f] = mean_s (xhat[f] - x[f])^2,
+    kl[f] = -0.5 * mean_l (1 + logvar - mu^2 - exp(logvar)). xhat [rows, S], mu / logvar [rows, L] may be row views
+    of wider buffers (a plan's workspace). Returns (rec, kl), fp32 [rows] (written into `rec` / `kl` if given)."""
+    lib = _lib.load()
+    if audio.dtype not in (torch.float32, torch.int16) or audio.dim() != 1:
+        raise _lib.RvaeError("audio must be a 1-D float32 or int16 tensor")
+    px, ldx = _rows(xhat, "xhat")
+    pm, ldm = _rows(mu, "mu")
+    pl, ldl = _rows(logvar, "logvar")
+    rows, S = xhat.shape
+    L = mu.shape[1]
+    if mu.shape != logvar.shape or mu.shape[0] != rows:
+        raise _lib.RvaeError("mu and logvar must be [rows, L] with the rows of xhat")
+    if ldm != ldl:
+        raise _lib.RvaeError("mu and logvar must share one row pitch")
+    dev = xhat.device
+    rec = torch.empty(rows, dtype=torch.float32, device=dev) if rec is None else rec
+    kl = torch.empty(rows, dtype=torch.float32, device=dev) if kl is None else kl
+    if rec.numel() != rows or kl.numel() != rows:
+        raise _lib.RvaeError("rec and kl must hold one value per frame")
+    if any(t.device != dev for t in (mu, logvar, audio, rec, kl)):
+        raise _lib.RvaeError("xhat, mu, logvar, audio, rec and kl must be on one device")
+    check(lib.rvae_frame_loss(ctx(dev), px, ldx, pm, pl, ldm, rows, S, L, _ptr(audio, None, "audio"),
+                              int(audio.dtype == torch.int16), audio.numel(), int(first_frame), int(hop),
+                              _ptr(rec, torch.float32, "rec"), _ptr(kl, torch.float32, "kl"), _stream()))
+    return rec, kl
+
+
 def loss_bwd(xhat, x, mu, logvar, beta: float, grad_out: Optional[torch.Tensor]):
     lib = _lib.load()
     B, S = xhat.shape

@@ -27,6 +27,7 @@ import torch
 
 from . import audio_io, dist as rdist
 from .dataset import AudioDataset, IterableAudioDataset, ToTensor
+from .inference import evaluate_audio
 from .model import VAE, FusedTrainStep
 from .optim import Adam
 from .stats import ParamHistogramLogger
@@ -122,6 +123,51 @@ def _precision(config) -> str:
     return config['VAE'].get('precision', fallback='bf16')
 
 
+def _test_loss_enabled(config) -> bool:
+    """[training] test_loss (optional, default False): score the held-out set at every checkpoint, log it and choose
+    best_model.pt by it. The held-out audio is only loaded when [dataset] generate_test is on."""
+    on = config['training'].getboolean('test_loss', fallback=False)
+    if on and not config['dataset'].getboolean('generate_test'):
+        raise ValueError("[training] test_loss = True needs [dataset] generate_test = True: the test set is only "
+                         "loaded for it")
+    return on
+
+
+def _evaluate_test(model, test_dataset, kl_beta, batch_size, writer, step_id):
+    """Held-out loss of the current weights (inference.evaluate_audio over the TestDataset, Philox seed 0, so every
+    checkpoint sees the same noise), logged under Loss/test*. batch_size = the training batch: the training plan is
+    reused, no new workspace."""
+    ev = evaluate_audio(model, test_dataset.audio_np, kl_beta, batch_size=batch_size, seed=0)
+    writer.add_scalar('Loss/test', ev.loss, step_id)
+    writer.add_scalar('Loss/test_reconstruction', ev.reconstruction_mean, step_id)
+    writer.add_scalar('Loss/test_kl', ev.kl_mean, step_id)
+    print('Test loss: {:.9f} - reconstruction: {:.9f} - KL: {:.9f}'.format(ev.loss, ev.reconstruction_mean,
+                                                                            ev.kl_mean))
+    return ev.loss
+
+
+def _keep_best_test(model, t_loss, best, workdir, config, key, step_id):
+    """best_model.pt by held-out loss: saves the model and records config[training][key] = step_id and best_test_loss
+    when t_loss beats `best`. Returns the best test loss so far."""
+    if t_loss >= best:
+        return best
+    save_path = workdir.joinpath('model').joinpath('best_model.pt')
+    torch.save(model, save_path)
+    print('{} {:05d}: Saved {} (test loss {:.9f})'.format(key, step_id, save_path, t_loss))
+    config['training'][key] = str(step_id)
+    config['training']['best_test_loss'] = str(t_loss)
+    return t_loss
+
+
+def _final_test_message(t_loss, best_test_loss):
+    if t_loss <= best_test_loss:
+        print("The last model is the best model.")
+    else:
+        print("Final test loss was not better than the best model.")
+        print("Final Test Loss: {}".format(t_loss))
+        print("Best Test Loss: {}".format(best_test_loss))
+
+
 def _with_next(iterable):
     """(item, next item or None) pairs: the device-side analogue of a prefetching DataLoader - the step functions
     gather the next batch on their background stream while the current step's GEMMs run."""
@@ -175,6 +221,7 @@ def run_epoch_trainer(argv=None):
     latent_dim = config['VAE'].getint('latent_dim')
     n_units = config['VAE'].getint('n_units')
     kl_beta = config['VAE'].getfloat('kl_beta')
+    test_loss = _test_loss_enabled(config)
     start_time = time.time()
     config['extra']['start'] = time.asctime(time.localtime(start_time))
 
@@ -224,6 +271,7 @@ def run_epoch_trainer(argv=None):
     train_loss_prev = 1000000
     best_loss = 1000000
     final_loss = 1000000
+    best_test_loss = float('inf')
     batch_id = 0
     for epoch in range(epochs):
         print('Epoch {}/{}'.format(epoch, epochs - 1))
@@ -262,7 +310,11 @@ def run_epoch_trainer(argv=None):
                 print('Audio examples generated: {}'.format(audio_out))
                 writer.add_audio('Reconstructed Audio', test_predictions_np, epoch, sample_rate=sampling_rate)
             torch.save(state, checkpoint_dir.joinpath('ckpt_{:05d}'.format(epoch)))
-            if (train_loss < train_loss_prev) and (epoch > save_best_model_after):
+            if test_loss:
+                t_loss = _evaluate_test(model, test_dataset, kl_beta, batch_size, writer, epoch)
+                if epoch > save_best_model_after:
+                    best_test_loss = _keep_best_test(model, t_loss, best_test_loss, workdir, config, 'best_epoch', epoch)
+            elif (train_loss < train_loss_prev) and (epoch > save_best_model_after):
                 save_path = workdir.joinpath('model').joinpath('best_model.pt')
                 torch.save(model, save_path)
                 print('Epoch {:05d}: Saved {}'.format(epoch, save_path))
@@ -286,7 +338,12 @@ def run_epoch_trainer(argv=None):
             print('Last Audio examples generated: {}'.format(audio_out))
             writer.add_audio('Reconstructed Audio', test_predictions_np, epochs, sample_rate=sampling_rate)
         torch.save(state, checkpoint_dir.joinpath('ckpt_{:05d}'.format(epochs)))
-        if final_loss > train_loss_prev:
+        if test_loss:
+            t_loss = _evaluate_test(model, test_dataset, kl_beta, batch_size, writer, epochs)
+            if epochs > save_best_model_after:
+                best_test_loss = _keep_best_test(model, t_loss, best_test_loss, workdir, config, 'best_epoch', epochs)
+            _final_test_message(t_loss, best_test_loss)
+        elif final_loss > train_loss_prev:
             print("Final loss was not better than the last best model.")
             print("Final Loss: {}".format(final_loss))
             print("Best Loss: {}".format(best_loss))
@@ -328,6 +385,7 @@ def run_stream_trainer(argv=None):
     latent_dim = config['VAE'].getint('latent_dim')
     n_units = config['VAE'].getint('n_units')
     kl_beta = config['VAE'].getfloat('kl_beta')
+    test_loss = _test_loss_enabled(config)
     if segment_length != 1024:
         raise ValueError("the streaming dataset frames at 1024 samples (rawvae/dataset.py:66); segment_length "
                          "= {} is not supported by train_iterable.py".format(segment_length))
@@ -380,6 +438,7 @@ def run_stream_trainer(argv=None):
 
         train_loss_prev = 1000000
         best_loss = 1000000
+        best_test_loss = float('inf')
         model.train()
         train_loss = 0.0
         batch_id = 0
@@ -408,7 +467,11 @@ def run_stream_trainer(argv=None):
                     print('Audio examples generated: {}'.format(audio_out))
                     writer.add_audio('Reconstructed Audio', test_predictions_np, batch_id, sample_rate=sampling_rate)
                 torch.save(state, checkpoint_dir.joinpath('ckpt_{:05d}'.format(batch_id)))
-                if train_loss < train_loss_prev:
+                if test_loss:
+                    t_loss = _evaluate_test(model, test_dataset, kl_beta, batch_size, writer, batch_id)
+                    best_test_loss = _keep_best_test(model, t_loss, best_test_loss, workdir, config, 'best_model',
+                                                     batch_id)
+                elif train_loss < train_loss_prev:
                     save_path = workdir.joinpath('model').joinpath('best_model.pt')
                     torch.save(model, save_path)
                     print('batch_id {:05d}: Saved {}'.format(batch_id, save_path))
@@ -434,7 +497,12 @@ def run_stream_trainer(argv=None):
                 print('Last Audio examples generated: {}'.format(audio_out))
                 writer.add_audio('Reconstructed Audio', test_predictions_np, batch_id, sample_rate=sampling_rate)
             torch.save(state, checkpoint_dir.joinpath('ckpt_{:05d}'.format(total_num_batches)))
-            if train_loss > train_loss_prev:
+            if test_loss:
+                t_loss = _evaluate_test(model, test_dataset, kl_beta, batch_size, writer, batch_id)
+                best_test_loss = _keep_best_test(model, t_loss, best_test_loss, workdir, config, 'best_model',
+                                                 total_num_batches)
+                _final_test_message(t_loss, best_test_loss)
+            elif train_loss > train_loss_prev:
                 print("Final loss was not better than the last best model.")
                 print("Final Loss: {}".format(final_loss))
                 print("Best Loss: {}".format(best_loss))
