@@ -410,6 +410,81 @@ int rvae_plan_adam_buckets(rvae_plan* plan, unsigned bucket_mask, double lr, dou
 int rvae_plan_train_step(rvae_plan* plan, float kl_beta, double lr, double beta1, double beta2, double eps,
                          double weight_decay, int zero_grads, float* loss_out, int ring_size, void* stream);
 
+/* ---------------------------------------------------------------------------------------------------------
+ * Scheduled hyper-parameters. The reference trains at a fixed learning rate (torch.optim.Adam, train.py:163,193)
+ * and a fixed KL weight (rawvae/model.py:45); this record adds a learning-rate warm-up and decay and a KL-weight
+ * ramp. It lives in device memory and the kernels of a step read it when they run, so a CUDA graph captured around
+ * rvae_plan_train_step_hp holds the record's ADDRESS: every replay follows the schedule at its own step, and any
+ * rewrite of the record that is stream-ordered before the replay.
+ *
+ * k = the device step counter (bufs.step) when the step starts; Adam's bias correction keeps t = k + 1.
+ * T = total_steps, W = warmup_steps. Learning rate:
+ *   k < W:       lr * (k + 1) / W
+ *   otherwise    D = max(T - W, 1), u = min(k - W, D) / D, and
+ *                constant lr | linear lr_min + (lr - lr_min) * (1 - u) | cosine lr_min + (lr - lr_min) * 0.5 * (1 + cos(pi u))
+ * KL weight, b0 = kl_beta_start, A = kl_anneal_steps, M = kl_cycles, R = kl_cycle_ratio:
+ *   constant kl_beta | linear b0 + (kl_beta - b0) * min(1, k / A)
+ *   cyclical C = ceil(T / M), tau = (k mod C) / C, b0 + (kl_beta - b0) * min(1, tau / R)
+ * Everything is evaluated in fp64, operation by operation in the order written, without FMA contraction. cos(pi u)
+ * is a fixed polynomial: the Taylor series of cos to x^22 at x = pi * min(u, 1 - u), negated for u > 0.5, evaluated
+ * by Horner's rule. So a host mirror that repeats these operations (rawaudiovae_kelsey_b200/schedule.py) gets the
+ * same doubles. lr(k) reaches Adam as a double; beta(k) is rounded to float, as the kl_beta argument of
+ * rvae_plan_train_step is. A record of kind constant / constant with W = 0 gives every kernel exactly the scalars
+ * rvae_plan_train_step gives it. */
+#define RVAE_LR_CONSTANT 0
+#define RVAE_LR_LINEAR 1
+#define RVAE_LR_COSINE 2
+#define RVAE_KL_CONSTANT 0
+#define RVAE_KL_LINEAR 1
+#define RVAE_KL_CYCLICAL 2
+
+typedef struct rvae_hparams {
+  double lr;               /*   0  peak learning rate */
+  double beta1;            /*   8 */
+  double beta2;            /*  16 */
+  double eps;              /*  24 */
+  double weight_decay;     /*  32 */
+  double kl_beta;          /*  40  target KL weight */
+  double lr_min;           /*  48 */
+  double kl_beta_start;    /*  56 */
+  double kl_cycle_ratio;   /*  64  R, in (0, 1] */
+  int64_t total_steps;     /*  72  T, >= 1 for a linear / cosine lr or a cyclical KL weight */
+  int64_t warmup_steps;    /*  80  W, >= 0 */
+  int64_t kl_anneal_steps; /*  88  A, >= 1 for a linear KL weight */
+  int64_t kl_cycles;       /*  96  M, >= 1 for a cyclical KL weight */
+  int32_t lr_schedule;     /* 104  RVAE_LR_* */
+  int32_t kl_anneal;       /* 108  RVAE_KL_* */
+} rvae_hparams;            /* 112 bytes, 8-byte aligned */
+
+#ifdef __cplusplus
+#define RVAE_STATIC_ASSERT(c, m) static_assert(c, m)
+#else
+#define RVAE_STATIC_ASSERT(c, m) _Static_assert(c, m)
+#endif
+RVAE_STATIC_ASSERT(sizeof(rvae_hparams) == 112, "rvae_hparams: 112 bytes");
+RVAE_STATIC_ASSERT(offsetof(rvae_hparams, kl_beta) == 40 && offsetof(rvae_hparams, kl_cycle_ratio) == 64,
+                   "rvae_hparams: double fields");
+RVAE_STATIC_ASSERT(offsetof(rvae_hparams, total_steps) == 72 && offsetof(rvae_hparams, kl_cycles) == 96,
+                   "rvae_hparams: integer fields");
+RVAE_STATIC_ASSERT(offsetof(rvae_hparams, lr_schedule) == 104 && offsetof(rvae_hparams, kl_anneal) == 108,
+                   "rvae_hparams: kinds");
+
+/* Validate a HOST copy of a record: 0 if it is usable, 1 for an unknown kind, W < 0, T < 1 with a linear / cosine
+ * learning rate or a cyclical KL weight, A < 1 with a linear KL weight, M < 1 with a cyclical one, R outside (0, 1]
+ * or a non-finite value. The device entries below cannot read the record without a synchronisation: check every
+ * record before it is uploaded. */
+int rvae_hparams_check(const rvae_hparams* host);
+/* rvae_plan_train_step with every hyper-parameter read from the device record hp_dev at run time (same data-parallel
+ * path, per-kernel timing mode and results for a constant record). Returns 1 for a null hp_dev or ring_size < 1
+ * (before the plan is used), 2 for the experiments-only fused latent epilogue, which takes its KL scale from the host. */
+int rvae_plan_train_step_hp(rvae_plan* plan, const rvae_hparams* hp_dev, int zero_grads, float* loss_out,
+                            int ring_size, void* stream);
+/* Evaluate the record's schedule at the n step indices k_dev[0..n) with the device function the training kernels
+ * use: lr_out[i] = lr(k_dev[i]), beta_out[i] = (float)beta(k_dev[i]). Returns 1 for null pointers or n < 1 (before
+ * ctx is used). */
+int rvae_hparams_eval(rvae_ctx* ctx, const rvae_hparams* hp_dev, const int64_t* k_dev, int n, double* lr_out,
+                      float* beta_out, void* stream);
+
 /* Device pointers into the workspace for the current batch (valid after forward): fp32 [batch, ...] at the plan's
  * padded row pitch - mu, logvar, eps [batch, Lp], xhat [batch, Sp] (rvae_param_layout_padded); only the first L (S)
  * columns of a row are the model's, the rest are zeros. */

@@ -32,6 +32,14 @@ class PlanBuffers(C.Structure):
                 ("params", "grads", "exp_avg", "exp_avg_sq", "step", "shadow_hi", "shadow_lo", "workspace")]
 
 
+class Hparams(C.Structure):
+    """rvae_hparams: the device-resident hyper-parameter record of a scheduled training step (112 bytes)."""
+    _fields_ = [(n, c_double) for n in ("lr", "beta1", "beta2", "eps", "weight_decay", "kl_beta", "lr_min",
+                                        "kl_beta_start", "kl_cycle_ratio")] + \
+               [(n, c_int64) for n in ("total_steps", "warmup_steps", "kl_anneal_steps", "kl_cycles")] + \
+               [(n, C.c_int32) for n in ("lr_schedule", "kl_anneal")]
+
+
 # name -> (restype, argtypes); every symbol declared in include/rvae_b200.h
 P = c_void_p
 SIGNATURES = {
@@ -109,6 +117,9 @@ SIGNATURES = {
     "rvae_plan_adam_buckets": (c_int, [P, C.c_uint, c_double, c_double, c_double, c_double, c_double, c_float, c_int, P]),
     "rvae_plan_adam": (c_int, [P, c_double, c_double, c_double, c_double, c_double, c_float, c_int, P]),
     "rvae_plan_train_step": (c_int, [P, c_float, c_double, c_double, c_double, c_double, c_double, c_int, P, c_int, P]),
+    "rvae_plan_train_step_hp": (c_int, [P, P, c_int, P, c_int, P]),
+    "rvae_hparams_check": (c_int, [C.POINTER(Hparams)]),
+    "rvae_hparams_eval": (c_int, [P, P, P, c_int, P, P, P]),
     "rvae_plan_mu": (P, [P]),
     "rvae_plan_logvar": (P, [P]),
     "rvae_plan_xhat": (P, [P]),

@@ -1,5 +1,6 @@
 // C ABI (include/rvae_b200.h): context, op-level entry points and the plan that issues a whole training or
 // inference step from C. No torch types cross this boundary.
+#include <cmath>
 #include <cstdlib>
 #include <dlfcn.h>
 #include <cstring>
@@ -491,7 +492,7 @@ int rvae_dgrad_latent(rvae_ctx* ctx, const void* da3_hi, const void* da3_lo, con
   d.B = op(w3_hi, w3_lo, MAJOR_MN, L);
   d.args.out_f32 = dz_scratch; d.args.ldo = L; d.args.accumulate = 1;
   RVAE_CHECK(gemm_launch(&ctx->c, d, S_(stream)));
-  return launch_latent_bwd(&ctx->c, dz_scratch, eps, logvar, mu, g_mu_ext, g_logvar_ext, kl_grad_scale, M, L,
+  return launch_latent_bwd(&ctx->c, dz_scratch, eps, logvar, mu, g_mu_ext, g_logvar_ext, kl_grad_value(kl_grad_scale), M, L,
                            BF(dml_hi), BF(dml_lo), bias_grad, 0, nullptr, S_(stream));
 }
 
@@ -625,6 +626,9 @@ struct rvae_plan {
                          // the ranks draw disjoint pieces of the single-process noise tensor (0 = single process)
   bool dp_enabled;       // rvae_plan_enable_dp: this plan's train steps all-reduce their gradients
   float kl_c0;           // kl_beta / (B L) of the last fused-loss forward (KL gradient scale of the latent backward)
+  double kl_bl;          // B L of that forward (global batch under data parallelism)
+  const rvae_hparams* hp_dev;   // during rvae_plan_train_step_hp: the device record the kernels read kl_beta from
+  int hp_early;                 // ... and the latent backward may read it before griddepcontrol.wait (two streams)
   bool dz_zeroed;        // the split-K latent dgrad accumulator holds zeros (left so by the latent backward kernel)
   bool grads_zeroed[5];  // gradient bucket s (0..3 weights, 4 biases) already holds zeros (left so by the fused Adam)
   // internal streams (created on first use): see rvae_plan_train_step
@@ -987,8 +991,8 @@ int ensure_side_stream(rvae_plan* p) {
 
 // Adam over the gradient buckets selected by `mask` (bit s = bucket s of rvae_plan_bucket): the selected buckets are
 // merged into contiguous segments of the flat buffer and updated with one launch per pair of segments.
-int adam_buckets(rvae_plan* p, unsigned mask, double lr, double beta1, double beta2, double eps, double weight_decay,
-                 float grad_scale, int zero_grads, int step_bias, bool advance_step, cudaStream_t st) {
+int adam_buckets(rvae_plan* p, unsigned mask, const HpArg& hp, float grad_scale, int zero_grads, int step_bias,
+                 bool advance_step, cudaStream_t st) {
   const rvae_layout& ly = p->lay;
   const rvae_plan_buffers& b = p->bufs;
   // flat order: W1 (bucket 3) | W2 (2) | W3 (1) | W4 (0) | biases (4)
@@ -1010,8 +1014,7 @@ int adam_buckets(rvae_plan* p, unsigned mask, double lr, double beta1, double be
     const bool pair = i + 1 < nseg;
     const bool last = i + 2 >= nseg;
     RVAE_CHECK(launch_adam2(&p->ctx->c, b.params + o, b.grads + o, b.exp_avg + o, b.exp_avg_sq + o, seg_n[i],
-                            pair ? seg_off[i + 1] - o : 0, pair ? seg_n[i + 1] : 0, lr, beta1, beta2, eps, weight_decay,
-                            grad_scale, b.step, step_bias, (advance_step && last) ? p->ticket : nullptr,
+                            pair ? seg_off[i + 1] - o : 0, pair ? seg_n[i + 1] : 0, hp, grad_scale, b.step, step_bias, (advance_step && last) ? p->ticket : nullptr,
                             BF(b.shadow_hi) + o, b.shadow_lo ? BF(b.shadow_lo) + o : nullptr, zero_grads, st));
   }
   for (int s = 0; s < 5; ++s)
@@ -1035,6 +1038,9 @@ struct LatentExt {
   const float* g_lv;
   const float* lv;
 };
+
+// KL gradient scale of the latent backward: the host's kl_c0, or beta(k) / (B L) from the record of a scheduled step
+KlGrad plan_kl(const rvae_plan* p) { return KlGrad{p->hp_dev, p->bufs.step, p->kl_bl, p->kl_c0, p->hp_early}; }
 
 // Fused launches read their tile schedule from the plan's one schedule buffer: usable by the batch size that owns it.
 bool sched_usable(const rvae_plan* p) { return p->sched_batch == 0 || p->sched_batch == p->batch; }
@@ -1130,7 +1136,7 @@ int backward_stage(rvae_plan* p, int stage, const LatentExt* ext, cudaStream_t s
       {
         TimedScope ts(p, T_LATENT, st);
         RVAE_CHECK(launch_latent_bwd(&p->ctx->c, p->dz, p->eps, ext ? ext->lv : p->lv, p->mu, ext ? ext->g_mu : nullptr,
-                                     ext ? ext->g_lv : nullptr, p->kl_c0, p->batch, L, p->dml.hi, p->dml.lo, grads + ly.b2,
+                                     ext ? ext->g_lv : nullptr, plan_kl(p), p->batch, L, p->dml.hi, p->dml.lo, grads + ly.b2,
                                      1, p->fin_pending ? &p->fin : nullptr, st));
       }
       p->fin_pending = false;
@@ -1168,7 +1174,7 @@ int backward_stage(rvae_plan* p, int stage, const LatentExt* ext, cudaStream_t s
     }
     TimedScope ts(p, T_LATENT, st);
     RVAE_CHECK(launch_latent_bwd(&p->ctx->c, p->dz, p->eps, ext ? ext->lv : p->lv, p->mu, ext ? ext->g_mu : nullptr,
-                                 ext ? ext->g_lv : nullptr, p->kl_c0, p->batch, L, p->dml.hi, p->dml.lo, grads + ly.b2, 1,
+                                 ext ? ext->g_lv : nullptr, plan_kl(p), p->batch, L, p->dml.hi, p->dml.lo, grads + ly.b2, 1,
                                  p->fin_pending ? &p->fin : nullptr, st));
     p->fin_pending = false;
     p->dz_zeroed = true;
@@ -1200,7 +1206,7 @@ int backward_stage(rvae_plan* p, int stage, const LatentExt* ext, cudaStream_t s
     };
     auto run_latent = [&]() -> int {
       return launch_latent_bwd(&p->ctx->c, p->dz, p->eps, ext ? ext->lv : p->lv, p->mu, ext ? ext->g_mu : nullptr,
-                               ext ? ext->g_lv : nullptr, p->kl_c0, p->batch, L, p->dml.hi, p->dml.lo, grads + ly.b2, 1,
+                               ext ? ext->g_lv : nullptr, plan_kl(p), p->batch, L, p->dml.hi, p->dml.lo, grads + ly.b2, 1,
                                p->fin_pending ? &p->fin : nullptr, s_l);
     };
     if (p->s1_order == 0) { RVAE_CHECK(run_wgrad()); RVAE_CHECK(run_latent()); }
@@ -1245,7 +1251,7 @@ int backward_stage(rvae_plan* p, int stage, const LatentExt* ext, cudaStream_t s
   if (stage == 1) {
     TimedScope ts(p, T_LATENT, st);
     RVAE_CHECK(launch_latent_bwd(&p->ctx->c, p->dz, p->eps, ext ? ext->lv : p->lv, p->mu, ext ? ext->g_mu : nullptr,
-                                 ext ? ext->g_lv : nullptr, p->kl_c0, p->batch, L, p->dml.hi, p->dml.lo, grads + ly.b2, 1,
+                                 ext ? ext->g_lv : nullptr, plan_kl(p), p->batch, L, p->dml.hi, p->dml.lo, grads + ly.b2, 1,
                                  p->fin_pending ? &p->fin : nullptr, st));
     p->fin_pending = false;
     p->dz_zeroed = true;
@@ -1272,7 +1278,7 @@ int rvae_plan_create(rvae_ctx* ctx, int S, int H, int L, int max_batch, int prec
   p->s_true = S; p->h_true = H; p->l_true = L;
   p->lay = lay; p->bound = false; p->batch = 0; p->have_eps = false; p->global_batch = 0; p->noise_row0 = 0;
   p->timing = false;
-  p->kl_c0 = 0.f; p->dz_zeroed = false; p->dp_enabled = false;
+  p->kl_c0 = 0.f; p->kl_bl = 0.0; p->hp_dev = nullptr; p->hp_early = 0; p->dz_zeroed = false; p->dp_enabled = false;
   p->cur = 0; p->ticket_zeroed = false; p->ticket = nullptr;
   p->x_pitch = 0; p->x_pitch_alt = 0;
   p->fuse_latent = false;
@@ -1592,6 +1598,7 @@ int rvae_plan_forward(rvae_plan* plan, float kl_beta, int fused_loss, int want_x
     }
     if (gs->fwd_state == 1) {
       p->kl_c0 = (float)((double)kl_beta / BL);
+      p->kl_bl = BL;
       RVAE_CHECK(ensure_bias_zeroed(p, st));   // F4's epilogue accumulates db4, the backward epilogues db3, db2, db1
       p->grads_zeroed[4] = false;
       RVAE_CUDA(cudaMemsetAsync(p->dep_flags, 0, sizeof(unsigned int) * 3 * 256, st));
@@ -1615,7 +1622,7 @@ int rvae_plan_forward(rvae_plan* plan, float kl_beta, int fused_loss, int want_x
     EpiArgs a = gs->g[G_F2].params.epi;
     if (p->out_mu && lat_direct) a.out_f32 = p->out_mu;
     if (p->out_lv && lat_direct) a.out_f32_b = p->out_lv;
-    if (fused_loss) p->kl_c0 = (float)((double)kl_beta / BL);
+    if (fused_loss) { p->kl_c0 = (float)((double)kl_beta / BL); p->kl_bl = BL; }
     else a.loss_acc = nullptr;
     RVAE_CHECK(run(p, G_F2, st, &a));
     if (!lat_direct) RVAE_CHECK(copy_latents_out(p, st));
@@ -1789,12 +1796,14 @@ int rvae_plan_adam_buckets(rvae_plan* plan, unsigned bucket_mask, double lr, dou
   // zero_grads: the kernel clears the gradient buffer after consuming it (what optimizer.zero_grad() does at the top
   // of the reference loop, train.py:184), so the next step's split-K weight gradients can reduce-add without memsets
   TimedScope ts(plan, T_ADAM, S_(stream));
-  return adam_buckets(plan, bucket_mask, lr, beta1, beta2, eps, weight_decay, grad_scale, zero_grads, 0, false,
-                      S_(stream));
+  return adam_buckets(plan, bucket_mask, hp_value(lr, beta1, beta2, eps, weight_decay), grad_scale, zero_grads, 0,
+                      false, S_(stream));
 }
 
-int rvae_plan_train_step(rvae_plan* plan, float kl_beta, double lr, double beta1, double beta2, double eps,
-                         double weight_decay, int zero_grads, float* loss_out, int ring_size, void* stream) {
+// The training step behind rvae_plan_train_step (hp by value, KL weight kl_beta) and rvae_plan_train_step_hp (hp.dev
+// = the device record, which the Adam launches, the latent backward and the loss finalisation read instead)
+static int train_step(rvae_plan* plan, float kl_beta, const HpArg& hp, int zero_grads, float* loss_out, int ring_size,
+               void* stream) {
   RVAE_CHECK(check_ready(plan, true));
   const rvae_plan_buffers& b = plan->bufs;
   RVAE_REQUIRE(b.grads && b.exp_avg && b.exp_avg_sq && b.step, RVAE_ERR_STATE,
@@ -1803,15 +1812,27 @@ int rvae_plan_train_step(rvae_plan* plan, float kl_beta, double lr, double beta1
   // The step counter t (Adam's bias correction, the loss-ring slot, the Philox offset) stays at its old value for
   // the whole step: every Adam launch uses t + 1, and the last block of the final launch advances it.
   const bool fork = plan->two_streams && !plan->timing;
+  // With a record bound, the latent backward evaluates it before griddepcontrol.wait, overlapping the GEMM before it,
+  // when the step runs on the internal streams. That is safe: (1) the record is written by a copy the caller orders
+  // before this call on `stream`, and every kernel of the step runs on `st` after cudaStreamWaitEvent(ev_hp_fork),
+  // which is recorded on `stream` after the copy; (2) the step counter was last written by the previous step's final
+  // Adam launch, an earlier operation of `st`; the wait on ev_hp_fork lies between it and this step's kernels, and a
+  // stream operation other than a kernel starts only when every earlier operation of its stream is complete, so that
+  // launch has completed before any kernel of this step starts (replays of a captured graph run one after the other:
+  // the same holds); (3) no kernel of this step writes the counter before its final Adam launch. On one stream
+  // (per-kernel timing, RVAE_TWO_STREAMS=0) only kernels separate the steps, and a chain of early starts could reach
+  // back to the previous step's last kernel, so the kernel reads the record after griddepcontrol.wait.
+  plan->hp_early = fork && plan->hp_dev != nullptr;
   if (!fork) {
     // (per-kernel timing / RVAE_TWO_STREAMS=0: a LOCAL step - no collectives are issued even when the context has a
     // communicator; bench.py's attribution pass runs this on rank 0 only)
     RVAE_CHECK(rvae_plan_forward(plan, kl_beta, 1, 0, stream));
     RVAE_CHECK(rvae_plan_finish_loss_deferred(plan, kl_beta, loss_out, ring_size));  // runs inside stage 1
     plan->fin.inc_step = 0;
+    plan->fin.hp = hp.dev;
     RVAE_CHECK(rvae_plan_backward(plan, -1, stream));
     TimedScope ts(plan, T_ADAM, S_(stream));
-    return adam_buckets(plan, 0x1f, lr, beta1, beta2, eps, weight_decay, 1.0f, zero_grads, 1, true, S_(stream));
+    return adam_buckets(plan, 0x1f, hp, 1.0f, zero_grads, 1, true, S_(stream));
   }
   // The critical chain (GEMMs) runs on a highest-priority stream; the HBM-bound side work (next batch + its noise,
   // Adam per bucket) on a lowest-priority background stream. The persistent GEMM grids leave the SMs that wave
@@ -1851,6 +1872,7 @@ int rvae_plan_train_step(rvae_plan* plan, float kl_beta, double lr, double beta1
   }
   RVAE_CHECK(rvae_plan_finish_loss_deferred(plan, kl_beta, loss_out, ring_size));  // runs inside stage 1
   plan->fin.inc_step = 0;
+  plan->fin.hp = hp.dev;
   // Adam per bucket as soon as the bucket's gradient is complete; the dgrad GEMM that reads the bucket's bf16
   // shadow weights runs before the weight-gradient GEMM of the same stage, so nothing of this step reads them again.
   // Data parallelism: bucket s is SUM all-reduced (NCCL over NVLink / NVSwitch) on the communication stream as soon
@@ -1918,7 +1940,7 @@ int rvae_plan_train_step(rvae_plan* plan, float kl_beta, double lr, double beta1
       RVAE_CUDA(cudaEventRecord(plan->ev_comm_done[s], cs));
       RVAE_CUDA(cudaStreamWaitEvent(bg, plan->ev_comm_done[s], 0));
       if (s == 0) RVAE_CHECK(finalize_on_bg());
-      RVAE_CHECK(adam_buckets(plan, kBucketMask[s] | extra, lr, beta1, beta2, eps, weight_decay, 1.0f, zero_grads, 1, false, bg));
+      RVAE_CHECK(adam_buckets(plan, kBucketMask[s] | extra, hp, 1.0f, zero_grads, 1, false, bg));
       continue;
     }
     // single process: only W4 (the first bucket to complete, with the most GEMM time left to hide under) is updated
@@ -1931,7 +1953,7 @@ int rvae_plan_train_step(rvae_plan* plan, float kl_beta, double lr, double beta1
       // (single process) held to adam_bg_blocks blocks: it then lives on the SMs the 128-CTA GEMM grids leave free
       // instead of taking every SM a finishing GEMM releases before the latent kernel of stage 1 gets there
       cx->c.aux_grid_cap = plan->adam_bg_blocks;
-      const int rc_bg = adam_buckets(plan, kBucketMask[0], lr, beta1, beta2, eps, weight_decay, 1.0f, zero_grads, 1, false, bg);
+      const int rc_bg = adam_buckets(plan, kBucketMask[0], hp, 1.0f, zero_grads, 1, false, bg);
       cx->c.aux_grid_cap = 0;
       RVAE_CHECK(rc_bg);
     }
@@ -1951,10 +1973,62 @@ int rvae_plan_train_step(rvae_plan* plan, float kl_beta, double lr, double beta1
     RVAE_CUDA(cudaStreamWaitEvent(st, plan->ev_comm_done[2], 0));   // the bias bucket travelled with exchange 2
   }
   RVAE_CUDA(cudaStreamWaitEvent(st, plan->ev_adam_join, 0));  // every earlier Adam launch has read the step counter
-  RVAE_CHECK(adam_buckets(plan, dp ? 0x18u : 0x1eu, lr, beta1, beta2, eps, weight_decay, 1.0f, zero_grads, 1, true, st));
+  RVAE_CHECK(adam_buckets(plan, dp ? 0x18u : 0x1eu, hp, 1.0f, zero_grads, 1, true, st));
   RVAE_CUDA(cudaEventRecord(plan->ev_hp_join, st));
   RVAE_CUDA(cudaStreamWaitEvent(S_(stream), plan->ev_hp_join, 0));
   return RVAE_OK;
+}
+
+int rvae_plan_train_step(rvae_plan* plan, float kl_beta, double lr, double beta1, double beta2, double eps,
+                         double weight_decay, int zero_grads, float* loss_out, int ring_size, void* stream) {
+  return train_step(plan, kl_beta, hp_value(lr, beta1, beta2, eps, weight_decay), zero_grads, loss_out, ring_size,
+                    stream);
+}
+
+int rvae_plan_train_step_hp(rvae_plan* plan, const rvae_hparams* hp_dev, int zero_grads, float* loss_out,
+                            int ring_size, void* stream) {
+  RVAE_REQUIRE(hp_dev != nullptr && ring_size >= 1, RVAE_ERR_INVALID, "plan_train_step_hp: null record or ring_size %d",
+               ring_size);
+  RVAE_CHECK(check_ready(plan, true));
+  // the experiments-only fused latent epilogue takes its KL scale from the host (EpiArgs::c0)
+  RVAE_REQUIRE(!latent_fused(plan), RVAE_ERR_UNSUPPORTED,
+               "plan_train_step_hp: the fused latent epilogue (RVAE_FUSE_LATENT) does not read the record");
+  struct HpGuard {   // the record is bound for the kernels of this call only
+    rvae_plan* p;
+    HpGuard(rvae_plan* p_, const rvae_hparams* hp) : p(p_) { p->hp_dev = hp; }
+    ~HpGuard() { p->hp_dev = nullptr; p->hp_early = 0; }
+  } guard(plan, hp_dev);
+  return train_step(plan, 0.0f, hp_device(hp_dev), zero_grads, loss_out, ring_size, stream);
+}
+
+int rvae_hparams_check(const rvae_hparams* h) {
+  RVAE_REQUIRE(h, RVAE_ERR_INVALID, "hparams_check: null record");
+  const double vals[9] = {h->lr, h->beta1, h->beta2, h->eps, h->weight_decay, h->kl_beta, h->lr_min, h->kl_beta_start,
+                          h->kl_cycle_ratio};
+  for (double v : vals) RVAE_REQUIRE(std::isfinite(v), RVAE_ERR_INVALID, "hparams_check: non-finite value");
+  RVAE_REQUIRE(h->lr_schedule >= RVAE_LR_CONSTANT && h->lr_schedule <= RVAE_LR_COSINE, RVAE_ERR_INVALID,
+               "hparams_check: lr_schedule %d", h->lr_schedule);
+  RVAE_REQUIRE(h->kl_anneal >= RVAE_KL_CONSTANT && h->kl_anneal <= RVAE_KL_CYCLICAL, RVAE_ERR_INVALID,
+               "hparams_check: kl_anneal %d", h->kl_anneal);
+  RVAE_REQUIRE(h->warmup_steps >= 0, RVAE_ERR_INVALID, "hparams_check: warmup_steps %lld", (long long)h->warmup_steps);
+  RVAE_REQUIRE(h->total_steps >= 1 || (h->lr_schedule == RVAE_LR_CONSTANT && h->kl_anneal != RVAE_KL_CYCLICAL),
+               RVAE_ERR_INVALID, "hparams_check: total_steps %lld", (long long)h->total_steps);
+  RVAE_REQUIRE(h->kl_anneal_steps >= 1 || h->kl_anneal != RVAE_KL_LINEAR, RVAE_ERR_INVALID,
+               "hparams_check: kl_anneal_steps %lld", (long long)h->kl_anneal_steps);
+  RVAE_REQUIRE(h->kl_cycles >= 1 || h->kl_anneal != RVAE_KL_CYCLICAL, RVAE_ERR_INVALID, "hparams_check: kl_cycles %lld",
+               (long long)h->kl_cycles);
+  RVAE_REQUIRE(h->kl_cycle_ratio > 0.0 && h->kl_cycle_ratio <= 1.0, RVAE_ERR_INVALID, "hparams_check: kl_cycle_ratio %g",
+               h->kl_cycle_ratio);
+  return RVAE_OK;
+}
+
+int rvae_hparams_eval(rvae_ctx* ctx, const rvae_hparams* hp_dev, const int64_t* k_dev, int n, double* lr_out,
+                      float* beta_out, void* stream) {
+  // arguments first: a malformed call is reported the same way with or without a device
+  RVAE_REQUIRE(hp_dev && k_dev && lr_out && beta_out && n > 0, RVAE_ERR_INVALID,
+               "hparams_eval: null buffer or n %d (need n > 0)", n);
+  CTX_OR_FAIL(ctx);
+  return launch_hparams_eval(&ctx->c, hp_dev, k_dev, n, lr_out, beta_out, S_(stream));
 }
 
 const float* rvae_plan_mu(const rvae_plan* plan) { return plan ? plan->mu : nullptr; }

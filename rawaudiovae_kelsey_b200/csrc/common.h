@@ -7,6 +7,7 @@
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
+#include "../../include/rvae_b200.h"
 #include "gemm.cuh"
 
 namespace rvae {
@@ -187,13 +188,22 @@ int launch_lerp_reparam(Ctx* ctx, const float* mu_a, const float* lv_a, const fl
                         cudaStream_t stream);
 int launch_loss_finalize(Ctx* ctx, double* acc, int64_t B, int S, int L, float beta, float* loss_out, int ring_size,
                          float* step, cudaStream_t stream);
+// The hyper-parameters of an Adam launch: the device record `dev` (read when the kernel runs), or the record `val`
+// passed by value when dev == nullptr
+struct HpArg {
+  const rvae_hparams* dev;
+  rvae_hparams val;
+};
+HpArg hp_value(double lr, double beta1, double beta2, double eps, double weight_decay);   // a constant record
+inline HpArg hp_device(const rvae_hparams* dev) { HpArg a = hp_value(0.0, 0.0, 0.0, 0.0, 0.0); a.dev = dev; return a; }
 int launch_adam(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, double lr, double beta1, double beta2,
                 double eps, double weight_decay, float grad_scale, const float* step, __nv_bfloat16* shadow_hi,
                 __nv_bfloat16* shadow_lo, int zero_grads, cudaStream_t stream);
-int launch_adam2(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, int64_t off_b, int64_t n_b, double lr,
-                 double beta1, double beta2, double eps, double weight_decay, float grad_scale, float* step, int step_bias,
-                 unsigned int* ticket, __nv_bfloat16* shadow_hi, __nv_bfloat16* shadow_lo, int zero_grads,
-                 cudaStream_t stream);
+int launch_adam2(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, int64_t off_b, int64_t n_b,
+                 const HpArg& hp, float grad_scale, float* step, int step_bias, unsigned int* ticket,
+                 __nv_bfloat16* shadow_hi, __nv_bfloat16* shadow_lo, int zero_grads, cudaStream_t stream);
+int launch_hparams_eval(Ctx* ctx, const rvae_hparams* hp, const int64_t* k, int n, double* lr_out, float* beta_out,
+                        cudaStream_t stream);
 int launch_step_inc(Ctx* ctx, float* step, cudaStream_t stream);
 // TensorBoard parameter histograms (rvae_param_histogram): record layout and size in include/rvae_b200.h
 size_t param_histogram_bytes(int n_segs, int n_edges);
@@ -229,6 +239,7 @@ struct P2PSegs {   // a bucket = concatenation of up to three segments of the fl
 };
 int launch_allreduce_p2p(Ctx* ctx, const P2PArgs& a, const P2PSegs& sg, int bucket, int ctas, cudaStream_t stream);
 // loss = acc[0]*inv_rec + kl_scale*acc[1] -> loss_out[step mod ring_size]; acc cleared; *step += 1
+//   hp != nullptr: kl_scale = -0.5 * beta(k) / kl_bl instead, beta(k) from the record at k = *step
 struct LossFinalize {
   double* acc;
   double inv_rec, kl_scale;
@@ -236,12 +247,23 @@ struct LossFinalize {
   int ring_size;
   float* step;
   int inc_step;  // 0: the step counter is advanced elsewhere (by the last Adam launch of the step)
+  const rvae_hparams* hp;
+  double kl_bl;  // B * L of the loss normalisation
 };
+// KL gradient scale of the latent backward: c, or (float)(beta(k) / bl) with beta(k) from the record at k = *step
+struct KlGrad {
+  const rvae_hparams* hp;
+  const float* step;
+  double bl;
+  float c;
+  int early;  // the record and the counter are final before the kernel starts: read them before griddepcontrol.wait
+};
+inline KlGrad kl_grad_value(float c) { return KlGrad{nullptr, nullptr, 0.0, c, 0}; }
 LossFinalize make_loss_finalize(double* acc, int64_t B, int S, int L, float beta, float* loss_out, int ring_size,
                                 float* step);
 int launch_loss_finalize_prepared(Ctx* ctx, const LossFinalize& f, cudaStream_t stream);
 int launch_latent_bwd(Ctx* ctx, float* dz, const float* eps, const float* lv, const float* mu, const float* g_mu_ext,
-                      const float* g_lv_ext, float kl_grad_scale, int64_t M, int L, __nv_bfloat16* dml_hi,
+                      const float* g_lv_ext, const KlGrad& kl, int64_t M, int L, __nv_bfloat16* dml_hi,
                       __nv_bfloat16* dml_lo, float* bias_grad, int clear_dz, const LossFinalize* fin,
                       cudaStream_t stream);
 

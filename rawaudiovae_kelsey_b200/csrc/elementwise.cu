@@ -569,6 +569,87 @@ __global__ void loss_fwd_kernel(const float* __restrict__ xhat, const float* __r
   }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Scheduled hyper-parameters (rvae_hparams, include/rvae_b200.h): lr(k) and beta(k) at step index k. Every operation
+// is an explicitly rounded fp64 intrinsic (no FMA contraction) in the order the header writes it, so schedule.py's
+// host mirror, which repeats them one by one, gets the same doubles.
+// ------------------------------------------------------------------------------------------------
+// cos(pi u) for u in [0, 1]: Taylor series to x^22 at x = pi * min(u, 1 - u) <= pi / 2 (truncation < 1e-19),
+// negated for u > 0.5 - a fixed polynomial instead of the libm cos, whose last bit differs between device and host
+__device__ __forceinline__ double cos_pi_unit(double u) {
+  const double c[12] = {1.0, -0.5, 0.041666666666666664, -0.001388888888888889, 2.48015873015873e-05,
+                        -2.755731922398589e-07, 2.08767569878681e-09, -1.1470745597729725e-11, 4.779477332387385e-14,
+                        -1.5619206968586225e-16, 4.110317623312165e-19, -8.896791392450574e-22};
+  const bool flip = u > 0.5;
+  if (flip) u = __dadd_rn(1.0, -u);
+  const double x = __dmul_rn(3.141592653589793, u);
+  const double x2 = __dmul_rn(x, x);
+  double r = c[11];
+#pragma unroll
+  for (int i = 10; i >= 0; --i) r = __dadd_rn(__dmul_rn(r, x2), c[i]);
+  return flip ? -r : r;
+}
+
+__device__ __forceinline__ void hparams_eval(const rvae_hparams& h, double k, double* lr_out, float* beta_out) {
+  const double lr = h.lr;
+  const double W = static_cast<double>(h.warmup_steps);
+  double a;
+  if (k < W) {
+    a = __ddiv_rn(__dmul_rn(lr, __dadd_rn(k, 1.0)), W);
+  } else if (h.lr_schedule == RVAE_LR_CONSTANT) {
+    a = lr;
+  } else {
+    const int64_t d = h.total_steps - h.warmup_steps;
+    const double D = static_cast<double>(d > 1 ? d : 1);
+    const double u = __ddiv_rn(fmin(__dadd_rn(k, -W), D), D);
+    const double span = __dadd_rn(lr, -h.lr_min);
+    if (h.lr_schedule == RVAE_LR_LINEAR)
+      a = __dadd_rn(h.lr_min, __dmul_rn(span, __dadd_rn(1.0, -u)));
+    else
+      a = __dadd_rn(h.lr_min, __dmul_rn(__dmul_rn(span, 0.5), __dadd_rn(1.0, cos_pi_unit(u))));
+  }
+  double b = h.kl_beta;
+  if (h.kl_anneal != RVAE_KL_CONSTANT) {
+    double f;
+    if (h.kl_anneal == RVAE_KL_LINEAR) {
+      f = fmin(1.0, __ddiv_rn(k, static_cast<double>(h.kl_anneal_steps)));
+    } else {
+      const int64_t C = (h.total_steps + h.kl_cycles - 1) / h.kl_cycles;
+      const double tau = __ddiv_rn(static_cast<double>(static_cast<int64_t>(k) % C), static_cast<double>(C));
+      f = fmin(1.0, __ddiv_rn(tau, h.kl_cycle_ratio));
+    }
+    b = __dadd_rn(h.kl_beta_start, __dmul_rn(__dadd_rn(h.kl_beta, -h.kl_beta_start), f));
+  }
+  *lr_out = a;
+  *beta_out = static_cast<float>(b);
+}
+
+__global__ void hparams_eval_kernel(const rvae_hparams* __restrict__ hp, const int64_t* __restrict__ k, int n,
+                                    double* __restrict__ lr_out, float* __restrict__ beta_out) {
+  ptx::pdl_launch_dependents();
+  ptx::pdl_wait();
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) hparams_eval(*hp, static_cast<double>(k[i]), lr_out + i, beta_out + i);
+}
+
+int launch_hparams_eval(Ctx* ctx, const rvae_hparams* hp, const int64_t* k, int n, double* lr_out, float* beta_out,
+                        cudaStream_t stream) {
+  RVAE_REQUIRE(hp && k && lr_out && beta_out && n > 0, RVAE_ERR_INVALID, "hparams_eval: null buffer or n %d", n);
+  RVAE_CUDA(launch_kernel(ctx, hparams_eval_kernel, dim3((n + 127) / 128), dim3(128), (size_t)0, stream, hp, k, n,
+                          lr_out, beta_out));
+  RVAE_LAUNCH_CHECK(ctx);
+  return RVAE_OK;
+}
+
+HpArg hp_value(double lr, double beta1, double beta2, double eps, double weight_decay) {
+  HpArg a;
+  memset(&a, 0, sizeof(a));
+  a.val.lr = lr; a.val.beta1 = beta1; a.val.beta2 = beta2; a.val.eps = eps; a.val.weight_decay = weight_decay;
+  a.val.kl_cycle_ratio = 1.0; a.val.kl_anneal_steps = 1; a.val.kl_cycles = 1;
+  a.val.lr_schedule = RVAE_LR_CONSTANT; a.val.kl_anneal = RVAE_KL_CONSTANT;
+  return a;
+}
+
 __device__ __forceinline__ void loss_finalize_body(double* acc, double inv_rec, double kl_scale, float* loss_out,
                                                    int ring_size, float* step, int inc_step) {
   const double loss = acc[0] * inv_rec + kl_scale * acc[1];
@@ -581,13 +662,20 @@ __device__ __forceinline__ void loss_finalize_body(double* acc, double inv_rec, 
   if (step && inc_step) *step += 1.0f;
 }
 
-__global__ void loss_finalize_kernel(double* __restrict__ acc, double inv_rec, double kl_scale,
-                                     float* __restrict__ loss_out, int ring_size, float* __restrict__ step,
-                                     int inc_step) {
+// kl_scale of a finalisation: the host's value, or -0.5 * beta(k) / (B L) from the record at k = *step
+__device__ __forceinline__ double loss_kl_scale(const LossFinalize& f) {
+  if (f.hp == nullptr) return f.kl_scale;
+  double lr;
+  float beta;
+  hparams_eval(*f.hp, static_cast<double>(*f.step), &lr, &beta);
+  return __ddiv_rn(__dmul_rn(-0.5, static_cast<double>(beta)), f.kl_bl);
+}
+
+__global__ void loss_finalize_kernel(LossFinalize f) {
   ptx::pdl_launch_dependents();
   ptx::pdl_wait();
   if (threadIdx.x == 0 && blockIdx.x == 0)
-    loss_finalize_body(acc, inv_rec, kl_scale, loss_out, ring_size, step, inc_step);
+    loss_finalize_body(f.acc, f.inv_rec, loss_kl_scale(f), f.loss_out, f.ring_size, f.step, f.inc_step);
 }
 
 LossFinalize make_loss_finalize(double* acc, int64_t B, int S, int L, float beta, float* loss_out, int ring_size,
@@ -600,6 +688,8 @@ LossFinalize make_loss_finalize(double* acc, int64_t B, int S, int L, float beta
   f.ring_size = ring_size;
   f.step = step;
   f.inc_step = 1;
+  f.hp = nullptr;
+  f.kl_bl = static_cast<double>(B) * L;
   return f;
 }
 
@@ -611,8 +701,8 @@ int launch_loss_finalize(Ctx* ctx, double* acc, int64_t B, int S, int L, float b
 
 int launch_loss_finalize_prepared(Ctx* ctx, const LossFinalize& f, cudaStream_t stream) {
   RVAE_REQUIRE(f.acc, RVAE_ERR_INVALID, "loss_finalize: null accumulator");
-  RVAE_CUDA(launch_kernel(ctx, loss_finalize_kernel, dim3(1), dim3(32), (size_t)0, stream, f.acc, f.inv_rec, f.kl_scale,
-                          f.loss_out, f.ring_size, f.step, f.inc_step));
+  RVAE_REQUIRE(f.hp == nullptr || f.step != nullptr, RVAE_ERR_INVALID, "loss_finalize: a record needs the step counter");
+  RVAE_CUDA(launch_kernel(ctx, loss_finalize_kernel, dim3(1), dim3(32), (size_t)0, stream, f));
   RVAE_LAUNCH_CHECK(ctx);
   return RVAE_OK;
 }
@@ -964,35 +1054,45 @@ int launch_lerp_reparam(Ctx* ctx, const float* mu_a, const float* lv_a, const fl
 // multiples of 4 then): the per-bucket launches of a training step (W3|W4, W2, W1 + bias block).
 // (4 blocks of 256 threads per SM need <= 64 registers: one register more costs a quarter of the occupancy and 30 % of
 // the bandwidth - measured when the hyper-parameters became doubles)
+// The hyper-parameters come from a record (HpArg: the device record of a scheduled step, read here when the kernel
+// runs, or a constant record passed by value); lr is the schedule's lr(k) at k = t - 1.
 template <int U>
 __global__ void __launch_bounds__(256, U == 4 ? 2 : 4) adam_kernel(float* __restrict__ p, float* __restrict__ g, float* __restrict__ m,
-                            float* __restrict__ v, int64_t n, int64_t off_b, int64_t n_b, double lr, double beta1_d,
-                            double beta2_d, double eps_d, double weight_decay_d, float grad_scale, float* step,
-                            int step_bias, unsigned int* ticket, __nv_bfloat16* __restrict__ sh_hi,
-                            __nv_bfloat16* __restrict__ sh_lo, int zero_grads, AuxTrace tr) {
+                            float* __restrict__ v, int64_t n, int64_t off_b, int64_t n_b, const __grid_constant__ HpArg hp,
+                            float grad_scale, float* step, int step_bias, unsigned int* ticket,
+                            __nv_bfloat16* __restrict__ sh_hi, __nv_bfloat16* __restrict__ sh_lo, int zero_grads,
+                            AuxTrace tr) {
   ptx::pdl_launch_dependents();
-  ptx::pdl_wait();
+  ptx::pdl_wait();   // (rvae_adam_step follows the launch that advances the step counter)
   aux_begin(tr, 4);
-  // The hyper-parameters arrive as doubles - what torch.optim.Adam holds (python floats) - and every scalar the
-  // update uses is derived from them exactly as torch derives it: 1 - beta in DOUBLE, then rounded to fp32 (the weight
-  // of lerp_ / the value of addcmul_; (1.f - 0.999f) would be off by 1.3e-5 relative), beta2 and eps rounded to fp32.
-  const float omb1 = static_cast<float>(1.0 - beta1_d), beta2 = static_cast<float>(beta2_d);
-  const float omb2 = static_cast<float>(1.0 - beta2_d), eps = static_cast<float>(eps_d);
-  const float weight_decay = static_cast<float>(weight_decay_d);
-  // bias corrections in double, as torch computes them on the host (python floats); one thread per block does the
-  // fp64 pow()s and broadcasts the two scalars
-  __shared__ float s_consts[2];
+  // The hyper-parameters are doubles - what torch.optim.Adam holds (python floats) - and every scalar the update uses
+  // is derived from them exactly as torch derives it: 1 - beta in DOUBLE, then rounded to fp32 (the weight of lerp_ /
+  // the value of addcmul_; (1.f - 0.999f) would be off by 1.3e-5 relative), beta2 and eps rounded to fp32. Bias
+  // corrections in double, as torch computes them on the host (python floats). One thread per block reads the record,
+  // does the fp64 pow()s and broadcasts the seven scalars.
+  __shared__ float s_consts[7];
   if (threadIdx.x == 0) {
+    const rvae_hparams& h = hp.dev != nullptr ? *hp.dev : hp.val;
     // t = *step + step_bias: step_bias = 1 when the step counter is advanced only at the end of the step (ticket)
     const double t = static_cast<double>(*reinterpret_cast<volatile float*>(step)) + step_bias;
-    const double bc1 = 1.0 - pow(beta1_d, t);
-    const double bc2 = 1.0 - pow(beta2_d, t);
+    double lr;
+    float beta_unused;
+    hparams_eval(h, t - 1.0, &lr, &beta_unused);
+    const double bc1 = 1.0 - pow(h.beta1, t);
+    const double bc2 = 1.0 - pow(h.beta2, t);
     s_consts[0] = static_cast<float>(lr / bc1);
     s_consts[1] = static_cast<float>(sqrt(bc2));
+    s_consts[2] = static_cast<float>(1.0 - h.beta1);
+    s_consts[3] = static_cast<float>(h.beta2);
+    s_consts[4] = static_cast<float>(1.0 - h.beta2);
+    s_consts[5] = static_cast<float>(h.eps);
+    s_consts[6] = static_cast<float>(h.weight_decay);
   }
   __syncthreads();
   const float step_size = s_consts[0];
   const float sqrt_bc2 = s_consts[1];
+  const float omb1 = s_consts[2], beta2 = s_consts[3], omb2 = s_consts[4], eps = s_consts[5];
+  const float weight_decay = s_consts[6];
   const int64_t nvec = n >> 2;
   const int64_t nvec_all = nvec + (n_b >> 2);
   const int64_t shift_b = (off_b >> 2) - nvec;
@@ -1084,14 +1184,13 @@ __global__ void __launch_bounds__(256, U == 4 ? 2 : 4) adam_kernel(float* __rest
 int launch_adam(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, double lr, double beta1, double beta2,
                 double eps, double weight_decay, float grad_scale, const float* step, __nv_bfloat16* shadow_hi,
                 __nv_bfloat16* shadow_lo, int zero_grads, cudaStream_t stream) {
-  return launch_adam2(ctx, p, g, m, v, n, 0, 0, lr, beta1, beta2, eps, weight_decay, grad_scale,
+  return launch_adam2(ctx, p, g, m, v, n, 0, 0, hp_value(lr, beta1, beta2, eps, weight_decay), grad_scale,
                       const_cast<float*>(step), 0, nullptr, shadow_hi, shadow_lo, zero_grads, stream);
 }
 
-int launch_adam2(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, int64_t off_b, int64_t n_b, double lr,
-                 double beta1, double beta2, double eps, double weight_decay, float grad_scale, float* step, int step_bias,
-                 unsigned int* ticket, __nv_bfloat16* shadow_hi, __nv_bfloat16* shadow_lo, int zero_grads,
-                 cudaStream_t stream) {
+int launch_adam2(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, int64_t off_b, int64_t n_b,
+                 const HpArg& hp, float grad_scale, float* step, int step_bias, unsigned int* ticket,
+                 __nv_bfloat16* shadow_hi, __nv_bfloat16* shadow_lo, int zero_grads, cudaStream_t stream) {
   RVAE_REQUIRE(p && g && m && v && step, RVAE_ERR_INVALID, "adam: null buffer");
   RVAE_REQUIRE(n_b == 0 || ((n & 3) == 0 && (off_b & 3) == 0 && (n_b & 3) == 0 && off_b >= n), RVAE_ERR_INVALID,
                "adam: segments must be multiples of 4 elements");
@@ -1111,8 +1210,8 @@ int launch_adam2(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, in
   if (ctx->aux_grid_cap > 0 && (int)grid.x > ctx->aux_grid_cap) grid.x = ctx->aux_grid_cap;
   auto kern = unroll == 1 ? adam_kernel<1> : (unroll == 4 ? adam_kernel<4> : adam_kernel<2>);
   RVAE_CUDA(launch_kernel(ctx, kern, grid, dim3(threads), (size_t)0,
-                          stream, p, g, m, v, n, off_b, n_b, lr, beta1, beta2, eps, weight_decay, grad_scale, step,
-                          step_bias, ticket, shadow_hi, shadow_lo, zero_grads, next_aux(ctx, 4)));
+                          stream, p, g, m, v, n, off_b, n_b, hp, grad_scale, step, step_bias, ticket, shadow_hi,
+                          shadow_lo, zero_grads, next_aux(ctx, 4)));
   RVAE_LAUNCH_CHECK(ctx);
   return RVAE_OK;
 }
@@ -1127,17 +1226,34 @@ int launch_adam2(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, in
 // strided set of rows: float4 loads, 8-byte bf16 stores, column sums in registers -> smem -> one atomic per column
 // and block.
 // ------------------------------------------------------------------------------------------------
+__device__ __forceinline__ float latent_kl_c(const KlGrad& kl) {
+  double lr;
+  float beta;
+  hparams_eval(*kl.hp, static_cast<double>(*kl.step), &lr, &beta);
+  return static_cast<float>(__ddiv_rn(static_cast<double>(beta), kl.bl));
+}
+
 __global__ void latent_bwd_kernel(float* __restrict__ dz, const float* __restrict__ eps, const float* __restrict__ lv,
                                   const float* __restrict__ mu, const float* __restrict__ g_mu_ext,
-                                  const float* __restrict__ g_lv_ext, float c, int64_t M, int L,
+                                  const float* __restrict__ g_lv_ext, KlGrad kl, int64_t M, int L,
                                   __nv_bfloat16* __restrict__ dml_hi, __nv_bfloat16* __restrict__ dml_lo,
                                   float* __restrict__ bias_grad, int clear_dz, LossFinalize fin, AuxTrace tr) {
   ptx::pdl_launch_dependents();
+  // c = (float)(beta(k) / (B L)), as the host rounds it for a kl_beta argument. kl.early: evaluated before
+  // griddepcontrol.wait, overlapping the previous kernel (see rvae_plan_train_step_hp for why that is safe)
+  __shared__ float s_c;
+  if (kl.hp != nullptr && kl.early && threadIdx.x == 0) s_c = latent_kl_c(kl);
   ptx::pdl_wait();
   aux_begin(tr, 3);
   // the deferred loss finalisation of this step rides along (the forward that filled the sums is long complete)
   if (fin.acc != nullptr && blockIdx.x == 0 && threadIdx.x == 0)
-    loss_finalize_body(fin.acc, fin.inv_rec, fin.kl_scale, fin.loss_out, fin.ring_size, fin.step, fin.inc_step);
+    loss_finalize_body(fin.acc, fin.inv_rec, loss_kl_scale(fin), fin.loss_out, fin.ring_size, fin.step, fin.inc_step);
+  float c = kl.c;
+  if (kl.hp != nullptr) {
+    if (!kl.early && threadIdx.x == 0) s_c = latent_kl_c(kl);
+    __syncthreads();
+    c = s_c;
+  }
   extern __shared__ float s_sum[];  // [rows_per_pass][2L]
   const int q = L >> 2;                    // float4 groups per row
   const int rpp = blockDim.x / q;          // rows per pass
@@ -1225,9 +1341,12 @@ __global__ void latent_bwd_kernel(float* __restrict__ dz, const float* __restric
 }
 
 int launch_latent_bwd(Ctx* ctx, float* dz, const float* eps, const float* lv, const float* mu, const float* g_mu_ext,
-                      const float* g_lv_ext, float kl_grad_scale, int64_t M, int L, __nv_bfloat16* dml_hi,
+                      const float* g_lv_ext, const KlGrad& kl, int64_t M, int L, __nv_bfloat16* dml_hi,
                       __nv_bfloat16* dml_lo, float* bias_grad, int clear_dz, const LossFinalize* fin,
                       cudaStream_t stream) {
+  // every block reads k = *step: the step counter must not advance inside this launch
+  RVAE_REQUIRE(kl.hp == nullptr || (kl.step != nullptr && (fin == nullptr || !fin->inc_step)), RVAE_ERR_INVALID,
+               "latent_bwd: a record needs a step counter that stays put during the launch");
   RVAE_REQUIRE(dz && eps && lv && dml_hi, RVAE_ERR_INVALID, "latent_bwd: null buffer");
   RVAE_REQUIRE((g_mu_ext != nullptr) == (g_lv_ext != nullptr), RVAE_ERR_INVALID,
                "latent_bwd: external gradients come in pairs");
@@ -1247,7 +1366,7 @@ int launch_latent_bwd(Ctx* ctx, float* dz, const float* eps, const float* lv, co
   memset(&f, 0, sizeof(f));
   if (fin) f = *fin;
   RVAE_CUDA(launch_kernel(ctx, latent_bwd_kernel, dim3(grid), dim3(threads), smem, stream, dz, eps, lv, mu, g_mu_ext,
-                          g_lv_ext, kl_grad_scale, M, L, dml_hi, dml_lo, bias_grad, clear_dz, f, next_aux(ctx, 3)));
+                          g_lv_ext, kl, M, L, dml_hi, dml_lo, bias_grad, clear_dz, f, next_aux(ctx, 3)));
   RVAE_LAUNCH_CHECK(ctx);
   return RVAE_OK;
 }

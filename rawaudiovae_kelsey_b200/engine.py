@@ -299,6 +299,14 @@ class Plan:
                                             loss_out.data_ptr() if loss_out is not None else None, ring_size,
                                             self._stream()))
 
+    def train_step_hp(self, hp: torch.Tensor, loss_out: Optional[torch.Tensor] = None, ring_size: int = 1,
+                      zero_grads: bool = True) -> None:
+        """train_step with every hyper-parameter read from the device record `hp` (schedule.Schedule) when the
+        kernels run: a captured graph of this call follows the schedule and any rewrite of the record."""
+        check(self.lib.rvae_plan_train_step_hp(self.handle, hp.data_ptr(), int(zero_grads),
+                                               loss_out.data_ptr() if loss_out is not None else None, ring_size,
+                                               self._stream()))
+
     def encode(self) -> None:
         check(self.lib.rvae_plan_encode(self.handle, self._stream()))
 

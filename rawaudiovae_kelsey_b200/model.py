@@ -22,6 +22,7 @@ import torch
 import torch.nn as nn
 
 from . import _lib, engine, ops
+from .schedule import DeviceRecord, Schedule
 
 _PRIVATE = ("_flat", "_plans", "_eps_counter")
 
@@ -380,10 +381,14 @@ class _StepBase:
     input signature (after `graph_warmup` eager steps) and replayed, so the host cost of a step drops from ~20
     kernel launches to one graph launch. Replays stay correct because everything that changes from step to step is
     read from device memory: frame indices from a static index buffer, the Philox offset and the loss-ring slot
-    from the optimizer's step counter."""
+    from the optimizer's step counter. The hyper-parameters too: the kernels read them from a device record
+    (schedule.DeviceRecord) that each call rewrites before the step when optimizer.param_groups[0], kl_beta or
+    `schedule` changed, so replays follow the schedule, a torch LR scheduler and any change made by hand."""
 
-    def __init__(self, model, optimizer, kl_beta, ring, graph, graph_warmup=1):
+    def __init__(self, model, optimizer, kl_beta, ring, graph, graph_warmup=1, schedule=None):
         self.model, self.optimizer, self.kl_beta = model, optimizer, float(kl_beta)
+        self.schedule = schedule if schedule is not None else Schedule()
+        self._record = None
         self.ring_size = int(ring)
         self.ring = None
         self.i = None            # host mirror of the device step counter (slot = i % ring_size)
@@ -410,6 +415,14 @@ class _StepBase:
         if hasattr(self.optimizer, "bind_flat"):
             self.optimizer.bind_flat(flat)
         return flat
+
+    def _hparams(self, device):
+        """Bring the device record up to date (outside any capture: a graph must hold its address, not a copy)."""
+        if self._record is None:
+            self._record = DeviceRecord(device)
+        g = self.optimizer.param_groups[0]
+        return self._record.update(self.schedule, g["lr"], g["betas"], g["eps"], g.get("weight_decay", 0.0),
+                                   self.kl_beta)
 
     def _slot(self):
         return self.ring[self.i % self.ring_size]
@@ -468,6 +481,7 @@ class _StepBase:
         """One step on `data`. `next_data` (optional FrameBatch): the batch of the NEXT call - it is gathered, and its
         noise drawn, on a background stream while this step's GEMMs run (pass the same object as `data` next time)."""
         flat = self._prepare()
+        self._hparams(flat.device)
         model = self.model
         graphable = self.graph and eps is None and model.eps_source == "philox"
         plan = self._take_prefetched(data) if eps is None else None
@@ -621,18 +635,18 @@ class FusedTrainStep(_StepBase):
     keep_grads=False (default): the Adam kernel clears the flat gradient buffer after consuming it, exactly what the
     reference's optimizer.zero_grad() does at the top of the next iteration; keep_grads=True leaves the step's
     gradients in model._flat.grads for inspection (costs memsets per step).
-    graph=True: replay a captured CUDA graph of the step (see _StepBase)."""
+    graph=True: replay a captured CUDA graph of the step (see _StepBase).
+    schedule (schedule.Schedule, default constant): learning rate and KL weight per step, with
+    optimizer.param_groups[0]['lr'] and kl_beta as the peak values."""
 
     def __init__(self, model: VAE, optimizer, kl_beta: float, ring: int = 64, keep_grads: bool = False,
-                 graph: bool = False):
-        super().__init__(model, optimizer, kl_beta, ring, graph)
+                 graph: bool = False, schedule: Optional[Schedule] = None):
+        super().__init__(model, optimizer, kl_beta, ring, graph, schedule=schedule)
         self.keep_grads = keep_grads
 
     def _enqueue(self, plan):
-        g = self.optimizer.param_groups[0]
-        b1, b2 = g["betas"]
-        plan.train_step(self.kl_beta, g["lr"], b1, b2, g["eps"], g.get("weight_decay", 0.0), loss_out=self.ring,
-                        ring_size=self.ring_size, zero_grads=not self.keep_grads)
+        plan.train_step_hp(self._record.tensor, loss_out=self.ring, ring_size=self.ring_size,
+                           zero_grads=not self.keep_grads)
 
     def __call__(self, data, eps: Optional[torch.Tensor] = None, next_data=None) -> torch.Tensor:
         return self._run(data, eps, next_data)

@@ -231,6 +231,22 @@ def frame_loss(xhat: torch.Tensor, mu: torch.Tensor, logvar: torch.Tensor, audio
     return rec, kl
 
 
+def hparams_eval(record: torch.Tensor, k: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Evaluate the schedule of a device rvae_hparams record (schedule.DeviceRecord.tensor) at the step indices k
+    (int64) with the device function of the training kernels. Returns (lr float64, beta float32), shaped like k."""
+    lib = _lib.load()
+    if record.dtype != torch.uint8 or record.numel() != C.sizeof(_lib.Hparams) or not record.is_cuda:
+        raise _lib.RvaeError("record must be a CUDA uint8 tensor of sizeof(rvae_hparams) bytes")
+    if k.dtype != torch.int64 or k.device != record.device:
+        raise _lib.RvaeError("k must be an int64 tensor on the record's device")
+    kc = k.contiguous()
+    lr = torch.empty(k.shape, dtype=torch.float64, device=k.device)
+    beta = torch.empty(k.shape, dtype=torch.float32, device=k.device)
+    check(lib.rvae_hparams_eval(ctx(k.device), record.data_ptr(), kc.data_ptr(), kc.numel(), lr.data_ptr(),
+                                beta.data_ptr(), _stream()))
+    return lr, beta
+
+
 def loss_bwd(xhat, x, mu, logvar, beta: float, grad_out: Optional[torch.Tensor]):
     lib = _lib.load()
     B, S = xhat.shape

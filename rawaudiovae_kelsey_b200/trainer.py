@@ -30,6 +30,7 @@ from .dataset import AudioDataset, IterableAudioDataset, ToTensor
 from .inference import evaluate_audio
 from .model import VAE, FusedTrainStep
 from .optim import Adam
+from .schedule import Schedule
 from .stats import ParamHistogramLogger
 from .testaudio import init_test_audio
 
@@ -131,6 +132,46 @@ def _test_loss_enabled(config) -> bool:
         raise ValueError("[training] test_loss = True needs [dataset] generate_test = True: the test set is only "
                          "loaded for it")
     return on
+
+
+def _schedule(config, total_steps: int) -> Schedule:
+    """The run's learning-rate and KL-weight schedule over total_steps steps: [training] lr_schedule, lr_warmup_steps,
+    lr_min and [VAE] kl_anneal, kl_beta_start, kl_anneal_steps (default: the whole run), kl_cycles, kl_cycle_ratio.
+    Missing keys give the constant schedule of the reference; bad values raise ValueError."""
+    tr, vae = config['training'], config['VAE']
+    return Schedule(lr_schedule=tr.get('lr_schedule', fallback='constant'),
+                    warmup_steps=tr.getint('lr_warmup_steps', fallback=0),
+                    total_steps=total_steps,
+                    lr_min=tr.getfloat('lr_min', fallback=0.0),
+                    kl_anneal=vae.get('kl_anneal', fallback='constant'),
+                    kl_beta_start=vae.getfloat('kl_beta_start', fallback=0.0),
+                    kl_anneal_steps=vae.getint('kl_anneal_steps', fallback=max(total_steps, 1)),
+                    kl_cycles=vae.getint('kl_cycles', fallback=1),
+                    kl_cycle_ratio=vae.getfloat('kl_cycle_ratio', fallback=0.5))
+
+
+def _epoch_steps(n_frames: int, batch_size: int, world: int = 1) -> int:
+    """Training steps per epoch of GpuFrameLoader (drop_last=False): a last global batch with fewer frames than ranks
+    is skipped."""
+    n = -(-n_frames // batch_size)
+    return n - 1 if n > 0 and n_frames - (n - 1) * batch_size < world else n
+
+
+def _epoch_trainer_steps(config, n_frames: int, world: int = 1) -> int:
+    """Steps of a run_epoch_trainer run over a training set of n_frames frames: epochs x steps per epoch."""
+    return config['training'].getint('epochs') * _epoch_steps(n_frames, config['training'].getint('batch_size'), world)
+
+
+def _stream_trainer_steps(config) -> int:
+    """Steps of a run_stream_trainer run: total_num_batches (train_iterable.py:74)."""
+    return int(config['training'].getint('total_num_frames') / config['training'].getint('batch_size'))
+
+
+def _log_hparams(writer, schedule, optimizer, kl_beta, batch_id):
+    """The learning rate the step at batch_id applies and, when it is annealed, its KL weight."""
+    writer.add_scalar('Learning Rate', schedule.lr_at(batch_id, optimizer.param_groups[0]['lr']), batch_id)
+    if schedule.kl_anneal != 'constant':
+        writer.add_scalar('KL Beta', schedule.beta_at(batch_id, kl_beta), batch_id)
 
 
 def _evaluate_test(model, test_dataset, kl_beta, batch_size, writer, step_id):
@@ -240,6 +281,7 @@ def run_epoch_trainer(argv=None):
                                     hop_size=hop_length, transform=ToTensor())
     loader = training_dataset.gpu_loader(batch_size, shuffle=True, device=device)
     loader.rank, loader.world = rank, world
+    schedule = _schedule(config, _epoch_trainer_steps(config, len(training_dataset), world))
 
     writer = _NullWriter()
     if rank == 0:
@@ -261,9 +303,9 @@ def run_epoch_trainer(argv=None):
     use_graph = config['training'].getboolean('cuda_graph', fallback=True)
     ring = max(64, log_interval)
     if world > 1:
-        step = rdist.DataParallelTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph)
+        step = rdist.DataParallelTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph, schedule=schedule)
     else:
-        step = FusedTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph)
+        step = FusedTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph, schedule=schedule)
 
     # parameter histograms on the GPU (rank 0 only): one launch + one small asynchronous copy per set
     hist = ParamHistogramLogger(model, writer) if rank == 0 else None
@@ -284,7 +326,7 @@ def run_epoch_trainer(argv=None):
                 step.global_batch = min(batch_size, len(training_dataset) - b * batch_size)
             loss = step(data, next_data=nxt)   # the next batch is gathered in the background of this step
             pending.append((batch_id, loss))
-            writer.add_scalar('Learning Rate', optimizer.param_groups[0]['lr'], batch_id)
+            _log_hparams(writer, schedule, optimizer, kl_beta, batch_id)
             batch_id += 1
             if len(pending) >= log_interval:
                 train_loss += _flush_losses(writer, pending, world=world)
@@ -379,7 +421,8 @@ def run_stream_trainer(argv=None):
     learning_rate = config['training'].getfloat('learning_rate')
     batch_size = config['training'].getint('batch_size')
     checkpoint_interval = config['training'].getint('checkpoint_interval')
-    total_num_batches = int(total_num_frames / batch_size)                      # train_iterable.py:74
+    total_num_batches = _stream_trainer_steps(config)
+    schedule = _schedule(config, total_num_batches)
     log_interval = config['training'].getint('log_interval', fallback=64)
     histogram_interval = config['training'].getint('histogram_interval', fallback=checkpoint_interval)
     latent_dim = config['VAE'].getint('latent_dim')
@@ -430,9 +473,9 @@ def run_stream_trainer(argv=None):
         ring = max(64, log_interval)
         if world > 1:
             step = rdist.DataParallelTrainStep(model, optimizer, kl_beta, global_batch=batch_size, ring=ring,
-                                               graph=use_graph)
+                                               graph=use_graph, schedule=schedule)
         else:
-            step = FusedTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph)
+            step = FusedTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph, schedule=schedule)
 
         hist = ParamHistogramLogger(model, writer) if rank == 0 and histogram_interval > 0 else None
 
@@ -447,7 +490,7 @@ def run_stream_trainer(argv=None):
         for data, nxt in _with_next(islice(stream, total_num_batches)):
             loss = step(data, next_data=nxt)   # the next batch is gathered in the background of this step
             pending.append((batch_id, loss))
-            writer.add_scalar('Learning Rate', optimizer.param_groups[0]['lr'], batch_id)
+            _log_hparams(writer, schedule, optimizer, kl_beta, batch_id)
             at_checkpoint = batch_id % checkpoint_interval == 0 and batch_id != 0
             if len(pending) >= log_interval or at_checkpoint:
                 train_loss += _flush_losses(writer, pending, fmt if rank == 0 else None, world=world)
