@@ -479,6 +479,22 @@ int rvae_hparams_check(const rvae_hparams* host);
  * (before the plan is used), 2 for the experiments-only fused latent epilogue, which takes its KL scale from the host. */
 int rvae_plan_train_step_hp(rvae_plan* plan, const rvae_hparams* hp_dev, int zero_grads, float* loss_out,
                             int ring_size, void* stream);
+/* Gradient-norm clipping of every later training step of the plan (rvae_plan_train_step, rvae_plan_train_step_hp),
+ * as torch.nn.utils.clip_grad_norm_ with norm type 2 between backward and Adam: norm = sqrt(sum g^2) over all ten
+ * parameters' gradients (after the all-reduce under data parallelism, before weight decay), and Adam consumes
+ * coef * g with coef = min(1, max_norm / (norm + 1e-6)). The sum of squares is fp64 in a fixed order (bitwise
+ * repeatable); coef is rounded to fp32 once. max_norm_dev: a device double, read when the kernels run, so a graph
+ * captured around a step follows any rewrite ordered before its replay; +inf measures without clipping; NULL
+ * switches clipping off (the step then issues exactly the launches it issues without this call). norm_out (may be
+ * NULL): the pre-clip norm of the step lands in norm_out[t mod ring_size], t = the step counter when the step starts.
+ * The gradients a step leaves with zero_grads = 0 are the unclipped ones. A non-finite norm propagates as in torch.
+ * Returns 1 for ring_size < 1 with a non-null norm_out (before the plan is used), 2 for the experiments-only fused
+ * latent epilogue. */
+int rvae_plan_set_grad_clip(rvae_plan* plan, const double* max_norm_dev, float* norm_out, int ring_size);
+/* The global L2 norm of the plan's bound gradient buffer with the kernels of a clipping step -> *norm_out (device
+ * float); not part of any step. Returns 1 for a null norm_out (before the plan is used). */
+int rvae_plan_grad_norm(rvae_plan* plan, float* norm_out, void* stream);
+
 /* Evaluate the record's schedule at the n step indices k_dev[0..n) with the device function the training kernels
  * use: lr_out[i] = lr(k_dev[i]), beta_out[i] = (float)beta(k_dev[i]). Returns 1 for null pointers or n < 1 (before
  * ctx is used). */

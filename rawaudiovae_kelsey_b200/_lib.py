@@ -118,6 +118,8 @@ SIGNATURES = {
     "rvae_plan_adam": (c_int, [P, c_double, c_double, c_double, c_double, c_double, c_float, c_int, P]),
     "rvae_plan_train_step": (c_int, [P, c_float, c_double, c_double, c_double, c_double, c_double, c_int, P, c_int, P]),
     "rvae_plan_train_step_hp": (c_int, [P, P, c_int, P, c_int, P]),
+    "rvae_plan_set_grad_clip": (c_int, [P, P, P, c_int]),
+    "rvae_plan_grad_norm": (c_int, [P, P, P]),
     "rvae_hparams_check": (c_int, [C.POINTER(Hparams)]),
     "rvae_hparams_eval": (c_int, [P, P, P, c_int, P, P, P]),
     "rvae_plan_mu": (P, [P]),

@@ -551,6 +551,10 @@ struct Planes {
   __nv_bfloat16* lo = nullptr;
 };
 
+// gradient-norm launches: W4 | W3 | W2 + biases | W1, in the order the backward stages complete them
+constexpr int kNormGroups = 4;
+constexpr int kNormMaxBlocks = 1024;
+
 enum GemmId { G_F1, G_F2, G_F3, G_F4_OUT, G_F4_LIN, G_B4W, G_B4D, G_B3W, G_B3D, G_B2W, G_B2D, G_B1W, G_COUNT };
 // timing slots of the non-GEMM kernels follow the GEMM slots
 enum AuxSlot { T_LOAD = G_COUNT, T_EPS, T_FINALIZE, T_COLSUM, T_ADAM, T_TANHBWD, T_LATENT, T_COUNT };
@@ -607,8 +611,16 @@ struct rvae_plan {
   bool fuse_forward;       // env RVAE_FUSE_FORWARD=1: forward pass as one chained launch (default off)
   bool fuse_latent;        // env RVAE_FUSE_LATENT: backward of reparameterize + KL inside the latent dgrad's epilogue
   int dual_pairs;          // CTA pairs a fused launch uses (0 = fused launches off)
-  unsigned int* ticket;    // last-block ticket of the step's final Adam launch (advances the step counter)
+  unsigned int* ticket;    // last-block ticket of the step's final Adam launch (advances the step counter); ticket[1]:
+                           // the gradient-norm finalisation's
   bool ticket_zeroed;
+  bool norm_ticket_zeroed;
+  // gradient-norm clipping (rvae_plan_set_grad_clip): clip_max != nullptr makes every training step clip
+  const double* clip_max;  // device max_norm
+  float* clip_norm_out;    // pre-clip norm ring (may be nullptr)
+  int clip_ring;
+  double* norm_parts;      // workspace: fp64 partials of the norm launches, [kNormGroups][kNormMaxBlocks]
+  float* clip_coef;        // workspace: the step's clipping factor, read by the Adam launch
   struct Prefetch {
     bool registered;       // rvae_plan_prefetch_frames called; consumed by the next rvae_plan_train_step
     int ready_batch;       // > 0: the alternate set holds this many frames (+ their noise), enqueued by a train step
@@ -712,6 +724,8 @@ size_t carve(rvae_plan* p, uint8_t* base) {
   p->ticket = reinterpret_cast<unsigned int*>(take(256));
   p->sched_dev = reinterpret_cast<int*>(take(sizeof(int) * 2 * 6 * 128 * kSchedMax));
   p->dep_flags = reinterpret_cast<unsigned int*>(take(sizeof(unsigned int) * 3 * 256));
+  p->norm_parts = reinterpret_cast<double*>(take(sizeof(double) * kNormGroups * kNormMaxBlocks));
+  p->clip_coef = reinterpret_cast<float*>(take(sizeof(float)));
   p->dz = reinterpret_cast<float*>(take(B * L * 4));
   p->xhat = reinterpret_cast<float*>(take(B * S * 4));
   p->loss_acc = reinterpret_cast<double*>(take(2 * sizeof(double)));
@@ -992,7 +1006,7 @@ int ensure_side_stream(rvae_plan* p) {
 // Adam over the gradient buckets selected by `mask` (bit s = bucket s of rvae_plan_bucket): the selected buckets are
 // merged into contiguous segments of the flat buffer and updated with one launch per pair of segments.
 int adam_buckets(rvae_plan* p, unsigned mask, const HpArg& hp, float grad_scale, int zero_grads, int step_bias,
-                 bool advance_step, cudaStream_t st) {
+                 bool advance_step, cudaStream_t st, const float* coef = nullptr) {
   const rvae_layout& ly = p->lay;
   const rvae_plan_buffers& b = p->bufs;
   // flat order: W1 (bucket 3) | W2 (2) | W3 (1) | W4 (0) | biases (4)
@@ -1014,12 +1028,53 @@ int adam_buckets(rvae_plan* p, unsigned mask, const HpArg& hp, float grad_scale,
     const bool pair = i + 1 < nseg;
     const bool last = i + 2 >= nseg;
     RVAE_CHECK(launch_adam2(&p->ctx->c, b.params + o, b.grads + o, b.exp_avg + o, b.exp_avg_sq + o, seg_n[i],
-                            pair ? seg_off[i + 1] - o : 0, pair ? seg_n[i + 1] : 0, hp, grad_scale, b.step, step_bias, (advance_step && last) ? p->ticket : nullptr,
+                            pair ? seg_off[i + 1] - o : 0, pair ? seg_n[i + 1] : 0, hp, grad_scale, coef, b.step, step_bias, (advance_step && last) ? p->ticket : nullptr,
                             BF(b.shadow_hi) + o, b.shadow_lo ? BF(b.shadow_lo) + o : nullptr, zero_grads, st));
   }
   for (int s = 0; s < 5; ++s)
     if (mask & (1u << s)) p->grads_zeroed[s] = zero_grads != 0;
   return RVAE_OK;
+}
+
+// Sum of squares of norm group k (0: W4, 1: W3, 2: W2 + biases, 3: W1) into its partial slots. The partition and the
+// grids are fixed, so the norm of a gradient buffer has the same bits on every path (two streams, one stream, data
+// parallel, rvae_plan_grad_norm). fin != nullptr: this is the last launch of the reduction; it finalises into *fin.
+int grad_norm_group(rvae_plan* p, int k, NormFinalize* fin, cudaStream_t st) {
+  const rvae_layout& ly = p->lay;
+  const int64_t off[kNormGroups][2] = {{ly.w4, 0}, {ly.w3, 0}, {ly.w2, ly.b1}, {ly.w1, 0}};
+  const int64_t len[kNormGroups][2] = {{ly.b1 - ly.w4, 0}, {ly.w4 - ly.w3, 0}, {ly.w3 - ly.w2, ly.total - ly.b1},
+                                       {ly.w2 - ly.w1, 0}};
+  // the groups' partials are packed in group order: group k starts after the blocks of groups 0..k-1
+  int base[kNormGroups + 1] = {0};
+  for (int j = 0; j < kNormGroups; ++j) base[j + 1] = base[j] + grad_norm_blocks(&p->ctx->c, len[j][0] + len[j][1]);
+  RVAE_REQUIRE(base[kNormGroups] <= kNormGroups * kNormMaxBlocks, RVAE_ERR_UNSUPPORTED, "grad_norm: %d blocks",
+               base[kNormGroups]);
+  if (fin != nullptr) {
+    if (!p->norm_ticket_zeroed) {
+      RVAE_CUDA(cudaMemsetAsync(p->ticket + 1, 0, sizeof(unsigned int), st));
+      p->norm_ticket_zeroed = true;
+    }
+    fin->parts = p->norm_parts;
+    fin->n_parts = base[kNormGroups];
+    fin->ticket = p->ticket + 1;
+  }
+  NormFinalize none;
+  memset(&none, 0, sizeof(none));
+  return launch_grad_norm(&p->ctx->c, p->bufs.grads + off[k][0], len[k][0], off[k][1] - off[k][0], len[k][1],
+                          p->norm_parts + base[k], fin ? *fin : none, st);
+}
+
+// The finalisation of a clipping training step: the pre-clip norm into the ring slot of the step, the factor into
+// the workspace slot the Adam launch reads
+NormFinalize clip_finalize(rvae_plan* p) {
+  NormFinalize f;
+  memset(&f, 0, sizeof(f));
+  f.step = p->bufs.step;
+  f.norm_out = p->clip_norm_out;
+  f.ring_size = p->clip_ring;
+  f.max_norm = p->clip_max;
+  f.coef_out = p->clip_coef;
+  return f;
 }
 
 // Backward stage s, in one stream: the dgrad GEMM that produces the next layer's pre-activation gradient (and, in its
@@ -1279,7 +1334,8 @@ int rvae_plan_create(rvae_ctx* ctx, int S, int H, int L, int max_batch, int prec
   p->lay = lay; p->bound = false; p->batch = 0; p->have_eps = false; p->global_batch = 0; p->noise_row0 = 0;
   p->timing = false;
   p->kl_c0 = 0.f; p->kl_bl = 0.0; p->hp_dev = nullptr; p->hp_early = 0; p->dz_zeroed = false; p->dp_enabled = false;
-  p->cur = 0; p->ticket_zeroed = false; p->ticket = nullptr;
+  p->cur = 0; p->ticket_zeroed = false; p->ticket = nullptr; p->norm_ticket_zeroed = false;
+  p->clip_max = nullptr; p->clip_norm_out = nullptr; p->clip_ring = 1;
   p->x_pitch = 0; p->x_pitch_alt = 0;
   p->fuse_latent = false;
   p->sched_batch = 0;
@@ -1402,7 +1458,7 @@ int rvae_plan_bind(rvae_plan* plan, const rvae_plan_buffers* b) {
   plan->sched_batch = 0;
   for (int i = 0; i < 5; ++i) plan->grads_zeroed[i] = false;
   plan->dz_zeroed = false;
-  plan->cur = 0; plan->ticket_zeroed = false;
+  plan->cur = 0; plan->ticket_zeroed = false; plan->norm_ticket_zeroed = false;
   memset(&plan->pf, 0, sizeof(plan->pf));
   if (plan->two_streams) RVAE_CHECK(ensure_side_stream(plan));
   plan->bound = true;
@@ -1812,6 +1868,10 @@ static int train_step(rvae_plan* plan, float kl_beta, const HpArg& hp, int zero_
   // The step counter t (Adam's bias correction, the loss-ring slot, the Philox offset) stays at its old value for
   // the whole step: every Adam launch uses t + 1, and the last block of the final launch advances it.
   const bool fork = plan->two_streams && !plan->timing;
+  // Gradient clipping: the global norm depends on every bucket and Adam is nonlinear in g, so no bucket is updated
+  // before the norm is known. Each bucket's norm partial takes the place of its background Adam launch; the last one
+  // finalises the clipping factor, and one Adam launch over all buckets reads it.
+  const bool clip = plan->clip_max != nullptr;
   // With a record bound, the latent backward evaluates it before griddepcontrol.wait, overlapping the GEMM before it,
   // when the step runs on the internal streams. That is safe: (1) the record is written by a copy the caller orders
   // before this call on `stream`, and every kernel of the step runs on `st` after cudaStreamWaitEvent(ev_hp_fork),
@@ -1831,8 +1891,13 @@ static int train_step(rvae_plan* plan, float kl_beta, const HpArg& hp, int zero_
     plan->fin.inc_step = 0;
     plan->fin.hp = hp.dev;
     RVAE_CHECK(rvae_plan_backward(plan, -1, stream));
-    TimedScope ts(plan, T_ADAM, S_(stream));
-    return adam_buckets(plan, 0x1f, hp, 1.0f, zero_grads, 1, true, S_(stream));
+    TimedScope ts(plan, T_ADAM, S_(stream));   // (gradient-norm launches are booked with Adam)
+    if (clip) {
+      NormFinalize fin = clip_finalize(plan);
+      for (int k = 0; k < kNormGroups; ++k)
+        RVAE_CHECK(grad_norm_group(plan, k, k == kNormGroups - 1 ? &fin : nullptr, S_(stream)));
+    }
+    return adam_buckets(plan, 0x1f, hp, 1.0f, zero_grads, 1, true, S_(stream), clip ? plan->clip_coef : nullptr);
   }
   // The critical chain (GEMMs) runs on a highest-priority stream; the HBM-bound side work (next batch + its noise,
   // Adam per bucket) on a lowest-priority background stream. The persistent GEMM grids leave the SMs that wave
@@ -1940,7 +2005,22 @@ static int train_step(rvae_plan* plan, float kl_beta, const HpArg& hp, int zero_
       RVAE_CUDA(cudaEventRecord(plan->ev_comm_done[s], cs));
       RVAE_CUDA(cudaStreamWaitEvent(bg, plan->ev_comm_done[s], 0));
       if (s == 0) RVAE_CHECK(finalize_on_bg());
-      RVAE_CHECK(adam_buckets(plan, kBucketMask[s] | extra, hp, 1.0f, zero_grads, 1, false, bg));
+      if (clip) {
+        if (extra) RVAE_CHECK(grad_norm_group(plan, 1, nullptr, bg));
+        RVAE_CHECK(grad_norm_group(plan, s, nullptr, bg));   // norm group s = the buckets of exchange s
+      } else {
+        RVAE_CHECK(adam_buckets(plan, kBucketMask[s] | extra, hp, 1.0f, zero_grads, 1, false, bg));
+      }
+      continue;
+    }
+    if (clip) {
+      // single process: the norm partial of each bucket on the background stream as soon as its stage completes it
+      if (s == 1 && w3_with_stage2) continue;   // W3's gradient is complete after stage 2
+      RVAE_CUDA(cudaEventRecord(plan->ev_adam_fork, st));
+      RVAE_CUDA(cudaStreamWaitEvent(bg, plan->ev_adam_fork, 0));
+      if (s == 0) RVAE_CHECK(finalize_on_bg());
+      if (s == 2 && w3_with_stage2) RVAE_CHECK(grad_norm_group(plan, 1, nullptr, bg));
+      RVAE_CHECK(grad_norm_group(plan, s, nullptr, bg));
       continue;
     }
     // single process: only W4 (the first bucket to complete, with the most GEMM time left to hide under) is updated
@@ -1973,7 +2053,14 @@ static int train_step(rvae_plan* plan, float kl_beta, const HpArg& hp, int zero_
     RVAE_CUDA(cudaStreamWaitEvent(st, plan->ev_comm_done[2], 0));   // the bias bucket travelled with exchange 2
   }
   RVAE_CUDA(cudaStreamWaitEvent(st, plan->ev_adam_join, 0));  // every earlier Adam launch has read the step counter
-  RVAE_CHECK(adam_buckets(plan, dp ? 0x18u : 0x1eu, hp, 1.0f, zero_grads, 1, true, st));
+  if (clip) {
+    // (the background norm partials are complete: the wait above)
+    NormFinalize fin = clip_finalize(plan);
+    RVAE_CHECK(grad_norm_group(plan, 3, &fin, st));
+    RVAE_CHECK(adam_buckets(plan, 0x1fu, hp, 1.0f, zero_grads, 1, true, st, plan->clip_coef));
+  } else {
+    RVAE_CHECK(adam_buckets(plan, dp ? 0x18u : 0x1eu, hp, 1.0f, zero_grads, 1, true, st));
+  }
   RVAE_CUDA(cudaEventRecord(plan->ev_hp_join, st));
   RVAE_CUDA(cudaStreamWaitEvent(S_(stream), plan->ev_hp_join, 0));
   return RVAE_OK;
@@ -1999,6 +2086,32 @@ int rvae_plan_train_step_hp(rvae_plan* plan, const rvae_hparams* hp_dev, int zer
     ~HpGuard() { p->hp_dev = nullptr; p->hp_early = 0; }
   } guard(plan, hp_dev);
   return train_step(plan, 0.0f, hp_device(hp_dev), zero_grads, loss_out, ring_size, stream);
+}
+
+int rvae_plan_set_grad_clip(rvae_plan* plan, const double* max_norm_dev, float* norm_out, int ring_size) {
+  RVAE_REQUIRE(norm_out == nullptr || ring_size >= 1, RVAE_ERR_INVALID, "plan_set_grad_clip: ring_size %d", ring_size);
+  RVAE_REQUIRE(plan, RVAE_ERR_INVALID, "null rvae_plan");
+  // the experiments-only fused latent epilogue runs its own stage-1 path, which this step layout does not cover
+  RVAE_REQUIRE(max_norm_dev == nullptr || !(plan->fuse_latent && plan->precision == RVAE_PRECISION_BF16),
+               RVAE_ERR_UNSUPPORTED,
+               "plan_set_grad_clip: the fused latent epilogue (RVAE_FUSE_LATENT) is not supported");
+  plan->clip_max = max_norm_dev;
+  plan->clip_norm_out = max_norm_dev ? norm_out : nullptr;
+  plan->clip_ring = norm_out ? ring_size : 1;
+  return RVAE_OK;
+}
+
+int rvae_plan_grad_norm(rvae_plan* plan, float* norm_out, void* stream) {
+  RVAE_REQUIRE(norm_out, RVAE_ERR_INVALID, "plan_grad_norm: null norm_out");
+  RVAE_CHECK(check_ready(plan, false));
+  RVAE_REQUIRE(plan->bufs.grads, RVAE_ERR_STATE, "plan_grad_norm: grads not bound");
+  NormFinalize fin;
+  memset(&fin, 0, sizeof(fin));
+  fin.norm_out = norm_out;
+  fin.ring_size = 1;
+  for (int k = 0; k < kNormGroups; ++k)
+    RVAE_CHECK(grad_norm_group(plan, k, k == kNormGroups - 1 ? &fin : nullptr, S_(stream)));
+  return RVAE_OK;
 }
 
 int rvae_hparams_check(const rvae_hparams* h) {

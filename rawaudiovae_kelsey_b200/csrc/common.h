@@ -200,8 +200,22 @@ int launch_adam(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, dou
                 double eps, double weight_decay, float grad_scale, const float* step, __nv_bfloat16* shadow_hi,
                 __nv_bfloat16* shadow_lo, int zero_grads, cudaStream_t stream);
 int launch_adam2(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, int64_t off_b, int64_t n_b,
-                 const HpArg& hp, float grad_scale, float* step, int step_bias, unsigned int* ticket,
+                 const HpArg& hp, float grad_scale, const float* coef, float* step, int step_bias, unsigned int* ticket,
                  __nv_bfloat16* shadow_hi, __nv_bfloat16* shadow_lo, int zero_grads, cudaStream_t stream);
+// Gradient norm for clipping (grad_norm_kernel): the last block of a launch with `ticket` set sums parts[0, n_parts)
+struct NormFinalize {
+  const double* parts;
+  int n_parts;
+  unsigned int* ticket;   // nullptr: the launch only writes its partials
+  const float* step;      // ring slot = *step mod ring_size (nullptr: slot 0)
+  float* norm_out;        // nullptr: not reported
+  int ring_size;
+  const double* max_norm; // nullptr: no clipping factor
+  float* coef_out;
+};
+int grad_norm_blocks(const Ctx* ctx, int64_t n);   // the fixed grid of a launch over n elements
+int launch_grad_norm(Ctx* ctx, const float* g, int64_t n, int64_t off_b, int64_t n_b, double* part,
+                     const NormFinalize& f, cudaStream_t stream);
 int launch_hparams_eval(Ctx* ctx, const rvae_hparams* hp, const int64_t* k, int n, double* lr_out, float* beta_out,
                         cudaStream_t stream);
 int launch_step_inc(Ctx* ctx, float* step, cudaStream_t stream);

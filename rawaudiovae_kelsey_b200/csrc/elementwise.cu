@@ -1059,7 +1059,7 @@ int launch_lerp_reparam(Ctx* ctx, const float* mu_a, const float* lv_a, const fl
 template <int U>
 __global__ void __launch_bounds__(256, U == 4 ? 2 : 4) adam_kernel(float* __restrict__ p, float* __restrict__ g, float* __restrict__ m,
                             float* __restrict__ v, int64_t n, int64_t off_b, int64_t n_b, const __grid_constant__ HpArg hp,
-                            float grad_scale, float* step, int step_bias, unsigned int* ticket,
+                            float grad_scale, const float* coef, float* step, int step_bias, unsigned int* ticket,
                             __nv_bfloat16* __restrict__ sh_hi, __nv_bfloat16* __restrict__ sh_lo, int zero_grads,
                             AuxTrace tr) {
   ptx::pdl_launch_dependents();
@@ -1069,8 +1069,9 @@ __global__ void __launch_bounds__(256, U == 4 ? 2 : 4) adam_kernel(float* __rest
   // is derived from them exactly as torch derives it: 1 - beta in DOUBLE, then rounded to fp32 (the weight of lerp_ /
   // the value of addcmul_; (1.f - 0.999f) would be off by 1.3e-5 relative), beta2 and eps rounded to fp32. Bias
   // corrections in double, as torch computes them on the host (python floats). One thread per block reads the record,
-  // does the fp64 pow()s and broadcasts the seven scalars.
-  __shared__ float s_consts[7];
+  // does the fp64 pow()s and broadcasts the seven scalars. coef != nullptr: the gradient-clipping factor of the step
+  // (grad_norm_kernel), folded into the gradient scale - g * coef in fp32, as torch.nn.utils.clip_grad_norm_ scales g.
+  __shared__ float s_consts[8];
   if (threadIdx.x == 0) {
     const rvae_hparams& h = hp.dev != nullptr ? *hp.dev : hp.val;
     // t = *step + step_bias: step_bias = 1 when the step counter is advanced only at the end of the step (ticket)
@@ -1087,8 +1088,10 @@ __global__ void __launch_bounds__(256, U == 4 ? 2 : 4) adam_kernel(float* __rest
     s_consts[4] = static_cast<float>(1.0 - h.beta2);
     s_consts[5] = static_cast<float>(h.eps);
     s_consts[6] = static_cast<float>(h.weight_decay);
+    s_consts[7] = coef != nullptr ? grad_scale * *coef : grad_scale;
   }
   __syncthreads();
+  grad_scale = s_consts[7];
   const float step_size = s_consts[0];
   const float sqrt_bc2 = s_consts[1];
   const float omb1 = s_consts[2], beta2 = s_consts[3], omb2 = s_consts[4], eps = s_consts[5];
@@ -1184,12 +1187,12 @@ __global__ void __launch_bounds__(256, U == 4 ? 2 : 4) adam_kernel(float* __rest
 int launch_adam(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, double lr, double beta1, double beta2,
                 double eps, double weight_decay, float grad_scale, const float* step, __nv_bfloat16* shadow_hi,
                 __nv_bfloat16* shadow_lo, int zero_grads, cudaStream_t stream) {
-  return launch_adam2(ctx, p, g, m, v, n, 0, 0, hp_value(lr, beta1, beta2, eps, weight_decay), grad_scale,
+  return launch_adam2(ctx, p, g, m, v, n, 0, 0, hp_value(lr, beta1, beta2, eps, weight_decay), grad_scale, nullptr,
                       const_cast<float*>(step), 0, nullptr, shadow_hi, shadow_lo, zero_grads, stream);
 }
 
 int launch_adam2(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, int64_t off_b, int64_t n_b,
-                 const HpArg& hp, float grad_scale, float* step, int step_bias, unsigned int* ticket,
+                 const HpArg& hp, float grad_scale, const float* coef, float* step, int step_bias, unsigned int* ticket,
                  __nv_bfloat16* shadow_hi, __nv_bfloat16* shadow_lo, int zero_grads, cudaStream_t stream) {
   RVAE_REQUIRE(p && g && m && v && step, RVAE_ERR_INVALID, "adam: null buffer");
   RVAE_REQUIRE(n_b == 0 || ((n & 3) == 0 && (off_b & 3) == 0 && (n_b & 3) == 0 && off_b >= n), RVAE_ERR_INVALID,
@@ -1210,8 +1213,108 @@ int launch_adam2(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, in
   if (ctx->aux_grid_cap > 0 && (int)grid.x > ctx->aux_grid_cap) grid.x = ctx->aux_grid_cap;
   auto kern = unroll == 1 ? adam_kernel<1> : (unroll == 4 ? adam_kernel<4> : adam_kernel<2>);
   RVAE_CUDA(launch_kernel(ctx, kern, grid, dim3(threads), (size_t)0,
-                          stream, p, g, m, v, n, off_b, n_b, hp, grad_scale, step, step_bias, ticket, shadow_hi,
+                          stream, p, g, m, v, n, off_b, n_b, hp, grad_scale, coef, step, step_bias, ticket, shadow_hi,
                           shadow_lo, zero_grads, next_aux(ctx, 4)));
+  RVAE_LAUNCH_CHECK(ctx);
+  return RVAE_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Global gradient norm for clipping (torch.nn.utils.clip_grad_norm_, norm type 2). A launch reads one or two segments
+// of the flat gradient buffer (4 B/param, float4 loads), squares each fp32 element in fp64 - a gradient of 1e-30 does
+// not underflow - and writes one fp64 partial per block to part[blockIdx.x]. Element-to-thread mapping, the grid
+// (grad_norm_blocks) and the reduction tree are fixed, with no atomics, so a gradient buffer gives the same bits every
+// time. With f.ticket set, the last block of the launch sums every partial of the reduction, f.parts[0 .. n_parts),
+// in index order (earlier launches are complete: stream- or event-ordered before this one) and writes
+//   norm = sqrt(sum) -> norm_out[*step mod ring_size] (fp32; slot 0 without a step counter),
+//   coef = min(1, max_norm / (norm + 1e-6)) in fp64, rounded to fp32 once -> *coef_out (when max_norm != nullptr).
+// A NaN norm gives a NaN coef (torch.clamp propagates it); inf gives 0, or NaN with max_norm = inf, as in torch.
+// ------------------------------------------------------------------------------------------------
+constexpr int kNormThreads = 256;
+
+__device__ __forceinline__ double block_sum_f64(double v, double* smem) {
+  // block total in thread 0, in a fixed order
+  v = warp_sum_f64(v);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  if (lane == 0) smem[warp] = v;
+  __syncthreads();
+  double t = 0.0;
+  if (warp == 0) t = warp_sum_f64(lane < kNormThreads / 32 ? smem[lane] : 0.0);
+  return t;
+}
+
+__global__ void __launch_bounds__(kNormThreads) grad_norm_kernel(const float* __restrict__ g, int64_t n, int64_t off_b,
+                                                                 int64_t n_b, double* __restrict__ part,
+                                                                 NormFinalize f) {
+  ptx::pdl_launch_dependents();
+  ptx::pdl_wait();
+  __shared__ double red[kNormThreads / 32];
+  __shared__ bool is_last;
+  constexpr int U = 4;   // float4 loads in flight per thread
+  const int64_t nvec = n >> 2, nvec_all = nvec + (n_b >> 2), shift_b = (off_b >> 2) - nvec;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  double acc = 0.0;
+  for (int64_t w0 = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; w0 < nvec_all; w0 += U * stride) {
+    float4 q[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int64_t w = w0 + u * stride;
+      q[u] = w < nvec_all ? __ldcg(reinterpret_cast<const float4*>(g) + (w < nvec ? w : w + shift_b))
+                          : make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      acc = fma((double)q[u].x, (double)q[u].x, acc);
+      acc = fma((double)q[u].y, (double)q[u].y, acc);
+      acc = fma((double)q[u].z, (double)q[u].z, acc);
+      acc = fma((double)q[u].w, (double)q[u].w, acc);
+    }
+  }
+  const double total = block_sum_f64(acc, red);
+  if (threadIdx.x == 0) part[blockIdx.x] = total;
+  if (f.ticket == nullptr) return;
+  if (threadIdx.x == 0) {
+    __threadfence();
+    is_last = atomicAdd(f.ticket, 1u) == gridDim.x - 1;
+  }
+  __syncthreads();
+  if (!is_last) return;
+  __threadfence();
+  double s = 0.0;
+  for (int i = threadIdx.x; i < f.n_parts; i += blockDim.x) s += __ldcg(f.parts + i);
+  __syncthreads();   // red[] is reused
+  s = block_sum_f64(s, red);
+  if (threadIdx.x == 0) {
+    *f.ticket = 0u;
+    const double norm = sqrt(s);
+    if (f.norm_out != nullptr) {
+      const int slot = (f.ring_size > 1 && f.step) ? static_cast<int>(static_cast<long long>(*f.step) % f.ring_size) : 0;
+      f.norm_out[slot] = static_cast<float>(norm);
+    }
+    if (f.max_norm != nullptr) {
+      const double c = *f.max_norm / (norm + 1e-6);
+      *f.coef_out = static_cast<float>(c > 1.0 ? 1.0 : c);   // (not fmin: a NaN must propagate)
+    }
+  }
+}
+
+int grad_norm_blocks(const Ctx* ctx, int64_t n) {
+  // a multiple of the SM count: one to four blocks per SM, by size
+  const int64_t per_wave = (int64_t)ctx->num_sms_total * kNormThreads * 4;   // elements one float4 per thread covers
+  const int64_t waves = std::min<int64_t>(4, std::max<int64_t>(1, (n + per_wave - 1) / per_wave));
+  return ctx->num_sms_total * (int)waves;
+}
+
+int launch_grad_norm(Ctx* ctx, const float* g, int64_t n, int64_t off_b, int64_t n_b, double* part,
+                     const NormFinalize& f, cudaStream_t stream) {
+  RVAE_REQUIRE(g && part, RVAE_ERR_INVALID, "grad_norm: null buffer");
+  RVAE_REQUIRE((n & 3) == 0 && (off_b & 3) == 0 && (n_b & 3) == 0 && (n_b == 0 || off_b >= n) &&
+                   (reinterpret_cast<uintptr_t>(g) & 15) == 0,
+               RVAE_ERR_INVALID, "grad_norm: segments must be 16-byte aligned multiples of 4 elements");
+  RVAE_REQUIRE(f.ticket == nullptr || (f.parts && f.n_parts > 0 && (f.max_norm == nullptr || f.coef_out)),
+               RVAE_ERR_INVALID, "grad_norm: bad finalize arguments");
+  RVAE_CUDA(launch_kernel(ctx, grad_norm_kernel, dim3(grad_norm_blocks(ctx, n + n_b)), dim3(kNormThreads), (size_t)0,
+                          stream, g, n, off_b, n_b, part, f));
   RVAE_LAUNCH_CHECK(ctx);
   return RVAE_OK;
 }

@@ -268,11 +268,13 @@ class DataParallelTrainStep(_StepBase):
     The returned loss is the mean over THIS rank's frames (an unbiased estimate of the global mean that needs no
     collective); reduce_loss=True additionally averages it over the ranks (exact for equal shards).
     graph=True captures the whole step, NCCL collectives included, into one CUDA graph per input signature.
-    schedule: as for FusedTrainStep; every rank evaluates it at the same step counter."""
+    schedule: as for FusedTrainStep; every rank evaluates it at the same step counter.
+    max_grad_norm: as for FusedTrainStep. The norm is taken over the all-reduced gradient, which is identical on every
+    rank, in a fixed order, so every rank clips by the same factor and the replicas stay bitwise equal."""
 
     def __init__(self, model, optimizer, kl_beta: float, global_batch: Optional[int] = None, group=None,
-                 ring: int = 64, reduce_loss: bool = False, graph: bool = False, schedule=None):
-        super().__init__(model, optimizer, kl_beta, ring, graph, schedule=schedule)
+                 ring: int = 64, reduce_loss: bool = False, graph: bool = False, schedule=None, max_grad_norm=None):
+        super().__init__(model, optimizer, kl_beta, ring, graph, schedule=schedule, max_grad_norm=max_grad_norm)
         self.group = group
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
@@ -320,7 +322,7 @@ class DataParallelTrainStep(_StepBase):
         return self._shared_seed if getattr(self, "_shared_seed", None) is not None else super()._seed()
 
     def _enqueue(self, plan):
-        plan.train_step_hp(self._record.tensor, loss_out=self.ring, ring_size=self.ring_size, zero_grads=True)
+        self._train_step(plan, zero_grads=True)
 
     def __call__(self, data, eps: Optional[torch.Tensor] = None, next_data=None) -> torch.Tensor:
         flat = self._prepare()

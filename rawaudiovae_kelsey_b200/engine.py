@@ -307,6 +307,20 @@ class Plan:
                                                loss_out.data_ptr() if loss_out is not None else None, ring_size,
                                                self._stream()))
 
+    def set_grad_clip(self, max_norm_ptr: Optional[int], norm_out: Optional[torch.Tensor] = None,
+                      ring_size: int = 1) -> None:
+        """Clip the gradient of every later training step by its global norm at the device double max_norm_ptr
+        (None = off); the pre-clip norm of each step goes to norm_out[step mod ring_size] when norm_out is given."""
+        check(self.lib.rvae_plan_set_grad_clip(self.handle, max_norm_ptr,
+                                               norm_out.data_ptr() if norm_out is not None else None, int(ring_size)))
+
+    def grad_norm(self, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Global L2 norm of the bound gradient buffer, with the kernels of a clipping step (0-dim float32 tensor)."""
+        if out is None:
+            out = torch.empty((), dtype=torch.float32, device=self.flat.device)
+        check(self.lib.rvae_plan_grad_norm(self.handle, out.data_ptr(), self._stream()))
+        return out
+
     def encode(self) -> None:
         check(self.lib.rvae_plan_encode(self.handle, self._stream()))
 

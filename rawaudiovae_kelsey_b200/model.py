@@ -15,6 +15,7 @@ so the fused Adam kernel and the gradient all-reduce see contiguous memory.
 """
 from __future__ import annotations
 
+import math
 import os
 from typing import Dict, List, Optional
 
@@ -375,6 +376,19 @@ def loss_function(recon_x, x, mu, logvar, kl_beta, segment_length):
     return _LossFunction.apply(c(recon_x), c(x), c(mu), c(logvar), float(kl_beta))
 
 
+def check_max_grad_norm(value) -> Optional[float]:
+    """A training step's gradient-clipping threshold: None (no clipping) or a float > 0, +inf included (the norm is
+    measured and logged, the update is unchanged). Raises ValueError for anything else."""
+    if value is None:
+        return None
+    if isinstance(value, bool) or not isinstance(value, (int, float)):
+        raise ValueError(f"max_grad_norm must be None or a number > 0, got {value!r}")
+    v = float(value)
+    if math.isnan(v) or v <= 0.0:
+        raise ValueError(f"max_grad_norm must be > 0 (inf allowed), got {value!r}")
+    return v
+
+
 class _StepBase:
     """Shared machinery of FusedTrainStep / dist.DataParallelTrainStep: the device-side loss ring and the CUDA-graph
     cache. A step is enqueued by `self._enqueue(plan)` (subclass); with graph=True the enqueue is captured once per
@@ -383,14 +397,21 @@ class _StepBase:
     read from device memory: frame indices from a static index buffer, the Philox offset and the loss-ring slot
     from the optimizer's step counter. The hyper-parameters too: the kernels read them from a device record
     (schedule.DeviceRecord) that each call rewrites before the step when optimizer.param_groups[0], kl_beta or
-    `schedule` changed, so replays follow the schedule, a torch LR scheduler and any change made by hand."""
+    `schedule` changed, so replays follow the schedule, a torch LR scheduler and any change made by hand.
 
-    def __init__(self, model, optimizer, kl_beta, ring, graph, graph_warmup=1, schedule=None):
+    max_grad_norm (None = off): clip the gradient by its global L2 norm before Adam, as torch.nn.utils.clip_grad_norm_
+    does, inside the step (rvae_plan_set_grad_clip). The threshold lives in the device record too, so changing
+    `step.max_grad_norm` reaches graph replays; switching clipping on or off captures a new graph. The pre-clip norm
+    of every step lands in a device ring of the loss ring's size; `grad_norm` is the last step's slot."""
+
+    def __init__(self, model, optimizer, kl_beta, ring, graph, graph_warmup=1, schedule=None, max_grad_norm=None):
+        self.max_grad_norm = max_grad_norm     # validated before any GPU work
         self.model, self.optimizer, self.kl_beta = model, optimizer, float(kl_beta)
         self.schedule = schedule if schedule is not None else Schedule()
         self._record = None
         self.ring_size = int(ring)
         self.ring = None
+        self.norm_ring = None    # pre-clip gradient norms, slot = step counter mod ring_size (allocated when clipping)
         self.i = None            # host mirror of the device step counter (slot = i % ring_size)
         self.graph = bool(graph)
         # eager calls per input signature before its graph is captured: ONE is needed (the first call of a signature
@@ -404,12 +425,30 @@ class _StepBase:
         self.stats = {"eager": 0, "captures": 0, "replays": 0}
         self.steady = 0
 
+    @property
+    def max_grad_norm(self) -> Optional[float]:
+        return self._max_grad_norm
+
+    @max_grad_norm.setter
+    def max_grad_norm(self, value):
+        self._max_grad_norm = check_max_grad_norm(value)
+
+    @property
+    def grad_norm(self) -> Optional[torch.Tensor]:
+        """The pre-clip gradient norm of the last step (0-dim device tensor, a slot of the norm ring), or None when
+        clipping is off or before the first step."""
+        if self.max_grad_norm is None or self.norm_ring is None or not self.i:
+            return None
+        return self.norm_ring[(self.i - 1) % self.ring_size]
+
     # -- helpers
     def _prepare(self):
         model = self.model
         flat = model._ensure_flat()
         if self.ring is None:
             self.ring = torch.zeros(self.ring_size, dtype=torch.float32, device=flat.device)
+        if self.norm_ring is None and self.max_grad_norm is not None:
+            self.norm_ring = torch.zeros(self.ring_size, dtype=torch.float32, device=flat.device)
         if self.i is None:
             self.i = int(flat.step.item())          # one sync, first call only (resumed optimizers start at t0 > 0)
         if hasattr(self.optimizer, "bind_flat"):
@@ -422,7 +461,18 @@ class _StepBase:
             self._record = DeviceRecord(device)
         g = self.optimizer.param_groups[0]
         return self._record.update(self.schedule, g["lr"], g["betas"], g["eps"], g.get("weight_decay", 0.0),
-                                   self.kl_beta)
+                                   self.kl_beta, self.max_grad_norm)
+
+    def _train_step(self, plan, zero_grads):
+        """The fused step from the device record, clipping when max_grad_norm is set (a plan setting for this call)."""
+        if self.max_grad_norm is None:
+            plan.train_step_hp(self._record.tensor, loss_out=self.ring, ring_size=self.ring_size, zero_grads=zero_grads)
+            return
+        plan.set_grad_clip(self._record.max_norm_ptr, self.norm_ring, self.ring_size)
+        try:
+            plan.train_step_hp(self._record.tensor, loss_out=self.ring, ring_size=self.ring_size, zero_grads=zero_grads)
+        finally:
+            plan.set_grad_clip(None)
 
     def _slot(self):
         return self.ring[self.i % self.ring_size]
@@ -490,7 +540,7 @@ class _StepBase:
             # ---- plain path: load inside the step (captured graph: from static index / input buffers)
             key = self._graph_key(data) if graphable else None
             if key is not None:
-                key = key + self._key_extra(data)
+                key = key + self._key_extra(data) + (self.max_grad_norm is not None,)
             if key is not None and key in self._graphs:
                 st = self._graphs[key]
                 self._load_static(key, data, st)
@@ -523,7 +573,7 @@ class _StepBase:
             if graphable and do_pf and isinstance(data, FrameBatch):
                 key = ("pf", plan.handle.value, next_data.audio.data_ptr(), plan.batch, next_data.n_frames,
                        next_data.hop, self._plan_cur(plan), plan.pitch, model._in_place(next_data)) \
-                    + self._key_extra(data) + self._key_extra(next_data)
+                    + self._key_extra(data) + self._key_extra(next_data) + (self.max_grad_norm is not None,)
             if key is not None and key in self._graphs:
                 st = self._graphs[key]
                 self._fill_idx(st, next_data)
@@ -634,19 +684,20 @@ class FusedTrainStep(_StepBase):
 
     keep_grads=False (default): the Adam kernel clears the flat gradient buffer after consuming it, exactly what the
     reference's optimizer.zero_grad() does at the top of the next iteration; keep_grads=True leaves the step's
-    gradients in model._flat.grads for inspection (costs memsets per step).
+    gradients in model._flat.grads for inspection (costs memsets per step). With clipping they are the raw,
+    unclipped gradients: the norm torch.nn.utils.clip_grad_norm_ returns, and step.grad_norm holds, is theirs.
     graph=True: replay a captured CUDA graph of the step (see _StepBase).
     schedule (schedule.Schedule, default constant): learning rate and KL weight per step, with
-    optimizer.param_groups[0]['lr'] and kl_beta as the peak values."""
+    optimizer.param_groups[0]['lr'] and kl_beta as the peak values.
+    max_grad_norm (None, or a float > 0, inf included): clip by the global gradient norm (see _StepBase)."""
 
     def __init__(self, model: VAE, optimizer, kl_beta: float, ring: int = 64, keep_grads: bool = False,
-                 graph: bool = False, schedule: Optional[Schedule] = None):
-        super().__init__(model, optimizer, kl_beta, ring, graph, schedule=schedule)
+                 graph: bool = False, schedule: Optional[Schedule] = None, max_grad_norm: Optional[float] = None):
+        super().__init__(model, optimizer, kl_beta, ring, graph, schedule=schedule, max_grad_norm=max_grad_norm)
         self.keep_grads = keep_grads
 
     def _enqueue(self, plan):
-        plan.train_step_hp(self._record.tensor, loss_out=self.ring, ring_size=self.ring_size,
-                           zero_grads=not self.keep_grads)
+        self._train_step(plan, zero_grads=not self.keep_grads)
 
     def __call__(self, data, eps: Optional[torch.Tensor] = None, next_data=None) -> torch.Tensor:
         return self._run(data, eps, next_data)

@@ -13,6 +13,7 @@ from __future__ import annotations
 
 import ctypes as C
 import math
+import struct
 from dataclasses import dataclass
 
 import torch
@@ -136,20 +137,29 @@ class Schedule:
 
 
 class DeviceRecord:
-    """The device copy of a training step's rvae_hparams record. `update` rewrites it - with one copy from pinned
-    memory, ordered on the current stream, without a device synchronisation - only when the schedule or a peak value
-    differs from what the record holds. The record keeps its address, so a captured graph reads the new values."""
+    """The device copy of a training step's rvae_hparams record, followed by the gradient-clipping threshold (a
+    double; rvae_plan_set_grad_clip). `update` rewrites both - with one copy from pinned memory, ordered on the
+    current stream, without a device synchronisation - only when the schedule, a peak value or the threshold differs
+    from what the record holds. The record keeps its address, so a captured graph reads the new values."""
 
     def __init__(self, device):
-        self.tensor = torch.zeros(C.sizeof(_lib.Hparams), dtype=torch.uint8, device=device)
+        self.tensor = torch.zeros(C.sizeof(_lib.Hparams) + 8, dtype=torch.uint8, device=device)
         self._key = None
 
-    def update(self, schedule: Schedule, lr, betas, eps, weight_decay, kl_beta) -> torch.Tensor:
-        key = (schedule, float(lr), float(betas[0]), float(betas[1]), float(eps), float(weight_decay), float(kl_beta))
+    @property
+    def max_norm_ptr(self) -> int:
+        """Device address of the clipping threshold."""
+        return self.tensor.data_ptr() + C.sizeof(_lib.Hparams)
+
+    def update(self, schedule: Schedule, lr, betas, eps, weight_decay, kl_beta, max_grad_norm=None) -> torch.Tensor:
+        max_norm = math.inf if max_grad_norm is None else float(max_grad_norm)
+        key = (schedule, float(lr), float(betas[0]), float(betas[1]), float(eps), float(weight_decay), float(kl_beta),
+               max_norm)
         if key != self._key:
             rec = schedule.record(lr, betas, eps, weight_decay, kl_beta)
             _lib.check(_lib.load().rvae_hparams_check(C.byref(rec)))
-            host = torch.frombuffer(bytearray(bytes(rec)), dtype=torch.uint8).pin_memory()
+            raw = bytes(rec) + struct.pack("<d", max_norm)
+            host = torch.frombuffer(bytearray(raw), dtype=torch.uint8).pin_memory()
             self.tensor.copy_(host, non_blocking=True)
             self._key = key
         return self.tensor

@@ -28,7 +28,7 @@ import torch
 from . import audio_io, dist as rdist
 from .dataset import AudioDataset, IterableAudioDataset, ToTensor
 from .inference import evaluate_audio
-from .model import VAE, FusedTrainStep
+from .model import VAE, FusedTrainStep, check_max_grad_norm
 from .optim import Adam
 from .schedule import Schedule
 from .stats import ParamHistogramLogger
@@ -150,6 +150,20 @@ def _schedule(config, total_steps: int) -> Schedule:
                     kl_cycle_ratio=vae.getfloat('kl_cycle_ratio', fallback=0.5))
 
 
+def _max_grad_norm(config):
+    """[training] max_grad_norm (optional): clip each step's gradient by its global L2 norm at this value, and log the
+    pre-clip norm as 'Grad Norm'; inf logs without clipping. Absent or empty: no clipping, no extra tag. Values <= 0,
+    NaN or text that is not a number raise ValueError."""
+    v = config['training'].get('max_grad_norm', fallback='').strip()
+    if not v:
+        return None
+    try:
+        f = float(v)
+    except ValueError:
+        raise ValueError(f"[training] max_grad_norm must be a number > 0 or inf, got {v!r}") from None
+    return check_max_grad_norm(f)
+
+
 def _epoch_steps(n_frames: int, batch_size: int, world: int = 1) -> int:
     """Training steps per epoch of GpuFrameLoader (drop_last=False): a last global batch with fewer frames than ranks
     is skipped."""
@@ -224,14 +238,21 @@ def _with_next(iterable):
 
 
 def _flush_losses(writer, pending, print_fmt=None, world=1):
-    """Read back a block of per-batch losses (device scalars) with one sync and log them under the reference's tag."""
+    """Read back a block of per-batch losses (device scalars) with one sync and log them under the reference's tag.
+    Entries are (step id, loss) or, when clipping, (step id, loss, gradient norm): the norms come back in the same
+    copy and are logged as 'Grad Norm'."""
     if not pending:
         return 0.0
-    vals = torch.stack([l for _, l in pending]).cpu().tolist()
+    norms = [e[2] for e in pending if len(e) > 2]
+    got = torch.stack([e[1] for e in pending] + norms).cpu().tolist()
+    vals, norm_vals = got[:len(pending)], got[len(pending):]
     if world > 1:
         rdist.check_health(pending[0][1].device)   # a rank that dropped out of the gradient exchange: fail loudly
-    for (step_id, _), v in zip(pending, vals):
+    for i, (e, v) in enumerate(zip(pending, vals)):
+        step_id = e[0]
         writer.add_scalar('Loss/Batch', v, step_id)
+        if norm_vals:
+            writer.add_scalar('Grad Norm', norm_vals[i], step_id)
         if print_fmt:
             print(print_fmt.format(step_id, v))
     pending.clear()
@@ -263,6 +284,7 @@ def run_epoch_trainer(argv=None):
     n_units = config['VAE'].getint('n_units')
     kl_beta = config['VAE'].getfloat('kl_beta')
     test_loss = _test_loss_enabled(config)
+    max_grad_norm = _max_grad_norm(config)
     start_time = time.time()
     config['extra']['start'] = time.asctime(time.localtime(start_time))
 
@@ -303,9 +325,11 @@ def run_epoch_trainer(argv=None):
     use_graph = config['training'].getboolean('cuda_graph', fallback=True)
     ring = max(64, log_interval)
     if world > 1:
-        step = rdist.DataParallelTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph, schedule=schedule)
+        step = rdist.DataParallelTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph, schedule=schedule,
+                                           max_grad_norm=max_grad_norm)
     else:
-        step = FusedTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph, schedule=schedule)
+        step = FusedTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph, schedule=schedule,
+                              max_grad_norm=max_grad_norm)
 
     # parameter histograms on the GPU (rank 0 only): one launch + one small asynchronous copy per set
     hist = ParamHistogramLogger(model, writer) if rank == 0 else None
@@ -325,7 +349,7 @@ def run_epoch_trainer(argv=None):
             if world > 1:  # the last batch of an epoch may be short: normalise by the true global batch size
                 step.global_batch = min(batch_size, len(training_dataset) - b * batch_size)
             loss = step(data, next_data=nxt)   # the next batch is gathered in the background of this step
-            pending.append((batch_id, loss))
+            pending.append((batch_id, loss) if max_grad_norm is None else (batch_id, loss, step.grad_norm))
             _log_hparams(writer, schedule, optimizer, kl_beta, batch_id)
             batch_id += 1
             if len(pending) >= log_interval:
@@ -429,6 +453,7 @@ def run_stream_trainer(argv=None):
     n_units = config['VAE'].getint('n_units')
     kl_beta = config['VAE'].getfloat('kl_beta')
     test_loss = _test_loss_enabled(config)
+    max_grad_norm = _max_grad_norm(config)
     if segment_length != 1024:
         raise ValueError("the streaming dataset frames at 1024 samples (rawvae/dataset.py:66); segment_length "
                          "= {} is not supported by train_iterable.py".format(segment_length))
@@ -473,9 +498,10 @@ def run_stream_trainer(argv=None):
         ring = max(64, log_interval)
         if world > 1:
             step = rdist.DataParallelTrainStep(model, optimizer, kl_beta, global_batch=batch_size, ring=ring,
-                                               graph=use_graph, schedule=schedule)
+                                               graph=use_graph, schedule=schedule, max_grad_norm=max_grad_norm)
         else:
-            step = FusedTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph, schedule=schedule)
+            step = FusedTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph, schedule=schedule,
+                                  max_grad_norm=max_grad_norm)
 
         hist = ParamHistogramLogger(model, writer) if rank == 0 and histogram_interval > 0 else None
 
@@ -489,7 +515,7 @@ def run_stream_trainer(argv=None):
         fmt = '====> Batch: {} - Loss: {:.9f}'
         for data, nxt in _with_next(islice(stream, total_num_batches)):
             loss = step(data, next_data=nxt)   # the next batch is gathered in the background of this step
-            pending.append((batch_id, loss))
+            pending.append((batch_id, loss) if max_grad_norm is None else (batch_id, loss, step.grad_norm))
             _log_hparams(writer, schedule, optimizer, kl_beta, batch_id)
             at_checkpoint = batch_id % checkpoint_interval == 0 and batch_id != 0
             if len(pending) >= log_interval or at_checkpoint:
