@@ -495,6 +495,34 @@ int rvae_plan_set_grad_clip(rvae_plan* plan, const double* max_norm_dev, float* 
  * float); not part of any step. Returns 1 for a null norm_out (before the plan is used). */
 int rvae_plan_grad_norm(rvae_plan* plan, float* norm_out, void* stream);
 
+/* Deterministic training steps (opt-in). With a scratch bound, every output of rvae_plan_train_step(_hp) - parameters,
+ * exp_avg, exp_avg_sq, bf16 shadows, the step counter, the loss ring, the norm ring and the gradients of zero_grads = 0
+ * - depends only on the inputs, the state, the hyper-parameters, the dims, the batch size, the precision and the
+ * world size: not on stream timing, on which CTA runs which tile, on the SM budget (RVAE_NUM_SMS,
+ * RVAE_S1_WGRAD_CTAS) or on whether a GEMM runs in a fused launch. Every sum the default step does with atomics or
+ * a TMA reduce-add has a fixed order instead:
+ *   - split-K weight gradients and latent dgrad: split 0 stores into the gradient (dz) buffer, split k >= 1 into its
+ *     own scratch slice, with plain TMA stores; the split count comes from the shapes against a fixed 74 CTA pairs.
+ *     After backward stage s one grad_sum launch adds the slices of bucket s to split 0 in split order;
+ *   - bias gradients: each epilogue warp writes the column sums of its 32 rows to partial row (row / 32) of the
+ *     scratch, the latent backward one row per block (fixed grid of min(ceil(rows / rows per pass), 592) blocks,
+ *     rows per pass = max(1, 1024 / Lp)); the grad_sum launch after stage 2 adds each bias column's rows into the
+ *     bias block in a fixed order (rows r = l mod 32 by lane l in ascending order, then a fixed 32-lane tree);
+ *   - dz: the latent backward adds the slices in split order;
+ *   - loss: each (32-row block, 64-column group) of the MSE and of the KL term has one fp64 slot; the finalisation
+ *     adds the slots in index order (fixed thread partition and tree).
+ * Scratch layout (256-byte aligned sections, sized at max_batch): weight-gradient slices (the largest bucket's) |
+ * latent-dgrad slices | bias partial rows [rows32][total - b1] | latent bias rows [592 max][2Lp] | MSE slots
+ * [rows32][Sp/64] (fp64) | KL slots [rows32][Lp/64] (fp64), rows32 = max_batch rounded up to 256, over 32.
+ * Data parallelism is covered with the peer-load all-reduce (it sums the ranks in rank order); a step whose gradients
+ * go through NVLS multicast or NCCL returns 2, as do the experiments-only paths (RVAE_FUSE_LATENT, RVAE_MERGE_B3W,
+ * RVAE_FUSE_FORWARD). Only the training step is covered: rvae_plan_forward / _backward / _backward_external called
+ * on their own run the default kernels. rvae_plan_workspace_bytes is unchanged. */
+size_t rvae_plan_deterministic_bytes(const rvae_plan* plan);   /* scratch bytes at the plan's max_batch */
+/* Bind the caller-owned scratch (>= rvae_plan_deterministic_bytes, 256-byte aligned); NULL switches the mode off.
+ * Returns 1 for a short or misaligned scratch. */
+int rvae_plan_set_deterministic(rvae_plan* plan, void* scratch, size_t bytes);
+
 /* Evaluate the record's schedule at the n step indices k_dev[0..n) with the device function the training kernels
  * use: lr_out[i] = lr(k_dev[i]), beta_out[i] = (float)beta(k_dev[i]). Returns 1 for null pointers or n < 1 (before
  * ctx is used). */

@@ -119,6 +119,8 @@ SIGNATURES = {
     "rvae_plan_train_step": (c_int, [P, c_float, c_double, c_double, c_double, c_double, c_double, c_int, P, c_int, P]),
     "rvae_plan_train_step_hp": (c_int, [P, P, c_int, P, c_int, P]),
     "rvae_plan_set_grad_clip": (c_int, [P, P, P, c_int]),
+    "rvae_plan_deterministic_bytes": (c_size_t, [P]),
+    "rvae_plan_set_deterministic": (c_int, [P, P, c_size_t]),
     "rvae_plan_grad_norm": (c_int, [P, P, P]),
     "rvae_hparams_check": (c_int, [C.POINTER(Hparams)]),
     "rvae_hparams_eval": (c_int, [P, P, P, c_int, P, P, P]),

@@ -1,5 +1,6 @@
 // C ABI (include/rvae_b200.h): context, op-level entry points and the plan that issues a whole training or
 // inference step from C. No torch types cross this boundary.
+#include <algorithm>
 #include <cmath>
 #include <cstdlib>
 #include <dlfcn.h>
@@ -605,8 +606,9 @@ struct rvae_plan {
   // maps. 0 = the planes hold dense [count, S] rows (gather / tensor input).
   int x_pitch, x_pitch_alt;
   int* sched_dev;          // schedules of the fused launches: [2 input sets][6 launches][128 pairs][kSchedMax]
-  int sched_batch;         // the batch size those schedules were built for (0 = none yet): the buffer holds ONE set of
-                           // schedules, so other batch sizes of this plan (a ragged last batch) run separate launches
+  int sched_batch;         // sched_owner() of the GEMM set those schedules were built for (0 = none yet): the buffer
+                           // holds ONE set of schedules, so other batch sizes of this plan (a ragged last batch), and
+                           // the other mode (deterministic or not) of the same batch size, run separate launches
   unsigned int* dep_flags; // row-block counters of the chained forward launch: [3 layer transitions][256]
   bool fuse_forward;       // env RVAE_FUSE_FORWARD=1: forward pass as one chained launch (default off)
   bool fuse_latent;        // env RVAE_FUSE_LATENT: backward of reparameterize + KL inside the latent dgrad's epilogue
@@ -680,6 +682,13 @@ struct rvae_plan {
   // loss finalisation deferred into the latent backward kernel (rvae_plan_finish_loss_deferred)
   LossFinalize fin;
   bool fin_pending;
+  // deterministic mode (rvae_plan_set_deterministic): the caller's scratch, carved by det_carve; det_on while a
+  // training step enqueues its kernels
+  uint8_t* det_scratch;
+  bool det_on;
+  float *det_w, *det_dz, *det_bpart, *det_lpart;
+  double *det_mse, *det_kl;
+  size_t det_w_cap, det_dz_cap;
   std::map<int64_t, GemmSet> sets;  // prepared GEMMs per (batch size, input set, frame pitch)
   // optional per-GEMM timing
   bool timing;
@@ -735,6 +744,45 @@ size_t carve(rvae_plan* p, uint8_t* base) {
     p->ext_gmu = reinterpret_cast<float*>(take(B * L * 4));
     p->ext_glv = reinterpret_cast<float*>(take(B * L * 4));
     p->ext_lv = reinterpret_cast<float*>(take(B * L * 4));
+  }
+  return off;
+}
+
+// Scratch of deterministic mode at max_batch, in this order (256-byte aligned sections; layout in rvae_b200.h):
+//   weight-gradient slices (splits 1.., the largest of the four buckets' needs: one bucket's slices are summed before
+//   the next stage starts) | latent-dgrad slices | bias partial rows [rows32][total - b1] (b1 | b2 | b3 | b4 columns)
+//   | latent-backward bias partial rows [blocks][2L] | MSE slots [rows32][S/64] | KL slots [rows32][L/64] (fp64)
+// rows32 = max_batch rounded up to 256, over 32. With base == nullptr only sizes are computed.
+size_t det_carve(rvae_plan* p, uint8_t* base) {
+  const Ctx* c = &p->ctx->c;
+  const int B = p->max_batch, S = p->S, H = p->H, L = p->L;
+  size_t wf = 0, dzf = 0;
+  for (int kb = 1; (kb - 1) * kBlockK < B; ++kb) {   // weight gradients: K = the batch
+    const int K = std::min(kb * kBlockK, B);
+    wf = std::max({wf, det_slice_floats(c, S, H, K), det_slice_floats(c, H, L, K), det_slice_floats(c, 2 * L, H, K),
+                   det_slice_floats(c, H, S, K)});
+  }
+  for (int m = kBlockM;; m += kBlockM) {              // latent dgrad: M = the batch
+    const int M = std::min(m, B);
+    dzf = std::max(dzf, det_slice_floats(c, M, L, H));
+    if (M == B) break;
+  }
+  const size_t rows32 = (size_t)(B + 255) / 256 * 8;
+  size_t off = 0;
+  auto take = [&](size_t bytes) -> uint8_t* {
+    uint8_t* r = base ? base + off : nullptr;
+    off += align_up(bytes, 256);
+    return r;
+  };
+  float* w = reinterpret_cast<float*>(take(wf * 4));
+  float* dz = reinterpret_cast<float*>(take(dzf * 4));
+  float* bpart = reinterpret_cast<float*>(take(rows32 * (size_t)(p->lay.total - p->lay.b1) * 4));
+  float* lpart = reinterpret_cast<float*>(take((size_t)latent_det_blocks(B, L) * 2 * L * 4));
+  double* mse = reinterpret_cast<double*>(take(rows32 * (S / 64) * 8));
+  double* kl = reinterpret_cast<double*>(take(rows32 * (L / 64) * 8));
+  if (base) {
+    p->det_w = w; p->det_dz = dz; p->det_bpart = bpart; p->det_lpart = lpart; p->det_mse = mse; p->det_kl = kl;
+    p->det_w_cap = wf; p->det_dz_cap = dzf;
   }
   return off;
 }
@@ -848,6 +896,25 @@ int prepare(rvae_plan* p, GemmSet& gs, int id) {
     default:
       return set_error(RVAE_ERR_INVALID, "plan: bad gemm id %d", id);
   }
+  if (p->det_on) {
+    // deterministic kinds: partial sums to fixed scratch slots, summed in fixed order by the latent backward and the
+    // per-bucket grad_sum launches
+    const int64_t nbias = ly.total - ly.b1;
+    switch (id) {
+      case G_F2: d.epi = EPI_HEAD_DET; d.args.loss_acc = p->det_kl; break;
+      case G_F4_OUT:
+        d.epi = EPI_OUT_DET; d.args.loss_acc = p->det_mse;
+        d.args.colsum = p->det_bpart + (ly.b4 - ly.b1); d.args.ldp = (int)nbias;
+        break;
+      case G_B4D: d.epi = EPI_DRELU_DET; d.args.colsum = p->det_bpart + (ly.b3 - ly.b1); d.args.ldp = (int)nbias; break;
+      case G_B2D: d.epi = EPI_DRELU_DET; d.args.colsum = p->det_bpart; d.args.ldp = (int)nbias; break;
+      case G_B3D: d.epi = EPI_SLICE; d.args.out_f32_b = p->det_dz; d.slice_cap = p->det_dz_cap; break;
+      case G_B4W: case G_B3W: case G_B2W: case G_B1W:
+        d.epi = EPI_SLICE; d.args.out_f32_b = p->det_w; d.slice_cap = p->det_w_cap;
+        break;
+      default: break;
+    }
+  }
   RVAE_CHECK(gemm_prepare(&p->ctx->c, d, &gs.g[id]));
   gs.ready[id] = true;
   return RVAE_OK;
@@ -855,7 +922,8 @@ int prepare(rvae_plan* p, GemmSet& gs, int id) {
 
 int get_set(rvae_plan* p, GemmSet** out) {
   // tensor maps bake in the addresses of the current input set and the row pitch of its frames
-  const int64_t key = ((int64_t)p->batch * 2 + p->cur) * 65536 + p->x_pitch;
+  // (and whether the step is deterministic: other epilogue kinds, split counts and scratch maps)
+  const int64_t key = (((int64_t)p->batch * 2 + p->cur) * 65536 + p->x_pitch) * 2 + (p->det_on ? 1 : 0);
   auto it = p->sets.find(key);
   if (it == p->sets.end()) {
     GemmSet gs;
@@ -1098,7 +1166,10 @@ struct LatentExt {
 KlGrad plan_kl(const rvae_plan* p) { return KlGrad{p->hp_dev, p->bufs.step, p->kl_bl, p->kl_c0, p->hp_early}; }
 
 // Fused launches read their tile schedule from the plan's one schedule buffer: usable by the batch size that owns it.
-bool sched_usable(const rvae_plan* p) { return p->sched_batch == 0 || p->sched_batch == p->batch; }
+// The owner is the batch size AND the mode: the deterministic and the default GEMM sets of one batch size may differ
+// in their split counts (units), so they must not share schedules either.
+int sched_owner(const rvae_plan* p) { return 2 * p->batch + (p->det_on ? 1 : 0); }
+bool sched_usable(const rvae_plan* p) { return p->sched_batch == 0 || p->sched_batch == sched_owner(p); }
 
 // Stage 1 runs the reparameterisation / KL backward inside the latent dgrad's epilogue (bf16 mode, fused loss)
 bool latent_fused(const rvae_plan* p) {
@@ -1130,7 +1201,7 @@ int backward_stage_latent_fused(rvae_plan* p, cudaStream_t st) {
       const int rc = gemm_prepare_chain(&p->ctx->c, both, 2, pairs, sched, &gs->dual_lat);
       gs->dual_lat_state = rc == RVAE_OK ? 1 : -1;
       if (rc != RVAE_OK && rc != RVAE_ERR_UNSUPPORTED) return rc;
-      if (rc == RVAE_OK) p->sched_batch = p->batch;
+      if (rc == RVAE_OK) p->sched_batch = sched_owner(p);
     }
     if (gs->dual_lat_state == 1) {
       PreparedChain d = gs->dual_lat;
@@ -1145,7 +1216,76 @@ int backward_stage_latent_fused(rvae_plan* p, cudaStream_t st) {
   return run(p, G_B3W, st);
 }
 
+// The latent backward of stage 1 (after the latent dgrad filled dz); it carries the deferred loss finalisation.
+// Deterministic mode: dz's split slices are added in split order and the bias / loss partials go to fixed slots.
+int latent_launch(rvae_plan* p, const LatentExt* ext, cudaStream_t st) {
+  const rvae_layout& ly = p->lay;
+  int rc;
+  if (p->det_on) {
+    RVAE_REQUIRE(ext == nullptr, RVAE_ERR_STATE, "plan_backward: deterministic mode covers the fused loss only");
+    GemmSet* gs;
+    RVAE_CHECK(get_set(p, &gs));
+    const GemmParams& g = gs->g[G_B3D].params;
+    const int rows32 = (p->batch + 31) / 32;
+    LatentDet det;
+    det.dz_slices = p->det_dz;
+    det.dz_stride = (int64_t)g.epi.ldp * p->L;
+    det.n_dz_slices = g.k_splits - 1;
+    det.bias_part = p->det_lpart;
+    det.mse = p->det_mse;
+    det.kl = p->det_kl;
+    det.n_mse = rows32 * (p->S / 64);
+    det.n_kl = rows32 * (p->L / 64);
+    rc = launch_latent_bwd_det(&p->ctx->c, p->dz, p->eps, p->lv, p->mu, plan_kl(p), p->batch, p->L, p->dml.hi,
+                               p->dml.lo, det, p->fin_pending ? &p->fin : nullptr, st);
+  } else {
+    rc = launch_latent_bwd(&p->ctx->c, p->dz, p->eps, ext ? ext->lv : p->lv, p->mu, ext ? ext->g_mu : nullptr,
+                           ext ? ext->g_lv : nullptr, plan_kl(p), p->batch, p->L, p->dml.hi, p->dml.lo,
+                           p->bufs.grads + ly.b2, 1, p->fin_pending ? &p->fin : nullptr, st);
+  }
+  p->fin_pending = false;
+  p->dz_zeroed = !p->det_on;   // (the deterministic kernel reads dz and leaves it)
+  return rc;
+}
+
+// Deterministic mode, after backward stage s on `st`: gradient bucket s = split 0 + the scratch slices in split order;
+// after stage 2 also the bias block = the fixed-order sums of its partial rows (db4 from the forward, db3, db2, db1 from stages
+// 0..2), so every later reader (Adam, the norm, the all-reduce) sees complete gradients.
+int grad_sum_stage(rvae_plan* p, int stage, cudaStream_t st) {
+  static const int kWgrad[4] = {G_B4W, G_B3W, G_B2W, G_B1W};
+  const rvae_layout& ly = p->lay;
+  const int64_t woff[4] = {ly.w4, ly.w3, ly.w2, ly.w1};
+  float* grads = p->bufs.grads;
+  GemmSet* gs;
+  RVAE_CHECK(get_set(p, &gs));
+  const GemmParams& g = gs->g[kWgrad[stage]].params;
+  GradSum a;
+  memset(&a, 0, sizeof(a));
+  a.w = grads + woff[stage];
+  a.w_slices = p->det_w;
+  a.w_count = (int64_t)g.M * g.N;
+  a.w_slice_stride = (int64_t)g.epi.ldp * g.N;
+  a.n_slices = g.k_splits - 1;
+  if (stage == 2) {
+    const int rows32 = (p->batch + 31) / 32;
+    const int64_t nbias = ly.total - ly.b1;
+    a.seg[0] = {grads + ly.b1, p->det_bpart, nbias, p->H, rows32};
+    a.seg[1] = {grads + ly.b2, p->det_lpart, 2 * p->L, 2 * p->L, latent_det_blocks(p->batch, p->L)};
+    a.seg[2] = {grads + ly.b3, p->det_bpart + (ly.b3 - ly.b1), nbias, p->H, rows32};
+    a.seg[3] = {grads + ly.b4, p->det_bpart + (ly.b4 - ly.b1), nbias, p->S, rows32};
+    a.n_seg = 4;
+  }
+  return launch_grad_sum(&p->ctx->c, a, st);
+}
+
+int backward_stage_gemms(rvae_plan* p, int stage, const LatentExt* ext, cudaStream_t st);
+
 int backward_stage(rvae_plan* p, int stage, const LatentExt* ext, cudaStream_t st) {
+  RVAE_CHECK(backward_stage_gemms(p, stage, ext, st));
+  return p->det_on ? grad_sum_stage(p, stage, st) : RVAE_OK;
+}
+
+int backward_stage_gemms(rvae_plan* p, int stage, const LatentExt* ext, cudaStream_t st) {
   const int S = p->S, H = p->H, L = p->L;
   const rvae_layout& ly = p->lay;
   float* grads = p->bufs.grads;
@@ -1154,11 +1294,13 @@ int backward_stage(rvae_plan* p, int stage, const LatentExt* ext, cudaStream_t s
   RVAE_REQUIRE(stage >= 0 && stage < 4, RVAE_ERR_INVALID, "plan_backward: stage %d not in -1..3", stage);
   float* wptr[4] = {grads + ly.w4, grads + ly.w3, grads + ly.w2, grads + ly.w1};
   const size_t wcount[4] = {(size_t)S * H, (size_t)H * L, (size_t)2 * L * H, (size_t)H * S};
-  if (!p->grads_zeroed[stage]) RVAE_CUDA(cudaMemsetAsync(wptr[stage], 0, sizeof(float) * wcount[stage], st));
+  // (deterministic mode: split 0 stores the whole bucket)
+  if (!p->grads_zeroed[stage] && !p->det_on)
+    RVAE_CUDA(cudaMemsetAsync(wptr[stage], 0, sizeof(float) * wcount[stage], st));
   p->grads_zeroed[stage] = false;
   // stage 1, bf16 mode, fused loss: the reparameterisation / KL backward runs inside the latent dgrad's epilogue
   if (stage == 1 && ext == nullptr && latent_fused(p)) return backward_stage_latent_fused(p, st);
-  if (stage == 1 && !p->dz_zeroed)
+  if (stage == 1 && !p->dz_zeroed && !p->det_on)
     RVAE_CUDA(cudaMemsetAsync(p->dz, 0, sizeof(float) * (size_t)p->max_batch * L, st));
   auto stage_pairs = [&](int st_idx) {
     // under data parallelism the fused launches leave the same spare SMs as the single GEMMs do: the exchange kernels
@@ -1184,18 +1326,14 @@ int backward_stage(rvae_plan* p, int stage, const LatentExt* ext, cudaStream_t s
       const int rc = gemm_prepare_chain(&p->ctx->c, three, 3, stage_pairs(2), sched, &gs->tri);
       gs->tri_state = rc == RVAE_OK ? 1 : -1;
       if (rc != RVAE_OK && rc != RVAE_ERR_UNSUPPORTED) return rc;
-      if (rc == RVAE_OK) p->sched_batch = p->batch;
+      if (rc == RVAE_OK) p->sched_batch = sched_owner(p);
     }
     if (gs->tri_state == 1) {
       RVAE_CHECK(run(p, G_B3D, st));
       {
         TimedScope ts(p, T_LATENT, st);
-        RVAE_CHECK(launch_latent_bwd(&p->ctx->c, p->dz, p->eps, ext ? ext->lv : p->lv, p->mu, ext ? ext->g_mu : nullptr,
-                                     ext ? ext->g_lv : nullptr, plan_kl(p), p->batch, L, p->dml.hi, p->dml.lo, grads + ly.b2,
-                                     1, p->fin_pending ? &p->fin : nullptr, st));
+        RVAE_CHECK(latent_launch(p, ext, st));
       }
-      p->fin_pending = false;
-      p->dz_zeroed = true;
       p->b3w_deferred = true;
       return RVAE_OK;
     }
@@ -1228,12 +1366,7 @@ int backward_stage(rvae_plan* p, int stage, const LatentExt* ext, cudaStream_t s
       RVAE_CHECK(gemm_run(&p->ctx->c, w, st));
     }
     TimedScope ts(p, T_LATENT, st);
-    RVAE_CHECK(launch_latent_bwd(&p->ctx->c, p->dz, p->eps, ext ? ext->lv : p->lv, p->mu, ext ? ext->g_mu : nullptr,
-                                 ext ? ext->g_lv : nullptr, plan_kl(p), p->batch, L, p->dml.hi, p->dml.lo, grads + ly.b2, 1,
-                                 p->fin_pending ? &p->fin : nullptr, st));
-    p->fin_pending = false;
-    p->dz_zeroed = true;
-    return RVAE_OK;
+    return latent_launch(p, ext, st);
   }
   if (stage == 1 && p->split_stage1 && p->two_streams && !p->timing && p->batch > kBlockM) {
     // latent dgrad, then the latent backward kernel (HBM-bound, feeds stage 2: the critical chain) on `st` while the fc3
@@ -1259,16 +1392,10 @@ int backward_stage(rvae_plan* p, int stage, const LatentExt* ext, cudaStream_t s
       if (w.grid > cap) w.grid = cap;
       return gemm_run(&p->ctx->c, w, s_w);
     };
-    auto run_latent = [&]() -> int {
-      return launch_latent_bwd(&p->ctx->c, p->dz, p->eps, ext ? ext->lv : p->lv, p->mu, ext ? ext->g_mu : nullptr,
-                               ext ? ext->g_lv : nullptr, plan_kl(p), p->batch, L, p->dml.hi, p->dml.lo, grads + ly.b2, 1,
-                               p->fin_pending ? &p->fin : nullptr, s_l);
-    };
+    auto run_latent = [&]() -> int { return latent_launch(p, ext, s_l); };
     if (p->s1_order == 0) { RVAE_CHECK(run_wgrad()); RVAE_CHECK(run_latent()); }
     else { RVAE_CHECK(run_latent()); RVAE_CHECK(run_wgrad()); }
     RVAE_CUDA(cudaEventRecord(p->ev_s1_join, p->hp2));
-    p->fin_pending = false;
-    p->dz_zeroed = true;
     RVAE_CUDA(cudaStreamWaitEvent(st, p->ev_s1_join, 0));
     return RVAE_OK;
   }
@@ -1287,7 +1414,7 @@ int backward_stage(rvae_plan* p, int stage, const LatentExt* ext, cudaStream_t s
       const int rc = gemm_prepare_chain(&p->ctx->c, both, 2, pairs, sched, &gs->dual[stage]);
       gs->dual_state[stage] = rc == RVAE_OK ? 1 : -1;
       if (rc != RVAE_OK && rc != RVAE_ERR_UNSUPPORTED) return rc;
-      if (rc == RVAE_OK) p->sched_batch = p->batch;
+      if (rc == RVAE_OK) p->sched_batch = sched_owner(p);
     }
     if (gs->dual_state[stage] == 1) {
       // per-kernel timing: the fused launch IS the kernel of this stage - its time and the flops of both problems are
@@ -1305,11 +1432,7 @@ int backward_stage(rvae_plan* p, int stage, const LatentExt* ext, cudaStream_t s
   if (!fused && kDgrad[stage] >= 0) RVAE_CHECK(run(p, kDgrad[stage], st));
   if (stage == 1) {
     TimedScope ts(p, T_LATENT, st);
-    RVAE_CHECK(launch_latent_bwd(&p->ctx->c, p->dz, p->eps, ext ? ext->lv : p->lv, p->mu, ext ? ext->g_mu : nullptr,
-                                 ext ? ext->g_lv : nullptr, plan_kl(p), p->batch, L, p->dml.hi, p->dml.lo, grads + ly.b2, 1,
-                                 p->fin_pending ? &p->fin : nullptr, st));
-    p->fin_pending = false;
-    p->dz_zeroed = true;
+    RVAE_CHECK(latent_launch(p, ext, st));
   }
   return fused ? RVAE_OK : run(p, kWgrad[stage], st);
 }
@@ -1339,6 +1462,9 @@ int rvae_plan_create(rvae_ctx* ctx, int S, int H, int L, int max_batch, int prec
   p->x_pitch = 0; p->x_pitch_alt = 0;
   p->fuse_latent = false;
   p->sched_batch = 0;
+  p->det_scratch = nullptr; p->det_on = false;
+  p->det_w = p->det_dz = p->det_bpart = p->det_lpart = nullptr; p->det_mse = p->det_kl = nullptr;
+  p->det_w_cap = p->det_dz_cap = 0;
   memset(&p->pf, 0, sizeof(p->pf));
   for (int i = 0; i < 5; ++i) p->grads_zeroed[i] = false;
   p->streams_ready = false; p->ev_fork = nullptr;
@@ -1442,6 +1568,32 @@ int rvae_plan_read_timing(rvae_plan* plan, float* ms, int64_t* launches, double*
 }
 
 size_t rvae_plan_workspace_bytes(const rvae_plan* plan) { return plan ? plan->ws_bytes : 0; }
+
+size_t rvae_plan_deterministic_bytes(const rvae_plan* plan) {
+  return plan ? det_carve(const_cast<rvae_plan*>(plan), nullptr) : 0;   // (sizes only: the plan is not modified)
+}
+
+int rvae_plan_set_deterministic(rvae_plan* plan, void* scratch, size_t bytes) {
+  RVAE_REQUIRE(plan, RVAE_ERR_INVALID, "null rvae_plan");
+  if (scratch == nullptr) {
+    plan->det_scratch = nullptr;
+    return RVAE_OK;
+  }
+  const size_t need = det_carve(plan, nullptr);
+  RVAE_REQUIRE(bytes >= need, RVAE_ERR_INVALID, "plan_set_deterministic: %zu bytes of scratch, %zu needed", bytes, need);
+  RVAE_REQUIRE((reinterpret_cast<uintptr_t>(scratch) & 255) == 0, RVAE_ERR_INVALID,
+               "plan_set_deterministic: scratch must be 256-byte aligned");
+  uint8_t* s = reinterpret_cast<uint8_t*>(scratch);
+  if (plan->det_w != nullptr && s != reinterpret_cast<uint8_t*>(plan->det_w) && !plan->sets.empty()) {
+    // prepared deterministic GEMMs bake in the old scratch: rebuild them - once nothing in flight reads it
+    RVAE_CUDA(cudaDeviceSynchronize());
+    plan->sets.clear();
+    plan->sched_batch = 0;
+  }
+  det_carve(plan, s);
+  plan->det_scratch = s;
+  return RVAE_OK;
+}
 
 int rvae_plan_bind(rvae_plan* plan, const rvae_plan_buffers* b) {
   RVAE_REQUIRE(plan && b, RVAE_ERR_INVALID, "plan_bind: null argument");
@@ -1650,7 +1802,7 @@ int rvae_plan_forward(rvae_plan* plan, float kl_beta, int fused_loss, int want_x
       const int rc = gemm_prepare_chain(&p->ctx->c, layers, 4, fpairs, sched, &gs->fwd, p->dep_flags);
       gs->fwd_state = rc == RVAE_OK ? 1 : -1;
       if (rc != RVAE_OK && rc != RVAE_ERR_UNSUPPORTED) return rc;
-      if (rc == RVAE_OK) p->sched_batch = p->batch;
+      if (rc == RVAE_OK) p->sched_batch = sched_owner(p);
     }
     if (gs->fwd_state == 1) {
       p->kl_c0 = (float)((double)kl_beta / BL);
@@ -1868,6 +2020,27 @@ static int train_step(rvae_plan* plan, float kl_beta, const HpArg& hp, int zero_
   // The step counter t (Adam's bias correction, the loss-ring slot, the Philox offset) stays at its old value for
   // the whole step: every Adam launch uses t + 1, and the last block of the final launch advances it.
   const bool fork = plan->two_streams && !plan->timing;
+  if (plan->det_scratch != nullptr) {
+    // deterministic mode: refused before anything is enqueued where a path has no deterministic form
+    RVAE_REQUIRE(!plan->fuse_latent && !plan->merge_b3w && !plan->fuse_forward, RVAE_ERR_UNSUPPORTED,
+                 "plan_train_step: deterministic mode does not cover the experiments paths RVAE_FUSE_LATENT, "
+                 "RVAE_MERGE_B3W and RVAE_FUSE_FORWARD");
+    const rvae_ctx* cx = plan->ctx;
+    if (fork && plan->dp_enabled && (cx->comm != nullptr || cx->p2p_ready) && cx->dp_world > 1) {
+      const uint8_t* g0 = reinterpret_cast<const uint8_t*>(b.grads);
+      const bool peer = cx->p2p_ready && cx->sym_base != nullptr && g0 >= cx->sym_base + kP2PFlagBytes &&
+                        g0 + sizeof(float) * (size_t)plan->lay.total <= cx->sym_base + kP2PFlagBytes + cx->sym_data_bytes;
+      RVAE_REQUIRE(peer && cx->p2p.mc_data == nullptr, RVAE_ERR_UNSUPPORTED,
+                   "plan_train_step: deterministic mode needs the peer-load all-reduce (it sums the ranks in rank "
+                   "order); this plan's gradients are exchanged by %s, which gives no order guarantee",
+                   peer ? "NVLS multicast" : "NCCL");
+    }
+  }
+  struct DetGuard {   // the deterministic kinds are enqueued by this call only
+    rvae_plan* p;
+    explicit DetGuard(rvae_plan* p_) : p(p_) { p->det_on = p->det_scratch != nullptr; }
+    ~DetGuard() { p->det_on = false; }
+  } det_guard(plan);
   // Gradient clipping: the global norm depends on every bucket and Adam is nonlinear in g, so no bucket is updated
   // before the norm is known. Each bucket's norm partial takes the place of its background Adam launch; the last one
   // finalises the clipping factor, and one Adam launch over all buckets reads it.

@@ -114,6 +114,7 @@ struct GemmDesc {
   int head_L;    // EPI_HEAD: latent width L (B holds 2L stacked rows, N must equal 2L)
   int k_splits;  // EPI_WGRAD: requested split-K (0 = choose)
   int side_cols; // EPI_OUT: > 0 = columns of the side input x that are data (as Operand::cols); 0 = N
+  size_t slice_cap;  // EPI_SLICE: fp32 elements of the scratch args.out_f32_b (splits 1..)
 };
 
 struct PreparedGemm {
@@ -127,6 +128,8 @@ struct PreparedGemm {
   int a_major, b_major, cg;
   int out_rows, out_cols_bf16, out_ld_bf16, out_cols_f32, out_ld_f32;
   int side_cols;  // GemmDesc::side_cols
+  int kind;       // the kernel's epilogue kind (epi is what it computes: epi_base(kind))
+  int slice_rows; // EPI_SLICE: rows of the scratch slices (splits 1..), 0 = one split
 };
 
 int gemm_bind_outputs(PreparedGemm* g, const EpiArgs& args, bool force);
@@ -151,6 +154,8 @@ int gemm_prepare_chain(const Ctx* ctx, const PreparedGemm* const* g, int count, 
 int gemm_run_chain(Ctx* ctx, const PreparedChain& g, cudaStream_t stream);
 
 int gemm_prepare(const Ctx* ctx, const GemmDesc& d, PreparedGemm* out);
+// fp32 elements of the scratch slices an EPI_SLICE GEMM [M, N] x K stores (0 for one split)
+size_t det_slice_floats(const Ctx* ctx, int M, int N, int K);
 int gemm_run(Ctx* ctx, const PreparedGemm& g, cudaStream_t stream);
 int gemm_launch(Ctx* ctx, const GemmDesc& d, cudaStream_t stream);  // prepare + run
 
@@ -280,5 +285,41 @@ int launch_latent_bwd(Ctx* ctx, float* dz, const float* eps, const float* lv, co
                       const float* g_lv_ext, const KlGrad& kl, int64_t M, int L, __nv_bfloat16* dml_hi,
                       __nv_bfloat16* dml_lo, float* bias_grad, int clear_dz, const LossFinalize* fin,
                       cudaStream_t stream);
+
+// Deterministic mode (rvae_plan_set_deterministic). A gradient bucket's sum, in fixed order:
+//   w[i] += slice_1[i] + ... + slice_{n_slices}[i]   (slice k at w_slices + (k - 1) * w_slice_stride; split 0 is w)
+//   bias segment s: dst[c] = sum over r < rows of src[r * pitch + c]: lane l of a warp adds rows l, l + 32, ... in
+//   ascending order, then the 32 lane sums meet in a fixed xor-butterfly tree
+struct GradSumSeg {
+  float* dst;
+  const float* src;
+  int64_t pitch;
+  int cols, rows;
+};
+struct GradSum {
+  float* w;
+  const float* w_slices;
+  int64_t w_count, w_slice_stride;
+  int n_slices;
+  GradSumSeg seg[4];
+  int n_seg;
+};
+int launch_grad_sum(Ctx* ctx, const GradSum& a, cudaStream_t stream);
+// The latent backward of a deterministic step: dz = dz + dz_slices[0] + ... (split order, slices at dz_stride
+// floats), the column sums of d_ml per block -> bias_part[block][2L] (grid latent_det_blocks), and the loss
+// finalisation from the fixed loss slots: acc = {sum mse[0, n_mse), sum kl[0, n_kl)} in index order.
+struct LatentDet {
+  const float* dz_slices;
+  int64_t dz_stride;
+  int n_dz_slices;
+  float* bias_part;
+  const double* mse;
+  const double* kl;
+  int n_mse, n_kl;
+};
+int latent_det_blocks(int64_t M, int L);
+int launch_latent_bwd_det(Ctx* ctx, float* dz, const float* eps, const float* lv, const float* mu, const KlGrad& kl,
+                          int64_t M, int L, __nv_bfloat16* dml_hi, __nv_bfloat16* dml_lo, const LatentDet& det,
+                          const LossFinalize* fin, cudaStream_t stream);
 
 }  // namespace rvae

@@ -1336,11 +1336,16 @@ __device__ __forceinline__ float latent_kl_c(const KlGrad& kl) {
   return static_cast<float>(__ddiv_rn(static_cast<double>(beta), kl.bl));
 }
 
-__global__ void latent_bwd_kernel(float* __restrict__ dz, const float* __restrict__ eps, const float* __restrict__ lv,
-                                  const float* __restrict__ mu, const float* __restrict__ g_mu_ext,
-                                  const float* __restrict__ g_lv_ext, KlGrad kl, int64_t M, int L,
-                                  __nv_bfloat16* __restrict__ dml_hi, __nv_bfloat16* __restrict__ dml_lo,
-                                  float* __restrict__ bias_grad, int clear_dz, LossFinalize fin, AuxTrace tr) {
+// kDet (launch_latent_bwd_det): dz is the sum of its split-K slices in split order, the block's column sums go to its
+// own row of det.bias_part, and the loss is finalised from the fixed loss slots - no atomics anywhere.
+template <bool kDet>
+__device__ __forceinline__ void latent_bwd_body(float* __restrict__ dz, const float* __restrict__ eps,
+                                                const float* __restrict__ lv, const float* __restrict__ mu,
+                                                const float* __restrict__ g_mu_ext, const float* __restrict__ g_lv_ext,
+                                                const KlGrad& kl, int64_t M, int L, __nv_bfloat16* __restrict__ dml_hi,
+                                                __nv_bfloat16* __restrict__ dml_lo, float* __restrict__ bias_grad,
+                                                int clear_dz, const LossFinalize& fin, const AuxTrace& tr,
+                                                const LatentDet& det) {
   ptx::pdl_launch_dependents();
   // c = (float)(beta(k) / (B L)), as the host rounds it for a kl_beta argument. kl.early: evaluated before
   // griddepcontrol.wait, overlapping the previous kernel (see rvae_plan_train_step_hp for why that is safe)
@@ -1349,8 +1354,30 @@ __global__ void latent_bwd_kernel(float* __restrict__ dz, const float* __restric
   ptx::pdl_wait();
   aux_begin(tr, 3);
   // the deferred loss finalisation of this step rides along (the forward that filled the sums is long complete)
-  if (fin.acc != nullptr && blockIdx.x == 0 && threadIdx.x == 0)
-    loss_finalize_body(fin.acc, fin.inv_rec, loss_kl_scale(fin), fin.loss_out, fin.ring_size, fin.step, fin.inc_step);
+  if constexpr (kDet) {
+    if (fin.acc != nullptr && blockIdx.x == 0) {
+      // the slots in index order: a fixed partition over the threads, then a fixed tree
+      __shared__ double red[2][32];
+      double a = 0.0, b = 0.0;
+      for (int i = threadIdx.x; i < det.n_mse; i += blockDim.x) a += det.mse[i];
+      for (int i = threadIdx.x; i < det.n_kl; i += blockDim.x) b += det.kl[i];
+      a = warp_sum_f64(a);
+      b = warp_sum_f64(b);
+      if ((threadIdx.x & 31) == 0) { red[0][threadIdx.x >> 5] = a; red[1][threadIdx.x >> 5] = b; }
+      __syncthreads();
+      if (threadIdx.x == 0) {
+        double ta = 0.0, tb = 0.0;
+        for (int w = 0; w < (int)(blockDim.x + 31) / 32; ++w) { ta += red[0][w]; tb += red[1][w]; }
+        fin.acc[0] = ta;
+        fin.acc[1] = tb;
+        loss_finalize_body(fin.acc, fin.inv_rec, loss_kl_scale(fin), fin.loss_out, fin.ring_size, fin.step,
+                           fin.inc_step);
+      }
+    }
+  } else {
+    if (fin.acc != nullptr && blockIdx.x == 0 && threadIdx.x == 0)
+      loss_finalize_body(fin.acc, fin.inv_rec, loss_kl_scale(fin), fin.loss_out, fin.ring_size, fin.step, fin.inc_step);
+  }
   float c = kl.c;
   if (kl.hp != nullptr) {
     if (!kl.early && threadIdx.x == 0) s_c = latent_kl_c(kl);
@@ -1378,6 +1405,12 @@ __global__ void latent_bwd_kernel(float* __restrict__ dz, const float* __restric
       idx[u] = (size_t)(ok[u] ? r : 0) * q + cx;
       if (ok[u]) {
         d4[u] = __ldcs(reinterpret_cast<const float4*>(dz) + idx[u]);
+        if constexpr (kDet) {
+          for (int k = 0; k < det.n_dz_slices; ++k) {   // split order
+            const float4 t = __ldcs(reinterpret_cast<const float4*>(det.dz_slices + k * det.dz_stride) + idx[u]);
+            d4[u].x += t.x; d4[u].y += t.y; d4[u].z += t.z; d4[u].w += t.w;
+          }
+        }
         e4[u] = __ldcs(reinterpret_cast<const float4*>(eps) + idx[u]);
         l4[u] = __ldcs(reinterpret_cast<const float4*>(lv) + idx[u]);
         b4[u] = make_float4(0.f, 0.f, 0.f, 0.f);  // additive term of d_lv
@@ -1437,10 +1470,28 @@ __global__ void latent_bwd_kernel(float* __restrict__ dz, const float* __restric
     for (int col = threadIdx.x; col < 2 * L; col += blockDim.x) {
       float t = 0.f;
       for (int y = 0; y < rpp; ++y) t += s_sum[(size_t)y * 2 * L + col];
-      atomicAdd(bias_grad + col, t);
+      if constexpr (kDet) bias_grad[(size_t)blockIdx.x * 2 * L + col] = t;
+      else atomicAdd(bias_grad + col, t);
     }
   }
   aux_end(tr);
+}
+
+__global__ void latent_bwd_kernel(float* __restrict__ dz, const float* __restrict__ eps, const float* __restrict__ lv,
+                                  const float* __restrict__ mu, const float* __restrict__ g_mu_ext,
+                                  const float* __restrict__ g_lv_ext, KlGrad kl, int64_t M, int L,
+                                  __nv_bfloat16* __restrict__ dml_hi, __nv_bfloat16* __restrict__ dml_lo,
+                                  float* __restrict__ bias_grad, int clear_dz, LossFinalize fin, AuxTrace tr) {
+  const LatentDet none = {};
+  latent_bwd_body<false>(dz, eps, lv, mu, g_mu_ext, g_lv_ext, kl, M, L, dml_hi, dml_lo, bias_grad, clear_dz, fin, tr,
+                         none);
+}
+
+__global__ void latent_bwd_det_kernel(float* __restrict__ dz, const float* __restrict__ eps,
+                                      const float* __restrict__ lv, const float* __restrict__ mu, KlGrad kl, int64_t M,
+                                      int L, __nv_bfloat16* __restrict__ dml_hi, __nv_bfloat16* __restrict__ dml_lo,
+                                      LossFinalize fin, AuxTrace tr, LatentDet det) {
+  latent_bwd_body<true>(dz, eps, lv, mu, nullptr, nullptr, kl, M, L, dml_hi, dml_lo, det.bias_part, 0, fin, tr, det);
 }
 
 int launch_latent_bwd(Ctx* ctx, float* dz, const float* eps, const float* lv, const float* mu, const float* g_mu_ext,
@@ -1470,6 +1521,132 @@ int launch_latent_bwd(Ctx* ctx, float* dz, const float* eps, const float* lv, co
   if (fin) f = *fin;
   RVAE_CUDA(launch_kernel(ctx, latent_bwd_kernel, dim3(grid), dim3(threads), smem, stream, dz, eps, lv, mu, g_mu_ext,
                           g_lv_ext, kl, M, L, dml_hi, dml_lo, bias_grad, clear_dz, f, next_aux(ctx, 3)));
+  RVAE_LAUNCH_CHECK(ctx);
+  return RVAE_OK;
+}
+
+// The deterministic launch's grid: four blocks per SM of a B200 whatever the SM budget, so the rows each block sums,
+// and with them the bits of its column sums, depend on the shapes alone.
+int latent_det_blocks(int64_t M, int L) {
+  const int q = L / 4;
+  const int rpp = q >= 256 ? 1 : 256 / q;
+  const int64_t want = (M + rpp - 1) / rpp;
+  return (int)(want < 148 * 4 ? want : 148 * 4);
+}
+
+int launch_latent_bwd_det(Ctx* ctx, float* dz, const float* eps, const float* lv, const float* mu, const KlGrad& kl,
+                          int64_t M, int L, __nv_bfloat16* dml_hi, __nv_bfloat16* dml_lo, const LatentDet& det,
+                          const LossFinalize* fin, cudaStream_t stream) {
+  RVAE_REQUIRE(kl.hp == nullptr || (kl.step != nullptr && (fin == nullptr || !fin->inc_step)), RVAE_ERR_INVALID,
+               "latent_bwd: a record needs a step counter that stays put during the launch");
+  RVAE_REQUIRE(dz && eps && lv && mu && dml_hi && det.bias_part && (det.n_dz_slices == 0 || det.dz_slices),
+               RVAE_ERR_INVALID, "latent_bwd_det: null buffer");
+  RVAE_REQUIRE(fin == nullptr || (det.mse && det.kl), RVAE_ERR_INVALID, "latent_bwd_det: no loss slots");
+  RVAE_REQUIRE(L > 0 && L % 4 == 0 && L / 4 <= 1024, RVAE_ERR_UNSUPPORTED, "latent_bwd: latent_dim=%d", L);
+  if (M <= 0) return RVAE_OK;
+  const int q = L / 4;
+  const int rpp = q >= 256 ? 1 : 256 / q;
+  LossFinalize f;
+  memset(&f, 0, sizeof(f));
+  if (fin) f = *fin;
+  RVAE_CUDA(launch_kernel(ctx, latent_bwd_det_kernel, dim3(latent_det_blocks(M, L)), dim3(q * rpp),
+                          (size_t)rpp * 2 * L * sizeof(float), stream, dz, eps, lv, mu, kl, M, L, dml_hi, dml_lo, f,
+                          next_aux(ctx, 3), det));
+  RVAE_LAUNCH_CHECK(ctx);
+  return RVAE_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Sum of one gradient bucket in deterministic mode (GradSum in common.h): the weight gradient's split-K slices added
+// to split 0 in split order (one thread per float4), and the bias partial rows of each column in a fixed order (one
+// warp per float4 of columns: lane-strided rows, then a butterfly tree). Neither the grid nor the SM budget enters
+// the order of any sum; HBM-bound (float4 loads, grid a multiple of the SM count).
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) grad_sum_kernel(const __grid_constant__ GradSum a) {
+  ptx::pdl_launch_dependents();
+  ptx::pdl_wait();
+  const int64_t tid = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  const int64_t nthreads = (int64_t)gridDim.x * blockDim.x;
+  // weights: one thread per float4, the slices in split order
+  const int64_t nw = a.n_slices > 0 ? a.w_count >> 2 : 0;
+  for (int64_t i = tid; i < nw; i += nthreads) {
+    float4 v = reinterpret_cast<const float4*>(a.w)[i];
+    for (int k = 0; k < a.n_slices; ++k) {
+      const float4 t = __ldcs(reinterpret_cast<const float4*>(a.w_slices + k * a.w_slice_stride) + i);
+      v.x += t.x; v.y += t.y; v.z += t.z; v.w += t.w;
+    }
+    reinterpret_cast<float4*>(a.w)[i] = v;
+  }
+  // biases: one WARP per float4 of columns. Lane l adds rows l, l + 32, l + 64, ... in ascending order, then the
+  // lanes' sums meet in a fixed butterfly tree: a fixed order whatever the grid, and 32 times the loads in flight of
+  // a thread walking every row alone
+  int64_t nb[4];
+  int64_t nbt = 0;
+#pragma unroll
+  for (int s = 0; s < 4; ++s) { nb[s] = s < a.n_seg ? a.seg[s].cols >> 2 : 0; nbt += nb[s]; }
+  const int lane = threadIdx.x & 31;
+  for (int64_t wi = tid >> 5; wi < nbt; wi += nthreads >> 5) {
+    int64_t j = wi;
+    GradSumSeg g = a.seg[0];
+    bool found = false;
+#pragma unroll
+    for (int s = 0; s < 4; ++s) {   // (unrolled: no dynamically indexed copy of the segment table)
+      if (!found && j < nb[s]) { g = a.seg[s]; found = true; }
+      else if (!found) j -= nb[s];
+    }
+    constexpr int kBatch = 4;
+    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int r0 = lane; r0 < g.rows; r0 += 32 * kBatch) {
+      float4 t[kBatch];
+#pragma unroll
+      for (int u = 0; u < kBatch; ++u) {
+        const int r = r0 + 32 * u;
+        t[u] = r < g.rows ? __ldcs(reinterpret_cast<const float4*>(g.src + r * g.pitch) + j)
+                          : make_float4(0.f, 0.f, 0.f, 0.f);
+      }
+#pragma unroll
+      for (int u = 0; u < kBatch; ++u) {
+        if (r0 + 32 * u < g.rows) { v.x += t[u].x; v.y += t[u].y; v.z += t[u].z; v.w += t[u].w; }
+      }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      v.x += __shfl_xor_sync(0xffffffffu, v.x, o);
+      v.y += __shfl_xor_sync(0xffffffffu, v.y, o);
+      v.z += __shfl_xor_sync(0xffffffffu, v.z, o);
+      v.w += __shfl_xor_sync(0xffffffffu, v.w, o);
+    }
+    if (lane == 0) reinterpret_cast<float4*>(g.dst)[j] = v;
+  }
+}
+
+int launch_grad_sum(Ctx* ctx, const GradSum& a, cudaStream_t stream) {
+  RVAE_REQUIRE(a.n_seg >= 0 && a.n_seg <= 4, RVAE_ERR_INVALID, "grad_sum: %d segments", a.n_seg);
+  uintptr_t align = reinterpret_cast<uintptr_t>(a.w) | reinterpret_cast<uintptr_t>(a.w_slices) |
+                    (uintptr_t)(a.w_count | a.w_slice_stride);
+  for (int s = 0; s < a.n_seg; ++s) {
+    const GradSumSeg& g = a.seg[s];
+    RVAE_REQUIRE(g.dst && g.src && g.rows >= 0, RVAE_ERR_INVALID, "grad_sum: bad bias segment %d", s);
+    align |= reinterpret_cast<uintptr_t>(g.dst) | reinterpret_cast<uintptr_t>(g.src) | (uintptr_t)(g.pitch | g.cols);
+  }
+  RVAE_REQUIRE((align & 3) == 0 && ((reinterpret_cast<uintptr_t>(a.w) | reinterpret_cast<uintptr_t>(a.w_slices)) & 15) == 0,
+               RVAE_ERR_INVALID, "grad_sum: buffers must be 16-byte aligned multiples of 4 elements");
+  RVAE_REQUIRE(a.n_slices == 0 || (a.w && a.w_slices), RVAE_ERR_INVALID, "grad_sum: null weight buffer");
+  for (int s = 0; s < a.n_seg; ++s)
+    RVAE_REQUIRE(((reinterpret_cast<uintptr_t>(a.seg[s].dst) | reinterpret_cast<uintptr_t>(a.seg[s].src)) & 15) == 0,
+                 RVAE_ERR_INVALID, "grad_sum: bias segments must be 16-byte aligned");
+  const int64_t nwork = (a.n_slices > 0 ? a.w_count / 4 : 0) + [&] {
+    int64_t t = 0;
+    for (int s = 0; s < a.n_seg; ++s) t += a.seg[s].cols / 4 * 32;   // a warp per float4 of bias columns
+    return t;
+  }();
+  const int threads = 256;
+  // a multiple of the SM count: one to four blocks per SM, by size (every thread covers >= one float4)
+  const int64_t per_sm = (int64_t)threads;
+  const int64_t blocks = std::min<int64_t>(4, std::max<int64_t>(1, (nwork + per_sm * ctx->num_sms_total - 1) /
+                                                                    (per_sm * ctx->num_sms_total)));
+  RVAE_CUDA(launch_kernel(ctx, grad_sum_kernel, dim3((unsigned)(blocks * ctx->num_sms_total)), dim3(threads),
+                          (size_t)0, stream, a));
   RVAE_LAUNCH_CHECK(ctx);
   return RVAE_OK;
 }

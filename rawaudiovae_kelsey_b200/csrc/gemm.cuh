@@ -52,6 +52,20 @@ constexpr int kSlotsPerTeam = 3;
 
 enum : int { MAJOR_K = 0, MAJOR_MN = 1 };
 enum : int { EPI_LINEAR = 0, EPI_HEAD = 1, EPI_OUT = 2, EPI_DRELU = 3, EPI_REDUCE = 5, EPI_DLATENT = 6 };
+// Deterministic kinds (rvae_plan_set_deterministic): the same epilogues with every cross-CTA or cross-warp sum moved
+// to fixed scratch slots, so the bits of a result never depend on which CTA ran which tile or in what order.
+//   SLICE      : REDUCE with a plain store per split: split 0 -> out_f32, split k >= 1 -> out_f32_b rows
+//                (k - 1) * ldp + m (ldp = the slice stride, rows)
+//   HEAD_DET   : HEAD; the KL partial of each (32-row block r, 64-latent-column group c) -> loss_acc[r * L/64 + c]
+//   OUT_DET    : OUT; the MSE partial of each (32-row block r, 64-column group c) -> loss_acc[r * N/64 + c], and the
+//                column sums of each warp's 32 rows -> colsum[r * ldp + n] (no atomics)
+//   DRELU_DET  : DRELU with the column sums as in OUT_DET
+enum : int { EPI_SLICE = 7, EPI_HEAD_DET = 8, EPI_OUT_DET = 9, EPI_DRELU_DET = 10 };
+__host__ __device__ constexpr int epi_base(int e) {
+  return e == EPI_SLICE ? EPI_REDUCE : e == EPI_HEAD_DET ? EPI_HEAD : e == EPI_OUT_DET ? EPI_OUT
+       : e == EPI_DRELU_DET ? EPI_DRELU : e;
+}
+__host__ __device__ constexpr bool epi_det(int e) { return e >= EPI_SLICE; }
 enum : int { ACT_NONE = 0, ACT_RELU = 1, ACT_TANH = 2, ACT_TANH_APPROX = 3 };
 
 // Epilogue arguments. Slot meaning per epilogue kind:
@@ -84,6 +98,7 @@ struct EpiArgs {
   int L;     // HEAD latent width
   int accumulate;
   float c0;
+  int ldp;   // deterministic kinds: SLICE slice stride (rows); OUT_DET / DRELU_DET row pitch of the colsum partials
 };
 
 struct alignas(64) GemmParams {
@@ -586,7 +601,8 @@ struct EpiState {
 template <class KD, int BLOCK_N, int CG>
 __device__ __forceinline__ void epilogue_unit(const GemmParams& p, int u, EpiState& es, const Shared& sh, int titer) {
   using Cfg = GemmCfg<BLOCK_N, CG>;
-  constexpr int EPI = KD::EPI;
+  constexpr int EPI = epi_base(KD::EPI);
+  constexpr bool kDet = epi_det(KD::EPI);
   const EpiArgs& e = p.epi;
   Team& tm = es.tm;
   const int team = es.team, row = es.row, team_tid = es.team_tid, lane = es.lane;
@@ -601,7 +617,8 @@ __device__ __forceinline__ void epilogue_unit(const GemmParams& p, int u, EpiSta
   const int m = m0 + row;
   const bool row_ok = m < p.M;
   const uint32_t t_acc = sh.tmem_base + es.lane_base + as * BLOCK_N;
-  (void)lane; (void)tr; (void)dual; (void)row_ok; (void)m;
+  const int r32 = m0 / 32 + es.quarter;   // deterministic kinds: this warp's 32-row block of the problem
+  (void)lane; (void)tr; (void)dual; (void)row_ok; (void)m; (void)r32;
 
       if constexpr (EPI == EPI_HEAD) {
         // ---- tile columns [0, kHalf) = mu, [kHalf, BLOCK_N) = logvar of latent columns n_blk*kHalf ..; a team owns
@@ -693,6 +710,11 @@ __device__ __forceinline__ void epilogue_unit(const GemmParams& p, int u, EpiSta
                 ptx::tma_store_commit();
               }
             }
+          }
+          if constexpr (kDet) {
+            const float kl = warp_sum(loss_local);
+            loss_local = 0.f;
+            if (lane == 0 && e.loss_acc) e.loss_acc[static_cast<size_t>(r32) * (L / 64) + col0 / 64] = kl;
           }
           if (e.out_hi && dual) {
             tm.drain();
@@ -821,7 +843,12 @@ __device__ __forceinline__ void epilogue_unit(const GemmParams& p, int u, EpiSta
           uint8_t* sl = tm.slot(tm.use);
 #pragma unroll
           for (int i = 0; i < 8; ++i) *slot_chunk(sl, row, i) = make_uint4(r[4 * i], r[4 * i + 1], r[4 * i + 2], r[4 * i + 3]);
-          tm.store(tm.use, &p.tmOutF32, n, m0, e.accumulate != 0);
+          if constexpr (kDet) {
+            if (tc.ks == 0) tm.store(tm.use, &p.tmOutF32, n, m0, false);
+            else tm.store(tm.use, &p.tmOutF32b, n, (tc.ks - 1) * e.ldp + m0, false);
+          } else {
+            tm.store(tm.use, &p.tmOutF32, n, m0, e.accumulate != 0);
+          }
           ++tm.use;
         }
       } else {
@@ -945,8 +972,18 @@ __device__ __forceinline__ void epilogue_unit(const GemmParams& p, int u, EpiSta
             if (do_colsum) {
               // bias gradient: column sums of this unit over the tile's 128 rows (rows >= M contribute zeros)
               warp_colsum64(v, lane);
-              atomicAdd(cs + 2 * lane, v[0]);
-              atomicAdd(cs + 2 * lane + 1, v[1]);
+              if constexpr (kDet) {   // this warp's 32 rows -> their own partial row, at a fixed index
+                *reinterpret_cast<float2*>(e.colsum + static_cast<size_t>(r32) * e.ldp + n0 + 2 * lane) =
+                    make_float2(v[0], v[1]);
+              } else {
+                atomicAdd(cs + 2 * lane, v[0]);
+                atomicAdd(cs + 2 * lane + 1, v[1]);
+              }
+            }
+            if constexpr (kDet && EPI == EPI_OUT) {
+              const float mse = warp_sum(loss_local);
+              loss_local = 0.f;
+              if (lane == 0 && e.loss_acc) e.loss_acc[static_cast<size_t>(r32) * (p.N / 64) + n0 / 64] = mse;
             }
             tm.store(tm.use, &p.tmOutHi, n0, m0, false);
             if (dual && tm.issuer) {
@@ -954,7 +991,7 @@ __device__ __forceinline__ void epilogue_unit(const GemmParams& p, int u, EpiSta
               ptx::tma_store_commit();
             }
             if (tr) trace_ev(p.trace, titer, j == 0 ? 13 : 15);
-            if (do_colsum) {
+            if (do_colsum && !kDet) {
               // the barrier inside store() ordered the four warps' smem atomics before this read; the strip is
               // cleared for its next use two units from now (the other strip serves the unit in between)
               if (team_tid < 64) {

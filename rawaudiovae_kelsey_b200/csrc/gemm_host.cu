@@ -89,6 +89,8 @@ int gemm_bind_outputs(PreparedGemm* g, const EpiArgs& a, bool force) {
     RVAE_CHECK(encode_2d(&p.tmOutF32, a.out_f32, true, g->out_cols_f32, g->out_rows, g->out_ld_f32, 32, 128));
   if (a.out_f32_b && g->epi == EPI_HEAD && (force || a.out_f32_b != old.out_f32_b))
     RVAE_CHECK(encode_2d(&p.tmOutF32b, a.out_f32_b, true, g->out_cols_f32, g->out_rows, g->out_ld_f32, 32, 128));
+  if (a.out_f32_b && g->slice_rows > 0 && (force || a.out_f32_b != old.out_f32_b))   // SLICE: splits 1.. in scratch
+    RVAE_CHECK(encode_2d(&p.tmOutF32b, a.out_f32_b, true, g->out_cols_f32, g->slice_rows, g->out_ld_f32, 32, 128));
   if (a.in0 && (force || a.in0 != old.in0 || a.ldi != old.ldi)) {
     if (g->epi == EPI_HEAD)  // eps, fp32 [M, L]
       RVAE_CHECK(encode_2d(&p.tmSide, a.in0, true, g->out_cols_f32, g->out_rows, g->out_ld_f32, 32, 128));
@@ -121,6 +123,12 @@ static const Variant kVariants[] = {
     RVAE_VARIANT(256, MAJOR_K, MAJOR_MN, EPI_DRELU),  RVAE_VARIANT(128, MAJOR_K, MAJOR_MN, EPI_DRELU),
     RVAE_VARIANT(256, MAJOR_K, MAJOR_MN, EPI_REDUCE),  RVAE_VARIANT(128, MAJOR_K, MAJOR_MN, EPI_REDUCE),
     RVAE_VARIANT(256, MAJOR_MN, MAJOR_MN, EPI_REDUCE), RVAE_VARIANT(128, MAJOR_MN, MAJOR_MN, EPI_REDUCE),
+    // deterministic kinds (EPI_SLICE ...): the training step with rvae_plan_set_deterministic
+    RVAE_VARIANT(256, MAJOR_K, MAJOR_K, EPI_HEAD_DET),   RVAE_VARIANT(128, MAJOR_K, MAJOR_K, EPI_HEAD_DET),
+    RVAE_VARIANT(256, MAJOR_K, MAJOR_K, EPI_OUT_DET),    RVAE_VARIANT(128, MAJOR_K, MAJOR_K, EPI_OUT_DET),
+    RVAE_VARIANT(256, MAJOR_K, MAJOR_MN, EPI_DRELU_DET), RVAE_VARIANT(128, MAJOR_K, MAJOR_MN, EPI_DRELU_DET),
+    RVAE_VARIANT(256, MAJOR_K, MAJOR_MN, EPI_SLICE),     RVAE_VARIANT(128, MAJOR_K, MAJOR_MN, EPI_SLICE),
+    RVAE_VARIANT(256, MAJOR_MN, MAJOR_MN, EPI_SLICE),    RVAE_VARIANT(128, MAJOR_MN, MAJOR_MN, EPI_SLICE),
 #if RVAE_EXPERIMENTS
     // latent dgrad with the reparameterisation / KL backward fused: pair tiles only
     {256, MAJOR_K, MAJOR_MN, EPI_DLATENT, 2, gemm_kernel_2cta<256, MAJOR_K, MAJOR_MN, EPI_DLATENT>,
@@ -174,11 +182,43 @@ static void choose_tile(const Ctx* ctx, int M, int N, bool allow128, bool allow2
   *block_n = (c128 < c256) ? 128 : 256;
 }
 
-int gemm_prepare(const Ctx* ctx, const GemmDesc& d, PreparedGemm* out) {
+// Split-K of a reduce GEMM: the smallest split (<= 8, >= 8 k-blocks each) whose last wave over `slots` tile slots is
+// >= 90% full; else the best seen
+static int split_rule(int tiles, int kb_total, int slots) {
+  int splits = 1;
+  double best = 0.0;
+  for (int s = 1; s <= 8 && kb_total / s >= 8; ++s) {
+    const int units = tiles * s;
+    const double eff = (double)units / (ceil_div(units, slots) * (double)slots);
+    if (eff > best + 1e-9) { best = eff; splits = s; }
+    if (eff >= 0.90) break;
+  }
+  return splits;
+}
+
+// Deterministic mode (EPI_SLICE): the split count comes from the shapes and this fixed slot count - the CTA pairs of a
+// B200 - never from the SM budget (RVAE_NUM_SMS), so the order of the split sums is a function of the problem alone.
+constexpr int kDetSlotSms = 148;
+
+// fp32 elements of the scratch slices (splits 1..) of a SLICE GEMM [M, N] x K with the tile choice of gemm_prepare
+size_t det_slice_floats(const Ctx* ctx, int M, int N, int K) {
+  int block_n, cg;
+  choose_tile(ctx, M, N, N % 256 != 0, true, &block_n, &cg);
+  const int m_blocks = ceil_div(M, kBlockM * cg), n_blocks = ceil_div(N, block_n), kb_total = ceil_div(K, kBlockK);
+  int splits = split_rule(m_blocks * n_blocks, kb_total, kDetSlotSms / cg);
+  if (splits > kb_total) splits = kb_total;
+  const int per = ceil_div(kb_total, splits);
+  splits = ceil_div(kb_total, per);
+  return (size_t)(splits - 1) * m_blocks * kBlockM * cg * N;
+}
+
+// d.epi: the epilogue the kernel computes (epi_base of `kind`); kind: the kernel's epilogue kind (EPI_SLICE, ...)
+static int prepare_impl(const Ctx* ctx, const GemmDesc& d, int kind, PreparedGemm* out) {
   RVAE_REQUIRE(d.M > 0 && d.N > 0 && d.K > 0, RVAE_ERR_INVALID, "gemm: empty problem %d x %d x %d", d.M, d.N, d.K);
   RVAE_REQUIRE(d.A.hi && d.B.hi, RVAE_ERR_INVALID, "gemm: null operand");
   RVAE_REQUIRE(d.N % 64 == 0, RVAE_ERR_UNSUPPORTED, "gemm: N=%d must be a multiple of 64", d.N);
   RVAE_CHECK(configure_variants());
+  const bool det = epi_det(kind);
 
   PreparedGemm& g = *out;
   memset(&g, 0, sizeof(g));
@@ -219,25 +259,32 @@ int gemm_prepare(const Ctx* ctx, const GemmDesc& d, PreparedGemm* out) {
   if (d.epi == EPI_REDUCE) {
     const int tiles = p.m_blocks * p.n_blocks;
     static const int env_splits = getenv("RVAE_WGRAD_SPLITS") ? atoi(getenv("RVAE_WGRAD_SPLITS")) : 0;
-    if (d.k_splits > 0) {
+    if (det) {
+      splits = split_rule(tiles, p.kb_total, kDetSlotSms / cg);
+    } else if (d.k_splits > 0) {
       splits = d.k_splits;
     } else if (env_splits > 0 && d.A.major == MAJOR_MN) {   // experiments: finer weight-gradient units
       splits = env_splits;
     } else {
-      // smallest split (<= 8, >= 8 k-blocks each) whose last wave is >= 90% full; else the best seen
-      double best = 0.0;
-      for (int s = 1; s <= 8 && p.kb_total / s >= 8; ++s) {
-        const int units = tiles * s;
-        const double eff = (double)units / (ceil_div(units, slots) * (double)slots);
-        if (eff > best + 1e-9) { best = eff; splits = s; }
-        if (eff >= 0.90) break;
-      }
+      splits = split_rule(tiles, p.kb_total, slots);
     }
     if (splits > p.kb_total) splits = p.kb_total;
-    RVAE_REQUIRE(splits == 1 || d.args.accumulate, RVAE_ERR_INVALID, "reduce gemm: split-K needs accumulate=1");
+    RVAE_REQUIRE(splits == 1 || d.args.accumulate || det, RVAE_ERR_INVALID, "reduce gemm: split-K needs accumulate=1");
   }
   p.kb_per_split = ceil_div(p.kb_total, splits);
   p.k_splits = ceil_div(p.kb_total, p.kb_per_split);  // every split owns >= 1 k-block
+  if (det && d.epi == EPI_REDUCE) {
+    // split k >= 1 stores rows (k - 1) * stride + m of the scratch: a stride of whole tiles keeps the rows a last,
+    // partly out-of-range tile stores inside its own slice
+    const int stride = p.m_blocks * kBlockM * cg;
+    p.epi.ldp = stride;
+    p.epi.accumulate = 0;
+    g.slice_rows = (p.k_splits - 1) * stride;
+    RVAE_REQUIRE(g.slice_rows == 0 || (d.args.out_f32_b != nullptr &&
+                                       (size_t)g.slice_rows * d.N <= d.slice_cap),
+                 RVAE_ERR_INVALID, "slice gemm: %d split rows x %d exceed the deterministic scratch (%zu floats)",
+                 g.slice_rows, d.N, d.slice_cap);
+  }
 
   // passes: hi*hi (+ hi*lo + lo*hi when both operands carry a residual plane)
   const Operand* pa[kMaxPasses];
@@ -288,9 +335,10 @@ int gemm_prepare(const Ctx* ctx, const GemmDesc& d, PreparedGemm* out) {
 
   g.block_n = block_n;
   g.a_major = d.A.major; g.b_major = d.B.major; g.cg = cg;
-  g.variant = find_variant(block_n, d.A.major, d.B.major, d.epi, cg);
+  g.kind = kind;
+  g.variant = find_variant(block_n, d.A.major, d.B.major, kind, cg);
   RVAE_REQUIRE(g.variant >= 0, RVAE_ERR_UNSUPPORTED, "gemm: no kernel for block_n=%d majors (%d,%d) epilogue %d",
-               block_n, d.A.major, d.B.major, d.epi);
+               block_n, d.A.major, d.B.major, kind);
   // Persistent grid: the fewest CTAs (pairs) that still finish in the same number of waves. What wave quantisation
   // would leave idle in the last wave is left idle for the whole kernel instead - those SMs run the concurrent
   // HBM-bound work of the step (noise, Adam, all-reduce) without taking anything from this GEMM.
@@ -300,6 +348,12 @@ int gemm_prepare(const Ctx* ctx, const GemmDesc& d, PreparedGemm* out) {
   g.grid = cg * (units < slots_eff ? units : slots_eff);
   g.smem_bytes = kVariants[g.variant].smem;
   return RVAE_OK;
+}
+
+int gemm_prepare(const Ctx* ctx, const GemmDesc& desc, PreparedGemm* out) {
+  GemmDesc d = desc;
+  d.epi = epi_base(desc.epi);
+  return prepare_impl(ctx, d, desc.epi, out);
 }
 
 int gemm_run(Ctx* ctx, const PreparedGemm& g, cudaStream_t stream) {
@@ -338,12 +392,19 @@ using KDlat = Kind<MAJOR_K, MAJOR_MN, EPI_DLATENT>;
 using KLinear = Kind<MAJOR_K, MAJOR_K, EPI_LINEAR>;
 using KHead = Kind<MAJOR_K, MAJOR_K, EPI_HEAD>;
 using KOut = Kind<MAJOR_K, MAJOR_K, EPI_OUT>;
+using KDreluDet = Kind<MAJOR_K, MAJOR_MN, EPI_DRELU_DET>;
+using KWgradSlice = Kind<MAJOR_MN, MAJOR_MN, EPI_SLICE>;
+using KDzSlice = Kind<MAJOR_K, MAJOR_MN, EPI_SLICE>;
 #define RVAE_KID(K) {K::A, K::B, K::EPI}
 static const ChainVariant kChainVariants[] = {
     // dgrad + ReLU mask | weight gradient            (backward stages 0 and 2)
     {2, {RVAE_KID(KDrelu), RVAE_KID(KWgrad)}, gemm_chain_kernel_2cta<256, KDrelu, KWgrad, NoKind, NoKind>},
     // split-K latent dgrad | weight gradient         (backward stage 1)
     {2, {RVAE_KID(KDz), RVAE_KID(KWgrad)}, gemm_chain_kernel_2cta<256, KDz, KWgrad, NoKind, NoKind>},
+    // the same two launches with the deterministic kinds
+    {2, {RVAE_KID(KDreluDet), RVAE_KID(KWgradSlice)},
+     gemm_chain_kernel_2cta<256, KDreluDet, KWgradSlice, NoKind, NoKind>},
+    {2, {RVAE_KID(KDzSlice), RVAE_KID(KWgradSlice)}, gemm_chain_kernel_2cta<256, KDzSlice, KWgradSlice, NoKind, NoKind>},
 
 #if RVAE_EXPERIMENTS
     // dgrad + ReLU mask | weight gradient | the previous stage's weight gradient   (stage 2 with B3w riding along:
@@ -402,7 +463,7 @@ int gemm_prepare_chain(const Ctx* ctx, const PreparedGemm* const* g, int count, 
     if (cv.count != count) continue;
     bool match = true;
     for (int i = 0; i < count; ++i)
-      match = match && cv.k[i].a == g[i]->a_major && cv.k[i].b == g[i]->b_major && cv.k[i].e == g[i]->epi;
+      match = match && cv.k[i].a == g[i]->a_major && cv.k[i].b == g[i]->b_major && cv.k[i].e == g[i]->kind;
     if (match) variant = v;
   }
   RVAE_REQUIRE(variant >= 0, RVAE_ERR_UNSUPPORTED, "chain gemm: no fused kernel for this combination of problems");

@@ -139,15 +139,43 @@ def _move_grads(model, flat, grads):
             p.grad = None
 
 
-def adopt_symmetric_grads(model, group=None) -> bool:
+def adopt_symmetric_grads(model, group=None, peer_loads: bool = False) -> bool:
     """Move the model's flat gradient buffer into a symmetric allocation that every rank of the group maps over
     CUDA IPC, so the gradient all-reduce can be done by librvae_b200's own NVLink peer-memory kernel instead of NCCL.
-    Returns False (and leaves NCCL in charge) when RVAE_DP_BACKEND=nccl or the group has more than 8 ranks."""
+    Returns False (and leaves NCCL in charge) when RVAE_DP_BACKEND=nccl or the group has more than 8 ranks.
+    peer_loads=True (deterministic steps): the peer-load exchange, which sums the ranks in rank order, whatever
+    RVAE_DP_BACKEND says; raises ValueError naming the backend when the group ends up on NVLS multicast or NCCL."""
+    from . import _lib, ops
+    if peer_loads:
+        if dist.get_world_size(group) > 8:     # (no GPU work yet: the peer-load kernel takes at most 8 ranks)
+            agree_peer_loads("nccl", group)
+        flat = model._ensure_flat()
+        ok = _adopt(model, group, "p2p")
+        agree_peer_loads(("nvls" if _lib.load().rvae_dp_uses_multicast(ops.ctx(flat.device)) else "p2p") if ok
+                         else "nccl", group)
+        return True
+    return _adopt(model, group, os.environ.get("RVAE_DP_BACKEND", "auto"))
+
+
+def agree_peer_loads(backend: str, group=None) -> None:
+    """Deterministic data parallelism: every rank passes the exchange its gradients ended up on ("p2p" = peer loads,
+    "nvls", "nccl"); all ranks raise ValueError naming the other backends unless every rank is on peer loads, so no
+    rank trains on while another refuses, and none trains non-deterministically."""
+    box = [None] * dist.get_world_size(group)
+    dist.all_gather_object(box, backend, group=group)
+    bad = sorted({b for b in box if b != "p2p"})
+    if bad:
+        raise ValueError(f"deterministic data parallelism needs the peer-load gradient all-reduce (ranks summed in "
+                         f"rank order); this group exchanges gradients by {' / '.join(bad)}, which gives no order "
+                         f"guarantee")
+
+
+def _adopt(model, group, backend) -> bool:
     from . import _lib, ops
     import ctypes as C
     flat = model._ensure_flat()
     world, rank = dist.get_world_size(group), dist.get_rank(group)
-    if os.environ.get("RVAE_DP_BACKEND", "auto") == "nccl" or world > 8:
+    if backend == "nccl" or world > 8:
         return False
     key = flat.device.index
     if key in _SYM_READY:
@@ -161,7 +189,6 @@ def adopt_symmetric_grads(model, group=None) -> bool:
         # Default ("auto"): from 3 ranks up. Measured on one box (profiles/README.md): N = 8 +5.4 %, N = 4 +2.6 %, N = 2
         # -3.5 % (with two ranks a rank's own slice travels to the switch and back for nothing), so two ranks keep the
         # library's own CUDA-IPC allocation and peer loads. RVAE_DP_BACKEND=nvls / p2p / nccl force one.
-        backend = os.environ.get("RVAE_DP_BACKEND", "auto")
         if backend == "nvls" or (backend == "auto" and world >= 3):
             grads = _adopt_torch_symmetric(lib, flat, group, rank, world)
             if grads is not None:
@@ -270,11 +297,20 @@ class DataParallelTrainStep(_StepBase):
     graph=True captures the whole step, NCCL collectives included, into one CUDA graph per input signature.
     schedule: as for FusedTrainStep; every rank evaluates it at the same step counter.
     max_grad_norm: as for FusedTrainStep. The norm is taken over the all-reduced gradient, which is identical on every
-    rank, in a fixed order, so every rank clips by the same factor and the replicas stay bitwise equal."""
+    rank, in a fixed order, so every rank clips by the same factor and the replicas stay bitwise equal.
+    deterministic: as for FusedTrainStep, with the gradients exchanged by the peer-load all-reduce whatever
+    RVAE_DP_BACKEND says (it sums the ranks in rank order). RVAE_DP_BACKEND=nvls or nccl raises ValueError here, and
+    so does a group that cannot use peer loads, at its first step: the step never trains non-deterministically."""
 
     def __init__(self, model, optimizer, kl_beta: float, global_batch: Optional[int] = None, group=None,
-                 ring: int = 64, reduce_loss: bool = False, graph: bool = False, schedule=None, max_grad_norm=None):
-        super().__init__(model, optimizer, kl_beta, ring, graph, schedule=schedule, max_grad_norm=max_grad_norm)
+                 ring: int = 64, reduce_loss: bool = False, graph: bool = False, schedule=None, max_grad_norm=None,
+                 deterministic: bool = False):
+        super().__init__(model, optimizer, kl_beta, ring, graph, schedule=schedule, max_grad_norm=max_grad_norm,
+                         deterministic=deterministic)
+        forced = os.environ.get("RVAE_DP_BACKEND", "auto")
+        if self.deterministic and forced in ("nvls", "nccl"):
+            raise ValueError(f"deterministic=True needs the peer-load gradient all-reduce; RVAE_DP_BACKEND={forced} "
+                             f"gives no order guarantee")
         self.group = group
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
@@ -328,7 +364,7 @@ class DataParallelTrainStep(_StepBase):
         flat = self._prepare()
         if not self._synced and self.world > 1:
             init_native_comm(flat.device, self.group)
-            adopt_symmetric_grads(self.model, self.group)
+            adopt_symmetric_grads(self.model, self.group, peer_loads=self.deterministic)
             flat = self._prepare()
             broadcast_parameters(flat.params, self.group)
             flat.sync_shadow()

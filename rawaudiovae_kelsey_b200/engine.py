@@ -314,6 +314,24 @@ class Plan:
         check(self.lib.rvae_plan_set_grad_clip(self.handle, max_norm_ptr,
                                                norm_out.data_ptr() if norm_out is not None else None, int(ring_size)))
 
+    def deterministic_bytes(self) -> int:
+        """Scratch bytes of the deterministic training step at this plan's max_batch (rvae_plan_deterministic_bytes)."""
+        return int(self.lib.rvae_plan_deterministic_bytes(self.handle))
+
+    def set_deterministic(self, on: bool) -> None:
+        """Make this plan's training steps bitwise reproducible (on) or use the default kernels (off). The scratch is
+        allocated on first use and kept with the plan, so a captured graph's addresses stay valid."""
+        if not on:
+            check(self.lib.rvae_plan_set_deterministic(self.handle, None, 0))
+            return
+        scratch = getattr(self, "_det_scratch", None)
+        if scratch is None:
+            nbytes = self.deterministic_bytes()
+            scratch = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.flat.device)
+            self._det_scratch = scratch
+        aligned = (scratch.data_ptr() + 255) // 256 * 256
+        check(self.lib.rvae_plan_set_deterministic(self.handle, aligned, scratch.numel() - (aligned - scratch.data_ptr())))
+
     def grad_norm(self, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Global L2 norm of the bound gradient buffer, with the kernels of a clipping step (0-dim float32 tensor)."""
         if out is None:

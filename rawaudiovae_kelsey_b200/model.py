@@ -376,6 +376,13 @@ def loss_function(recon_x, x, mu, logvar, kl_beta, segment_length):
     return _LossFunction.apply(c(recon_x), c(x), c(mu), c(logvar), float(kl_beta))
 
 
+def check_deterministic(value) -> bool:
+    """A training step's deterministic switch: True or False. Raises ValueError for anything else."""
+    if not isinstance(value, bool):
+        raise ValueError(f"deterministic must be True or False, got {value!r}")
+    return value
+
+
 def check_max_grad_norm(value) -> Optional[float]:
     """A training step's gradient-clipping threshold: None (no clipping) or a float > 0, +inf included (the norm is
     measured and logged, the update is unchanged). Raises ValueError for anything else."""
@@ -402,10 +409,19 @@ class _StepBase:
     max_grad_norm (None = off): clip the gradient by its global L2 norm before Adam, as torch.nn.utils.clip_grad_norm_
     does, inside the step (rvae_plan_set_grad_clip). The threshold lives in the device record too, so changing
     `step.max_grad_norm` reaches graph replays; switching clipping on or off captures a new graph. The pre-clip norm
-    of every step lands in a device ring of the loss ring's size; `grad_norm` is the last step's slot."""
+    of every step lands in a device ring of the loss ring's size; `grad_norm` is the last step's slot.
 
-    def __init__(self, model, optimizer, kl_beta, ring, graph, graph_warmup=1, schedule=None, max_grad_norm=None):
+    deterministic (bool, fixed at construction): bitwise reproducible steps (rvae_plan_set_deterministic). Every
+    output of a step - parameters, Adam moments, bf16 shadows, the step counter, the loss and norm rings, kept
+    gradients - then depends only on the inputs, the state, the hyper-parameters, the dims, the batch size, the
+    precision and the world size, never on scheduling or the SM budget. Each plan the step uses gets its own scratch
+    (rvae_plan_deterministic_bytes: 35.9 MB at the default dims and 8192 frames). The unfused path (loss_function +
+    loss.backward()) is not covered."""
+
+    def __init__(self, model, optimizer, kl_beta, ring, graph, graph_warmup=1, schedule=None, max_grad_norm=None,
+                 deterministic=False):
         self.max_grad_norm = max_grad_norm     # validated before any GPU work
+        self.deterministic = check_deterministic(deterministic)
         self.model, self.optimizer, self.kl_beta = model, optimizer, float(kl_beta)
         self.schedule = schedule if schedule is not None else Schedule()
         self._record = None
@@ -465,6 +481,16 @@ class _StepBase:
 
     def _train_step(self, plan, zero_grads):
         """The fused step from the device record, clipping when max_grad_norm is set (a plan setting for this call)."""
+        if self.deterministic:
+            plan.set_deterministic(True)
+            try:
+                self._train_step_clip(plan, zero_grads)
+            finally:
+                plan.set_deterministic(False)
+            return
+        self._train_step_clip(plan, zero_grads)
+
+    def _train_step_clip(self, plan, zero_grads):
         if self.max_grad_norm is None:
             plan.train_step_hp(self._record.tensor, loss_out=self.ring, ring_size=self.ring_size, zero_grads=zero_grads)
             return
@@ -540,7 +566,7 @@ class _StepBase:
             # ---- plain path: load inside the step (captured graph: from static index / input buffers)
             key = self._graph_key(data) if graphable else None
             if key is not None:
-                key = key + self._key_extra(data) + (self.max_grad_norm is not None,)
+                key = key + self._key_extra(data) + (self.max_grad_norm is not None, self.deterministic)
             if key is not None and key in self._graphs:
                 st = self._graphs[key]
                 self._load_static(key, data, st)
@@ -573,7 +599,8 @@ class _StepBase:
             if graphable and do_pf and isinstance(data, FrameBatch):
                 key = ("pf", plan.handle.value, next_data.audio.data_ptr(), plan.batch, next_data.n_frames,
                        next_data.hop, self._plan_cur(plan), plan.pitch, model._in_place(next_data)) \
-                    + self._key_extra(data) + self._key_extra(next_data) + (self.max_grad_norm is not None,)
+                    + self._key_extra(data) + self._key_extra(next_data) + (self.max_grad_norm is not None,
+                                                                             self.deterministic)
             if key is not None and key in self._graphs:
                 st = self._graphs[key]
                 self._fill_idx(st, next_data)
@@ -689,11 +716,14 @@ class FusedTrainStep(_StepBase):
     graph=True: replay a captured CUDA graph of the step (see _StepBase).
     schedule (schedule.Schedule, default constant): learning rate and KL weight per step, with
     optimizer.param_groups[0]['lr'] and kl_beta as the peak values.
-    max_grad_norm (None, or a float > 0, inf included): clip by the global gradient norm (see _StepBase)."""
+    max_grad_norm (None, or a float > 0, inf included): clip by the global gradient norm (see _StepBase).
+    deterministic (bool, default False): bitwise reproducible steps (see _StepBase)."""
 
     def __init__(self, model: VAE, optimizer, kl_beta: float, ring: int = 64, keep_grads: bool = False,
-                 graph: bool = False, schedule: Optional[Schedule] = None, max_grad_norm: Optional[float] = None):
-        super().__init__(model, optimizer, kl_beta, ring, graph, schedule=schedule, max_grad_norm=max_grad_norm)
+                 graph: bool = False, schedule: Optional[Schedule] = None, max_grad_norm: Optional[float] = None,
+                 deterministic: bool = False):
+        super().__init__(model, optimizer, kl_beta, ring, graph, schedule=schedule, max_grad_norm=max_grad_norm,
+                         deterministic=deterministic)
         self.keep_grads = keep_grads
 
     def _enqueue(self, plan):

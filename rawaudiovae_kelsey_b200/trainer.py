@@ -17,6 +17,7 @@ from __future__ import annotations
 import argparse
 import configparser
 import os
+import random
 import sys
 import time
 from itertools import islice
@@ -164,6 +165,37 @@ def _max_grad_norm(config):
     return check_max_grad_norm(f)
 
 
+def _deterministic(config) -> bool:
+    """[training] deterministic (optional bool, default False): bitwise reproducible training steps (FusedTrainStep /
+    DataParallelTrainStep deterministic=True). A value that is not a boolean raises ValueError."""
+    v = config['training'].get('deterministic', fallback='').strip()
+    if not v:
+        return False
+    try:
+        return config['training'].getboolean('deterministic')
+    except ValueError:
+        raise ValueError(f"[training] deterministic must be a boolean (True / False), got {v!r}") from None
+
+
+def _seed(config):
+    """[training] seed (optional int): seeds torch and random at start-up, which fixes the initial weights, the
+    sampler permutation, the stream's file order and the noise seed. Absent or empty: unseeded. Text that is not an
+    integer raises ValueError."""
+    v = config['training'].get('seed', fallback='').strip()
+    if not v:
+        return None
+    try:
+        return int(v)
+    except ValueError:
+        raise ValueError(f"[training] seed must be an integer, got {v!r}") from None
+
+
+def _apply_seed(seed) -> None:
+    if seed is not None:
+        torch.manual_seed(seed)
+        random.seed(seed)
+
+
 def _epoch_steps(n_frames: int, batch_size: int, world: int = 1) -> int:
     """Training steps per epoch of GpuFrameLoader (drop_last=False): a last global batch with fewer frames than ranks
     is skipped."""
@@ -285,6 +317,8 @@ def run_epoch_trainer(argv=None):
     kl_beta = config['VAE'].getfloat('kl_beta')
     test_loss = _test_loss_enabled(config)
     max_grad_norm = _max_grad_norm(config)
+    deterministic = _deterministic(config)
+    _apply_seed(_seed(config))
     start_time = time.time()
     config['extra']['start'] = time.asctime(time.localtime(start_time))
 
@@ -326,10 +360,10 @@ def run_epoch_trainer(argv=None):
     ring = max(64, log_interval)
     if world > 1:
         step = rdist.DataParallelTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph, schedule=schedule,
-                                           max_grad_norm=max_grad_norm)
+                                           max_grad_norm=max_grad_norm, deterministic=deterministic)
     else:
         step = FusedTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph, schedule=schedule,
-                              max_grad_norm=max_grad_norm)
+                              max_grad_norm=max_grad_norm, deterministic=deterministic)
 
     # parameter histograms on the GPU (rank 0 only): one launch + one small asynchronous copy per set
     hist = ParamHistogramLogger(model, writer) if rank == 0 else None
@@ -454,9 +488,12 @@ def run_stream_trainer(argv=None):
     kl_beta = config['VAE'].getfloat('kl_beta')
     test_loss = _test_loss_enabled(config)
     max_grad_norm = _max_grad_norm(config)
+    deterministic = _deterministic(config)
+    seed = _seed(config)
     if segment_length != 1024:
         raise ValueError("the streaming dataset frames at 1024 samples (rawvae/dataset.py:66); segment_length "
                          "= {} is not supported by train_iterable.py".format(segment_length))
+    _apply_seed(seed)
     start_time = time.time()
     config['extra']['start'] = time.asctime(time.localtime(start_time))
 
@@ -498,10 +535,11 @@ def run_stream_trainer(argv=None):
         ring = max(64, log_interval)
         if world > 1:
             step = rdist.DataParallelTrainStep(model, optimizer, kl_beta, global_batch=batch_size, ring=ring,
-                                               graph=use_graph, schedule=schedule, max_grad_norm=max_grad_norm)
+                                               graph=use_graph, schedule=schedule, max_grad_norm=max_grad_norm,
+                                               deterministic=deterministic)
         else:
             step = FusedTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph, schedule=schedule,
-                                  max_grad_norm=max_grad_norm)
+                                  max_grad_norm=max_grad_norm, deterministic=deterministic)
 
         hist = ParamHistogramLogger(model, writer) if rank == 0 and histogram_interval > 0 else None
 
