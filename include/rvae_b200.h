@@ -523,6 +523,29 @@ size_t rvae_plan_deterministic_bytes(const rvae_plan* plan);   /* scratch bytes 
  * Returns 1 for a short or misaligned scratch. */
 int rvae_plan_set_deterministic(rvae_plan* plan, void* scratch, size_t bytes);
 
+/* Exponential moving average (EMA) of the weights, as torch.optim.swa_utils.AveragedModel with
+ * multi_avg_fn = get_ema_multi_avg_fn(decay) and update_parameters(model) after every optimizer step, kept inside the
+ * training step. With an EMA set, every Adam launch of every later rvae_plan_train_step(_hp) of the plan also updates
+ * ema[i] for the elements it updates, from the parameter it has just computed:
+ *   n_averaged == 0: ema = p;   else ema = lerp(ema, p, w), w = (float)(1 - decay), 1 - decay formed in double;
+ *   lerp(e, p, w) = |w| < 0.5 ? e + w (p - e) : p - (p - e)(1 - w)   (torch's formula), in fp32;
+ * and the last block of the step's final Adam launch, which advances the step counter, does *count_dev += 1. The
+ * step issues the same launches as without an EMA (the EMA is 8 more bytes per parameter in each), and parameters,
+ * Adam moments, shadows and the step counter are the same bit for bit. It composes with gradient clipping,
+ * deterministic mode and data parallelism (each rank updates its own EMA from the all-reduced update).
+ * ema: fp32, 16-byte aligned, the flat layout of the plan's parameters (rvae_param_layout_padded; padding elements
+ * stay 0 when they are 0 in ema and params). decay_dev: a device double in [0, 1], read when the kernels run, so a
+ * graph captured around a step follows any rewrite ordered before its replay. count_dev: the device int64 n_averaged.
+ * ema == NULL switches the EMA off. rvae_plan_adam / rvae_plan_adam_buckets called on their own do not update it.
+ * Returns 1 for a non-null ema with a null decay_dev or count_dev, or a misaligned ema (before the plan is used). */
+int rvae_plan_set_ema(rvae_plan* plan, float* ema, const double* decay_dev, int64_t* count_dev);
+/* The same EMA update as one launch over n elements: ema = lerp(ema, params, w) (a copy when *count_dev == 0), then
+ * *count_dev += 1 - what follows an optimizer step of the unfused path. ema and params: 16-byte aligned fp32. Calls on
+ * one ctx must be ordered (one stream, or event-ordered): they share one device ticket. Returns 1 for a null
+ * pointer, n < 0, a misaligned buffer or a null ctx. */
+int rvae_ema_update(rvae_ctx* ctx, float* ema, const float* params, int64_t n, const double* decay_dev,
+                    int64_t* count_dev, void* stream);
+
 /* Evaluate the record's schedule at the n step indices k_dev[0..n) with the device function the training kernels
  * use: lr_out[i] = lr(k_dev[i]), beta_out[i] = (float)beta(k_dev[i]). Returns 1 for null pointers or n < 1 (before
  * ctx is used). */

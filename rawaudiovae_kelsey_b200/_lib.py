@@ -122,6 +122,8 @@ SIGNATURES = {
     "rvae_plan_deterministic_bytes": (c_size_t, [P]),
     "rvae_plan_set_deterministic": (c_int, [P, P, c_size_t]),
     "rvae_plan_grad_norm": (c_int, [P, P, P]),
+    "rvae_plan_set_ema": (c_int, [P, P, P, P]),
+    "rvae_ema_update": (c_int, [P, P, P, c_int64, P, P, P]),
     "rvae_hparams_check": (c_int, [C.POINTER(Hparams)]),
     "rvae_hparams_eval": (c_int, [P, P, P, c_int, P, P, P]),
     "rvae_plan_mu": (P, [P]),

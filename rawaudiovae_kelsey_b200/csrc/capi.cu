@@ -47,6 +47,7 @@ struct rvae_ctx {
   bool p2p_ready;
   int p2p_ctas;        // CTAs of an all-reduce that runs under the GEMMs (they live on the spare SMs)
   int p2p_ctas_last;   // CTAs of the step's last, exposed all-reduce
+  unsigned int* ema_ticket;   // device word: last-block ticket of rvae_ema_update (zero between launches)
 };
 
 static inline cudaStream_t S_(void* s) { return reinterpret_cast<cudaStream_t>(s); }
@@ -106,6 +107,19 @@ int rvae_ctx_create(int device, rvae_ctx** out) {
   if (const char* e = getenv("RVAE_DEBUG")) ctx->c.debug = atoi(e);
   ctx->c.use_pdl = 1;
   if (const char* e = getenv("RVAE_PDL")) ctx->c.use_pdl = atoi(e);
+  {
+    int prev = 0;
+    RVAE_CUDA(cudaGetDevice(&prev));
+    RVAE_CUDA(cudaSetDevice(device));
+    const cudaError_t e1 = cudaMalloc(&ctx->ema_ticket, 256);
+    const cudaError_t e2 = e1 == cudaSuccess ? cudaMemset(ctx->ema_ticket, 0, 256) : e1;
+    RVAE_CUDA(cudaSetDevice(prev));
+    if (e2 != cudaSuccess) {
+      if (e1 == cudaSuccess) cudaFree(ctx->ema_ticket);
+      delete ctx;
+      RVAE_CUDA(e2);
+    }
+  }
   *out = ctx;
   return RVAE_OK;
 }
@@ -117,6 +131,7 @@ void rvae_ctx_destroy(rvae_ctx* ctx) {
       if (ctx->peer_base[p] && p != ctx->dp_rank) cudaIpcCloseMemHandle(ctx->peer_base[p]);
     if (ctx->sym_base) cudaFree(ctx->sym_base);
   }
+  if (ctx->ema_ticket) cudaFree(ctx->ema_ticket);
   delete ctx;
 }
 
@@ -623,6 +638,12 @@ struct rvae_plan {
   int clip_ring;
   double* norm_parts;      // workspace: fp64 partials of the norm launches, [kNormGroups][kNormMaxBlocks]
   float* clip_coef;        // workspace: the step's clipping factor, read by the Adam launch
+  // exponential moving average of the parameters (rvae_plan_set_ema): ema != nullptr makes every Adam launch of a
+  // training step update it; ema_on while a training step enqueues its kernels
+  float* ema;
+  const double* ema_decay;
+  int64_t* ema_count;
+  bool ema_on;
   struct Prefetch {
     bool registered;       // rvae_plan_prefetch_frames called; consumed by the next rvae_plan_train_step
     int ready_batch;       // > 0: the alternate set holds this many frames (+ their noise), enqueued by a train step
@@ -1095,9 +1116,11 @@ int adam_buckets(rvae_plan* p, unsigned mask, const HpArg& hp, float grad_scale,
     const int64_t o = seg_off[i];
     const bool pair = i + 1 < nseg;
     const bool last = i + 2 >= nseg;
+    // a training step with an EMA set: the same launch also updates the EMA of its segments
+    const EmaArg ema = {p->ema_on ? p->ema + o : nullptr, p->ema_decay, p->ema_count};
     RVAE_CHECK(launch_adam2(&p->ctx->c, b.params + o, b.grads + o, b.exp_avg + o, b.exp_avg_sq + o, seg_n[i],
                             pair ? seg_off[i + 1] - o : 0, pair ? seg_n[i + 1] : 0, hp, grad_scale, coef, b.step, step_bias, (advance_step && last) ? p->ticket : nullptr,
-                            BF(b.shadow_hi) + o, b.shadow_lo ? BF(b.shadow_lo) + o : nullptr, zero_grads, st));
+                            BF(b.shadow_hi) + o, b.shadow_lo ? BF(b.shadow_lo) + o : nullptr, zero_grads, ema, st));
   }
   for (int s = 0; s < 5; ++s)
     if (mask & (1u << s)) p->grads_zeroed[s] = zero_grads != 0;
@@ -1459,6 +1482,7 @@ int rvae_plan_create(rvae_ctx* ctx, int S, int H, int L, int max_batch, int prec
   p->kl_c0 = 0.f; p->kl_bl = 0.0; p->hp_dev = nullptr; p->hp_early = 0; p->dz_zeroed = false; p->dp_enabled = false;
   p->cur = 0; p->ticket_zeroed = false; p->ticket = nullptr; p->norm_ticket_zeroed = false;
   p->clip_max = nullptr; p->clip_norm_out = nullptr; p->clip_ring = 1;
+  p->ema = nullptr; p->ema_decay = nullptr; p->ema_count = nullptr; p->ema_on = false;
   p->x_pitch = 0; p->x_pitch_alt = 0;
   p->fuse_latent = false;
   p->sched_batch = 0;
@@ -2041,6 +2065,11 @@ static int train_step(rvae_plan* plan, float kl_beta, const HpArg& hp, int zero_
     explicit DetGuard(rvae_plan* p_) : p(p_) { p->det_on = p->det_scratch != nullptr; }
     ~DetGuard() { p->det_on = false; }
   } det_guard(plan);
+  struct EmaGuard {   // the EMA Adam launches are enqueued by this call only
+    rvae_plan* p;
+    explicit EmaGuard(rvae_plan* p_) : p(p_) { p->ema_on = p->ema != nullptr; }
+    ~EmaGuard() { p->ema_on = false; }
+  } ema_guard(plan);
   // Gradient clipping: the global norm depends on every bucket and Adam is nonlinear in g, so no bucket is updated
   // before the norm is known. Each bucket's norm partial takes the place of its background Adam launch; the last one
   // finalises the clipping factor, and one Adam launch over all buckets reads it.
@@ -2272,6 +2301,27 @@ int rvae_plan_set_grad_clip(rvae_plan* plan, const double* max_norm_dev, float* 
   plan->clip_norm_out = max_norm_dev ? norm_out : nullptr;
   plan->clip_ring = norm_out ? ring_size : 1;
   return RVAE_OK;
+}
+
+int rvae_plan_set_ema(rvae_plan* plan, float* ema, const double* decay_dev, int64_t* count_dev) {
+  RVAE_REQUIRE(ema == nullptr || (decay_dev != nullptr && count_dev != nullptr), RVAE_ERR_INVALID,
+               "plan_set_ema: an EMA buffer needs its decay and count");
+  RVAE_REQUIRE((reinterpret_cast<uintptr_t>(ema) & 15) == 0, RVAE_ERR_INVALID,
+               "plan_set_ema: the EMA buffer must be 16-byte aligned");
+  RVAE_REQUIRE(plan, RVAE_ERR_INVALID, "null rvae_plan");
+  plan->ema = ema;
+  plan->ema_decay = ema ? decay_dev : nullptr;
+  plan->ema_count = ema ? count_dev : nullptr;
+  return RVAE_OK;
+}
+
+int rvae_ema_update(rvae_ctx* ctx, float* ema, const float* params, int64_t n, const double* decay_dev,
+                    int64_t* count_dev, void* stream) {
+  RVAE_REQUIRE(ema && params && decay_dev && count_dev && n >= 0, RVAE_ERR_INVALID,
+               "ema_update: null buffer or n = %lld", (long long)n);
+  CTX_OR_FAIL(ctx);
+  const EmaArg e = {ema, decay_dev, count_dev};
+  return launch_ema_update(&ctx->c, params, n, e, ctx->ema_ticket, S_(stream));
 }
 
 int rvae_plan_grad_norm(rvae_plan* plan, float* norm_out, void* stream) {

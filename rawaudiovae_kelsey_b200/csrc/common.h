@@ -201,12 +201,24 @@ struct HpArg {
 };
 HpArg hp_value(double lr, double beta1, double beta2, double eps, double weight_decay);   // a constant record
 inline HpArg hp_device(const rvae_hparams* dev) { HpArg a = hp_value(0.0, 0.0, 0.0, 0.0, 0.0); a.dev = dev; return a; }
+// The exponential moving average an Adam launch also updates (rvae_plan_set_ema), or the buffer rvae_ema_update
+// updates: the fp32 average e over the same elements as the parameters, the device decay and the device update count
+// n_averaged. e == nullptr: none.
+struct EmaArg {
+  float* e;
+  const double* decay;
+  int64_t* count;
+};
 int launch_adam(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, double lr, double beta1, double beta2,
                 double eps, double weight_decay, float grad_scale, const float* step, __nv_bfloat16* shadow_hi,
                 __nv_bfloat16* shadow_lo, int zero_grads, cudaStream_t stream);
 int launch_adam2(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, int64_t off_b, int64_t n_b,
                  const HpArg& hp, float grad_scale, const float* coef, float* step, int step_bias, unsigned int* ticket,
-                 __nv_bfloat16* shadow_hi, __nv_bfloat16* shadow_lo, int zero_grads, cudaStream_t stream);
+                 __nv_bfloat16* shadow_hi, __nv_bfloat16* shadow_lo, int zero_grads, const EmaArg& ema,
+                 cudaStream_t stream);
+// e = lerp(e, p, 1 - decay) over n elements (a copy when n_averaged == 0), then n_averaged += 1 by the last block
+int launch_ema_update(Ctx* ctx, const float* p, int64_t n, const EmaArg& ema, unsigned int* ticket,
+                      cudaStream_t stream);
 // Gradient norm for clipping (grad_norm_kernel): the last block of a launch with `ticket` set sums parts[0, n_parts)
 struct NormFinalize {
   const double* parts;

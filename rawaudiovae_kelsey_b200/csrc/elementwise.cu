@@ -1056,12 +1056,45 @@ int launch_lerp_reparam(Ctx* ctx, const float* mu_a, const float* lv_a, const fl
 // the bandwidth - measured when the hyper-parameters became doubles)
 // The hyper-parameters come from a record (HpArg: the device record of a scheduled step, read here when the kernel
 // runs, or a constant record passed by value); lr is the schedule's lr(k) at k = t - 1.
-template <int U>
+// EMA = true (the training step with rvae_plan_set_ema): the launch also moves the exponential moving average e of the
+// parameters toward the p it has just computed (ema_lerp), 8 more bytes per parameter; p, m and v come from the same
+// adam_update as without it, so they do not change by a bit.
+
+// One Adam update of an element, shared by both instantiations of adam_kernel
+__device__ __forceinline__ void adam_update(float& p, float& m, float& v, float g, float grad_scale,
+                                            float weight_decay, float omb1, float beta2, float omb2, float sqrt_bc2,
+                                            float eps, float step_size) {
+  float gr = g * grad_scale;
+  if (weight_decay != 0.f) gr = fmaf(weight_decay, p, gr);
+  m = m + omb1 * (gr - m);
+  v = beta2 * v + omb2 * gr * gr;
+  const float denom = sqrtf(v) / sqrt_bc2 + eps;
+  p = p - step_size * (m / denom);
+}
+
+// One EMA update of an element, as torch.optim.swa_utils.AveragedModel with get_ema_multi_avg_fn: a copy of p on the
+// first update, else torch.lerp(e, p, w) with w = 1 - decay (torch's two-branch formula, contracted as nvcc
+// contracts torch's CUDA lerp)
+__device__ __forceinline__ float ema_lerp(float e, float p, float w, bool first) {
+  if (first) return p;
+  const float d = p - e;
+  return fabsf(w) < 0.5f ? fmaf(w, d, e) : fmaf(-d, 1.0f - w, p);
+}
+
+// The EMA's scalars, read by thread 0 of a block: w = fp32(1 - decay) (formed in double, rounded once, as a python
+// float reaches torch._foreach_lerp_) and whether this is the first update (n_averaged == 0)
+__device__ __forceinline__ void ema_consts(const EmaArg& ema, float* w, float* first) {
+  const double decay = *reinterpret_cast<const volatile double*>(ema.decay);
+  *w = static_cast<float>(1.0 - decay);
+  *first = *reinterpret_cast<const volatile int64_t*>(ema.count) == 0 ? 1.f : 0.f;
+}
+
+template <int U, bool EMA>
 __global__ void __launch_bounds__(256, U == 4 ? 2 : 4) adam_kernel(float* __restrict__ p, float* __restrict__ g, float* __restrict__ m,
                             float* __restrict__ v, int64_t n, int64_t off_b, int64_t n_b, const __grid_constant__ HpArg hp,
                             float grad_scale, const float* coef, float* step, int step_bias, unsigned int* ticket,
                             __nv_bfloat16* __restrict__ sh_hi, __nv_bfloat16* __restrict__ sh_lo, int zero_grads,
-                            AuxTrace tr) {
+                            AuxTrace tr, const __grid_constant__ EmaArg ema) {
   ptx::pdl_launch_dependents();
   ptx::pdl_wait();   // (rvae_adam_step follows the launch that advances the step counter)
   aux_begin(tr, 4);
@@ -1071,8 +1104,9 @@ __global__ void __launch_bounds__(256, U == 4 ? 2 : 4) adam_kernel(float* __rest
   // corrections in double, as torch computes them on the host (python floats). One thread per block reads the record,
   // does the fp64 pow()s and broadcasts the seven scalars. coef != nullptr: the gradient-clipping factor of the step
   // (grad_norm_kernel), folded into the gradient scale - g * coef in fp32, as torch.nn.utils.clip_grad_norm_ scales g.
-  __shared__ float s_consts[8];
+  __shared__ float s_consts[EMA ? 10 : 8];
   if (threadIdx.x == 0) {
+    if constexpr (EMA) ema_consts(ema, &s_consts[8], &s_consts[9]);
     const rvae_hparams& h = hp.dev != nullptr ? *hp.dev : hp.val;
     // t = *step + step_bias: step_bias = 1 when the step counter is advanced only at the end of the step (ticket)
     const double t = static_cast<double>(*reinterpret_cast<volatile float*>(step)) + step_bias;
@@ -1096,6 +1130,8 @@ __global__ void __launch_bounds__(256, U == 4 ? 2 : 4) adam_kernel(float* __rest
   const float sqrt_bc2 = s_consts[1];
   const float omb1 = s_consts[2], beta2 = s_consts[3], omb2 = s_consts[4], eps = s_consts[5];
   const float weight_decay = s_consts[6];
+  const float ema_w = EMA ? s_consts[EMA ? 8 : 0] : 0.f;
+  const bool ema_first = EMA && s_consts[EMA ? 9 : 0] != 0.f;
   const int64_t nvec = n >> 2;
   const int64_t nvec_all = nvec + (n_b >> 2);
   const int64_t shift_b = (off_b >> 2) - nvec;
@@ -1108,6 +1144,7 @@ __global__ void __launch_bounds__(256, U == 4 ? 2 : 4) adam_kernel(float* __rest
   for (int64_t w0 = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; w0 < nvec_all; w0 += U * stride) {
     int64_t idx[U];
     float4 pp[U], gg[U], mm[U], vv[U];
+    float4 ee[EMA ? U : 1];
 #pragma unroll
     for (int u = 0; u < U; ++u) {
       const int64_t w = w0 + u * stride;
@@ -1117,6 +1154,7 @@ __global__ void __launch_bounds__(256, U == 4 ? 2 : 4) adam_kernel(float* __rest
         gg[u] = __ldcs(reinterpret_cast<const float4*>(g) + idx[u]);
         mm[u] = __ldcs(reinterpret_cast<const float4*>(m) + idx[u]);
         vv[u] = __ldcs(reinterpret_cast<const float4*>(v) + idx[u]);
+        if constexpr (EMA) ee[u] = __ldcs(reinterpret_cast<const float4*>(ema.e) + idx[u]);
       }
     }
 #pragma unroll
@@ -1128,17 +1166,17 @@ __global__ void __launch_bounds__(256, U == 4 ? 2 : 4) adam_kernel(float* __rest
       float* ma = reinterpret_cast<float*>(&mm[u]);
       float* va = reinterpret_cast<float*>(&vv[u]);
 #pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        float gr = ga[j] * grad_scale;
-        if (weight_decay != 0.f) gr = fmaf(weight_decay, pa[j], gr);
-        ma[j] = ma[j] + omb1 * (gr - ma[j]);
-        va[j] = beta2 * va[j] + omb2 * gr * gr;
-        const float denom = sqrtf(va[j]) / sqrt_bc2 + eps;
-        pa[j] = pa[j] - step_size * (ma[j] / denom);
-      }
+      for (int j = 0; j < 4; ++j)
+        adam_update(pa[j], ma[j], va[j], ga[j], grad_scale, weight_decay, omb1, beta2, omb2, sqrt_bc2, eps, step_size);
       __stcs(reinterpret_cast<float4*>(p) + i, pp[u]);
       __stcs(reinterpret_cast<float4*>(m) + i, mm[u]);
       __stcs(reinterpret_cast<float4*>(v) + i, vv[u]);
+      if constexpr (EMA) {
+        float* ea = reinterpret_cast<float*>(&ee[EMA ? u : 0]);
+#pragma unroll
+        for (int j = 0; j < 4; ++j) ea[j] = ema_lerp(ea[j], pa[j], ema_w, ema_first);
+        __stcs(reinterpret_cast<float4*>(ema.e) + i, ee[EMA ? u : 0]);
+      }
       // zero_grads: the next step's split-K weight gradients reduce-add into this buffer (saves 4 memsets / step)
       if (zero_grads) reinterpret_cast<float4*>(g)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
       if (sh_hi) {
@@ -1154,12 +1192,11 @@ __global__ void __launch_bounds__(256, U == 4 ? 2 : 4) adam_kernel(float* __rest
   }
   if (blockIdx.x == 0) {
     for (int64_t j = (nvec << 2) + threadIdx.x; j < n; j += blockDim.x) {
-      float gr = g[j] * grad_scale;
-      if (weight_decay != 0.f) gr = fmaf(weight_decay, p[j], gr);
-      const float mj = m[j] + omb1 * (gr - m[j]);
-      const float vj = beta2 * v[j] + omb2 * gr * gr;
-      const float pj = p[j] - step_size * (mj / (sqrtf(vj) / sqrt_bc2 + eps));
+      const float gj = g[j];
+      float pj = p[j], mj = m[j], vj = v[j];
+      adam_update(pj, mj, vj, gj, grad_scale, weight_decay, omb1, beta2, omb2, sqrt_bc2, eps, step_size);
       m[j] = mj; v[j] = vj; p[j] = pj;
+      if constexpr (EMA) ema.e[j] = ema_lerp(ema.e[j], pj, ema_w, ema_first);
       if (zero_grads) g[j] = 0.f;
       if (sh_hi) {
         const __nv_bfloat16 h = __float2bfloat16_rn(pj);
@@ -1179,6 +1216,8 @@ __global__ void __launch_bounds__(256, U == 4 ? 2 : 4) adam_kernel(float* __rest
       if (done == gridDim.x - 1) {
         *ticket = 0u;
         *step = *reinterpret_cast<volatile float*>(step) + 1.0f;
+        // n_averaged advances with the step counter, once per step, after every EMA launch of the step has read it
+        if constexpr (EMA) *ema.count = *reinterpret_cast<volatile int64_t*>(ema.count) + 1;
       }
     }
   }
@@ -1188,13 +1227,16 @@ int launch_adam(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, dou
                 double eps, double weight_decay, float grad_scale, const float* step, __nv_bfloat16* shadow_hi,
                 __nv_bfloat16* shadow_lo, int zero_grads, cudaStream_t stream) {
   return launch_adam2(ctx, p, g, m, v, n, 0, 0, hp_value(lr, beta1, beta2, eps, weight_decay), grad_scale, nullptr,
-                      const_cast<float*>(step), 0, nullptr, shadow_hi, shadow_lo, zero_grads, stream);
+                      const_cast<float*>(step), 0, nullptr, shadow_hi, shadow_lo, zero_grads, EmaArg{}, stream);
 }
 
 int launch_adam2(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, int64_t off_b, int64_t n_b,
                  const HpArg& hp, float grad_scale, const float* coef, float* step, int step_bias, unsigned int* ticket,
-                 __nv_bfloat16* shadow_hi, __nv_bfloat16* shadow_lo, int zero_grads, cudaStream_t stream) {
+                 __nv_bfloat16* shadow_hi, __nv_bfloat16* shadow_lo, int zero_grads, const EmaArg& ema,
+                 cudaStream_t stream) {
   RVAE_REQUIRE(p && g && m && v && step, RVAE_ERR_INVALID, "adam: null buffer");
+  RVAE_REQUIRE(ema.e == nullptr || (ema.decay && ema.count && (reinterpret_cast<uintptr_t>(ema.e) & 15) == 0),
+               RVAE_ERR_INVALID, "adam: the EMA buffer must be 16-byte aligned, with its decay and count");
   RVAE_REQUIRE(n_b == 0 || ((n & 3) == 0 && (off_b & 3) == 0 && (n_b & 3) == 0 && off_b >= n), RVAE_ERR_INVALID,
                "adam: segments must be multiples of 4 elements");
   RVAE_REQUIRE(((reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(m) |
@@ -1211,10 +1253,79 @@ int launch_adam2(Ctx* ctx, float* p, float* g, float* m, float* v, int64_t n, in
   const int64_t groups = (n + n_b + 3) / 4;
   dim3 grid(grid_for(ctx, (groups + unroll - 1) / unroll, threads, bps > 0 ? bps : 4));
   if (ctx->aux_grid_cap > 0 && (int)grid.x > ctx->aux_grid_cap) grid.x = ctx->aux_grid_cap;
-  auto kern = unroll == 1 ? adam_kernel<1> : (unroll == 4 ? adam_kernel<4> : adam_kernel<2>);
+  auto kern = unroll == 1 ? adam_kernel<1, false> : (unroll == 4 ? adam_kernel<4, false> : adam_kernel<2, false>);
+  if (ema.e != nullptr)
+    kern = unroll == 1 ? adam_kernel<1, true> : (unroll == 4 ? adam_kernel<4, true> : adam_kernel<2, true>);
   RVAE_CUDA(launch_kernel(ctx, kern, grid, dim3(threads), (size_t)0,
                           stream, p, g, m, v, n, off_b, n_b, hp, grad_scale, coef, step, step_bias, ticket, shadow_hi,
-                          shadow_lo, zero_grads, next_aux(ctx, 4)));
+                          shadow_lo, zero_grads, next_aux(ctx, 4), ema));
+  RVAE_LAUNCH_CHECK(ctx);
+  return RVAE_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Standalone EMA update (rvae_ema_update): e = ema_lerp(e, p) over a flat buffer, with the device function of the EMA
+// Adam launch - the update that follows an optimizer step of the unfused path. float4 loads and stores (12 B/param,
+// streaming), a grid of 1 to 4 blocks per SM; the last block to finish advances n_averaged (ticket).
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) ema_update_kernel(const float* __restrict__ p, int64_t n,
+                                                         const __grid_constant__ EmaArg ema, unsigned int* ticket) {
+  ptx::pdl_launch_dependents();
+  ptx::pdl_wait();
+  __shared__ float s_consts[2];
+  if (threadIdx.x == 0) ema_consts(ema, &s_consts[0], &s_consts[1]);
+  __syncthreads();
+  const float w = s_consts[0];
+  const bool first = s_consts[1] != 0.f;
+  constexpr int U = 4;
+  const int64_t nvec = n >> 2;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  float4* e4 = reinterpret_cast<float4*>(ema.e);
+  for (int64_t w0 = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; w0 < nvec; w0 += U * stride) {
+    float4 pp[U], ee[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int64_t i = w0 + u * stride;
+      if (i < nvec) {
+        pp[u] = __ldcs(reinterpret_cast<const float4*>(p) + i);
+        ee[u] = __ldcs(e4 + i);
+      }
+    }
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int64_t i = w0 + u * stride;
+      if (i >= nvec) continue;
+      ee[u].x = ema_lerp(ee[u].x, pp[u].x, w, first);
+      ee[u].y = ema_lerp(ee[u].y, pp[u].y, w, first);
+      ee[u].z = ema_lerp(ee[u].z, pp[u].z, w, first);
+      ee[u].w = ema_lerp(ee[u].w, pp[u].w, w, first);
+      __stcs(e4 + i, ee[u]);
+    }
+  }
+  if (blockIdx.x == 0)
+    for (int64_t j = (nvec << 2) + threadIdx.x; j < n; j += blockDim.x) ema.e[j] = ema_lerp(ema.e[j], p[j], w, first);
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    __threadfence();
+    if (atomicAdd(ticket, 1u) == gridDim.x - 1) {
+      *ticket = 0u;
+      *ema.count = *reinterpret_cast<volatile int64_t*>(ema.count) + 1;
+    }
+  }
+}
+
+int launch_ema_update(Ctx* ctx, const float* p, int64_t n, const EmaArg& ema, unsigned int* ticket,
+                      cudaStream_t stream) {
+  RVAE_REQUIRE(p && ema.e && ema.decay && ema.count && ticket, RVAE_ERR_INVALID, "ema_update: null buffer");
+  RVAE_REQUIRE(n >= 0, RVAE_ERR_INVALID, "ema_update: n = %lld", (long long)n);
+  RVAE_REQUIRE(((reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(ema.e)) & 15) == 0, RVAE_ERR_INVALID,
+               "ema_update: ema and params must be 16-byte aligned");
+  const int threads = 256;
+  // a multiple of the SM count: one to four blocks per SM, by size (each thread covers 4 float4 groups per trip)
+  const int64_t per_wave = (int64_t)ctx->num_sms_total * threads * 4 * 4;
+  const int64_t waves = std::min<int64_t>(4, std::max<int64_t>(1, (n + per_wave - 1) / per_wave));
+  RVAE_CUDA(launch_kernel(ctx, ema_update_kernel, dim3(ctx->num_sms_total * (int)waves), dim3(threads), (size_t)0,
+                          stream, p, n, ema, ticket));
   RVAE_LAUNCH_CHECK(ctx);
   return RVAE_OK;
 }

@@ -300,13 +300,15 @@ class DataParallelTrainStep(_StepBase):
     rank, in a fixed order, so every rank clips by the same factor and the replicas stay bitwise equal.
     deterministic: as for FusedTrainStep, with the gradients exchanged by the peer-load all-reduce whatever
     RVAE_DP_BACKEND says (it sums the ranks in rank order). RVAE_DP_BACKEND=nvls or nccl raises ValueError here, and
-    so does a group that cannot use peer loads, at its first step: the step never trains non-deterministically."""
+    so does a group that cannot use peer loads, at its first step: the step never trains non-deterministically.
+    ema: as for FusedTrainStep. Each rank updates its own average from the all-reduced update, which is identical on
+    every rank, so the averages stay bitwise equal without any communication."""
 
     def __init__(self, model, optimizer, kl_beta: float, global_batch: Optional[int] = None, group=None,
                  ring: int = 64, reduce_loss: bool = False, graph: bool = False, schedule=None, max_grad_norm=None,
-                 deterministic: bool = False):
+                 deterministic: bool = False, ema=None):
         super().__init__(model, optimizer, kl_beta, ring, graph, schedule=schedule, max_grad_norm=max_grad_norm,
-                         deterministic=deterministic)
+                         deterministic=deterministic, ema=ema)
         forced = os.environ.get("RVAE_DP_BACKEND", "auto")
         if self.deterministic and forced in ("nvls", "nccl"):
             raise ValueError(f"deterministic=True needs the peer-load gradient all-reduce; RVAE_DP_BACKEND={forced} "

@@ -314,6 +314,19 @@ class Plan:
         check(self.lib.rvae_plan_set_grad_clip(self.handle, max_norm_ptr,
                                                norm_out.data_ptr() if norm_out is not None else None, int(ring_size)))
 
+    def set_ema(self, ema: Optional[torch.Tensor], decay_ptr: Optional[int] = None,
+                n_averaged: Optional[torch.Tensor] = None) -> None:
+        """Update the fp32 EMA buffer `ema` (the flat layout of the parameters) in every Adam launch of every later
+        training step, with the device double decay at decay_ptr and the device int64 count n_averaged (None = off)."""
+        if ema is None:
+            check(self.lib.rvae_plan_set_ema(self.handle, None, None, None))
+            return
+        if ema.dtype != torch.float32 or ema.numel() != self.flat.total or ema.device != self.flat.device:
+            raise _lib.RvaeError("the EMA buffer must be a float32 tensor of the flat parameter layout")
+        if n_averaged is None or n_averaged.dtype != torch.int64 or n_averaged.device != self.flat.device:
+            raise _lib.RvaeError("n_averaged must be an int64 tensor on the plan's device")
+        check(self.lib.rvae_plan_set_ema(self.handle, ema.data_ptr(), decay_ptr, n_averaged.data_ptr()))
+
     def deterministic_bytes(self) -> int:
         """Scratch bytes of the deterministic training step at this plan's max_batch (rvae_plan_deterministic_bytes)."""
         return int(self.lib.rvae_plan_deterministic_bytes(self.handle))

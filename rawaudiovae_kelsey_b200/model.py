@@ -383,6 +383,14 @@ def check_deterministic(value) -> bool:
     return value
 
 
+def check_ema(value):
+    """A training step's EMA: None or an ema.ExponentialMovingAverage. Raises ValueError for anything else."""
+    from .ema import ExponentialMovingAverage
+    if value is not None and not isinstance(value, ExponentialMovingAverage):
+        raise ValueError(f"ema must be None or an ExponentialMovingAverage, got {value!r}")
+    return value
+
+
 def check_max_grad_norm(value) -> Optional[float]:
     """A training step's gradient-clipping threshold: None (no clipping) or a float > 0, +inf included (the norm is
     measured and logged, the update is unchanged). Raises ValueError for anything else."""
@@ -416,12 +424,18 @@ class _StepBase:
     gradients - then depends only on the inputs, the state, the hyper-parameters, the dims, the batch size, the
     precision and the world size, never on scheduling or the SM budget. Each plan the step uses gets its own scratch
     (rvae_plan_deterministic_bytes: 35.9 MB at the default dims and 8192 frames). The unfused path (loss_function +
-    loss.backward()) is not covered."""
+    loss.backward()) is not covered.
+
+    ema (ema.ExponentialMovingAverage of this model, or None): every step also updates the moving average of the
+    weights, inside its Adam launches (rvae_plan_set_ema), from the parameters they have just computed. The decay lives
+    in the device record, so changing `ema.decay` reaches graph replays; switching the EMA on or off captures a new
+    graph. Parameters, moments and everything else a step computes are the same bit for bit with and without it."""
 
     def __init__(self, model, optimizer, kl_beta, ring, graph, graph_warmup=1, schedule=None, max_grad_norm=None,
-                 deterministic=False):
+                 deterministic=False, ema=None):
         self.max_grad_norm = max_grad_norm     # validated before any GPU work
         self.deterministic = check_deterministic(deterministic)
+        self.ema = check_ema(ema)
         self.model, self.optimizer, self.kl_beta = model, optimizer, float(kl_beta)
         self.schedule = schedule if schedule is not None else Schedule()
         self._record = None
@@ -469,6 +483,8 @@ class _StepBase:
             self.i = int(flat.step.item())          # one sync, first call only (resumed optimizers start at t0 > 0)
         if hasattr(self.optimizer, "bind_flat"):
             self.optimizer.bind_flat(flat)
+        if self.ema is not None and self.ema.target().numel() != flat.total:
+            raise _lib.RvaeError("the EMA does not have the model's parameter layout")
         return flat
 
     def _hparams(self, device):
@@ -477,10 +493,22 @@ class _StepBase:
             self._record = DeviceRecord(device)
         g = self.optimizer.param_groups[0]
         return self._record.update(self.schedule, g["lr"], g["betas"], g["eps"], g.get("weight_decay", 0.0),
-                                   self.kl_beta, self.max_grad_norm)
+                                   self.kl_beta, self.max_grad_norm,
+                                   self.ema.decay if self.ema is not None else None)
 
     def _train_step(self, plan, zero_grads):
-        """The fused step from the device record, clipping when max_grad_norm is set (a plan setting for this call)."""
+        """The fused step from the device record, with the EMA, deterministic mode and clipping when they are on
+        (plan settings for this call)."""
+        if self.ema is None:
+            self._train_step_det(plan, zero_grads)
+            return
+        plan.set_ema(self.ema.target(), self._record.ema_decay_ptr, self.ema.n_averaged)
+        try:
+            self._train_step_det(plan, zero_grads)
+        finally:
+            plan.set_ema(None)
+
+    def _train_step_det(self, plan, zero_grads):
         if self.deterministic:
             plan.set_deterministic(True)
             try:
@@ -566,7 +594,8 @@ class _StepBase:
             # ---- plain path: load inside the step (captured graph: from static index / input buffers)
             key = self._graph_key(data) if graphable else None
             if key is not None:
-                key = key + self._key_extra(data) + (self.max_grad_norm is not None, self.deterministic)
+                key = key + self._key_extra(data) + (self.max_grad_norm is not None, self.deterministic,
+                                                     self._ema_key())
             if key is not None and key in self._graphs:
                 st = self._graphs[key]
                 self._load_static(key, data, st)
@@ -600,7 +629,7 @@ class _StepBase:
                 key = ("pf", plan.handle.value, next_data.audio.data_ptr(), plan.batch, next_data.n_frames,
                        next_data.hop, self._plan_cur(plan), plan.pitch, model._in_place(next_data)) \
                     + self._key_extra(data) + self._key_extra(next_data) + (self.max_grad_norm is not None,
-                                                                             self.deterministic)
+                                                                             self.deterministic, self._ema_key())
             if key is not None and key in self._graphs:
                 st = self._graphs[key]
                 self._fill_idx(st, next_data)
@@ -620,9 +649,15 @@ class _StepBase:
                 self._enqueue(plan)
                 if do_pf:
                     self._pf = (plan, next_data)
+        if self.ema is not None:
+            self.ema.mark_updated()
         slot = self._slot()
         self.i += 1
         return slot
+
+    def _ema_key(self):
+        """The EMA buffer a captured graph writes (None: no EMA)."""
+        return self.ema.target().data_ptr() if self.ema is not None else None
 
     # -- hooks of the data-parallel subclass
     def _configure(self, plan, data):
@@ -717,13 +752,14 @@ class FusedTrainStep(_StepBase):
     schedule (schedule.Schedule, default constant): learning rate and KL weight per step, with
     optimizer.param_groups[0]['lr'] and kl_beta as the peak values.
     max_grad_norm (None, or a float > 0, inf included): clip by the global gradient norm (see _StepBase).
-    deterministic (bool, default False): bitwise reproducible steps (see _StepBase)."""
+    deterministic (bool, default False): bitwise reproducible steps (see _StepBase).
+    ema (ema.ExponentialMovingAverage, default None): also update this moving average of the weights (see _StepBase)."""
 
     def __init__(self, model: VAE, optimizer, kl_beta: float, ring: int = 64, keep_grads: bool = False,
                  graph: bool = False, schedule: Optional[Schedule] = None, max_grad_norm: Optional[float] = None,
-                 deterministic: bool = False):
+                 deterministic: bool = False, ema=None):
         super().__init__(model, optimizer, kl_beta, ring, graph, schedule=schedule, max_grad_norm=max_grad_norm,
-                         deterministic=deterministic)
+                         deterministic=deterministic, ema=ema)
         self.keep_grads = keep_grads
 
     def _enqueue(self, plan):

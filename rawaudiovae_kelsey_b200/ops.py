@@ -294,6 +294,17 @@ def adam_step(p, g, m, v, step, lr, beta1=0.9, beta2=0.999, eps=1e-8, weight_dec
                              _ptr(shadow_lo, torch.bfloat16), _stream()))
 
 
+def ema_update(ema: torch.Tensor, params: torch.Tensor, decay: torch.Tensor, n_averaged: torch.Tensor) -> None:
+    """ema = lerp(ema, params, 1 - decay) in place (a copy when n_averaged == 0), then n_averaged += 1: one launch
+    over flat fp32 buffers. decay: a device float64 scalar tensor, n_averaged a device int64 one."""
+    if ema.numel() != params.numel():
+        raise _lib.RvaeError(f"ema has {ema.numel()} elements, params {params.numel()}")
+    check(_lib.load().rvae_ema_update(ctx(ema.device), _ptr(ema, torch.float32, "ema"),
+                                      _ptr(params, torch.float32, "params"), ema.numel(),
+                                      _ptr(decay, torch.float64, "decay"), _ptr(n_averaged, torch.int64, "n_averaged"),
+                                      _stream()))
+
+
 def histogram_record_layout(n_segs: int, n_edges: int) -> dict:
     """Byte offsets of the fields of an rvae_param_histogram record (include/rvae_b200.h); "bytes" = results only,
     "total" = results + the kernel's scratch (what the device buffer must hold)."""

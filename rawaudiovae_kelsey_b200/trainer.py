@@ -29,6 +29,7 @@ import torch
 from . import audio_io, dist as rdist
 from .dataset import AudioDataset, IterableAudioDataset, ToTensor
 from .inference import evaluate_audio
+from .ema import ExponentialMovingAverage, check_ema_decay
 from .model import VAE, FusedTrainStep, check_max_grad_norm
 from .optim import Adam
 from .schedule import Schedule
@@ -163,6 +164,33 @@ def _max_grad_norm(config):
     except ValueError:
         raise ValueError(f"[training] max_grad_norm must be a number > 0 or inf, got {v!r}") from None
     return check_max_grad_norm(f)
+
+
+def _ema_decay(config):
+    """[training] ema_decay (optional): keep an exponential moving average of the weights with this decay, in [0, 1]
+    (ema.ExponentialMovingAverage, updated inside every training step). The test reconstructions, the test loss,
+    best_model.pt and last_model.pt then use the averaged weights, and each checkpoint also holds them
+    ('ema_state_dict', 'ema_n_averaged'). Absent or empty: no average. Values outside [0, 1], NaN or text that is not a
+    number raise ValueError."""
+    v = config['training'].get('ema_decay', fallback='').strip()
+    if not v:
+        return None
+    try:
+        f = float(v)
+    except ValueError:
+        raise ValueError(f"[training] ema_decay must be a number in [0, 1], got {v!r}") from None
+    try:
+        return check_ema_decay(f)
+    except ValueError:
+        raise ValueError(f"[training] ema_decay must be in [0, 1], got {v!r}") from None
+
+
+def _with_ema(state, ema):
+    """A checkpoint dict, plus the average's weights and update count when an EMA is kept."""
+    if ema is not None:
+        state['ema_state_dict'] = ema.state_dict()
+        state['ema_n_averaged'] = int(ema.n_averaged.item())
+    return state
 
 
 def _deterministic(config) -> bool:
@@ -317,6 +345,7 @@ def run_epoch_trainer(argv=None):
     kl_beta = config['VAE'].getfloat('kl_beta')
     test_loss = _test_loss_enabled(config)
     max_grad_norm = _max_grad_norm(config)
+    ema_decay = _ema_decay(config)
     deterministic = _deterministic(config)
     _apply_seed(_seed(config))
     start_time = time.time()
@@ -358,12 +387,14 @@ def run_epoch_trainer(argv=None):
     optimizer = Adam(model.parameters(), lr=learning_rate)
     use_graph = config['training'].getboolean('cuda_graph', fallback=True)
     ring = max(64, log_interval)
+    ema = ExponentialMovingAverage(model, ema_decay) if ema_decay is not None else None
+    served = ema.module if ema is not None else model   # the weights that are evaluated, listened to and saved
     if world > 1:
         step = rdist.DataParallelTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph, schedule=schedule,
-                                           max_grad_norm=max_grad_norm, deterministic=deterministic)
+                                           max_grad_norm=max_grad_norm, deterministic=deterministic, ema=ema)
     else:
         step = FusedTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph, schedule=schedule,
-                              max_grad_norm=max_grad_norm, deterministic=deterministic)
+                              max_grad_norm=max_grad_norm, deterministic=deterministic, ema=ema)
 
     # parameter histograms on the GPU (rank 0 only): one launch + one small asynchronous copy per set
     hist = ParamHistogramLogger(model, writer) if rank == 0 else None
@@ -402,21 +433,22 @@ def run_epoch_trainer(argv=None):
         if rank == 0 and epoch % checkpoint_interval == 0 and epoch != 0:
             print('Checkpoint - Epoch {}'.format(epoch))
             hist.flush(wait=True)
-            state = {'epoch': epoch, 'state_dict': model.state_dict(), 'optimizer': optimizer.state_dict()}
+            state = _with_ema({'epoch': epoch, 'state_dict': model.state_dict(),
+                              'optimizer': optimizer.state_dict()}, ema)
             if generate_test:
                 audio_out = audio_log_dir.joinpath('test_reconst_{:05d}.wav'.format(epoch))
-                test_predictions_np = _reconstruct_test(model, test_dataset, batch_size, device)
+                test_predictions_np = _reconstruct_test(served, test_dataset, batch_size, device)
                 audio_io.write_wav(audio_out, test_predictions_np, sampling_rate)
                 print('Audio examples generated: {}'.format(audio_out))
                 writer.add_audio('Reconstructed Audio', test_predictions_np, epoch, sample_rate=sampling_rate)
             torch.save(state, checkpoint_dir.joinpath('ckpt_{:05d}'.format(epoch)))
             if test_loss:
-                t_loss = _evaluate_test(model, test_dataset, kl_beta, batch_size, writer, epoch)
+                t_loss = _evaluate_test(served, test_dataset, kl_beta, batch_size, writer, epoch)
                 if epoch > save_best_model_after:
-                    best_test_loss = _keep_best_test(model, t_loss, best_test_loss, workdir, config, 'best_epoch', epoch)
+                    best_test_loss = _keep_best_test(served, t_loss, best_test_loss, workdir, config, 'best_epoch', epoch)
             elif (train_loss < train_loss_prev) and (epoch > save_best_model_after):
                 save_path = workdir.joinpath('model').joinpath('best_model.pt')
-                torch.save(model, save_path)
+                torch.save(served, save_path)
                 print('Epoch {:05d}: Saved {}'.format(epoch, save_path))
                 config['training']['best_epoch'] = str(epoch)
                 best_loss = train_loss
@@ -430,18 +462,19 @@ def run_epoch_trainer(argv=None):
     if rank == 0:
         hist.flush(wait=True)
         print('Last Checkpoint - Epoch {}'.format(epochs))
-        state = {'epoch': epochs, 'state_dict': model.state_dict(), 'optimizer': optimizer.state_dict()}
+        state = _with_ema({'epoch': epochs, 'state_dict': model.state_dict(),
+                          'optimizer': optimizer.state_dict()}, ema)
         if generate_test:
             audio_out = audio_log_dir.joinpath('test_reconst_{:05d}.wav'.format(epochs))
-            test_predictions_np = _reconstruct_test(model, test_dataset, batch_size, device)
+            test_predictions_np = _reconstruct_test(served, test_dataset, batch_size, device)
             audio_io.write_wav(audio_out, test_predictions_np, sampling_rate)
             print('Last Audio examples generated: {}'.format(audio_out))
             writer.add_audio('Reconstructed Audio', test_predictions_np, epochs, sample_rate=sampling_rate)
         torch.save(state, checkpoint_dir.joinpath('ckpt_{:05d}'.format(epochs)))
         if test_loss:
-            t_loss = _evaluate_test(model, test_dataset, kl_beta, batch_size, writer, epochs)
+            t_loss = _evaluate_test(served, test_dataset, kl_beta, batch_size, writer, epochs)
             if epochs > save_best_model_after:
-                best_test_loss = _keep_best_test(model, t_loss, best_test_loss, workdir, config, 'best_epoch', epochs)
+                best_test_loss = _keep_best_test(served, t_loss, best_test_loss, workdir, config, 'best_epoch', epochs)
             _final_test_message(t_loss, best_test_loss)
         elif final_loss > train_loss_prev:
             print("Final loss was not better than the last best model.")
@@ -450,7 +483,7 @@ def run_epoch_trainer(argv=None):
         else:
             print("The last model is the best model.")
         save_path = workdir.joinpath('model').joinpath('last_model.pt')
-        torch.save(model, save_path)
+        torch.save(served, save_path)
         print('Training Finished: Saved the last model')
         config['extra']['end'] = time.asctime(time.localtime(time.time()))
         config['extra']['time_elapsed'] = str(time.time() - start_time)
@@ -488,6 +521,7 @@ def run_stream_trainer(argv=None):
     kl_beta = config['VAE'].getfloat('kl_beta')
     test_loss = _test_loss_enabled(config)
     max_grad_norm = _max_grad_norm(config)
+    ema_decay = _ema_decay(config)
     deterministic = _deterministic(config)
     seed = _seed(config)
     if segment_length != 1024:
@@ -533,13 +567,15 @@ def run_stream_trainer(argv=None):
         optimizer = Adam(model.parameters(), lr=learning_rate)
         use_graph = config['training'].getboolean('cuda_graph', fallback=True)
         ring = max(64, log_interval)
+        ema = ExponentialMovingAverage(model, ema_decay) if ema_decay is not None else None
+        served = ema.module if ema is not None else model   # the weights that are evaluated, listened to and saved
         if world > 1:
             step = rdist.DataParallelTrainStep(model, optimizer, kl_beta, global_batch=batch_size, ring=ring,
                                                graph=use_graph, schedule=schedule, max_grad_norm=max_grad_norm,
-                                               deterministic=deterministic)
+                                               deterministic=deterministic, ema=ema)
         else:
             step = FusedTrainStep(model, optimizer, kl_beta, ring=ring, graph=use_graph, schedule=schedule,
-                                  max_grad_norm=max_grad_norm, deterministic=deterministic)
+                                  max_grad_norm=max_grad_norm, deterministic=deterministic, ema=ema)
 
         hist = ParamHistogramLogger(model, writer) if rank == 0 and histogram_interval > 0 else None
 
@@ -566,21 +602,22 @@ def run_stream_trainer(argv=None):
                 print('Checkpoint - Epoch {}'.format(batch_id))
                 if hist is not None:
                     hist.flush(wait=True)
-                state = {'batch_id': batch_id, 'state_dict': model.state_dict(), 'optimizer': optimizer.state_dict()}
+                state = _with_ema({'batch_id': batch_id, 'state_dict': model.state_dict(),
+                                  'optimizer': optimizer.state_dict()}, ema)
                 if generate_test:
                     audio_out = audio_log_dir.joinpath('test_reconst_{:05d}.wav'.format(batch_id))
-                    test_predictions_np = _reconstruct_test(model, test_dataset, batch_size, device)
+                    test_predictions_np = _reconstruct_test(served, test_dataset, batch_size, device)
                     audio_io.write_wav(audio_out, test_predictions_np, sampling_rate)
                     print('Audio examples generated: {}'.format(audio_out))
                     writer.add_audio('Reconstructed Audio', test_predictions_np, batch_id, sample_rate=sampling_rate)
                 torch.save(state, checkpoint_dir.joinpath('ckpt_{:05d}'.format(batch_id)))
                 if test_loss:
-                    t_loss = _evaluate_test(model, test_dataset, kl_beta, batch_size, writer, batch_id)
-                    best_test_loss = _keep_best_test(model, t_loss, best_test_loss, workdir, config, 'best_model',
+                    t_loss = _evaluate_test(served, test_dataset, kl_beta, batch_size, writer, batch_id)
+                    best_test_loss = _keep_best_test(served, t_loss, best_test_loss, workdir, config, 'best_model',
                                                      batch_id)
                 elif train_loss < train_loss_prev:
                     save_path = workdir.joinpath('model').joinpath('best_model.pt')
-                    torch.save(model, save_path)
+                    torch.save(served, save_path)
                     print('batch_id {:05d}: Saved {}'.format(batch_id, save_path))
                     config['training']['best_model'] = str(batch_id)
                     best_loss = train_loss
@@ -596,17 +633,18 @@ def run_stream_trainer(argv=None):
             if hist is not None:
                 hist.flush(wait=True)
             print('Last Checkpoint - batch_id {}'.format(batch_id))
-            state = {'batch_id': batch_id, 'state_dict': model.state_dict(), 'optimizer': optimizer.state_dict()}
+            state = _with_ema({'batch_id': batch_id, 'state_dict': model.state_dict(),
+                              'optimizer': optimizer.state_dict()}, ema)
             if generate_test:
                 audio_out = audio_log_dir.joinpath('test_reconst_{:05d}.wav'.format(total_num_batches))
-                test_predictions_np = _reconstruct_test(model, test_dataset, batch_size, device)
+                test_predictions_np = _reconstruct_test(served, test_dataset, batch_size, device)
                 audio_io.write_wav(audio_out, test_predictions_np, sampling_rate)
                 print('Last Audio examples generated: {}'.format(audio_out))
                 writer.add_audio('Reconstructed Audio', test_predictions_np, batch_id, sample_rate=sampling_rate)
             torch.save(state, checkpoint_dir.joinpath('ckpt_{:05d}'.format(total_num_batches)))
             if test_loss:
-                t_loss = _evaluate_test(model, test_dataset, kl_beta, batch_size, writer, batch_id)
-                best_test_loss = _keep_best_test(model, t_loss, best_test_loss, workdir, config, 'best_model',
+                t_loss = _evaluate_test(served, test_dataset, kl_beta, batch_size, writer, batch_id)
+                best_test_loss = _keep_best_test(served, t_loss, best_test_loss, workdir, config, 'best_model',
                                                  total_num_batches)
                 _final_test_message(t_loss, best_test_loss)
             elif train_loss > train_loss_prev:
@@ -616,7 +654,7 @@ def run_stream_trainer(argv=None):
             else:
                 print("The last model is the best model.")
             save_path = workdir.joinpath('model').joinpath('last_model.pt')
-            torch.save(model, save_path)
+            torch.save(served, save_path)
             print('Training Finished: Saved the last model')
             config['extra']['end'] = time.asctime(time.localtime(time.time()))
             config['extra']['time_elapsed'] = str(time.time() - start_time)
